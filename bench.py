@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py — the headline benchmark of the D-VQVAE hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1)
+
+--dump-outputs DIR writes what the last timed step returned on rank 0 as DIR/<name>.npy (see dump_outputs): the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workload (BASELINE.json configs[1]): fused VQ lookup, N = 4 194 304 fp32 latents PER GPU,
 e_dim = 64, n_e = 512, train path (indices + z_q + loss + perplexity + usage histogram),
@@ -36,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "d-vqvae_b200"))
 
@@ -44,6 +48,7 @@ E_DIM = 64
 N_E = 512
 E2E_CHUNK_ROWS = 262144          # rows per chunk of the host-buffer pipeline (e2e leg)
 AL, BETA = 1.0, 0.25
+DUMP_ZQ_ROWS = 65536             # z_q rows written by --dump-outputs: all 4M rows would be 1 GiB
 METRIC = "vq_latents_per_sec"
 UNIT = "latents/s"
 WORKLOAD = ("BASELINE config 2: fused VQ lookup, N=4194304 fp32 latents per GPU, e_dim=64, n_e=512, "
@@ -164,6 +169,27 @@ def cpu_port_rate(target_seconds: float, max_rows: int):
     dt = time.perf_counter() - t0
     rows = n_chunks * chunk
     return rows / dt, torch.get_num_threads(), "%d rows (%d chunks of 65536) of the config-2 workload, train path, %.1f s" % (rows, n_chunks, dt)
+
+
+def dump_outputs(out_dir, vq, out):
+    """Write one train step's results as float32 / float64 .npy files, 48.5 MiB in all: the code index of every row
+    (min_encodings is the lazy one-hot of it), z_q at a fixed seeded sample of rows (and those row numbers), loss,
+    perplexity and the usage histogram."""
+    import numpy as np
+    import torch
+    loss, z_q, ppl, _, idx = out
+    rows = np.sort(np.random.RandomState(0).choice(z_q.shape[0], DUMP_ZQ_ROWS, replace=False))
+    arrays = {
+        "loss": loss.cpu().numpy().astype(np.float32),
+        "perplexity": ppl.cpu().numpy().astype(np.float32),
+        "indices": idx.reshape(-1).cpu().numpy().astype(np.float64),
+        "z_q_rows": rows.astype(np.float64),
+        "z_q_sample": z_q[torch.from_numpy(rows).to(z_q.device)].cpu().numpy().astype(np.float32),
+        "usage_histogram": vq.last_stats[:vq.n_e].cpu().numpy().astype(np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_reference(args, rank):
@@ -343,7 +369,12 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the rank to the GPU's NUMA node")
     ap.add_argument("--raw-nccl", action="store_true", help="all-reduce (hist, sse) through dvq_allreduce_stats instead of torch.distributed")
     ap.add_argument("--e2e-chunk-rows", type=int, default=E2E_CHUNK_ROWS, help="rows per chunk of the host-buffer pipeline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -419,6 +450,8 @@ def main():
         elapsed_ms = float(t.item())
     loss, z_q, ppl, enc, idx = out
     value = N_PER_GPU * world * args.steps / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, vq, out)
 
     # ---- e2e: host buffers through dvq_vq_forward_host --------------------------------------------
     e2e_steps = args.e2e_steps or min(args.steps, 10)

@@ -38,7 +38,19 @@ def vq_inputs(name):
 
 
 def load_gold(name):
-    return np.load(os.path.join(GOLD, name + ".npz"))
+    """Where a VQ case's z_q arrays would make its file larger than 1 MB, the file keeps their SHA-256 instead: they
+    are rebuilt from the seeded inputs and the reference's indices (z_q is bit-exact given the index) and must match."""
+    g = np.load(os.path.join(GOLD, name + ".npz"))
+    if name not in VQ_CASES or "zq_train" in g.files:
+        return g
+    g = dict(g)
+    z, E, _, _ = vq_inputs(name)
+    for key, zq in (("zq_train", vo.zq_train_from_idx(z, E, g["idx_train"].astype(np.int64))),
+                    ("zq_infer", vo.zq_infer_from_idx(E, g["idx_infer"].astype(np.int64)))):
+        zq = np.ascontiguousarray(zq.reshape(z.shape))
+        assert hashlib.sha256(zq.tobytes()).hexdigest() == str(g.pop(key + "_sha256")), (name, key)
+        g[key] = zq
+    return g
 
 
 def rel_err(a, b):

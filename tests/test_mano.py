@@ -1,51 +1,18 @@
 """MANO hand layer (SURVEY §8 f4; reference call site network/gen_net.py:116-118, layer created at
 gen_diverse_grasp_obman.py:355-360 by the un-vendored package `mano`).
 
-CPU: the oracle (oracle/mano_oracle.py, a restatement of smplx/lbs.py's published algorithm) against the invariants the
-reference's own asset carries — only where /root/reference exists (the build container); the asset is not copied into the repo.
-GPU: the CUDA kernel behind `dvq.ManoLayer` against the oracle on a synthetic model of the same structure (the GPU box has no
-asset), through the reference's call signature.  Bar: 2e-6 of the hand size (FP32 kernel vs float64 oracle).
+CPU: the oracle (oracle/mano_oracle.py, a restatement of smplx/lbs.py's published algorithm) on a synthetic model.
+GPU: the CUDA kernel behind `dvq.ManoLayer` against the oracle on a synthetic model of MANO's structure (the MANO asset is
+licensed separately and not part of the repository), through the reference's call signature.  Bar: 2e-6 of the hand size
+(FP32 kernel vs float64 oracle).
 """
-import os
-
 import numpy as np
 import pytest
 import torch
 
 from oracle import mano_oracle as mo
 
-ASSET = "/root/reference/models/mano/MANO_RIGHT.pkl"
 TOL = 2e-6
-
-
-@pytest.mark.skipif(not os.path.exists(ASSET), reason="the reference's MANO asset is only present in the build container")
-def test_oracle_reproduces_the_invariants_of_the_reference_asset():
-    m = mo.load_pkl(ASSET)
-    assert m["v_template"].shape == (778, 3) and m["shapedirs"].shape == (778, 3, 10) and m["posedirs"].shape == (778, 3, 135)
-    assert list(m["parents"][1:]) == [0, 1, 2, 0, 4, 5, 0, 7, 8, 0, 10, 11, 0, 13, 14]
-    assert np.abs(m["weights"].sum(1) - 1.0).max() < 1e-6
-    # zero shape and pose (flat_hand_mean=True) -> the template; the regressed rest joints are the pickled J
-    v, j = mo.mano_forward(m, np.zeros((2, 10)), None, np.zeros((2, 45)))
-    assert np.abs(v - m["v_template"][None]).max() < 1e-12
-    assert np.abs(j - m["J"][None]).max() < 1e-12 and np.abs(m["J_regressor"] @ m["v_template"] - m["J"]).max() < 1e-12
-    # flat_hand_mean=False with hand_pose = -hands_mean (full 45-dim pose) is the flat hand again
-    v2, _ = mo.mano_forward(m, np.zeros((1, 10)), None, -m["hands_mean"][None], use_pca=False, flat_hand_mean=False)
-    assert np.abs(v2 - m["v_template"][None]).max() < 1e-12
-    # a rigid global rotation + translation moves the posed hand rigidly (joint 0 is the root of every chain)
-    rs = np.random.RandomState(3)
-    betas, pose = rs.randn(1, 10), 0.5 * rs.randn(1, 45)
-    v0, j0 = mo.mano_forward(m, betas, None, pose)
-    go, tr = rs.randn(1, 3), rs.randn(1, 3)
-    v1, j1 = mo.mano_forward(m, betas, go, pose, tr)
-    R = mo.rodrigues(go)[0]
-    root = j0[0, 0]
-    assert np.abs((v0[0] - root) @ R.T + root + tr[0] - v1[0]).max() < 1e-7      # (1e-8 epsilon inside rodrigues)
-    # the product module reads the same arrays
-    import dvq
-    layer = dvq.ManoLayer.from_pkl(ASSET, model_type="mano", use_pca=True, num_pca_comps=45, batch_size=1, flat_hand_mean=True)
-    assert np.abs(layer.v_template.numpy().reshape(778, 3) - m["v_template"]).max() < 1e-8
-    assert np.abs(layer.posedirs.numpy().reshape(135, 778, 3).transpose(1, 2, 0) - m["posedirs"]).max() < 1e-8
-    assert layer.faces.shape == (1538, 3)
 
 
 def test_oracle_synthetic_model_sanity():
