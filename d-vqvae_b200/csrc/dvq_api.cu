@@ -129,6 +129,15 @@ int dvq_debug_tc_pair_layout(long long N, int K, int D, int* out8) {
   return DVQ_OK;
 }
 
+int dvq_debug_tc_layout_ex(long long N, int K, int D, int flags, int* out8) {
+  if (!out8) return fail(DVQ_ERR_BAD_ARG, "out8 is NULL");
+  if (K <= 0 || D <= 0) return fail(DVQ_ERR_BAD_SHAPE, "need K > 0, D > 0");
+  const int zbytes = (flags & DVQ_Z_BF16) ? 2 : 4;
+  if (vq_tc_pair_selected((int64_t)N, K, D)) vq_tc_pair_layout_info((int64_t)N, K, D, out8, zbytes);
+  else vq_tc_layout_info(K, D, out8, zbytes);
+  return DVQ_OK;
+}
+
 long long dvq_debug_tc_image_offset(int k, int d, int K, int D, int pair, long long* image_bytes) {
   if (K <= 0 || D <= 0 || k < 0 || k >= K || d < 0 || d >= D + 16 || !vq_tc_supported(1, K, D)) return -1;
   return vq_tc_image_offset(k, d, K, D, pair, image_bytes);
@@ -193,9 +202,10 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
   if (N > 0 && (!z || !z_q || !idx)) return fail(DVQ_ERR_BAD_ARG, "z, z_q and idx must not be NULL");
   if (train && (!hist || !sse)) return fail(DVQ_ERR_BAD_ARG, "DVQ_TRAIN needs hist and sse");
   if ((flags & DVQ_WRITE_ONEHOT) && !onehot) return fail(DVQ_ERR_BAD_ARG, "DVQ_WRITE_ONEHOT needs onehot");
-  if ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(E) | reinterpret_cast<uintptr_t>(z_q)) % 4 != 0 ||
+  const bool zbf = (flags & DVQ_Z_BF16) != 0;   // z / z_q are bf16 rows
+  if ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(z_q)) % (zbf ? 2 : 4) != 0 || reinterpret_cast<uintptr_t>(E) % 4 != 0 ||
       reinterpret_cast<uintptr_t>(idx) % 8 != 0 || reinterpret_cast<uintptr_t>(workspace) % 256 != 0)
-    return fail(DVQ_ERR_BAD_ALIGN, "z/E/z_q need 4-byte, idx 8-byte, workspace 256-byte alignment");
+    return fail(DVQ_ERR_BAD_ALIGN, "z/z_q need %d-byte, E 4-byte, idx 8-byte, workspace 256-byte alignment", zbf ? 2 : 4);
   const VqWorkspace w = vq_workspace_layout(N, K, D, flags);
   if (workspace_bytes < w.total)
     return fail(DVQ_ERR_WORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, w.total);
@@ -227,7 +237,7 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
       int* cand_list = reinterpret_cast<int*>(ws + w.off_rowlist + align_up(sizeof(int) * (size_t)N, 256));
       profile_mark(1, true, s);
       rc = launch_vq_tc(z, E, ee, N, K, D, train, z_q, idx, hist, sse, ws + w.off_bop, counters, row_list, cand_list,
-                        reinterpret_cast<int*>(ws + w.off_binned), (int)(vq_refine_binned_zero_bytes() / sizeof(int)), cached, s);
+                        reinterpret_cast<int*>(ws + w.off_binned), (int)(vq_refine_binned_zero_bytes() / sizeof(int)), cached, zbf, s);
       profile_mark(1, false, s);
       if (rc) return rc;
       // exact FP32 refine of the rows the filter flagged (device-side count, no host sync): restricted to
@@ -250,21 +260,21 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
         const bool per_row_only = force_per_row || (!force_binned && vq_refine_codebook_in_smem(K, D));
         if (!per_row_only)
           rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, cand_list, counters, list_mode ? 1 : 0,
-                                       ws + w.off_binned, s);
+                                       ws + w.off_binned, zbf, s);
         if (!rc)
           rc = launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, row_list, cand_list, per_row_only ? counters : counters + 5,
                                 vq_tc_cand_gshift(K), list_mode ? row_list + (N - 1) : nullptr,
-                                list_mode ? (per_row_only ? counters + 2 : counters + 6) : nullptr, s);
+                                list_mode ? (per_row_only ? counters + 2 : counters + 6) : nullptr, zbf, s);
       } else {
-        rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, counters, 1, s);
+        rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, counters, 1, zbf, s);
         if (!rc && list_mode)
-          rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list + (N - 1), counters + 2, -1, s);
+          rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list + (N - 1), counters + 2, -1, zbf, s);
       }
       profile_mark(2, false, s);
       if (rc) return rc;
     } else {
       profile_mark(1, true, s);
-      rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, nullptr, nullptr, 1, s);
+      rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, nullptr, nullptr, 1, zbf, s);
       profile_mark(1, false, s);
       if (rc) return rc;
     }
@@ -337,26 +347,40 @@ int dvq_gather(const float* E, const int64_t* idx, int64_t N, int K, int D, floa
   return launch_gather(E, idx, N, K, D, out, oob, static_cast<cudaStream_t>(stream));
 }
 
-int dvq_vq_backward(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
-                    const float* rows, int64_t N, int K, int D, float al, float beta, float* dz, float* dE, void* stream) {
+int dvq_vq_backward_ex(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
+                       const float* rows, int64_t N, int K, int D, float al, float beta, int flags, float* dz, float* dE,
+                       void* stream) {
   if (N < 0 || K <= 0 || D <= 0 || (D & 3)) return fail(DVQ_ERR_BAD_SHAPE, "need N >= 0, K > 0, D a positive multiple of 4");
+  if (flags & ~DVQ_Z_BF16) return fail(DVQ_ERR_BAD_ARG, "dvq_vq_backward_ex accepts DVQ_Z_BF16 only");
   if (!g_loss || !rows || (N > 0 && (!z || !E || !idx))) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
-  if ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(E) | reinterpret_cast<uintptr_t>(g_zq) |
-       reinterpret_cast<uintptr_t>(dz) | reinterpret_cast<uintptr_t>(dE)) % 16 != 0)
-    return fail(DVQ_ERR_BAD_ALIGN, "dvq_vq_backward needs 16-byte aligned tensors");
+  const bool zbf = (flags & DVQ_Z_BF16) != 0;   // z, g_zq and dz move 4 elements at a time: 16 bytes fp32, 8 bytes bf16
+  if ((reinterpret_cast<uintptr_t>(E) | reinterpret_cast<uintptr_t>(dE)) % 16 != 0 ||
+      (reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(g_zq) | reinterpret_cast<uintptr_t>(dz)) % (zbf ? 8 : 16) != 0)
+    return fail(DVQ_ERR_BAD_ALIGN, "dvq_vq_backward needs 16-byte aligned E / dE and %d-byte aligned z / g_zq / dz", zbf ? 8 : 16);
   int rc = require_sm100();
   if (rc) return rc;
-  return launch_vq_backward(z, E, idx, g_zq, g_loss, rows, N, D, al, beta, dz, dE, static_cast<cudaStream_t>(stream));
+  return launch_vq_backward(z, E, idx, g_zq, g_loss, rows, N, D, al, beta, dz, dE, zbf, static_cast<cudaStream_t>(stream));
+}
+
+int dvq_vq_backward(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
+                    const float* rows, int64_t N, int K, int D, float al, float beta, float* dz, float* dE, void* stream) {
+  return dvq_vq_backward_ex(z, E, idx, g_zq, g_loss, rows, N, K, D, al, beta, 0, dz, dE, stream);
+}
+
+int dvq_vq_code_sums_ex(const float* z, const int64_t* idx, int64_t N, int K, int D, int flags, float* sums, void* stream) {
+  if (N < 0 || K <= 0 || D <= 0 || (D & 3)) return fail(DVQ_ERR_BAD_SHAPE, "need N >= 0, K > 0, D a positive multiple of 4");
+  if (flags & ~DVQ_Z_BF16) return fail(DVQ_ERR_BAD_ARG, "dvq_vq_code_sums_ex accepts DVQ_Z_BF16 only");
+  if (N > 0 && (!z || !idx || !sums)) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
+  const bool zbf = (flags & DVQ_Z_BF16) != 0;
+  if (reinterpret_cast<uintptr_t>(sums) % 16 != 0 || reinterpret_cast<uintptr_t>(z) % (zbf ? 8 : 16) != 0)
+    return fail(DVQ_ERR_BAD_ALIGN, "dvq_vq_code_sums needs 16-byte aligned sums and a %d-byte aligned z", zbf ? 8 : 16);
+  int rc = require_sm100();
+  if (rc) return rc;
+  return launch_vq_code_sums(z, idx, N, D, sums, zbf, static_cast<cudaStream_t>(stream));
 }
 
 int dvq_vq_code_sums(const float* z, const int64_t* idx, int64_t N, int K, int D, float* sums, void* stream) {
-  if (N < 0 || K <= 0 || D <= 0 || (D & 3)) return fail(DVQ_ERR_BAD_SHAPE, "need N >= 0, K > 0, D a positive multiple of 4");
-  if (N > 0 && (!z || !idx || !sums)) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
-  if ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(sums)) % 16 != 0)
-    return fail(DVQ_ERR_BAD_ALIGN, "dvq_vq_code_sums needs 16-byte aligned tensors");
-  int rc = require_sm100();
-  if (rc) return rc;
-  return launch_vq_code_sums(z, idx, N, D, sums, static_cast<cudaStream_t>(stream));
+  return dvq_vq_code_sums_ex(z, idx, N, K, D, 0, sums, stream);
 }
 
 int dvq_gather_multi(const float* const* E, int G, const int64_t* codes, int64_t N, int K, int D, float* out, int64_t out_stride,
@@ -569,6 +593,7 @@ int dvq_vq_forward_host(DvqHostCtx* c, const float* z_host, const float* E_host,
   if (K > c->K_max || D > c->D_max)
     return fail(DVQ_ERR_BAD_SHAPE, "K=%d D=%d exceed the context limits K_max=%d D_max=%d", K, D, c->K_max, c->D_max);
   if (flags & DVQ_WRITE_ONEHOT) return fail(DVQ_ERR_BAD_ARG, "the host-buffer entry does not materialise the one-hot matrix");
+  if (flags & DVQ_Z_BF16) return fail(DVQ_ERR_BAD_ARG, "the host-buffer entry takes fp32 rows only (DVQ_Z_BF16 is not accepted)");
   if (!E_host || (N > 0 && (!z_host || !zq_host || !idx_host))) return fail(DVQ_ERR_BAD_ARG, "NULL host pointer");
   const int train = (flags & DVQ_TRAIN) ? 1 : 0;
   if (train && (!loss_host || !perplexity_host)) return fail(DVQ_ERR_BAD_ARG, "DVQ_TRAIN needs loss_host and perplexity_host");

@@ -1,6 +1,7 @@
 // Shared internals of libdvq_sm100.so (not part of the public ABI).
 #pragma once
 
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -52,47 +53,48 @@ int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s);
 
 // Exact FP32 CUDA-core path.  row_list == nullptr: rows [0,N).  Otherwise rows
 // row_list[0 .. *n_list) (device-side count), used as the refine stage of the tcgen05 path.
-int launch_vq_simt(const float* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                   float* z_q, int64_t* idx, unsigned long long* hist, double* sse,
-                   const int* row_list, const int* n_list, int list_stride, cudaStream_t s);
+// zbf: z / z_q are bf16 rows (DVQ_Z_BF16), else fp32 — every VQ kernel below computes in fp32 on the upcast rows
+int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
+                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse,
+                   const int* row_list, const int* n_list, int list_stride, bool zbf, cudaStream_t s);
 
 // tcgen05 filter kernel (vq_tc_sm100.cu); supported(K,D) says whether the shape is handled.
 bool vq_tc_supported(int64_t N, int K, int D);
-void vq_tc_layout_info(int K, int D, int* out8);   // dvq_debug_tc_layout
+void vq_tc_layout_info(int K, int D, int* out8, int zbytes = 4);   // dvq_debug_tc_layout (zbytes: size of a z element)
 bool vq_tc_pair_selected(int64_t N, int K, int D);   // CTA-pair (cta_group::2) kernel for this shape?
-void vq_tc_pair_layout_info(int64_t N, int K, int D, int* out8);   // dvq_debug_tc_pair_layout
+void vq_tc_pair_layout_info(int64_t N, int K, int D, int* out8, int zbytes = 4);   // dvq_debug_tc_pair_layout
 long long vq_tc_image_offset(int k, int d, int K, int D, int pair, long long* image_bytes);   // dvq_debug_tc_image_offset
 size_t vq_tc_operand_bytes(int K, int D);
-int launch_vq_tc(const float* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                 float* z_q, int64_t* idx, unsigned long long* hist, double* sse,
+int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
+                 void* z_q, int64_t* idx, unsigned long long* hist, double* sse,
                  void* bop, int* counters, int* row_list, int* cand_list, int* zero_ints, int zero_n,
-                 bool codebook_cached, cudaStream_t s);
+                 bool codebook_cached, bool zbf, cudaStream_t s);
 
 // candidate-restricted exact refine (vq_refine.cu); cand_list[i] = bit mask of 32*2^gshift-code groups
 bool vq_refine_supported(int K, int D);
 bool vq_refine_codebook_in_smem(int K, int D);
 int vq_tc_cand_gshift(int K);
-int launch_vq_refine(const float* z, const float* E, const float* ee, int K, int D, int train, float* z_q, int64_t* idx,
+int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
                      unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                     const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, cudaStream_t s);
+                     const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, bool zbf, cudaStream_t s);
 
 // binned exact refine (vq_refine_binned.cu): (row, sub-chunk) pairs bucketed by sub-chunk; hands the list to
 // launch_vq_refine through counters[5] / counters[6] when the pairs do not fit its workspace
 long long refine_pair_cap_override();   // dvq_vq_set_refine (dvq_api.cu); 0 = default
 size_t vq_refine_binned_bytes(int64_t N);
 size_t vq_refine_binned_zero_bytes();
-int launch_vq_refine_binned(const float* z, const float* E, const float* ee, int64_t N, int K, int D, int train, float* z_q,
+int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
                             int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                            int* counters, int list_mode, void* ws, cudaStream_t s);
+                            int* counters, int list_mode, void* ws, bool zbf, cudaStream_t s);
 
 int launch_onehot(const int64_t* idx, int64_t N, int K, float* onehot, cudaStream_t s);
 int launch_finalize(const unsigned long long* hist, const double* sse, int64_t N, int K, int D, float al,
                     float beta, float* loss, float* ppl, cudaStream_t s);
-int launch_vq_backward(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
-                       const float* rows, int64_t N, int D, float al, float beta, float* dz, float* dE, cudaStream_t s);
+int launch_vq_backward(const void* z, const float* E, const int64_t* idx, const void* g_zq, const float* g_loss,
+                       const float* rows, int64_t N, int D, float al, float beta, void* dz, float* dE, bool zbf, cudaStream_t s);
 int launch_gather_multi(const float* const* E, int G, const int64_t* codes, int64_t N, int K, int D, float* out, int64_t out_stride,
                         int* oob, cudaStream_t s);
-int launch_vq_code_sums(const float* z, const int64_t* idx, int64_t N, int D, float* sums, cudaStream_t s);
+int launch_vq_code_sums(const void* z, const int64_t* idx, int64_t N, int D, float* sums, bool zbf, cudaStream_t s);
 int launch_gather(const float* E, const int64_t* idx, int64_t N, int K, int D, float* out, int* oob,
                   cudaStream_t s);
 
@@ -120,6 +122,33 @@ int launch_pointnet_tc_trunk(const float* x, const float* trans, const float* w1
 
 // ---- small device helpers ----------------------------------------------------------------
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+
+// z rows as fp32 or bf16 (DVQ_Z_BF16).  A bf16 value upcasts exactly (a 16-bit shift), so every kernel runs the fp32
+// arithmetic of the fp32 call on the upcast values; stores round to nearest even once.  The 4-element forms need
+// 16-byte (fp32) / 8-byte (bf16) alignment.
+__device__ __forceinline__ float zf(float v) { return v; }
+__device__ __forceinline__ float zf(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float4 bf4_to_f4(uint2 u) {
+  return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
+                     __uint_as_float(u.y & 0xffff0000u));
+}
+__device__ __forceinline__ uint32_t f2_to_bf2(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+__device__ __forceinline__ uint2 f4_to_bf4(float4 v) { return make_uint2(f2_to_bf2(v.x, v.y), f2_to_bf2(v.z, v.w)); }
+__device__ __forceinline__ float4 zld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+__device__ __forceinline__ float4 zld4(const __nv_bfloat16* p) { return bf4_to_f4(*reinterpret_cast<const uint2*>(p)); }
+__device__ __forceinline__ float4 zldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ float4 zldg4(const __nv_bfloat16* p) { return bf4_to_f4(__ldg(reinterpret_cast<const uint2*>(p))); }
+__device__ __forceinline__ float4 zldcs4(const float* p) { return __ldcs(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ float4 zldcs4(const __nv_bfloat16* p) { return bf4_to_f4(__ldcs(reinterpret_cast<const uint2*>(p))); }
+__device__ __forceinline__ void zst4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ void zst4(__nv_bfloat16* p, float4 v) { *reinterpret_cast<uint2*>(p) = f4_to_bf4(v); }
+__device__ __forceinline__ void zstcs4(float* p, float4 v) { __stcs(reinterpret_cast<float4*>(p), v); }
+__device__ __forceinline__ void zstcs4(__nv_bfloat16* p, float4 v) { __stcs(reinterpret_cast<uint2*>(p), f4_to_bf4(v)); }
+__device__ __forceinline__ void zst1(float* p, float v) { *p = v; }
+__device__ __forceinline__ void zst1(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

@@ -20,18 +20,20 @@ namespace {
 
 constexpr int RTHREADS = 1024;
 
-template <int DT, bool TRAIN, bool SMEM_E>
+// ZT: element type of z / z_q (float, or __nv_bfloat16 under DVQ_Z_BF16: the z rows are staged as bf16 and upcast on read)
+template <int DT, bool TRAIN, bool SMEM_E, typename ZT>
 __global__ void __launch_bounds__(RTHREADS, 1)
-vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K,
-                 float* __restrict__ zq, int64_t* __restrict__ idx_out, unsigned long long* __restrict__ hist,
+vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K,
+                 ZT* __restrict__ zq, int64_t* __restrict__ idx_out, unsigned long long* __restrict__ hist,
                  double* __restrict__ sse, const int* __restrict__ row_list, const int* __restrict__ cand_list,
                  const int* __restrict__ n_list, int gshift, const int* __restrict__ ovf_last, const int* __restrict__ n_ovf) {
-  extern __shared__ __align__(16) float smem_f[];   // zbuf[warps][2][DT] | es[K][DT+1] when SMEM_E
+  extern __shared__ __align__(16) float smem_f[];   // zbuf[warps][2][DT] (ZT) | es[K][DT+4] when SMEM_E
   constexpr int PITCH = DT + 4;
   constexpr int NW = RTHREADS / 32;
+  constexpr int ZE = 16 / (int)sizeof(ZT);          // z elements per 16-byte piece
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  float* zbuf = smem_f + warp * 2 * DT;             // double-buffered z row of this warp
-  float* es = smem_f + NW * 2 * DT;
+  ZT* zbuf = reinterpret_cast<ZT*>(smem_f) + warp * 2 * DT;   // double-buffered z row of this warp
+  float* es = reinterpret_cast<float*>(reinterpret_cast<ZT*>(smem_f) + NW * 2 * DT);
   // nothing listed (the usual case when the binned kernels ran first): leave before staging the codebook
   if (*n_list == 0 && (n_ovf == nullptr || *n_ovf == 0)) return;
   if (SMEM_E) {
@@ -51,30 +53,30 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
   // cp.async prefetch of the next undecided row of this warp hides its (random-access) global latency
   auto prefetch = [&](int i, int buf) {
     if (i < n) {
-      const float* src = z + (int64_t)row_list[i] * DT;
+      const ZT* src = z + (int64_t)row_list[i] * DT;
 #pragma unroll
-      for (int v = lane; v < DT / 4; v += 32) {
-        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zbuf + buf * DT + v * 4);
-        asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src + v * 4) : "memory");
+      for (int v = lane; v < DT / ZE; v += 32) {
+        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zbuf + buf * DT + v * ZE);
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src + v * ZE) : "memory");
       }
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
   };
   // outputs of one row (vq_simt_fp32.cu's epilogue), executed by one warp
-  auto emit_row = [&](int64_t row, int bidx, const float* zsrc) {
-    float* orow = zq + row * DT;
+  auto emit_row = [&](int64_t row, int bidx, const ZT* zsrc) {
+    ZT* orow = zq + row * DT;
     const float* erow = E + (int64_t)bidx * DT;
     for (int c = lane * 4; c < DT; c += 128) {
       const float4 e4 = ldg4(erow + c);
       float4 o4 = e4;
       if (TRAIN) {
-        const float4 z4 = *reinterpret_cast<const float4*>(zsrc + c);
+        const float4 z4 = zld4(zsrc + c);
         const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
         const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
         lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
         o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
       }
-      *reinterpret_cast<float4*>(orow + c) = o4;
+      zst4(orow + c, o4);
     }
     if (lane == 0) {
       idx_out[row] = (int64_t)bidx;
@@ -89,11 +91,11 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
     __syncwarp();
     const int64_t row = row_list[i];
     const unsigned cand = (unsigned)cand_list[i];
-    const float* zb = zbuf + buf * DT;
+    const ZT* zb = zbuf + buf * DT;
     float s2 = 0.f;   // ||z||^2 exactly as vq_simt_fp32.cu computes it
 #pragma unroll
     for (int c = 0; c < DT; c += 32) {
-      if (c + lane < DT) { const float v = zb[c + lane]; s2 = fmaf(v, v, s2); }
+      if (c + lane < DT) { const float v = zf(zb[c + lane]); s2 = fmaf(v, v, s2); }
     }
     const float zz = warp_sum(s2);
     float best = INFINITY;
@@ -163,7 +165,7 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
         const float* ea = es + (va ? code_a : 0) * PITCH;
 #pragma unroll
         for (int d = 0; d < DT; d += 4) {
-          const float4 z4 = *reinterpret_cast<const float4*>(zb + d);   // broadcast read
+          const float4 z4 = zld4(zb + d);   // broadcast read
           const float4 a4 = *reinterpret_cast<const float4*>(ea + d);
           acc_a = fmaf(z4.x, a4.x, acc_a); acc_a = fmaf(z4.y, a4.y, acc_a);
           acc_a = fmaf(z4.z, a4.z, acc_a); acc_a = fmaf(z4.w, a4.w, acc_a);
@@ -173,7 +175,7 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
         const float* eb = es + (vb ? code_b : 0) * PITCH;
 #pragma unroll
         for (int d = 0; d < DT; d += 4) {
-          const float4 z4 = *reinterpret_cast<const float4*>(zb + d);   // broadcast read
+          const float4 z4 = zld4(zb + d);   // broadcast read
           const float4 a4 = *reinterpret_cast<const float4*>(ea + d);
           const float4 b4 = *reinterpret_cast<const float4*>(eb + d);
           acc_a = fmaf(z4.x, a4.x, acc_a); acc_b = fmaf(z4.x, b4.x, acc_b);
@@ -186,7 +188,7 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
         const float* eb = E + (int64_t)(vb ? code_b : 0) * DT;
 #pragma unroll
         for (int d = 0; d < DT; d += 4) {
-          const float4 z4 = *reinterpret_cast<const float4*>(zb + d);
+          const float4 z4 = zld4(zb + d);
           const float4 a4 = ldg4(ea + d);
           const float4 b4 = ldg4(eb + d);
           acc_a = fmaf(z4.x, a4.x, acc_a); acc_b = fmaf(z4.x, b4.x, acc_b);
@@ -212,16 +214,16 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
     __shared__ float red_d[NW];
     __shared__ int red_k[NW];
     const int n2 = *n_ovf;
-    float* zrow = smem_f;   // every warp is done with its z buffers after the barrier below
+    ZT* zrow = reinterpret_cast<ZT*>(smem_f);   // every warp is done with its z buffers after the barrier below
     for (int j = blockIdx.x; j < n2; j += gridDim.x) {
       __syncthreads();
       const int64_t row = ovf_last[-(int64_t)j];   // the list is stored downwards from the end of the buffer
-      for (int v = tid; v < DT / 4; v += RTHREADS) reinterpret_cast<float4*>(zrow)[v] = ldg4(z + row * DT + v * 4);
+      for (int v = tid; v < DT / ZE; v += RTHREADS) reinterpret_cast<uint4*>(zrow)[v] = __ldg(reinterpret_cast<const uint4*>(z + row * DT) + v);
       __syncthreads();
       float s2 = 0.f;
 #pragma unroll
       for (int c = 0; c < DT; c += 32) {
-        if (c + lane < DT) { const float v = zrow[c + lane]; s2 = fmaf(v, v, s2); }
+        if (c + lane < DT) { const float v = zf(zrow[c + lane]); s2 = fmaf(v, v, s2); }
       }
       const float zz = warp_sum(s2);
       float best = INFINITY;
@@ -234,7 +236,7 @@ vq_refine_kernel(const float* __restrict__ z, const float* __restrict__ E, const
           float acc = 0.f;
 #pragma unroll 8
           for (int d = 0; d < DT; d += 4) {
-            const float4 z4 = *reinterpret_cast<const float4*>(zrow + d);
+            const float4 z4 = zld4(zrow + d);
             const float4 e4 = SMEM_E ? *reinterpret_cast<const float4*>(er + d) : ldg4(er + d);
             acc = fmaf(z4.x, e4.x, acc); acc = fmaf(z4.y, e4.y, acc);
             acc = fmaf(z4.z, e4.z, acc); acc = fmaf(z4.w, e4.w, acc);
@@ -279,18 +281,18 @@ bool vq_refine_codebook_in_smem(int K, int D) {
 
 bool vq_refine_supported(int K, int D) { return (D == 16 || D == 32 || D == 64 || D == 128 || D == 256 || D == 512) && K >= 32; }
 
-template <int DT>
-static int launch_refine_dt(const float* z, const float* E, const float* ee, int K, int train, float* z_q, int64_t* idx,
+template <int DT, typename ZT>
+static int launch_refine_dt(const ZT* z, const float* E, const float* ee, int K, int train, ZT* z_q, int64_t* idx,
                             unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
                             const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, int sm_count, cudaStream_t s) {
-  const size_t zbuf_bytes = (size_t)(RTHREADS / 32) * 2 * DT * sizeof(float);
+  const size_t zbuf_bytes = (size_t)(RTHREADS / 32) * 2 * DT * sizeof(ZT);
   const size_t smem_e = (size_t)K * (DT + 4) * sizeof(float);
   const bool in_smem = vq_refine_codebook_in_smem(K, DT);
 #define DVQ_LAUNCH_REFINE(TR_, SM_)                                                                                      \
   do {                                                                                                                   \
     const size_t bytes = zbuf_bytes + (SM_ ? smem_e : 0);                                                                \
-    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_refine_kernel<DT, TR_, SM_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)); \
-    vq_refine_kernel<DT, TR_, SM_><<<sm_count, RTHREADS, bytes, s>>>(z, E, ee, K, z_q, idx, hist, sse, row_list,         \
+    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_refine_kernel<DT, TR_, SM_, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)); \
+    vq_refine_kernel<DT, TR_, SM_, ZT><<<sm_count, RTHREADS, bytes, s>>>(z, E, ee, K, z_q, idx, hist, sse, row_list,         \
                                                                       cand_list, n_list, gshift, ovf_last, n_ovf);      \
   } while (0)
   if (train) { if (in_smem) DVQ_LAUNCH_REFINE(true, true); else DVQ_LAUNCH_REFINE(true, false); }
@@ -301,12 +303,10 @@ static int launch_refine_dt(const float* z, const float* E, const float* ee, int
   return DVQ_OK;
 }
 
-int launch_vq_refine(const float* z, const float* E, const float* ee, int K, int D, int train, float* z_q, int64_t* idx,
-                     unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                     const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, cudaStream_t s) {
-  DeviceProps dp;
-  int rc = device_props(&dp);
-  if (rc) return rc;
+template <typename ZT>
+static int launch_refine_t(const ZT* z, const float* E, const float* ee, int K, int D, int train, ZT* z_q, int64_t* idx,
+                           unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
+                           const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, const DeviceProps& dp, cudaStream_t s) {
   switch (D) {
     case 16: return launch_refine_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
     case 32: return launch_refine_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
@@ -316,6 +316,19 @@ int launch_vq_refine(const float* z, const float* E, const float* ee, int K, int
     case 512: return launch_refine_dt<512>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
     default: return fail(DVQ_ERR_BAD_SHAPE, "candidate refine kernel is instantiated for e_dim 16..512 (powers of two) only");
   }
+}
+
+int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
+                     unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
+                     const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, bool zbf, cudaStream_t s) {
+  DeviceProps dp;
+  int rc = device_props(&dp);
+  if (rc) return rc;
+  if (zbf)
+    return launch_refine_t(static_cast<const __nv_bfloat16*>(z), E, ee, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
+                           row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp, s);
+  return launch_refine_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, row_list, cand_list,
+                         n_list, gshift, ovf_last, n_ovf, dp, s);
 }
 
 }  // namespace dvq

@@ -71,8 +71,14 @@ __device__ __forceinline__ bool cand_is_all(unsigned cand, bool listed_normal, b
   return cand == 0u || cand == 0x7fffffffu;
 }
 
+// ||z||^2 of a listed row is stashed as a float in the first 4 bytes of its z_q row (rewritten by the emit kernel): 2 D >= 32
+// bytes of a bf16 row (DVQ_Z_BF16), at a 32-byte aligned offset
+template <typename ZT>
+__device__ __forceinline__ float* zz_stash(ZT* zq, int64_t row, int D) { return reinterpret_cast<float*>(zq + row * D); }
+
+template <typename ZT>
 __global__ void __launch_bounds__(PREP_THREADS, 1)
-refine_prep_kernel(const float* __restrict__ z, int D, int K, float* __restrict__ zq, unsigned long long* __restrict__ idx64,
+refine_prep_kernel(const ZT* __restrict__ z, int D, int K, ZT* __restrict__ zq, unsigned long long* __restrict__ idx64,
                    const int* __restrict__ row_list, const int* __restrict__ cand_list, const int* __restrict__ ovf_last,
                    int* __restrict__ counters, BinTables bt, int list_mode) {
   __shared__ int s_cnt[MAX_BINS];
@@ -94,13 +100,13 @@ refine_prep_kernel(const float* __restrict__ z, int D, int K, float* __restrict_
     const bool active = i < n + n2;
     const int64_t row = active ? listed_row(i, n, row_list, ovf_last) : 0;
     const unsigned cand = (active && i < n) ? (unsigned)cand_list[i] : 0u;
-    const float* zr = z + row * D;
+    const ZT* zr = z + row * D;
     float pm[4] = {0.f, 0.f, 0.f, 0.f};
     for (int c = 0; c < D; c += 32) {
 #pragma unroll
       for (int m = 0; m < 4; ++m) {
         const int d = c + j + 8 * m;
-        if (d < D) { const float v = __ldg(zr + d); pm[m] = fmaf(v, v, pm[m]); }
+        if (d < D) { const float v = zf(__ldg(zr + d)); pm[m] = fmaf(v, v, pm[m]); }
       }
     }
     float zz = (pm[0] + pm[2]) + (pm[1] + pm[3]);
@@ -109,7 +115,7 @@ refine_prep_kernel(const float* __restrict__ z, int D, int K, float* __restrict_
     zz += __shfl_xor_sync(0xffffffffu, zz, 1);
     if (active) {
       if (j == 0) {
-        zq[row * D] = zz;              // the row's z_q is rewritten by the emit kernel
+        *zz_stash(zq, row, D) = zz;    // the row's z_q is rewritten by the emit kernel
         idx64[row] = ~0ull;
       }
       const bool all = cand_is_all(cand, i < n, list_mode != 0);
@@ -218,13 +224,13 @@ __device__ __forceinline__ uint32_t float_key(float d) {
   return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
 
-template <int DS>
+template <int DS, typename ZT>
 __global__ void __launch_bounds__(PAIR_THREADS, DS <= 32 ? 2 : 1)
-refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K, int D,
-                    const float* __restrict__ zq, unsigned long long* __restrict__ idx64, const int* __restrict__ row_list,
+refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K, int D,
+                    ZT* __restrict__ zq, unsigned long long* __restrict__ idx64, const int* __restrict__ row_list,
                     const int* __restrict__ ovf_last, const int* __restrict__ pairs, const int* __restrict__ counters,
                     BinTables bt, long long pair_cap, int list_mode) {
-  extern __shared__ __align__(16) float smem_f[];   // zs[warps][2][RB][DS]
+  extern __shared__ __align__(16) float smem_f[];   // zs[warps][2][RB][DS] (ZT: bf16 rows are staged as bf16) | es
   __shared__ int s_start[MAX_BINS + 1];
   __shared__ int s_items[MAX_BINS + 1];
   constexpr int NW = PAIR_THREADS / 32;
@@ -237,7 +243,8 @@ refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, co
   __syncthreads();
   const int ch = bt.item_start[MAX_BINS + 1];
   const int items = s_items[nbins];
-  float* zs = smem_f + warp * 2 * RB * DS;   // two halves: one being read, one being filled
+  constexpr int ZE = 16 / (int)sizeof(ZT);    // z elements per 16-byte piece
+  ZT* zs = reinterpret_cast<ZT*>(smem_f) + warp * 2 * RB * DS;   // two halves: one being read, one being filled
   const int ns = D / DS;
   // sliced e_dim: the 32 code rows' slices are staged too ([32][DS + 4] floats, single-buffered: filled by coalesced
   // cp.async for the next step as soon as every lane has copied its own row into registers — conflict-free 128-bit loads —,
@@ -245,7 +252,7 @@ refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, co
   // Each lane fetching its own row straight from global memory — 32 different lines per load instruction — took two
   // thirds of the LSU data pipe, which the ncu capture showed to be the kernel's bound (74 % busy, FMA pipe 24 %).
   constexpr int EP = DS + 4;
-  float* es = smem_f + NW * 2 * RB * DS + warp * 32 * EP;
+  float* es = reinterpret_cast<float*>(reinterpret_cast<ZT*>(smem_f) + NW * 2 * RB * DS) + warp * 32 * EP;
   for (int item = blockIdx.x * NW + warp; item < items; item += gridDim.x * NW) {
     // bucket of this item: the last b with item_start[b] <= item
     int lo = 0, hi = nbins;   // invariant: s_items[lo] <= item < s_items[hi]
@@ -271,12 +278,12 @@ refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, co
     // Software pipeline over the (batch, slice) steps of the item: the z rows of the next step are copied into the
     // other half of the warp's staging buffer with cp.async (zero-filled for missing rows), and the
     // (row, ||z||^2) records of the next batch are read, while the current step is computed.
-    constexpr int ZL = RB * (DS / 4) / 32;   // 16-byte pieces per lane of one staged slice
+    constexpr int ZL = RB * (DS / ZE) / 32;   // 16-byte pieces per lane of one staged slice
     auto fetch_rows = [&](int p, int64_t& row_, float& zz_) {
       row_ = -1; zz_ = 0.f;
       if (p < p1 && lane < min(RB, p1 - p)) {
         row_ = listed_row(pairs[p + lane], n, row_list, ovf_last);
-        zz_ = zq[row_ * D];
+        zz_ = *zz_stash(zq, row_, D);
       }
     };
     auto stage_e = [&](int sl) {   // (no commit of its own)
@@ -294,10 +301,10 @@ refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, co
 #pragma unroll
       for (int k = 0; k < ZL; ++k) {
         const int f = k * 32 + lane;
-        const int r = f / (DS / 4), c4 = f - r * (DS / 4);
+        const int r = f / (DS / ZE), c4 = f - r * (DS / ZE);
         const long long rr = __shfl_sync(0xffffffffu, (long long)row_, r);
-        const float* src = rr >= 0 ? z + rr * D + sl * DS + c4 * 4 : z;
-        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zs + buf * RB * DS + r * DS + c4 * 4);
+        const ZT* src = rr >= 0 ? z + rr * D + sl * DS + c4 * ZE : z;
+        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zs + buf * RB * DS + r * DS + c4 * ZE);
         asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(rr >= 0 ? 16 : 0) : "memory");
       }
       asm volatile("cp.async.commit_group;" ::: "memory");
@@ -335,13 +342,13 @@ refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, co
             asm volatile("cp.async.commit_group;" ::: "memory");
           }
         }
-        const float* zb = zs + buf * RB * DS;
+        const ZT* zb = zs + buf * RB * DS;
         buf ^= 1;
 #pragma unroll
         for (int d = 0; d < DS; d += 4) {
 #pragma unroll
           for (int r = 0; r < RB; ++r) {
-            const float4 z4 = *reinterpret_cast<const float4*>(zb + r * DS + d);   // broadcast read
+            const float4 z4 = zld4(zb + r * DS + d);   // broadcast read
             acc[r] = fmaf(z4.x, e[d], acc[r]);
             acc[r] = fmaf(z4.y, e[d + 1], acc[r]);
             acc[r] = fmaf(z4.z, e[d + 2], acc[r]);
@@ -367,9 +374,9 @@ refine_pairs_kernel(const float* __restrict__ z, const float* __restrict__ E, co
   }
 }
 
-template <bool TRAIN>
+template <bool TRAIN, typename ZT>
 __global__ void __launch_bounds__(PREP_THREADS, 1)
-refine_emit_kernel(const float* __restrict__ z, const float* __restrict__ E, int D, float* __restrict__ zq,
+refine_emit_kernel(const ZT* __restrict__ z, const float* __restrict__ E, int D, ZT* __restrict__ zq,
                    unsigned long long* __restrict__ idx64, unsigned long long* __restrict__ hist, double* __restrict__ sse,
                    const int* __restrict__ row_list, const int* __restrict__ ovf_last, const int* __restrict__ counters,
                    long long pair_cap, int list_mode) {
@@ -386,21 +393,21 @@ refine_emit_kernel(const float* __restrict__ z, const float* __restrict__ E, int
     const int64_t row = active ? listed_row(i, n, row_list, ovf_last) : 0;
     const unsigned long long best = active ? idx64[row] : 0ull;
     const int bidx = best == ~0ull ? 0 : (int)(best & 0xffffffffull);
-    float* orow = zq + row * D;
+    ZT* orow = zq + row * D;
     const float* erow = E + (int64_t)bidx * D;
-    const float* zsrc = z + row * D;
+    const ZT* zsrc = z + row * D;
     if (active) {
       for (int c = j * 4; c < D; c += 32) {
         const float4 e4 = ldg4(erow + c);
         float4 o4 = e4;
         if (TRAIN) {
-          const float4 z4 = ldg4(zsrc + c);
+          const float4 z4 = zldg4(zsrc + c);
           const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
           const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
           lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
           o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
         }
-        *reinterpret_cast<float4*>(orow + c) = o4;
+        zst4(orow + c, o4);
       }
     }
     __syncwarp();   // every lane of the group has read idx64[row] before it is overwritten
@@ -424,9 +431,10 @@ size_t vq_refine_binned_bytes(int64_t N) {
 // the bin tables are zeroed by the caller (count, cursor: the first 2 * MAX_BINS ints of `ws`)
 size_t vq_refine_binned_zero_bytes() { return sizeof(int) * 2 * MAX_BINS; }
 
-int launch_vq_refine_binned(const float* z, const float* E, const float* ee, int64_t N, int K, int D, int train, float* z_q,
-                            int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                            int* counters, int list_mode, void* ws, cudaStream_t s) {
+template <typename ZT>
+static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t N, int K, int D, int train, ZT* z_q,
+                           int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
+                           int* counters, int list_mode, void* ws, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
@@ -454,11 +462,11 @@ int launch_vq_refine_binned(const float* z, const float* E, const float* ee, int
   DVQ_CUDA_CHECK(cudaGetLastError());
   refine_scatter_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(K, cand_list, counters, bt, pairs, pair_cap, list_mode, pair_warps);
   DVQ_CUDA_CHECK(cudaGetLastError());
-  const size_t smem = (size_t)(PAIR_THREADS / 32) * (2 * RB * DS + (D > DS ? 32 * (DS + 4) : 0)) * sizeof(float);
+  const size_t smem = (size_t)(PAIR_THREADS / 32) * (2 * RB * DS * sizeof(ZT) + (D > DS ? 32 * (DS + 4) * sizeof(float) : 0));
 #define DVQ_LAUNCH_PAIRS(DS_)                                                                                              \
   do {                                                                                                                     \
-    DVQ_CUDA_CHECK(cudaFuncSetAttribute(refine_pairs_kernel<DS_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    refine_pairs_kernel<DS_><<<pair_grid, PAIR_THREADS, smem, s>>>(z, E, ee, K, D, z_q, idx64, row_list, ovf_last, pairs,  \
+    DVQ_CUDA_CHECK(cudaFuncSetAttribute(refine_pairs_kernel<DS_, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    refine_pairs_kernel<DS_, ZT><<<pair_grid, PAIR_THREADS, smem, s>>>(z, E, ee, K, D, z_q, idx64, row_list, ovf_last, pairs,  \
                                                                    counters, bt, pair_cap, list_mode);                     \
   } while (0)
   if (DS == 64) DVQ_LAUNCH_PAIRS(64);
@@ -468,12 +476,22 @@ int launch_vq_refine_binned(const float* z, const float* E, const float* ee, int
 #undef DVQ_LAUNCH_PAIRS
   DVQ_CUDA_CHECK(cudaGetLastError());
   if (train)
-    refine_emit_kernel<true><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, row_list, ovf_last, counters, pair_cap, list_mode);
+    refine_emit_kernel<true, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, row_list, ovf_last, counters, pair_cap, list_mode);
   else
-    refine_emit_kernel<false><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, row_list, ovf_last, counters, pair_cap, list_mode);
+    refine_emit_kernel<false, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, row_list, ovf_last, counters, pair_cap, list_mode);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch(4);
   return DVQ_OK;
+}
+
+int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
+                            int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
+                            int* counters, int list_mode, void* ws, bool zbf, cudaStream_t s) {
+  if (zbf)
+    return launch_binned_t(static_cast<const __nv_bfloat16*>(z), E, ee, N, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
+                           row_list, cand_list, counters, list_mode, ws, s);
+  return launch_binned_t(static_cast<const float*>(z), E, ee, N, K, D, train, static_cast<float*>(z_q), idx, hist, sse, row_list,
+                         cand_list, counters, list_mode, ws, s);
 }
 
 }  // namespace dvq

@@ -25,26 +25,27 @@ constexpr int BK = 16;
 constexpr int LDT = 132;  // padded leading dim (floats); multiple of 4 keeps float4 reads aligned
 constexpr int NTHREADS = 256;
 
-template <bool VEC>
-__device__ __forceinline__ float4 load4(const float* __restrict__ base, int64_t row, int D, int k) {
+// T = float (codebook, fp32 z) or __nv_bfloat16 (DVQ_Z_BF16 z, upcast exactly)
+template <bool VEC, typename T>
+__device__ __forceinline__ float4 load4(const T* __restrict__ base, int64_t row, int D, int k) {
   float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
   if (row < 0) return v;
-  const float* p = base + row * (int64_t)D + k;
+  const T* p = base + row * (int64_t)D + k;
   if (VEC) {
-    if (k < D) v = __ldg(reinterpret_cast<const float4*>(p));
+    if (k < D) v = zldg4(p);
   } else {
-    if (k + 0 < D) v.x = __ldg(p + 0);
-    if (k + 1 < D) v.y = __ldg(p + 1);
-    if (k + 2 < D) v.z = __ldg(p + 2);
-    if (k + 3 < D) v.w = __ldg(p + 3);
+    if (k + 0 < D) v.x = zf(__ldg(p + 0));
+    if (k + 1 < D) v.y = zf(__ldg(p + 1));
+    if (k + 2 < D) v.z = zf(__ldg(p + 2));
+    if (k + 3 < D) v.w = zf(__ldg(p + 3));
   }
   return v;
 }
 
-template <bool VEC>
+template <bool VEC, typename ZT>
 __global__ void __launch_bounds__(NTHREADS, 2)
-vq_simt_kernel(const float* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee,
-               int64_t N, int K, int D, int train, float* __restrict__ zq, int64_t* __restrict__ idx_out,
+vq_simt_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee,
+               int64_t N, int K, int D, int train, ZT* __restrict__ zq, int64_t* __restrict__ idx_out,
                unsigned long long* __restrict__ hist, double* __restrict__ sse,
                const int* __restrict__ row_list, const int* __restrict__ n_list, int list_stride) {
   __shared__ __align__(16) float zs[BK][LDT];
@@ -77,8 +78,8 @@ vq_simt_kernel(const float* __restrict__ z, const float* __restrict__ E, const f
       const int64_t grow = srow[r];
       float s2 = 0.f;
       if (grow >= 0) {
-        const float* zrow = z + grow * (int64_t)D;
-        for (int c = lane; c < D; c += 32) { const float v = __ldg(zrow + c); s2 = fmaf(v, v, s2); }
+        const ZT* zrow = z + grow * (int64_t)D;
+        for (int c = lane; c < D; c += 32) { const float v = zf(__ldg(zrow + c)); s2 = fmaf(v, v, s2); }
       }
       s2 = warp_sum(s2);
       if (lane == 0) szz[r] = s2;
@@ -171,32 +172,32 @@ vq_simt_kernel(const float* __restrict__ z, const float* __restrict__ E, const f
       if (grow < 0) continue;
       const int k = sidx[r];
       const float* erow = E + (int64_t)k * D;
-      const float* zrow = z + grow * (int64_t)D;
-      float* orow = zq + grow * (int64_t)D;
+      const ZT* zrow = z + grow * (int64_t)D;
+      ZT* orow = zq + grow * (int64_t)D;
       if (VEC) {
         for (int c = lane * 4; c < D; c += 128) {
           const float4 e4 = ldg4(erow + c);
           float4 o4 = e4;
           if (train) {
-            const float4 z4 = ldg4(zrow + c);
+            const float4 z4 = zldg4(zrow + c);
             const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
             const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
             lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
             o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
           }
-          *reinterpret_cast<float4*>(orow + c) = o4;
+          zst4(orow + c, o4);
         }
       } else {
         for (int c = lane; c < D; c += 32) {
           const float e1 = __ldg(erow + c);
           float o1 = e1;
           if (train) {
-            const float z1 = __ldg(zrow + c);
+            const float z1 = zf(__ldg(zrow + c));
             const float dx = __fsub_rn(e1, z1);
             lsse += (double)dx * dx;
             o1 = __fadd_rn(z1, dx);
           }
-          orow[c] = o1;
+          zst1(orow + c, o1);
         }
       }
       if (lane == 0) {
@@ -240,9 +241,9 @@ int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s) {
   return DVQ_OK;
 }
 
-int launch_vq_simt(const float* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                   float* z_q, int64_t* idx, unsigned long long* hist, double* sse, const int* row_list,
-                   const int* n_list, int list_stride, cudaStream_t s) {
+int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
+                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse, const int* row_list,
+                   const int* n_list, int list_stride, bool zbf, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
@@ -250,12 +251,15 @@ int launch_vq_simt(const float* z, const float* E, const float* ee, int64_t N, i
   int64_t grid = (int64_t)dp.sm_count * 2;
   if (!row_list && tiles < grid) grid = tiles;
   if (grid < 1) grid = 1;
-  const bool vec = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(E) |
-                                     reinterpret_cast<uintptr_t>(z_q)) % 16 == 0);
-  if (vec)
-    vq_simt_kernel<true><<<(unsigned)grid, NTHREADS, 0, s>>>(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, n_list, list_stride);
-  else
-    vq_simt_kernel<false><<<(unsigned)grid, NTHREADS, 0, s>>>(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, n_list, list_stride);
+  // 128-bit codebook loads; z / z_q rows move 4 elements at a time (16 bytes fp32, 8 bytes bf16)
+  const bool vec = (D % 4 == 0) && reinterpret_cast<uintptr_t>(E) % 16 == 0 &&
+                   (reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(z_q)) % (zbf ? 8 : 16) == 0;
+#define DVQ_LAUNCH_SIMT(V_, T_)                                                                                             \
+  vq_simt_kernel<V_, T_><<<(unsigned)grid, NTHREADS, 0, s>>>(static_cast<const T_*>(z), E, ee, N, K, D, train,          \
+                                                             static_cast<T_*>(z_q), idx, hist, sse, row_list, n_list, list_stride)
+  if (zbf) { if (vec) DVQ_LAUNCH_SIMT(true, __nv_bfloat16); else DVQ_LAUNCH_SIMT(false, __nv_bfloat16); }
+  else     { if (vec) DVQ_LAUNCH_SIMT(true, float); else DVQ_LAUNCH_SIMT(false, float); }
+#undef DVQ_LAUNCH_SIMT
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;

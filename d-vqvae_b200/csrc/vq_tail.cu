@@ -106,10 +106,12 @@ __global__ void gather_kernel(const float* __restrict__ E, const int64_t* __rest
 __device__ __forceinline__ void red_add_v4(float* addr, float4 v) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
-template <bool HAS_GZQ, bool WANT_DZ, bool WANT_DE>
-__global__ void vq_backward_kernel(const float* __restrict__ z, const float* __restrict__ E, const int64_t* __restrict__ idx,
-                                   const float* __restrict__ g_zq, const float* __restrict__ g_loss, const float* __restrict__ rows,
-                                   int64_t N, int D, float al, float beta, float* __restrict__ dz, float* __restrict__ dE) {
+// ZT = __nv_bfloat16 (DVQ_Z_BF16): z, g_zq and dz are bf16 rows, the arithmetic is the same fp32 on the upcast values and dz is
+// rounded once when stored.
+template <bool HAS_GZQ, bool WANT_DZ, bool WANT_DE, typename ZT>
+__global__ void vq_backward_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const int64_t* __restrict__ idx,
+                                   const ZT* __restrict__ g_zq, const float* __restrict__ g_loss, const float* __restrict__ rows,
+                                   int64_t N, int D, float al, float beta, ZT* __restrict__ dz, float* __restrict__ dE) {
   const float scale = 2.0f * __ldg(g_loss) / (__ldg(rows) * (float)D);
   const float sz = scale * al, se = scale * beta;
   const int nv = D >> 2;
@@ -118,16 +120,16 @@ __global__ void vq_backward_kernel(const float* __restrict__ z, const float* __r
     const int64_t row = i / nv;
     const int c = (int)(i - row * nv) << 2;
     const int64_t k = __ldg(idx + row);
-    const float4 z4 = __ldcs(reinterpret_cast<const float4*>(z + row * D + c));
+    const float4 z4 = zldcs4(z + row * D + c);
     const float4 e4 = ldg4(E + k * D + c);
     const float4 d4 = make_float4(z4.x - e4.x, z4.y - e4.y, z4.z - e4.z, z4.w - e4.w);
     if (WANT_DZ) {
       float4 o = make_float4(sz * d4.x, sz * d4.y, sz * d4.z, sz * d4.w);
       if (HAS_GZQ) {
-        const float4 g4 = __ldcs(reinterpret_cast<const float4*>(g_zq + row * D + c));
+        const float4 g4 = zldcs4(g_zq + row * D + c);
         o.x += g4.x; o.y += g4.y; o.z += g4.z; o.w += g4.w;
       }
-      __stcs(reinterpret_cast<float4*>(dz + row * D + c), o);
+      zstcs4(dz + row * D + c, o);
     }
     if (WANT_DE) red_add_v4(dE + k * D + c, make_float4(-se * d4.x, -se * d4.y, -se * d4.z, -se * d4.w));
   }
@@ -157,20 +159,21 @@ __global__ void gather_multi_kernel(const GatherMultiParams gp, const int64_t* _
 }
 
 // sums[k,:] += sum over the rows assigned to code k of z[n,:]  (the per-code input sums of an EMA codebook update)
-__global__ void vq_code_sums_kernel(const float* __restrict__ z, const int64_t* __restrict__ idx, int64_t N, int D,
+template <typename ZT>
+__global__ void vq_code_sums_kernel(const ZT* __restrict__ z, const int64_t* __restrict__ idx, int64_t N, int D,
                                     float* __restrict__ sums) {
   const int nv = D >> 2;
   const int64_t total = N * (int64_t)nv;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t row = i / nv;
     const int c = (int)(i - row * nv) << 2;
-    red_add_v4(sums + __ldg(idx + row) * D + c, __ldcs(reinterpret_cast<const float4*>(z + row * D + c)));
+    red_add_v4(sums + __ldg(idx + row) * D + c, zldcs4(z + row * D + c));
   }
 }
 }  // namespace
 
-int launch_vq_backward(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
-                       const float* rows, int64_t N, int D, float al, float beta, float* dz, float* dE, cudaStream_t s) {
+int launch_vq_backward(const void* z, const float* E, const int64_t* idx, const void* g_zq, const float* g_loss,
+                       const float* rows, int64_t N, int D, float al, float beta, void* dz, float* dE, bool zbf, cudaStream_t s) {
   if (N == 0 || (!dz && !dE)) return DVQ_OK;
   DeviceProps dp;
   int rc = device_props(&dp);
@@ -178,10 +181,18 @@ int launch_vq_backward(const float* z, const float* E, const int64_t* idx, const
   const int threads = 256;
   int64_t blocks = (N * (D / 4) + threads - 1) / threads;
   if (blocks > (int64_t)dp.sm_count * 16) blocks = (int64_t)dp.sm_count * 16;
-#define DVQ_BWD(G_, Z_, E_) vq_backward_kernel<G_, Z_, E_><<<(unsigned)blocks, threads, 0, s>>>(z, E, idx, g_zq, g_loss, rows, N, D, al, beta, dz, dE)
-  if (dz && dE) { if (g_zq) DVQ_BWD(true, true, true); else DVQ_BWD(false, true, true); }
-  else if (dz) { if (g_zq) DVQ_BWD(true, true, false); else DVQ_BWD(false, true, false); }
-  else DVQ_BWD(false, false, true);
+#define DVQ_BWD(G_, Z_, E_, T_)                                                                                    \
+  vq_backward_kernel<G_, Z_, E_, T_><<<(unsigned)blocks, threads, 0, s>>>(static_cast<const T_*>(z), E, idx,        \
+      static_cast<const T_*>(g_zq), g_loss, rows, N, D, al, beta, static_cast<T_*>(dz), dE)
+#define DVQ_BWD_T(T_)                                                                                              \
+  do {                                                                                                             \
+    if (dz && dE) { if (g_zq) DVQ_BWD(true, true, true, T_); else DVQ_BWD(false, true, true, T_); }                 \
+    else if (dz) { if (g_zq) DVQ_BWD(true, true, false, T_); else DVQ_BWD(false, true, false, T_); }                \
+    else DVQ_BWD(false, false, true, T_);                                                                          \
+  } while (0)
+  if (zbf) DVQ_BWD_T(__nv_bfloat16);
+  else DVQ_BWD_T(float);
+#undef DVQ_BWD_T
 #undef DVQ_BWD
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
@@ -206,7 +217,7 @@ int launch_gather_multi(const float* const* E, int G, const int64_t* codes, int6
   return DVQ_OK;
 }
 
-int launch_vq_code_sums(const float* z, const int64_t* idx, int64_t N, int D, float* sums, cudaStream_t s) {
+int launch_vq_code_sums(const void* z, const int64_t* idx, int64_t N, int D, float* sums, bool zbf, cudaStream_t s) {
   if (N == 0) return DVQ_OK;
   DeviceProps dp;
   int rc = device_props(&dp);
@@ -214,7 +225,8 @@ int launch_vq_code_sums(const float* z, const int64_t* idx, int64_t N, int D, fl
   const int threads = 256;
   int64_t blocks = (N * (D / 4) + threads - 1) / threads;
   if (blocks > (int64_t)dp.sm_count * 16) blocks = (int64_t)dp.sm_count * 16;
-  vq_code_sums_kernel<<<(unsigned)blocks, threads, 0, s>>>(z, idx, N, D, sums);
+  if (zbf) vq_code_sums_kernel<__nv_bfloat16><<<(unsigned)blocks, threads, 0, s>>>(static_cast<const __nv_bfloat16*>(z), idx, N, D, sums);
+  else vq_code_sums_kernel<float><<<(unsigned)blocks, threads, 0, s>>>(static_cast<const float*>(z), idx, N, D, sums);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;

@@ -108,13 +108,13 @@ __host__ __device__ inline int cb_magic(int K, int D, bool pair = false) { retur
 struct TcParams {
   CUtensorMap ztile;      // z as a [N, D] tensor, box = (slice columns, 128 rows): the staged slices of e_dim > 64 (one TMA load each)
   CUtensorMap bmap[2];    // CTA-pair kernel: the operand image as [bytes / 1024, 256] int32, box = one half block without ([0]) / with ([1]) the fold columns
-  const float* z;
+  const void* z;          // [N, D] fp32 or bf16 (the kernel's ZT)
   const float* E;
   const uint8_t* bimg;
   const CbMeta* cb;
   int64_t N;
   int K, D, train;
-  float* zq;
+  void* zq;               // [N, D] ZT
   int64_t* idx;
   unsigned long long* hist;
   double* sse;
@@ -162,7 +162,9 @@ __host__ __device__ inline uint32_t smem_place(SmemLayout& L, int K) {
 // `ovr` != 0 forces (A images, z staging slots, ring slots) = (ovr / 100, ovr / 10 % 10, ovr % 10) for a streamed image
 // (experiments: DVQ_TC_LAYOUT; the launch passes it to the kernel so that both sides agree)
 // `pair`: layout of the CTA-pair kernel (cta_group::2) — always streamed, a ring slot holds this CTA's half (128 codes) of a block
-__host__ __device__ inline SmemLayout smem_layout(int K, int D, int ovr = 0, bool pair = false) {
+// `zbytes`: size of a z element (4 fp32, 2 bf16): a staging slot holds 128 rows of one slice.  Which kernel and layout class a shape
+// gets is decided on the fp32 plan (vq_tc_supported, vq_tc_pair_selected); the smaller bf16 slots only re-run the search below.
+__host__ __device__ inline SmemLayout smem_layout(int K, int D, int ovr = 0, bool pair = false, int zbytes = 4) {
   SmemLayout L;
   L.ds = (uint32_t)slice_width(D);
   L.ns = (uint32_t)D / L.ds;
@@ -171,7 +173,7 @@ __host__ __device__ inline SmemLayout smem_layout(int K, int D, int ovr = 0, boo
   L.bslice_bytes = kc_s * L.bcodes * 16u;
   L.bchunk_bytes = (kc_s + 2u) * L.bcodes * 16u;
   L.a_bytes = kc_a * A_CHUNK_BYTES;
-  L.stage_bytes = (uint32_t)TM * L.ds * 4;
+  L.stage_bytes = (uint32_t)TM * L.ds * (uint32_t)zbytes;
   const uint32_t nchunks = (uint32_t)(K + 255) / 256;
   if (!pair && nchunks * L.ns <= 2) {
     // resident operand image (two slots hold it for the life of the CTA).  Preference order when shared memory is
@@ -454,6 +456,23 @@ __device__ __forceinline__ float half_minus_float(uint32_t h16, float a) {
   return r;
 }
 
+// Reads of one staged z row: 4 elements at column 4 * c4 (one float4 / one 8-byte word of bf16, upcast exactly with a shift),
+// and the 8-wide k-chunk c8 as two float4 (two 16-byte loads of fp32, one of bf16)
+__device__ __forceinline__ void stage_ld8(const float4* row, int c8, float4& v0, float4& v1) {
+  v0 = row[2 * c8];
+  v1 = row[2 * c8 + 1];
+}
+__device__ __forceinline__ void stage_ld8(const uint2* row, int c8, float4& v0, float4& v1) {
+  const uint4 u = reinterpret_cast<const uint4*>(row)[c8];
+  v0 = bf4_to_f4(make_uint2(u.x, u.y));
+  v1 = bf4_to_f4(make_uint2(u.z, u.w));
+}
+// four z elements of a gather lane as loaded (float4 / packed bf16: the bf16 form holds half the registers while in flight)
+__device__ __forceinline__ float4 zraw_ldcs(const float* p) { return __ldcs(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ uint2 zraw_ldcs(const __nv_bfloat16* p) { return __ldcs(reinterpret_cast<const uint2*>(p)); }
+__device__ __forceinline__ float4 zup(float4 v) { return v; }
+__device__ __forceinline__ float4 zup(uint2 u) { return bf4_to_f4(u); }
+
 // All barriers live in one shared struct so that a site addresses its barrier as base + immediate.
 // (B_PEER_*: CTA-pair kernel, used in the leader CTA only — the peer CTA arrives on them remotely: its warp 1 once per tile
 // on B_PEER_A_FULL, each of its filter warps once per chunk on B_PEER_ACC_EMPTY)
@@ -666,10 +685,13 @@ __device__ __forceinline__ void filter_subchunk2(uint32_t (&va)[32], uint32_t (&
 // peer's warp 1 forwards "A image full" once per tile (remote arrive, release / acquire at cluster scope), the peer's filter
 // warps announce a freed accumulator stage with one remote arrive each; completions are committed to both CTAs' barriers
 // (multicast).
-template <int DT, bool TRAIN, bool LIST, bool CE, bool ST, bool PAIR = false>
+// ZT: element type of z / z_q — float, or __nv_bfloat16 (DVQ_Z_BF16: half the staging bytes, the converters and the gather
+// warps upcast exactly and run the fp32 arithmetic unchanged, z_q is rounded to bf16 when stored).
+template <int DT, bool TRAIN, bool LIST, bool CE, bool ST, bool PAIR = false, typename ZT = float>
 __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constant__ TcParams p) {
   static_assert(!(CE && ST), "the converter warps cannot hold the two-sub-chunk filter in 64 registers");
   static_assert(!PAIR || DT == 0, "the CTA-pair kernel is the generic streamed kernel");
+  using ZRaw = decltype(zraw_ldcs(static_cast<const ZT*>(nullptr)));   // four z elements as loaded: float4 / uint2 (bf16)
   constexpr int EPQX = CE ? EPQ + 1 : EPQ;       // filter warps per TMEM lane quarter
   constexpr int NB_ACC_THREADS = nb_acc_threads(EPQX), NB_ACC_HLP_THREADS = nb_acc_hlp_threads(EPQX), NB_FIN_THREADS = nb_fin_threads(EPQX);
   extern __shared__ __align__(128) uint8_t smem[];
@@ -683,7 +705,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
 
   const int D = DT > 0 ? DT : p.D;
   const int K = p.K;
-  const SmemLayout L = smem_layout(K, D, p.layout_ovr, PAIR);
+  const SmemLayout L = smem_layout(K, D, p.layout_ovr, PAIR, (int)sizeof(ZT));
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t crank = PAIR ? tc::cluster_ctarank() : 0u;   // 0 = leader (issues the MMAs), 1 = peer
   const int ns = DT > 0 ? (DT > DSLICE ? DT / DSLICE : 1) : (int)L.ns;   // e_dim slices
@@ -842,12 +864,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
           { STAT_T0(); wait_or_trap(BAR(B_STAGE_EMPTY, s), ph ^ 1u, err_out, ERR_STAGE_EMPTY); STAT_ADD(0); }
           if (ns == 1) {
             if (lane == 0) {   // the whole tile is one contiguous block
-              const uint32_t bytes = (uint32_t)rows * D * 4;
+              const uint32_t bytes = (uint32_t)rows * D * (uint32_t)sizeof(ZT);
               if (PAIR && rows == 0) tc::mbar_arrive_a(BAR(B_STAGE_FULL, s));   // the pair's tile past the end: nothing to load
               else {
                 tc::mbar_arrive_expect_tx_a(BAR(B_STAGE_FULL, s), bytes);
-                if (TRAIN) tc::bulk_g2s_keep_a(smem0 + L.stage[s], p.z + row0 * D, bytes, BAR(B_STAGE_FULL, s));
-                else tc::bulk_g2s_a(smem0 + L.stage[s], p.z + row0 * D, bytes, BAR(B_STAGE_FULL, s));
+                if (TRAIN) tc::bulk_g2s_keep_a(smem0 + L.stage[s], static_cast<const ZT*>(p.z) + row0 * D, bytes, BAR(B_STAGE_FULL, s));
+                else tc::bulk_g2s_a(smem0 + L.stage[s], static_cast<const ZT*>(p.z) + row0 * D, bytes, BAR(B_STAGE_FULL, s));
               }
             }
           } else {
@@ -855,7 +877,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
             // the barrier counts the whole box.  (As one bulk copy per 128- / 256-byte row segment — 128 per slice — this
             // was the bound of the sliced shapes: 2.1x the filter time at K = 512, e_dim 512.)
             if (lane == 0) {
-              tc::mbar_arrive_expect_tx_a(BAR(B_STAGE_FULL, s), (uint32_t)TM * ds * 4);
+              tc::mbar_arrive_expect_tx_a(BAR(B_STAGE_FULL, s), (uint32_t)TM * ds * (uint32_t)sizeof(ZT));
               if (TRAIN) tc::tma_load_2d_keep_a(smem0 + L.stage[s], &p.ztile, sl * ds, (int)row0, BAR(B_STAGE_FULL, s));
               else tc::tma_load_2d_a(smem0 + L.stage[s], &p.ztile, sl * ds, (int)row0, BAR(B_STAGE_FULL, s));
             }
@@ -1063,7 +1085,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
         const int s = L.nstage == 2 ? (int)(js & 1u) : 0;
         { STAT_T0(); wait_or_trap(BAR(B_STAGE_FULL, s), L.nstage == 2 ? (js >> 1) & 1u : js & 1u, err_out, ERR_STAGE_FULL); STAT_ADD(0); }
         if (warp == CONV_WARP0) TRACE(3, 0, 0);
-        const float4* src = reinterpret_cast<const float4*>(smem + L.stage[s]) + (size_t)r * nvs;
+        const ZRaw* src = reinterpret_cast<const ZRaw*>(smem + L.stage[s]) + (size_t)r * nvs;
 #ifdef DVQ_KO_NORM   // knock-out (timing experiment, wrong results): skip the norm pass
         if (r < rows) nsq = 64.f;
         if (false) {
@@ -1074,7 +1096,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
           uint64_t n01 = pack_f32x2(0.f, 0.f), n23 = n01;
           for (int i = 0; i < nvs; ++i) {
             const int c4 = (i + lane) & (nvs - 1);
-            const float4 v = src[c4];
+            const float4 v = zup(src[c4]);
             const uint64_t v01 = pack_f32x2(v.x, v.y), v23 = pack_f32x2(v.z, v.w);
             n01 = ffma2(v01, v01, n01); n23 = ffma2(v23, v23, n23);
           }
@@ -1104,7 +1126,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
       for (int sl = 0; sl < ns; ++sl, ++js) {
         const int s = L.nstage == 2 ? (int)(js & 1u) : 0;
         if (sl > 0) { STAT_T0(); wait_or_trap(BAR(B_STAGE_FULL, s), L.nstage == 2 ? (js >> 1) & 1u : js & 1u, err_out, ERR_STAGE_FULL); STAT_ADD(0); }
-        const float4* src = reinterpret_cast<const float4*>(smem + L.stage[s]) + (size_t)r * nvs;
+        const ZRaw* src = reinterpret_cast<const ZRaw*>(smem + L.stage[s]) + (size_t)r * nvs;
         uint8_t* aslice = aimg + (size_t)(sl * (nvs / 2)) * A_CHUNK_BYTES;
 #ifdef DVQ_KO_CONV   // knock-out: skip the FP16 conversion of the tile (the A image keeps stale data)
         for (int i = 0; i < 0; ++i) {
@@ -1112,7 +1134,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
         for (int i = 0; i < nvs / 2; ++i) {
 #endif
           const int c8 = (i + lane) & (nvs / 2 - 1);                       // 8-wide k-chunk
-          const float4 v0 = src[2 * c8], v1 = src[2 * c8 + 1];
+          float4 v0, v1;
+          stage_ld8(src, c8, v0, v1);
           // scale by the power-of-two s_n, two elements per FMUL2 (exact)
           const uint64_t xp[4] = {fmul2(pack_f32x2(v0.x, v0.y), s_n2), fmul2(pack_f32x2(v0.z, v0.w), s_n2),
                                   fmul2(pack_f32x2(v1.x, v1.y), s_n2), fmul2(pack_f32x2(v1.z, v1.w), s_n2)};
@@ -1305,14 +1328,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
       // Two batches of UH row-steps are kept in flight (software pipeline: the loads of batch b + 1 are issued
       // before batch b is consumed), and the z rows of the first batch — they do not depend on the codes — are
       // requested before this tile's codes arrive, so that only one L2 round trip per tile is exposed.
-      float4 eA[UH], zA[UH], eB[UH], zB[UH];
+      float4 eA[UH], eB[UH];
+      ZRaw zA[UH], zB[UH];
       int kA[UH], kB[UH];
       const bool full_tile = rows == TM;
       const bool piped = full_tile && (nsteps % (2 * UH)) == 0;
-      const float* zp0 = p.z + (row0 + rbase) * D + c4_lane * 4;
+      const ZT* zp0 = static_cast<const ZT*>(p.z) + (row0 + rbase) * D + c4_lane * 4;
       if (TRAIN && piped && PREFETCH_Z) {
 #pragma unroll
-        for (int u = 0; u < UH; ++u) zA[u] = __ldcs(reinterpret_cast<const float4*>(zp0 + (int64_t)(u * rps) * D));
+        for (int u = 0; u < UH; ++u) zA[u] = zraw_ldcs(zp0 + (int64_t)(u * rps) * D);
       }
       { STAT_T0(); nb_sync(NB_SIDX_FULL + slot, NB_SIDX_THREADS); STAT_ADD(0); }
       if (gw == 0) TRACE(4, 0, 0);
@@ -1355,20 +1379,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
 #endif
         const int c4 = (part << 5) | c4_lane;
         const char* ec = reinterpret_cast<const char*>(p.E + c4 * 4);
-        const float* zp = p.z + (row0 + rbase) * D + c4 * 4;
-        float* op = p.zq + (row0 + rbase) * D + c4 * 4;
+        const ZT* zp = static_cast<const ZT*>(p.z) + (row0 + rbase) * D + c4 * 4;
+        ZT* op = static_cast<ZT*>(p.zq) + (row0 + rbase) * D + c4 * 4;
         if (piped) {
           // fast path: no per-row checks
-          auto issue = [&](int t0, float4 (&e4)[UH], float4 (&z4)[UH], int (&kk)[UH], bool have_z) {
+          auto issue = [&](int t0, float4 (&e4)[UH], ZRaw (&z4)[UH], int (&kk)[UH], bool have_z) {
 #pragma unroll
             for (int u = 0; u < UH; ++u) kk[u] = sp[(t0 + u) * rps];
 #pragma unroll
             for (int u = 0; u < UH; ++u) {
               e4[u] = __ldg(reinterpret_cast<const float4*>(ec + (uint32_t)max(kk[u], 0)));   // undecided: any valid row
-              if (TRAIN && !have_z) z4[u] = __ldcs(reinterpret_cast<const float4*>(zp + (int64_t)((t0 + u) * rps) * D));   // last use of this tile
+              if (TRAIN && !have_z) z4[u] = zraw_ldcs(zp + (int64_t)((t0 + u) * rps) * D);   // last use of this tile
             }
           };
-          auto finish = [&](int t0, const float4 (&e4)[UH], const float4 (&z4)[UH], const int (&kk)[UH]) {
+          auto finish = [&](int t0, const float4 (&e4)[UH], const ZRaw (&z4)[UH], const int (&kk)[UH]) {
 #pragma unroll
             for (int u = 0; u < UH; ++u) {
               float4 o4 = e4[u];
@@ -1376,7 +1400,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
                 // packed FP32 (FADD2 / FMUL2 / FFMA2): d = fl(e - z), z_q = fl(z + d), two elements per instruction,
                 // each half an ordinary IEEE operation (bit-identical to the scalar form, no contraction)
                 const uint64_t e01 = pack_f32x2(e4[u].x, e4[u].y), e23 = pack_f32x2(e4[u].z, e4[u].w);
-                const uint64_t z01 = pack_f32x2(z4[u].x, z4[u].y), z23 = pack_f32x2(z4[u].z, z4[u].w);
+                const float4 zu = zup(z4[u]);
+                const uint64_t z01 = pack_f32x2(zu.x, zu.y), z23 = pack_f32x2(zu.z, zu.w);
                 const uint64_t d01 = fsub2(e01, z01), d23 = fsub2(e23, z23);
                 const uint64_t s2 = ffma2(d23, d23, fmul2(d01, d01));
                 float s0, s1;
@@ -1385,7 +1410,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
                 unpack_f32x2(fadd2(z01, d01), o4.x, o4.y);
                 unpack_f32x2(fadd2(z23, d23), o4.z, o4.w);
               }
-              __stcs(reinterpret_cast<float4*>(op + (int64_t)((t0 + u) * rps) * D), o4);   // streaming: never re-read
+              zstcs4(op + (int64_t)((t0 + u) * rps) * D, o4);   // streaming: never re-read
             }
           };
           issue(0, eA, zA, kA, PREFETCH_Z && part == 0);   // part 0: the z rows of the first batch were requested before the barrier
@@ -1405,14 +1430,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
             const float4 e1 = __ldg(reinterpret_cast<const float4*>(ec + (uint32_t)max(kv, 0)));
             float4 o4 = e1;
             if (TRAIN) {
-              const float4 z1 = __ldcs(reinterpret_cast<const float4*>(zp + (int64_t)ro * D));
+              const float4 z1 = zldcs4(zp + (int64_t)ro * D);
               const float dx = __fsub_rn(e1.x, z1.x), dy = __fsub_rn(e1.y, z1.y);
               const float dz = __fsub_rn(e1.z, z1.z), dw = __fsub_rn(e1.w, z1.w);
               const float ss = fmaf(dw, dw, fmaf(dz, dz, fmaf(dy, dy, dx * dx)));
               lsse = fmaf(kv < 0 ? 0.f : 1.f, ss, lsse);
               o4 = make_float4(__fadd_rn(z1.x, dx), __fadd_rn(z1.y, dy), __fadd_rn(z1.z, dz), __fadd_rn(z1.w, dw));
             }
-            __stcs(reinterpret_cast<float4*>(op + (int64_t)ro * D), o4);
+            zstcs4(op + (int64_t)ro * D, o4);
           }
         }
       }
@@ -1454,9 +1479,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
 
 }  // namespace
 
-// z [N, D] fp32 row-major as a 2-D tensor map with box (ds columns, TM rows), no swizzle: a slice of a row tile lands as
-// [row][ds floats], the layout the converter warps read
-static int encode_ztile(CUtensorMap* map, const float* z, int64_t N, int D, int ds) {
+// z [N, D] fp32 / bf16 row-major as a 2-D tensor map with box (ds columns, TM rows), no swizzle: a slice of a row tile lands as
+// [row][ds elements], the layout the converter warps read
+static int encode_ztile(CUtensorMap* map, const void* z, int64_t N, int D, int ds, bool zbf) {
   typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
   static EncodeFn encode = nullptr;
@@ -1468,10 +1493,11 @@ static int encode_ztile(CUtensorMap* map, const float* z, int64_t N, int D, int 
     encode = reinterpret_cast<EncodeFn>(fn);
   }
   const cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)N};
-  const cuuint64_t strides[1] = {(cuuint64_t)D * sizeof(float)};
+  const cuuint64_t strides[1] = {(cuuint64_t)D * (zbf ? 2u : 4u)};
   const cuuint32_t box[2] = {(cuuint32_t)ds, (cuuint32_t)TM};
   const cuuint32_t estr[2] = {1u, 1u};
-  const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(z), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  const CUresult r = encode(map, zbf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(z), dims, strides,
+                            box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for z [%lld, %d]", (int)r, (long long)N, D);
   return DVQ_OK;
@@ -1533,20 +1559,20 @@ bool vq_tc_pair_selected(int64_t N, int K, int D) {
 
 // dvq_debug_tc_pair_layout: out8 = { CTA-pair kernel selected for (N, K, D) (0/1), slice width, slices, A images, ring
 // slots, z staging slots, dynamic shared memory, codes per ring slot } of the pair layout (host-only)
-void vq_tc_pair_layout_info(int64_t N, int K, int D, int* out8) {
+void vq_tc_pair_layout_info(int64_t N, int K, int D, int* out8, int zbytes) {
   for (int i = 0; i < 8; ++i) out8[i] = 0;
   if (!vq_tc_supported(N > 0 ? N : 1, K, D)) return;
-  const SmemLayout L = smem_layout(K, D, 0, true);
+  const SmemLayout L = smem_layout(K, D, 0, true, zbytes);
   out8[0] = vq_tc_pair_selected(N, K, D) ? 1 : 0;
   out8[1] = (int)L.ds; out8[2] = (int)L.ns; out8[3] = (int)L.a_bufs; out8[4] = (int)L.nslots; out8[5] = (int)L.nstage;
   out8[6] = (int)L.total + 128; out8[7] = (int)L.bcodes;
 }
 
-void vq_tc_layout_info(int K, int D, int* out8) {
+void vq_tc_layout_info(int K, int D, int* out8, int zbytes) {
   const bool shape_ok = D >= 16 && D <= 512 && (D & (D - 1)) == 0 && K % 32 == 0 && K >= 32 && K <= 32704;
   for (int i = 0; i < 8; ++i) out8[i] = 0;
   if (!shape_ok) return;
-  const SmemLayout L = smem_layout(K, D);
+  const SmemLayout L = smem_layout(K, D, 0, false, zbytes);
   out8[0] = L.total <= SMEM_LIMIT ? 1 : 0;
   out8[1] = (int)L.ds; out8[2] = (int)L.ns; out8[3] = (int)L.a_bufs; out8[4] = (int)L.nslots; out8[5] = (int)L.nstage;
   out8[6] = (int)L.total + 128; out8[7] = (int)L.hist_in_smem;
@@ -1561,9 +1587,9 @@ size_t vq_tc_operand_bytes(int K, int D) {
   return align_up(sizeof(CbMeta), 256) + align_up((size_t)((K + 255) / 256) * L.ns * L.bchunk_bytes, 256);
 }
 
-int launch_vq_tc(const float* z, const float* E, const float* ee, int64_t N, int K, int D, int train, float* z_q,
+int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
                  int64_t* idx, unsigned long long* hist, double* sse, void* bop, int* counters, int* row_list,
-                 int* cand_list, int* zero_ints, int zero_n, bool codebook_cached, cudaStream_t s) {
+                 int* cand_list, int* zero_ints, int zero_n, bool codebook_cached, bool zbf, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
@@ -1573,7 +1599,8 @@ int launch_vq_tc(const float* z, const float* E, const float* ee, int64_t N, int
   uint8_t* bimg = static_cast<uint8_t*>(bop) + align_up(sizeof(CbMeta), 256);
   static const char* lay_env = getenv("DVQ_TC_LAYOUT");   // experiment: "a st sl" digits, e.g. 123 = 1 A image, 2 staging slots, 3 ring slots
   int ovr = lay_env ? atoi(lay_env) : 0;
-  if (ovr && (((K + 255) / 256) * (D / slice_width(D)) <= 2 || smem_layout(K, D, ovr).total > SMEM_LIMIT || ovr / 100 < 1 || ovr / 100 > 2 ||
+  const int zbytes = zbf ? 2 : 4;
+  if (ovr && (((K + 255) / 256) * (D / slice_width(D)) <= 2 || smem_layout(K, D, ovr, false, zbytes).total > SMEM_LIMIT || ovr / 100 < 1 || ovr / 100 > 2 ||
               ovr / 10 % 10 < 1 || ovr / 10 % 10 > 2 || ovr % 10 < 2 || ovr % 10 > MAX_BSLOTS_SOLO))
     ovr = 0;   // resident images keep their layout; impossible requests are ignored
   // CTA-pair kernel (cta_group::2) for streamed codebooks: on by default, DVQ_TC_PAIR=0 selects the single-CTA kernel (A/B runs).
@@ -1582,12 +1609,12 @@ int launch_vq_tc(const float* z, const float* E, const float* ee, int64_t N, int
   static const char* st_env = getenv("DVQ_TC_ST");
   int pair_ovr = lay_env ? atoi(lay_env) : 0;   // the pair kernel accepts rings of up to MAX_BSLOTS slots
   if (pair_ovr && (pair_ovr / 100 < 1 || pair_ovr / 100 > 2 || pair_ovr / 10 % 10 < 1 || pair_ovr / 10 % 10 > 2 || pair_ovr % 10 < 2 || pair_ovr % 10 > MAX_BSLOTS ||
-                   smem_layout(K, D, pair_ovr, true).total > SMEM_LIMIT))
+                   smem_layout(K, D, pair_ovr, true, zbytes).total > SMEM_LIMIT))
     pair_ovr = 0;
-  const SmemLayout L1 = smem_layout(K, D, ovr);
+  const SmemLayout L1 = smem_layout(K, D, ovr, false, zbytes);
   const bool streamed = ((K + 255) / 256) * (int)L1.ns > 2;
-  const bool pair = vq_tc_pair_selected(N, K, D) && dp.sm_count >= 2;
-  const SmemLayout L = pair ? smem_layout(K, D, pair_ovr, true) : L1;
+  const bool pair = vq_tc_pair_selected(N, K, D) && dp.sm_count >= 2;   // chosen on (N, K, D) alone, whatever the z type
+  const SmemLayout L = pair ? smem_layout(K, D, pair_ovr, true, zbytes) : L1;
   const size_t image_bytes = (size_t)((K + 255) / 256) * L1.ns * L1.bchunk_bytes;   // the same for both image layouts
   if (codebook_cached) {
     // DVQ_CODEBOOK_CACHED: CbMeta and the operand image in `bop` are those of this codebook; only the per-call
@@ -1607,7 +1634,7 @@ int launch_vq_tc(const float* z, const float* E, const float* ee, int64_t N, int
   TcParams p;
   memset(&p.ztile, 0, sizeof(p.ztile));
   if (D > DSLICE) {
-    rc = encode_ztile(&p.ztile, z, N, D, (int)L.ds);
+    rc = encode_ztile(&p.ztile, z, N, D, (int)L.ds, zbf);
     if (rc) return rc;
   }
   memset(p.bmap, 0, sizeof(p.bmap));
@@ -1630,43 +1657,58 @@ int launch_vq_tc(const float* z, const float* E, const float* ee, int64_t N, int
   // Converters join the filter as a fourth warp per TMEM lane quarter (DVQ_TC_CE=1; needs a streamed codebook and a
   // double-buffered A image).  It paid +4 % at e_dim 64, K >= 4096 while the filter was the bound; with the list-mode
   // early-out the filter is cheap and the variant is 5 % behind the default there, so it is not selected automatically.
-  const bool ce = streamed && L.a_bufs == 2 && ce_env && ce_env[0] == '1';
-#define DVQ_LAUNCH_TC(DT_, TR_, LS_, CE_, ST_)                                                                              \
+  // (the bf16 kernels are instantiated without the CE / ST experiment variants: a bf16 call ignores DVQ_TC_CE / DVQ_TC_ST)
+  const bool ce = !zbf && streamed && L.a_bufs == 2 && ce_env && ce_env[0] == '1';
+#define DVQ_LAUNCH_TC(DT_, TR_, LS_, CE_, ST_, ZT_)                                                                         \
   do {                                                                                                                 \
-    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<DT_, TR_, LS_, CE_, ST_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    vq_tc_kernel<DT_, TR_, LS_, CE_, ST_><<<(unsigned)grid, NTHREADS, smem, s>>>(p);                                        \
+    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<DT_, TR_, LS_, CE_, ST_, false, ZT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    vq_tc_kernel<DT_, TR_, LS_, CE_, ST_, false, ZT_><<<(unsigned)grid, NTHREADS, smem, s>>>(p);                           \
   } while (0)
-#define DVQ_LAUNCH_TC_PAIR(TR_, LS_, CE_, ST_)                                                                              \
+#define DVQ_LAUNCH_TC_PAIR(TR_, LS_, CE_, ST_, ZT_)                                                                         \
   do {                                                                                                                 \
-    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<0, TR_, LS_, CE_, ST_, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<0, TR_, LS_, CE_, ST_, true, ZT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     cudaLaunchConfig_t cfg = {};                                                                                       \
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;     \
     cudaLaunchAttribute at[1];                                                                                         \
     at[0].id = cudaLaunchAttributeClusterDimension;                                                                    \
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;                                 \
     cfg.attrs = at; cfg.numAttrs = 1;                                                                                  \
-    DVQ_CUDA_CHECK(cudaLaunchKernelEx(&cfg, vq_tc_kernel<0, TR_, LS_, CE_, ST_, true>, p));                             \
+    DVQ_CUDA_CHECK(cudaLaunchKernelEx(&cfg, vq_tc_kernel<0, TR_, LS_, CE_, ST_, true, ZT_>, p));                        \
   } while (0)
 #define DVQ_LAUNCH_TC_GENERIC(TR_, LS_)                                      \
   do {                                                                       \
-    if (pair && st) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, true);               \
-    else if (pair && ce) DVQ_LAUNCH_TC_PAIR(TR_, LS_, true, false);          \
-    else if (pair) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, false);               \
-    else if (st) DVQ_LAUNCH_TC(0, TR_, LS_, false, true);                    \
-    else if (ce) DVQ_LAUNCH_TC(0, TR_, LS_, true, false);                    \
-    else DVQ_LAUNCH_TC(0, TR_, LS_, false, false);                           \
+    if (pair && st) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, true, float);        \
+    else if (pair && ce) DVQ_LAUNCH_TC_PAIR(TR_, LS_, true, false, float);   \
+    else if (pair) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, false, float);        \
+    else if (st) DVQ_LAUNCH_TC(0, TR_, LS_, false, true, float);             \
+    else if (ce) DVQ_LAUNCH_TC(0, TR_, LS_, true, false, float);             \
+    else DVQ_LAUNCH_TC(0, TR_, LS_, false, false, float);                    \
+  } while (0)
+#define DVQ_LAUNCH_TC_GENERIC_BF16(TR_, LS_)                                 \
+  do {                                                                       \
+    if (pair) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, false, __nv_bfloat16);     \
+    else DVQ_LAUNCH_TC(0, TR_, LS_, false, false, __nv_bfloat16);            \
   } while (0)
   // two-sub-chunk filter with the epilogue-heavy register split (DVQ_TC_ST=1; streamed codebooks only).  Measured
   // within +-2 % of the default at every K >= 2048 shape of the sweep, so it is not selected automatically.
-  const bool st = streamed && st_env && st_env[0] == '1';
+  const bool st = !zbf && streamed && st_env && st_env[0] == '1';
   const bool list = p.cand_gshift < 0;
-  if (D == 64 && !list && !streamed) {
-    if (train) DVQ_LAUNCH_TC(64, true, false, false, false); else DVQ_LAUNCH_TC(64, false, false, false, false);
+  if (zbf) {
+    if (D == 64 && !list && !streamed) {
+      if (train) DVQ_LAUNCH_TC(64, true, false, false, false, __nv_bfloat16); else DVQ_LAUNCH_TC(64, false, false, false, false, __nv_bfloat16);
+    } else if (!list) {
+      if (train) DVQ_LAUNCH_TC_GENERIC_BF16(true, false); else DVQ_LAUNCH_TC_GENERIC_BF16(false, false);
+    } else {
+      if (train) DVQ_LAUNCH_TC_GENERIC_BF16(true, true); else DVQ_LAUNCH_TC_GENERIC_BF16(false, true);
+    }
+  } else if (D == 64 && !list && !streamed) {
+    if (train) DVQ_LAUNCH_TC(64, true, false, false, false, float); else DVQ_LAUNCH_TC(64, false, false, false, false, float);
   } else if (!list) {
     if (train) DVQ_LAUNCH_TC_GENERIC(true, false); else DVQ_LAUNCH_TC_GENERIC(false, false);
   } else {
     if (train) DVQ_LAUNCH_TC_GENERIC(true, true); else DVQ_LAUNCH_TC_GENERIC(false, true);
   }
+#undef DVQ_LAUNCH_TC_GENERIC_BF16
 #undef DVQ_LAUNCH_TC_GENERIC
 #undef DVQ_LAUNCH_TC_PAIR
 #undef DVQ_LAUNCH_TC

@@ -23,6 +23,7 @@ DVQ_PATH_AUTO = 0x00
 DVQ_PATH_SIMT = 0x10
 DVQ_PATH_TC = 0x20
 DVQ_HOST_COPY_ONLY = 0x100
+DVQ_Z_BF16 = 0x400          # z / z_q (g_zq / dz) are bf16 rows; the codebook stays fp32
 
 STATUS_NAMES = {0: "DVQ_OK", -1: "DVQ_ERR_BAD_SHAPE", -2: "DVQ_ERR_BAD_ALIGN", -3: "DVQ_ERR_UNSUPPORTED_ARCH",
                 -4: "DVQ_ERR_WORKSPACE", -5: "DVQ_ERR_CUDA", -6: "DVQ_ERR_NCCL", -7: "DVQ_ERR_BAD_ARG"}
@@ -37,6 +38,7 @@ SYMBOLS = {
     "dvq_vq_set_refine": (_i, [_i, C.c_longlong]),
     "dvq_debug_tc_layout": (_i, [_i, _i, C.POINTER(_i)]),
     "dvq_debug_tc_pair_layout": (_i, [C.c_longlong, _i, _i, C.POINTER(_i)]),
+    "dvq_debug_tc_layout_ex": (_i, [C.c_longlong, _i, _i, _i, C.POINTER(_i)]),
     "dvq_debug_tc_image_offset": (C.c_longlong, [_i, _i, _i, _i, _i, C.POINTER(C.c_longlong)]),
     "dvq_profile_mean": (_i, [C.POINTER(_f), C.POINTER(_i), _i]),
     "dvq_debug_umma": (_i, [_vp, C.c_uint32, _vp, C.c_uint32, _i, C.POINTER(C.c_uint32), C.c_uint32, _i, _vp, _vp, _vp]),
@@ -47,6 +49,8 @@ SYMBOLS = {
     "dvq_vq_finalize": (_i, [_vp, _vp, _i64, _i, _i, _f, _f, _vp, _vp, _vp]),
     "dvq_vq_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _f, _f, _vp, _vp, _vp]),
     "dvq_vq_code_sums": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp]),
+    "dvq_vq_backward_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _f, _f, _i, _vp, _vp, _vp]),
+    "dvq_vq_code_sums_ex": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp]),
     "dvq_pcnn_gemm": (_i, [_vp, _vp]),
     "dvq_pcnn_embed": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp]),
     "dvq_pcnn_rows_to_image": (_i, [_vp, _i, _i, _vp, _i, _i, _vp, _vp]),

@@ -6,9 +6,15 @@ return order — train path ``(loss, z_q, perplexity, min_encodings, min_encodin
 (:67), inference path ``(min_encoding_indices, z_q)`` (:54) — and ``get_emb(idx, dim)`` (:68).
 Everything between is one call into the C ABI (``dvq_vq_forward`` + ``dvq_vq_finalize``):
 the N x K distance matrix, the host-built one-hot and the second GEMM of the reference do not
-exist here.  There is no CPU path: inputs must be fp32 CUDA tensors.
+exist here.  There is no CPU path: inputs must be fp32 or bf16 CUDA tensors.
 
 Differences that are deliberate and documented (SURVEY §0.7, §0.8):
+* bf16 latents (what an encoder produces under ``torch.autocast(..., dtype=torch.bfloat16)``) are
+  quantized natively, without an fp32 copy: the call is the fp32 call on ``z.float()`` — the same
+  indices and histogram, loss and perplexity as fp32 scalars — with ``z_q`` returned in bf16 (the fp32
+  result rounded to nearest even).  The codebook stays an fp32 parameter; in the backward ``dz`` is
+  bf16 (the fp32 formulas on the upcast values, rounded once) and the codebook gradient fp32.  Other
+  dtypes (fp16, fp64) raise ``TypeError``.
 * ``min_encodings`` ([N,K] fp32 one-hot, 1 TiB at BASELINE config 4) is materialised only while
   it is at most ``onehot_limit_bytes`` (default 2 GiB); above that the 5-tuple carries a
   ``LazyOneHot`` that can still produce it on demand.  Both reference callers discard it
@@ -64,7 +70,7 @@ class _VQFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, z, weight, module):
-        loss, z_q, ppl, idx = module._forward_train_raw(z, weight)
+        loss, z_q, ppl, idx = module._forward_train_raw(z, weight)   # z_q has the dtype of z (fp32 or bf16)
         # rows the returned loss is a mean over: the local count, or — row-sharded — the all-reduced histogram total
         # (a device scalar: no host sync).  The gradients below are the exact partial derivatives of the RETURNED
         # (global) loss with respect to the local rows of z and the local rows' contribution to dE; summing dE over
@@ -89,29 +95,33 @@ class _VQFunction(torch.autograd.Function):
         rows = n_rows.reshape(1).contiguous()
         flat = z.detach().reshape(-1, d)
         n = flat.shape[0]
+        # bf16 z: g_zq arrives in bf16 (the dtype of z_q) and dz is returned in bf16; the arithmetic is fp32
+        bf16 = z.dtype == torch.bfloat16
         gq = None
         if g_zq is not None:
-            gq = g_zq.detach().to(torch.float32).reshape(-1, d).contiguous()
-        if d % 4 == 0 and flat.data_ptr() % 16 == 0 and weight.data_ptr() % 16 == 0 and (gq is None or gq.data_ptr() % 16 == 0):
-            # one fused pass (dvq_vq_backward): dz written once, dE by vector reductions
+            gq = g_zq.detach().to(z.dtype).reshape(-1, d).contiguous()
+        zal = 8 if bf16 else 16   # the kernel moves 4 elements of z / g_zq / dz at a time
+        if d % 4 == 0 and flat.data_ptr() % zal == 0 and weight.data_ptr() % 16 == 0 and (gq is None or gq.data_ptr() % zal == 0):
+            # one fused pass (dvq_vq_backward_ex): dz written once, dE by vector reductions
             gz = torch.empty_like(flat) if want_z else None
             gw = torch.zeros_like(weight) if want_e else None
             with torch.cuda.device(z.device):
-                _cabi.check(_cabi.lib.dvq_vq_backward(
+                _cabi.check(_cabi.lib.dvq_vq_backward_ex(
                     flat.data_ptr(), weight.detach().data_ptr(), idx.data_ptr(), gq.data_ptr() if gq is not None else None,
-                    gl.data_ptr(), rows.data_ptr(), n, weight.shape[0], d, ctx.al, ctx.beta,
+                    gl.data_ptr(), rows.data_ptr(), n, weight.shape[0], d, ctx.al, ctx.beta, _cabi.DVQ_Z_BF16 if bf16 else 0,
                     gz.data_ptr() if gz is not None else None, gw.data_ptr() if gw is not None else None,
-                    _stream_ptr(z.device)), "dvq_vq_backward")
+                    _stream_ptr(z.device)), "dvq_vq_backward_ex")
             return (gz.view_as(z) if gz is not None else None), gw, None
-        # shapes the vector kernel does not take (e_dim not a multiple of 4, odd storage offsets): same formulas in torch
+        # shapes the vector kernel does not take (e_dim not a multiple of 4, odd storage offsets): same formulas in torch,
+        # in fp32 (dz is cast to the dtype of z once)
         e = weight.detach().index_select(0, idx.view(-1))
-        diff = (flat - e) * (2.0 / (rows * d))
+        diff = (flat.float() - e) * (2.0 / (rows * d))
         gz = gw = None
         if want_z:
             gz = (gl * ctx.al) * diff
             if gq is not None:
-                gz = gz + gq
-            gz = gz.view_as(z)
+                gz = gz + gq.float()
+            gz = gz.to(z.dtype).view_as(z)
         if want_e:
             gw = torch.zeros_like(weight)
             gw.index_add_(0, idx.view(-1), (-(gl * ctx.beta)) * diff)
@@ -165,8 +175,8 @@ class VectorQuantizer(nn.Module):
     def _check(self, z: torch.Tensor, weight: torch.Tensor):
         if not isinstance(z, torch.Tensor):
             raise TypeError("z must be a torch.Tensor")
-        if z.dtype != torch.float32:
-            raise TypeError("dvq.VectorQuantizer computes in fp32; got %s" % z.dtype)
+        if z.dtype != torch.float32 and z.dtype != torch.bfloat16:
+            raise TypeError("dvq.VectorQuantizer computes in fp32 and takes fp32 or bf16 latents; got %s" % z.dtype)
         if not z.is_cuda or not weight.is_cuda:
             raise ValueError("dvq.VectorQuantizer has no CPU path: z and the codebook must be CUDA tensors "
                              "(got z on %s, codebook on %s)" % (z.device, weight.device))
@@ -187,11 +197,14 @@ class VectorQuantizer(nn.Module):
 
     def _launch(self, z, weight, flags, z_q, idx, onehot, stats):
         n = z.numel() // self.e_dim
+        if z.dtype == torch.bfloat16:
+            flags |= _cabi.DVQ_Z_BF16
         ws = self._workspace(n, flags, z.device)
         # (the 16-byte alignment of z decides between the tcgen05 and the FP32 kernel under AUTO: part of the key, since
-        #  only the former builds the operand image)
+        #  only the former builds the operand image; so is the dtype of z, so that a preparation is reused only by a call
+        #  of the same kind)
         key = (weight.data_ptr(), weight._version, ws.data_ptr(), n, flags & _cabi.DVQ_PATH_MASK, str(z.device),
-               z.data_ptr() % 16 == 0 and z_q.data_ptr() % 16 == 0)
+               z.data_ptr() % 16 == 0 and z_q.data_ptr() % 16 == 0, z.dtype)
         if self.cache_codebook and key == self._cb_key:
             flags |= _cabi.DVQ_CODEBOOK_CACHED
         self._cb_key = None          # (stays None if the launch raises)
@@ -211,6 +224,7 @@ class VectorQuantizer(nn.Module):
         if self._ws is None:
             return 0, 0
         out = (C.c_int * 4)()
+        # (the counters do not depend on the dtype of z: DVQ_Z_BF16 may be set in `flags` or not)
         with torch.cuda.device(self._ws.device):
             _cabi.check(_cabi.lib.dvq_vq_read_counters(self._ws.data_ptr(), n, self.n_e, self.e_dim,
                                                        self.path if flags is None else flags, out), "dvq_vq_read_counters")
@@ -278,14 +292,16 @@ class VectorQuantizer(nn.Module):
         """[n_e, e_dim] sum of the latents assigned to each code (``dvq_vq_code_sums``); summed over the ranks of a
         row-sharded module."""
         flat = z.detach().reshape(-1, self.e_dim).contiguous()
-        if self.e_dim % 4 != 0 or flat.data_ptr() % 16 != 0:
+        bf16 = flat.dtype == torch.bfloat16   # bf16 latents are summed in fp32 (sums stay fp32)
+        if self.e_dim % 4 != 0 or flat.data_ptr() % (8 if bf16 else 16) != 0:
             sums = torch.zeros(self.n_e, self.e_dim, device=flat.device)
-            sums.index_add_(0, idx.view(-1), flat)
+            sums.index_add_(0, idx.view(-1), flat.float())
         else:
             sums = torch.zeros(self.n_e, self.e_dim, device=flat.device)
             with torch.cuda.device(flat.device):
-                _cabi.check(_cabi.lib.dvq_vq_code_sums(flat.data_ptr(), idx.contiguous().data_ptr(), flat.shape[0], self.n_e,
-                                                       self.e_dim, sums.data_ptr(), _stream_ptr(flat.device)), "dvq_vq_code_sums")
+                _cabi.check(_cabi.lib.dvq_vq_code_sums_ex(flat.data_ptr(), idx.contiguous().data_ptr(), flat.shape[0], self.n_e,
+                                                          self.e_dim, _cabi.DVQ_Z_BF16 if bf16 else 0, sums.data_ptr(),
+                                                          _stream_ptr(flat.device)), "dvq_vq_code_sums_ex")
         if self.process_group is not None and _dist.world_size(self.process_group) > 1:
             _dist.all_reduce_sum(sums, self.process_group)
         return sums
@@ -318,7 +334,7 @@ class VectorQuantizer(nn.Module):
             return 0
         flat = z.detach().reshape(-1, self.e_dim)
         pick = torch.randint(0, flat.shape[0], (dead.numel(),), device=flat.device, generator=generator)
-        new_rows = flat[pick].contiguous()
+        new_rows = flat[pick].float().contiguous()   # (bf16 latents: the codebook stays fp32)
         if self.process_group is not None and _dist.world_size(self.process_group) > 1:
             _dist.broadcast0(new_rows, self.process_group)
         self.embedding.weight[dead] = new_rows

@@ -59,6 +59,11 @@ typedef enum DvqStatus {
                                    * reused instead of rebuilt (three small launches fewer per call) */
 #define DVQ_HOST_COPY_ONLY 0x100 /* dvq_vq_forward_host only: run the chunk pipeline's H2D / D2H copies without the
                                     kernels (outputs are undefined) - the copy-only ceiling of the host-buffer path */
+#define DVQ_Z_BF16 0x400      /* dvq_vq_forward / _workspace_bytes / _read_counters, dvq_vq_backward_ex, dvq_vq_code_sums_ex,
+                               * dvq_debug_tc_layout_ex: the `z` / `z_q` (and `g_zq` / `dz`) pointers are reinterpreted as
+                               * bf16 rows (2-byte alignment; the tcgen05 path needs 16 bytes as in fp32).  The call is the fp32
+                               * call on the upcast rows: same indices, histogram and SSE; z_q is its result rounded to
+                               * nearest-even bf16.  The codebook stays fp32.  Not accepted by dvq_vq_forward_host. */
 
 DVQ_API int dvq_abi_version(void);
 DVQ_API const char* dvq_last_error(void);
@@ -92,6 +97,13 @@ DVQ_API int dvq_debug_tc_layout(int K, int D, int* out8);
  * honours DVQ_TC_PAIR=0/1), e_dim slice width, slices per row, A images, ring slots (2-8), z staging slots, dynamic
  * shared memory in bytes, codes per ring slot (128) } of the pair kernel's plan. */
 DVQ_API int dvq_debug_tc_pair_layout(long long N, int K, int D, int* out8);
+
+/* Diagnostic (host-only): the plan of the tcgen05 kernel variant dvq_vq_forward would launch for (N, K, D, flags) (flags:
+ * DVQ_Z_BF16 or 0; other bits are ignored).  When the CTA-pair kernel is selected, out8 is filled as by
+ * dvq_debug_tc_pair_layout, otherwise as by dvq_debug_tc_layout — with flags = 0 exactly their output — with the plan
+ * of the z element type: the dynamic shared memory out8[6] includes the z staging slots of 128 rows x (slice width)
+ * x (4 bytes fp32 / 2 bytes bf16) each. */
+DVQ_API int dvq_debug_tc_layout_ex(long long N, int K, int D, int flags, int* out8);
 
 /* Diagnostic (host-only): byte offset of element (code k, column d) of the FP16 operand image the tcgen05 VQ kernel keeps in
  * its workspace — d in [0, D) the scaled code, d in [D, D + 16) the fold columns — for the single-CTA layout (pair = 0: blocks
@@ -142,10 +154,17 @@ DVQ_API int dvq_vq_finalize(const unsigned long long* hist, const double* sse, i
  * all-reduced histogram total on a row-sharded run); g_zq may be NULL (no gradient reaches z_q).  D % 4 == 0. */
 DVQ_API int dvq_vq_backward(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
                     const float* rows, int64_t N, int K, int D, float al, float beta, float* dz, float* dE, void* stream);
+/* The same with flags: DVQ_Z_BF16 = z, g_zq and dz are bf16 rows (8-byte aligned; E and dE stay fp32, 16-byte aligned).
+ * The formulas are evaluated in fp32 on the upcast values and dz is rounded to bf16 once.  flags = 0 is dvq_vq_backward. */
+DVQ_API int dvq_vq_backward_ex(const float* z, const float* E, const int64_t* idx, const float* g_zq, const float* g_loss,
+                               const float* rows, int64_t N, int K, int D, float al, float beta, int flags, float* dz, float* dE,
+                               void* stream);
 
 /* sums[k,:] += sum of the rows z[n,:] with idx[n] == k — the per-code input sums of an EMA codebook update
  * (together with the usage histogram of dvq_vq_forward).  sums [K,D] must be zeroed by the caller.  D % 4 == 0. */
 DVQ_API int dvq_vq_code_sums(const float* z, const int64_t* idx, int64_t N, int K, int D, float* sums, void* stream);
+/* The same with flags: DVQ_Z_BF16 = z is bf16 rows (8-byte aligned), summed in fp32.  flags = 0 is dvq_vq_code_sums. */
+DVQ_API int dvq_vq_code_sums_ex(const float* z, const int64_t* idx, int64_t N, int K, int D, int flags, float* sums, void* stream);
 
 /* VectorQuantizer.get_emb — quantizer.py:68-75 (batched meaning: out[n,:] = E[idx[n],:]).
  * Out-of-range indices set *oob (device int, may be NULL) and write zeros. */
