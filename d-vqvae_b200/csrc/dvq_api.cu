@@ -109,7 +109,7 @@ const char* dvq_last_error(void) { return g_err; }
 long long dvq_launch_count(void) { return __atomic_load_n(&g_launches, __ATOMIC_RELAXED); }
 
 int dvq_vq_set_refine(int mode, long long pair_cap) {
-  if (mode < 0 || mode > 2) return fail(DVQ_ERR_BAD_ARG, "refine mode must be 0 (auto), 1 (per-row) or 2 (binned)");
+  if (mode < 0 || mode > 3) return fail(DVQ_ERR_BAD_ARG, "refine mode must be 0 (auto), 1 (per-row), 2 (binned) or 3 (code-stationary)");
   __atomic_store_n(&g_refine_mode, mode, __ATOMIC_RELAXED);
   __atomic_store_n(&g_refine_pair_cap, pair_cap > 0 ? pair_cap : 0, __ATOMIC_RELAXED);
   return DVQ_OK;
@@ -247,21 +247,28 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
       //  list stored downwards from the end of the same buffer; both kernels re-evaluate them against every code)
       const bool list_mode = vq_tc_cand_gshift(K) < 0;
       if (vq_refine_supported(K, D)) {
-        // Two exact refine paths with identical results: the per-row kernel (one warp per undecided row) is the
-        // faster one while the FP32 codebook fits its shared memory (measured at K = 512, e_dim = 64: 0.105 vs
-        // 0.128 ms for 108 k rows); beyond that the binned kernels win by 2-5x (code rows register-resident per
-        // bucket instead of re-read from L2 per row).  The binned path hands its list back to the per-row kernel
-        // through counters[5] / counters[6] when the pairs do not fit its workspace (normally both stay zero and
-        // the per-row kernel exits at once).  dvq_vq_set_refine / DVQ_REFINE_PER_ROW / DVQ_REFINE_BINNED force one path.
+        // Three exact refine paths with identical results.  The code-stationary kernel (code rows register-resident, one
+        // warp per 32-code sub-chunk, z rows streamed past them) covers mask-mode codebooks whose K/32 warps hold e_dim
+        // floats per lane; the automatic choice takes it where it measured faster than the per-row kernel
+        // (vq_refine_stationary_default: K >= 128 up to e_dim 64, K = 256 at e_dim 128; config 2: 0.077 vs 0.101 ms).
+        // Otherwise the per-row kernel (one warp per undecided row) while the FP32 codebook fits its shared memory
+        // (measured at K = 512, e_dim = 64: 0.105 vs 0.128 ms for 108 k rows against the binned kernels); beyond that the
+        // binned kernels win by 2-5x (code rows register-resident per bucket instead of re-read from L2 per row).  The
+        // binned path hands its list back to the per-row kernel through counters[5] / counters[6] when the pairs do not
+        // fit its workspace (normally both stay zero and the per-row kernel exits at once).  dvq_vq_set_refine /
+        // DVQ_REFINE_PER_ROW / DVQ_REFINE_BINNED force one path.
         static const bool env_per_row = getenv("DVQ_REFINE_PER_ROW") != nullptr;
         static const bool env_binned = getenv("DVQ_REFINE_BINNED") != nullptr;
         const int mode = __atomic_load_n(&g_refine_mode, __ATOMIC_RELAXED);
         const bool force_per_row = env_per_row || mode == 1, force_binned = env_binned || mode == 2;
+        const bool stationary = mode == 3 || (!force_per_row && !force_binned && vq_refine_stationary_default(K, D));
         const bool per_row_only = force_per_row || (!force_binned && vq_refine_codebook_in_smem(K, D));
-        if (!per_row_only)
+        if (stationary)
+          rc = launch_vq_refine_stationary(z, E, ee, K, D, train, z_q, idx, hist, sse, row_list, cand_list, counters, zbf, s);
+        else if (!per_row_only)
           rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, cand_list, counters, list_mode ? 1 : 0,
                                        ws + w.off_binned, zbf, s);
-        if (!rc)
+        if (!rc && !stationary)
           rc = launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, row_list, cand_list, per_row_only ? counters : counters + 5,
                                 vq_tc_cand_gshift(K), list_mode ? row_list + (N - 1) : nullptr,
                                 list_mode ? (per_row_only ? counters + 2 : counters + 6) : nullptr, zbf, s);

@@ -78,6 +78,14 @@ int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int 
                      unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
                      const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, bool zbf, cudaStream_t s);
 
+// code-stationary exact refine (vq_refine_stationary.cu): mask-mode codebooks whose K/32 warps hold e_dim code floats
+// per lane in registers
+bool vq_refine_stationary_supported(int K, int D);
+bool vq_refine_stationary_default(int K, int D);   // the subset the automatic refine choice gives it (measured faster)
+int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
+                                unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
+                                const int* n_list, bool zbf, cudaStream_t s);
+
 // binned exact refine (vq_refine_binned.cu): (row, sub-chunk) pairs bucketed by sub-chunk; hands the list to
 // launch_vq_refine through counters[5] / counters[6] when the pairs do not fit its workspace
 long long refine_pair_cap_override();   // dvq_vq_set_refine (dvq_api.cu); 0 = default

@@ -78,9 +78,11 @@ DVQ_API long long dvq_launch_count(void);
 DVQ_API int dvq_profile_enable(int on);
 DVQ_API int dvq_profile_mean(float* ms, int* count, int n);
 
-/* Test / measurement hook for the exact refine stage of the tcgen05 path (both variants give identical
- * results): mode 0 = automatic (per-row kernel while the FP32 codebook fits its shared memory, binned
- * kernels otherwise), 1 = per-row kernel only, 2 = binned kernels; pair_cap > 0 overrides the capacity
+/* Test / measurement hook for the exact refine stage of the tcgen05 path (all variants give identical
+ * results): mode 0 = automatic (the code-stationary kernel on the mask-mode codebooks that fit in registers
+ * where it is the faster one, else the per-row kernel while the FP32 codebook fits its shared memory, binned
+ * kernels otherwise), 1 = per-row kernel only, 2 = binned kernels, 3 = code-stationary kernel
+ * (dvq_vq_forward fails with DVQ_ERR_BAD_SHAPE on a shape it does not cover); pair_cap > 0 overrides the capacity
  * of the binned (row, sub-chunk) pair list (default 2 N) so that tests can exercise the device-side
  * hand-back to the per-row kernel, <= 0 restores the default.  Process-wide. */
 DVQ_API int dvq_vq_set_refine(int mode, long long pair_cap);
