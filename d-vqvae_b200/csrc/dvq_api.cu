@@ -403,18 +403,33 @@ int dvq_gather_multi(const float* const* E, int G, const int64_t* codes, int64_t
   return launch_gather_multi(E, G, codes, N, K, D, out, out_stride, oob, static_cast<cudaStream_t>(stream));
 }
 
-int dvq_mano_forward(const DvqManoModel* model, const float* betas, const float* global_orient, const float* hand_pose,
-                     const float* transl, int B, float* vertices, float* joints, void* stream) {
-  if (B < 0) return fail(DVQ_ERR_BAD_SHAPE, "B must be >= 0");
-  if (!model || (B > 0 && (!betas || !hand_pose || !vertices))) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
+static int check_mano_model(const DvqManoModel* model) {
   if (!model->v_template || !model->shapedirs || !model->posedirs || !model->j_regressor || !model->weights || !model->pose_mean ||
       !model->parents || (model->ncomps > 0 && !model->hands_components))
     return fail(DVQ_ERR_BAD_ARG, "DvqManoModel has a NULL table");
   if (model->ncomps < 0 || model->ncomps > 45) return fail(DVQ_ERR_BAD_SHAPE, "ncomps must be in [0, 45]");
   if (reinterpret_cast<uintptr_t>(model->weights) % 16) return fail(DVQ_ERR_BAD_ALIGN, "the skinning weights need 16-byte alignment");
-  int rc = require_sm100();
+  return require_sm100();
+}
+
+int dvq_mano_forward(const DvqManoModel* model, const float* betas, const float* global_orient, const float* hand_pose,
+                     const float* transl, int B, float* vertices, float* joints, void* stream) {
+  if (B < 0) return fail(DVQ_ERR_BAD_SHAPE, "B must be >= 0");
+  if (!model || (B > 0 && (!betas || !hand_pose || !vertices))) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
+  int rc = check_mano_model(model);
   if (rc) return rc;
   return launch_mano(model, betas, global_orient, hand_pose, transl, B, vertices, joints, static_cast<cudaStream_t>(stream));
+}
+
+int dvq_mano_backward(const DvqManoModel* model, const float* betas, const float* global_orient, const float* hand_pose, int B,
+                      const float* grad_vertices, const float* grad_joints, float* grad_betas, float* grad_global_orient,
+                      float* grad_hand_pose, float* grad_transl, void* stream) {
+  if (B < 0) return fail(DVQ_ERR_BAD_SHAPE, "B must be >= 0");
+  if (!model || (B > 0 && (!betas || !hand_pose))) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
+  int rc = check_mano_model(model);
+  if (rc) return rc;
+  return launch_mano_backward(model, betas, global_orient, hand_pose, B, grad_vertices, grad_joints, grad_betas, grad_global_orient,
+                              grad_hand_pose, grad_transl, static_cast<cudaStream_t>(stream));
 }
 
 int dvq_pcnn_gemm(const DvqPcnnGemm* g, void* stream) {

@@ -118,6 +118,9 @@ int launch_pcnn_rows_to_image(const int64_t* label, int B, int Bp, const float* 
 // MANO hand layer (mano_sm100.cu)
 int launch_mano(const DvqManoModel* m, const float* betas, const float* global_orient, const float* hand_pose, const float* transl, int B,
                 float* vertices, float* joints, cudaStream_t s);
+int launch_mano_backward(const DvqManoModel* m, const float* betas, const float* global_orient, const float* hand_pose, int B,
+                         const float* grad_vertices, const float* grad_joints, float* grad_betas, float* grad_global_orient,
+                         float* grad_hand_pose, float* grad_transl, cudaStream_t s);
 
 // PointNet
 size_t pointnet_workspace_bytes(int B, int C, int P, int flags);

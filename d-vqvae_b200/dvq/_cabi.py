@@ -66,6 +66,7 @@ SYMBOLS = {
     "dvq_pointnet_forward_ex": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "dvq_allreduce_stats": (_i, [_vp, _vp, _vp, _i, _vp]),
     "dvq_mano_forward": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "dvq_mano_backward": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -8,7 +8,8 @@
 as one CUDA kernel behind the same call signature, so ``GenNet.set_rh_mano(dvq.ManoLayer.from_pkl(...))`` is the whole
 change and the decoder's 55 parameters reach the 778-point PointNet without leaving the device.  The arithmetic is the
 linear blend skinning of ``smplx/lbs.py`` (which ``mano`` wraps); ``oracle/mano_oracle.py`` restates it for the tests.
-Inference only (no autograd), CUDA tensors only.
+CUDA tensors only.  Gradients with respect to betas, global_orient, hand_pose and transl are opt-in
+(``ManoLayer(..., differentiable=True)``): a second kernel, ``dvq_mano_backward``, computes the vector-Jacobian product.
 """
 from __future__ import annotations
 
@@ -21,6 +22,7 @@ from types import SimpleNamespace
 import numpy as np
 import torch
 from torch import nn
+from torch.autograd.function import once_differentiable
 
 from . import _cabi
 from .quantizer import _stream_ptr
@@ -70,12 +72,53 @@ def read_mano_pkl(path):
             "faces": np.asarray(d["f"]).astype(np.int64)}
 
 
+class _ManoLBS(torch.autograd.Function):
+    """(betas, global_orient, hand_pose, transl) -> (vertices, joints) through ``dvq_mano_forward``.  The backward is
+    ``dvq_mano_backward``: it recomputes the forward intermediates from the saved inputs, so nothing else is kept.  The inputs
+    arrive as contiguous fp32 tensors; global_orient and transl may be None."""
+
+    @staticmethod
+    def forward(ctx, layer, betas, global_orient, hand_pose, transl):
+        ctx.layer = layer
+        ctx.set_materialize_grads(False)          # an unused output gives None: the kernel reads NULL as zero
+        ctx.save_for_backward(betas, global_orient, hand_pose)
+        return layer._launch_forward(betas, global_orient, hand_pose, transl)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_vertices, g_joints):
+        betas, global_orient, hand_pose = ctx.saved_tensors
+        layer = ctx.layer
+        _, want_betas, want_orient, want_pose, want_transl = ctx.needs_input_grad
+        B, dev = betas.shape[0], betas.device
+        new = lambda cols, want: torch.empty(B, cols, device=dev, dtype=torch.float32) if want else None
+        g_betas, g_orient, g_pose, g_transl = new(10, want_betas), new(3, want_orient), new(hand_pose.shape[1], want_pose), new(3, want_transl)
+        gv = g_vertices.to(torch.float32).contiguous() if g_vertices is not None else None
+        gj = g_joints.to(torch.float32).contiguous() if g_joints is not None else None
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        m = layer._model_struct()
+        with torch.cuda.device(dev):
+            _cabi.check(_cabi.lib.dvq_mano_backward(C.byref(m), betas.data_ptr(), ptr(global_orient), hand_pose.data_ptr(), B,
+                                                    ptr(gv), ptr(gj), ptr(g_betas), ptr(g_orient), ptr(g_pose), ptr(g_transl),
+                                                    _stream_ptr(dev)), "dvq_mano_backward")
+        return None, g_betas, g_orient, g_pose, g_transl
+
+
 class ManoLayer(nn.Module):
     """MANO linear blend skinning: ``layer(betas=[B,10], global_orient=[B,3], hand_pose=[B,ncomps], transl=[B,3])`` returns an
-    object with ``.vertices [B,778,3]`` and ``.joints [B,16,3]`` (the posed joints of the kinematic tree)."""
+    object with ``.vertices [B,778,3]`` and ``.joints [B,16,3]`` (the posed joints of the kinematic tree).
 
-    def __init__(self, model: dict, use_pca: bool = True, num_pca_comps: int = 45, flat_hand_mean: bool = True):
+    ``differentiable=False`` (the default) detaches the inputs: the outputs never carry a ``grad_fn``.  That keeps the drop-in
+    flow working where the hand parameters come out of a decoder that requires grad (``GenNet.gen`` outside ``no_grad``):
+    the vertices feed ``dvq.PointNetEncoder``, which refuses an input that requires grad.  With ``differentiable=True``, a
+    call in grad mode where some input requires grad returns vertices and joints with gradients to betas, global_orient,
+    hand_pose and transl (fp32 arithmetic; each gradient comes back in its input's dtype), e.g. for test-time refinement of a
+    grasp with Adam.  Every other call runs the same inference path as the default."""
+
+    def __init__(self, model: dict, use_pca: bool = True, num_pca_comps: int = 45, flat_hand_mean: bool = True,
+                 differentiable: bool = False):
         super().__init__()
+        self.differentiable = bool(differentiable)
         nv = 778
         f32 = lambda a, shape: torch.from_numpy(np.ascontiguousarray(np.asarray(a, dtype=np.float64).reshape(shape), dtype=np.float32))
         parents = np.asarray(model["parents"]).astype(np.int64).copy()
@@ -99,9 +142,27 @@ class ManoLayer(nn.Module):
         self.faces = np.asarray(model.get("faces", np.zeros((0, 3))), dtype=np.int64)
 
     @classmethod
-    def from_pkl(cls, model_path, use_pca=True, num_pca_comps=45, flat_hand_mean=True, **_ignored):
-        """Same keyword arguments as ``mano.load`` (``model_type``, ``batch_size`` ... are accepted and ignored)."""
-        return cls(read_mano_pkl(model_path), use_pca=use_pca, num_pca_comps=num_pca_comps, flat_hand_mean=flat_hand_mean)
+    def from_pkl(cls, model_path, use_pca=True, num_pca_comps=45, flat_hand_mean=True, differentiable=False, **_ignored):
+        """Same keyword arguments as ``mano.load`` (``model_type``, ``batch_size`` ... are accepted and ignored), plus
+        ``differentiable``."""
+        return cls(read_mano_pkl(model_path), use_pca=use_pca, num_pca_comps=num_pca_comps, flat_hand_mean=flat_hand_mean,
+                   differentiable=differentiable)
+
+    def _model_struct(self):
+        return _cabi.ManoModel(self.v_template.data_ptr(), self.shapedirs.data_ptr(), self.posedirs.data_ptr(), self.j_regressor.data_ptr(),
+                               self.weights.data_ptr(), self.hands_components.data_ptr(), self.pose_mean.data_ptr(), self.parents.data_ptr(),
+                               self.num_pca_comps if self.use_pca else 0)
+
+    def _launch_forward(self, betas, global_orient, hand_pose, transl):
+        dev, B = betas.device, betas.shape[0]
+        vertices = torch.empty(B, 778, 3, device=dev, dtype=torch.float32)
+        joints = torch.empty(B, 16, 3, device=dev, dtype=torch.float32)
+        m = self._model_struct()
+        with torch.cuda.device(dev):
+            _cabi.check(_cabi.lib.dvq_mano_forward(C.byref(m), betas.data_ptr(), global_orient.data_ptr() if global_orient is not None else None,
+                                                   hand_pose.data_ptr(), transl.data_ptr() if transl is not None else None, B,
+                                                   vertices.data_ptr(), joints.data_ptr(), _stream_ptr(dev)), "dvq_mano_forward")
+        return vertices, joints
 
     def forward(self, betas=None, global_orient=None, hand_pose=None, transl=None, **_ignored):
         dev = self.v_template.device
@@ -111,6 +172,8 @@ class ManoLayer(nn.Module):
         if hand_pose is None and betas is None:
             raise ValueError("need betas or hand_pose to infer the batch size")
         B = int((betas if betas is not None else hand_pose).shape[0])
+        grad = self.differentiable and torch.is_grad_enabled() and any(
+            t is not None and t.requires_grad for t in (betas, global_orient, hand_pose, transl))
 
         def prep(t, cols, name):
             if t is None:
@@ -119,19 +182,15 @@ class ManoLayer(nn.Module):
                 raise ValueError("%s is on %s, the layer on %s" % (name, t.device, dev))
             if tuple(t.shape) != (B, cols):
                 raise RuntimeError("%s must be [%d, %d], got %s" % (name, B, cols, tuple(t.shape)))
-            return t.detach().to(torch.float32).contiguous()
+            # the differentiable path casts in the graph, so each gradient comes back in its input's dtype
+            return (t if grad else t.detach()).to(torch.float32).contiguous()
 
         betas = prep(betas, 10, "betas") if betas is not None else torch.zeros(B, 10, device=dev)
         hand_pose = prep(hand_pose, ncols, "hand_pose") if hand_pose is not None else torch.zeros(B, ncols, device=dev)
         global_orient = prep(global_orient, 3, "global_orient")
         transl = prep(transl, 3, "transl")
-        vertices = torch.empty(B, 778, 3, device=dev, dtype=torch.float32)
-        joints = torch.empty(B, 16, 3, device=dev, dtype=torch.float32)
-        m = _cabi.ManoModel(self.v_template.data_ptr(), self.shapedirs.data_ptr(), self.posedirs.data_ptr(), self.j_regressor.data_ptr(),
-                            self.weights.data_ptr(), self.hands_components.data_ptr(), self.pose_mean.data_ptr(), self.parents.data_ptr(),
-                            self.num_pca_comps if self.use_pca else 0)
-        with torch.cuda.device(dev):
-            _cabi.check(_cabi.lib.dvq_mano_forward(C.byref(m), betas.data_ptr(), global_orient.data_ptr() if global_orient is not None else None,
-                                                   hand_pose.data_ptr(), transl.data_ptr() if transl is not None else None, B,
-                                                   vertices.data_ptr(), joints.data_ptr(), _stream_ptr(dev)), "dvq_mano_forward")
+        if grad:
+            vertices, joints = _ManoLBS.apply(self, betas, global_orient, hand_pose, transl)
+        else:
+            vertices, joints = self._launch_forward(betas, global_orient, hand_pose, transl)
         return SimpleNamespace(vertices=vertices, joints=joints)

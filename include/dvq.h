@@ -239,6 +239,14 @@ typedef struct DvqManoModel {
  * -> vertices [B,778,3], joints [B,16,3] (posed joints; NULL to skip). */
 DVQ_API int dvq_mano_forward(const DvqManoModel* model, const float* betas, const float* global_orient, const float* hand_pose,
                              const float* transl, int B, float* vertices, float* joints, void* stream);
+/* Vector-Jacobian product of dvq_mano_forward with respect to betas, global_orient, hand_pose and transl (the forward is
+ * recomputed from the same inputs; transl does not enter it).  grad_vertices [B,778,3] and grad_joints [B,16,3] are the
+ * upstream gradients, NULL meaning zero.  Each of grad_betas [B,10], grad_global_orient [B,3],
+ * grad_hand_pose [B, ncomps ? ncomps : 45] and grad_transl [B,3] is written when non-NULL.  An ordinary stream launch
+ * (no host synchronisation, no allocation; CUDA-graph capturable), deterministic run to run. */
+DVQ_API int dvq_mano_backward(const DvqManoModel* model, const float* betas, const float* global_orient, const float* hand_pose,
+                              int B, const float* grad_vertices, const float* grad_joints, float* grad_betas,
+                              float* grad_global_orient, float* grad_hand_pose, float* grad_transl, void* stream);
 
 /* Host-buffer (end-to-end) form of the same forward: z_host/E_host/zq_host/idx_host are
  * HOST pointers (pinned for full overlap).  Rows are streamed through the GPU in chunks on
