@@ -84,7 +84,7 @@ VqWorkspace vq_workspace_layout(int64_t N, int K, int D, int flags) {
   w.off_ee = off;
   off = align_up(off + sizeof(float) * (size_t)K, 256);
   w.off_counters = off;
-  off = align_up(off + sizeof(int) * 64, 256);   // [0..7] counters, [8..63] optional wait-time stats
+  off = align_up(off + sizeof(int) * CNT_WORDS, 256);
   const bool may_tc = (flags & DVQ_PATH_MASK) != DVQ_PATH_SIMT && vq_tc_supported(N, K, D);
   w.off_rowlist = off;
   if (may_tc) off = align_up(off + 2 * align_up(sizeof(int) * (size_t)N, 256), 256);
@@ -245,7 +245,9 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
       profile_mark(2, true, s);
       // (large codebooks: rows with too many candidates for the list record, and degenerate rows, sit in a second
       //  list stored downwards from the end of the same buffer; both kernels re-evaluate them against every code)
-      const bool list_mode = vq_tc_cand_gshift(K) < 0;
+      const bool list_mode = cand_list_mode(K);
+      const RefineList list{row_list, cand_list, counters + CNT_LISTED, list_mode ? row_list + (N - 1) : nullptr,
+                            list_mode ? counters + CNT_OVF : nullptr, list_mode};
       if (vq_refine_supported(K, D)) {
         // Three exact refine paths with identical results.  The code-stationary kernel (code rows register-resident, one
         // warp per 32-code sub-chunk, z rows streamed past them) covers mask-mode codebooks whose K/32 warps hold e_dim
@@ -254,7 +256,7 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
         // Otherwise the per-row kernel (one warp per undecided row) while the FP32 codebook fits its shared memory
         // (measured at K = 512, e_dim = 64: 0.105 vs 0.128 ms for 108 k rows against the binned kernels); beyond that the
         // binned kernels win by 2-5x (code rows register-resident per bucket instead of re-read from L2 per row).  The
-        // binned path hands its list back to the per-row kernel through counters[5] / counters[6] when the pairs do not
+        // binned path hands its list back to the per-row kernel through the hand-back counters when the pairs do not
         // fit its workspace (normally both stay zero and the per-row kernel exits at once).  dvq_vq_set_refine /
         // DVQ_REFINE_PER_ROW / DVQ_REFINE_BINNED force one path.
         static const bool env_per_row = getenv("DVQ_REFINE_PER_ROW") != nullptr;
@@ -263,19 +265,19 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
         const bool force_per_row = env_per_row || mode == 1, force_binned = env_binned || mode == 2;
         const bool stationary = mode == 3 || (!force_per_row && !force_binned && vq_refine_stationary_default(K, D));
         const bool per_row_only = force_per_row || (!force_binned && vq_refine_codebook_in_smem(K, D));
+        RefineList handback = list;
+        handback.n = counters + CNT_HANDBACK;
+        if (list_mode) handback.n_ovf = counters + CNT_HANDBACK_OVF;
         if (stationary)
-          rc = launch_vq_refine_stationary(z, E, ee, K, D, train, z_q, idx, hist, sse, row_list, cand_list, counters, zbf, s);
+          rc = launch_vq_refine_stationary(z, E, ee, K, D, train, z_q, idx, hist, sse, list, zbf, s);
         else if (!per_row_only)
-          rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, cand_list, counters, list_mode ? 1 : 0,
-                                       ws + w.off_binned, zbf, s);
+          rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list, counters, ws + w.off_binned, zbf, s);
         if (!rc && !stationary)
-          rc = launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, row_list, cand_list, per_row_only ? counters : counters + 5,
-                                vq_tc_cand_gshift(K), list_mode ? row_list + (N - 1) : nullptr,
-                                list_mode ? (per_row_only ? counters + 2 : counters + 6) : nullptr, zbf, s);
+          rc = launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, per_row_only ? list : handback, zbf, s);
       } else {
-        rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list, counters, 1, zbf, s);
+        rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list.rows, list.n, 1, zbf, s);
         if (!rc && list_mode)
-          rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, row_list + (N - 1), counters + 2, -1, zbf, s);
+          rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list.ovf_last, list.n_ovf, -1, zbf, s);
       }
       profile_mark(2, false, s);
       if (rc) return rc;
@@ -306,7 +308,8 @@ int dvq_vq_read_counters(const void* workspace, int64_t N, int K, int D, int fla
   DVQ_CUDA_CHECK(cudaMemcpy(out4, static_cast<const char*>(workspace) + w.off_counters, 4 * sizeof(int), cudaMemcpyDeviceToHost));
   if (getenv("DVQ_TC_STATS_PRINT")) {
     unsigned long long st[17];
-    DVQ_CUDA_CHECK(cudaMemcpy(st, static_cast<const char*>(workspace) + w.off_counters + 32, sizeof(st), cudaMemcpyDeviceToHost));
+    DVQ_CUDA_CHECK(cudaMemcpy(st, static_cast<const char*>(workspace) + w.off_counters + CNT_STATS * sizeof(int), sizeof(st),
+                              cudaMemcpyDeviceToHost));
     static const char* names[17] = {"producer.wait_stage_empty", "mma.wait_a_full", "mma.wait_acc_empty", "mma.total",
                                     "conv.wait_stage_full", "conv.wait_a_empty", "conv.total", "epi0.wait_acc_full",
                                     "epi4.wait_fin_empty", "epi0.wait_fin_full", "epi0.wait_sidx_empty", "epi0.total",

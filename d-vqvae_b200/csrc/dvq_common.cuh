@@ -39,13 +39,73 @@ static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; 
 // ---- workspace layout of dvq_vq_forward (all offsets 256-byte aligned) -------------------
 struct VqWorkspace {
   size_t off_ee;        // float [K]            ||e_k||^2
-  size_t off_counters;  // int   [8]            refine-list length, overflow flags
-  size_t off_rowlist;   // int   [2][N]         rows the tensor-core filter could not decide + their candidate masks
+  size_t off_counters;  // int   [CNT_WORDS]    see CounterSlot
+  size_t off_rowlist;   // int   [2][N]         rows the tensor-core filter could not decide + their candidate records
   size_t off_bop;       // operand image of the codebook for the tcgen05 path
   size_t off_binned;    // bin tables + (row, sub-chunk) pair list of the binned refine (vq_refine_binned.cu)
   size_t total;
 };
 VqWorkspace vq_workspace_layout(int64_t N, int K, int D, int flags);
+
+// ---- the refine list: how the tcgen05 filter (vq_tc_sm100.cu) hands its undecided rows to the exact kernels ----------
+// Slots of the int counters in the workspace, reset on every call.
+enum CounterSlot {
+  CNT_LISTED = 0,         // rows in the refine list: row_list[0 .. n)
+  CNT_ERROR = 1,          // pipeline protocol error of the filter kernel (0 = none)
+  CNT_OVF = 2,            // list mode: rows in the overflow list, stored downwards from row_list[N - 1]
+  CNT_PAIRS = 4,          // binned refine: (row, sub-chunk) pairs
+  CNT_HANDBACK = 5,       // binned refine: listed rows handed to the per-row kernel (the pairs did not fit)
+  CNT_HANDBACK_OVF = 6,   //   and overflow rows
+  CNT_STATS = 8,          // DVQ_TC_STATS builds: 64-bit wait-time accounting from here on
+  CNT_WORDS = 64
+};
+
+// Candidate record of a listed row (cand_list[i]).  In the filter's hand-off word, CAND_UNDECIDED marks an undecided row
+// and the low 31 bits hold the record.  Mask mode (K <= 992): bit g <-> 32-code sub-chunk g held a key inside the row's
+// error band.  List mode (larger codebooks, where 31 bits would be too coarse): up to three CAND_ENTRY_BITS-bit entries
+// (sub-chunk index + 1, 0 = empty, packed from the low bits, in no particular order); CAND_LIST_OVERFLOW = more than three,
+// such a row goes to the overflow list.  Every code: 0 in either mode, CAND_MASK_ALL (a degenerate row) in mask mode,
+// CAND_LIST_OVERFLOW in list mode.
+constexpr uint32_t CAND_UNDECIDED = 0x80000000u;
+constexpr uint32_t CAND_MASK_ALL = 0x7fffffffu;
+constexpr uint32_t CAND_LIST_OVERFLOW = 0x3fffffffu;
+constexpr int CAND_ENTRY_BITS = 10;
+__host__ __device__ inline bool cand_list_mode(int K) { return K > 31 * 32; }
+
+// sub-chunk of list entry k (0..2) of a record, -1 when empty
+__device__ __forceinline__ int cand_entry(uint32_t cand, int k) {
+  return (int)((cand >> (CAND_ENTRY_BITS * k)) & ((1u << CAND_ENTRY_BITS) - 1u)) - 1;
+}
+__device__ __forceinline__ bool cand_is_all(uint32_t cand, bool list_mode) {
+  return cand == 0u || cand == (list_mode ? CAND_LIST_OVERFLOW : CAND_MASK_ALL);
+}
+// the candidate sub-chunks of a record (every one of the nsc sub-chunks when `all`), spread over a group of `gs` lanes
+// (gl = lane in the group)
+template <typename F>
+__device__ __forceinline__ void for_each_candidate(uint32_t cand, bool all, bool list_mode, int nsc, int gl, int gs, F&& f) {
+  if (all) {
+    for (int b = gl; b < nsc; b += gs) f(b);
+  } else if (list_mode) {
+    for (int k = gl; k < 3; k += gs) {
+      const int e = cand_entry(cand, k);
+      if (e >= 0 && e < nsc) f(e);
+    }
+  } else {
+    for (int b = gl; b < 31 && b < nsc; b += gs)
+      if ((cand >> b) & 1u) f(b);
+  }
+}
+
+// The refine list as the exact kernels read it, counts on the device: rows[0 .. *n) with their records cand[0 .. *n), and in
+// list mode the overflow rows ovf_last[0], ovf_last[-1], ... ovf_last[-(*n_ovf - 1)] (ovf_last = row_list + N - 1).
+struct RefineList {
+  const int* rows;
+  const int* cand;
+  const int* n;
+  const int* ovf_last;   // nullptr in mask mode
+  const int* n_ovf;      // nullptr in mask mode
+  bool list_mode;
+};
 
 // ---- kernels launched by the API layer ---------------------------------------------------
 // ee[k] = sum_d E[k,d]^2
@@ -70,30 +130,27 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
                  void* bop, int* counters, int* row_list, int* cand_list, int* zero_ints, int zero_n,
                  bool codebook_cached, bool zbf, cudaStream_t s);
 
-// candidate-restricted exact refine (vq_refine.cu); cand_list[i] = bit mask of 32*2^gshift-code groups
+// candidate-restricted exact refine (vq_refine.cu): one warp per listed row
 bool vq_refine_supported(int K, int D);
 bool vq_refine_codebook_in_smem(int K, int D);
-int vq_tc_cand_gshift(int K);
 int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                     unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                     const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, bool zbf, cudaStream_t s);
+                     unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s);
 
 // code-stationary exact refine (vq_refine_stationary.cu): mask-mode codebooks whose K/32 warps hold e_dim code floats
 // per lane in registers
 bool vq_refine_stationary_supported(int K, int D);
 bool vq_refine_stationary_default(int K, int D);   // the subset the automatic refine choice gives it (measured faster)
 int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                                unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                                const int* n_list, bool zbf, cudaStream_t s);
+                                unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s);
 
 // binned exact refine (vq_refine_binned.cu): (row, sub-chunk) pairs bucketed by sub-chunk; hands the list to
-// launch_vq_refine through counters[5] / counters[6] when the pairs do not fit its workspace
+// launch_vq_refine through counters[CNT_HANDBACK] / [CNT_HANDBACK_OVF] when the pairs do not fit its workspace
 long long refine_pair_cap_override();   // dvq_vq_set_refine (dvq_api.cu); 0 = default
 size_t vq_refine_binned_bytes(int64_t N);
 size_t vq_refine_binned_zero_bytes();
 int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                            int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                            int* counters, int list_mode, void* ws, bool zbf, cudaStream_t s);
+                            int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
+                            void* ws, bool zbf, cudaStream_t s);
 
 int launch_onehot(const int64_t* idx, int64_t N, int K, float* onehot, cudaStream_t s);
 int launch_finalize(const unsigned long long* hist, const double* sse, int64_t N, int K, int D, float al,

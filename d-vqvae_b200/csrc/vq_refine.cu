@@ -1,19 +1,17 @@
 // Exact FP32 re-evaluation of the rows the tcgen05 filter could not decide, restricted to the
-// candidate code groups the filter recorded (a bit per group of 32*2^gshift codes that held a key
-// inside the row's error band).  One warp per undecided row; lane = code inside a 32-code group.
+// candidate sub-chunks the filter recorded (the 32-code sub-chunks that held a key inside the row's
+// error band).  One warp per undecided row; lane = code inside a sub-chunk.
 //
-// Arithmetic is bit-identical to vq_simt_fp32.cu: per (row, code) the dot product is a sequential
-// fmaf over d = 0..D-1, zz = lane-strided fmaf partials + xor-shuffle tree, d = fma(-2, dot,
-// fl(zz + ee_k)), winner = lexicographic minimum of (distance, index) — so a row refined here gets
-// exactly the index the all-FP32 kernel would give it (the true minimiser is always inside the
-// candidate groups: every key outside the band is provably farther, DESIGN.md §4.1).
+// Arithmetic: the contract of vq_exact.cuh, so a row refined here gets exactly the index the all-FP32
+// kernel would give it (the true minimiser is always inside the candidate sub-chunks: every key outside
+// the band is provably farther, DESIGN.md §4.1).
 //
 // The codebook is staged once per CTA in shared memory with a (D+4)-float row pitch: 16-byte aligned
 // rows whose 128-bit reads are conflict-free for lane = code (a quarter-warp covers all 32 banks).  The
 // z row stays in shared memory too (broadcast 128-bit reads), so a thread needs ~40 registers and 32
 // warps per SM hide the latency of the sequential FMA chain; each undecided row then costs ~2 groups
 // x (32 LDS.128 + 64 FMAs) per lane instead of the K x D of the full kernel.
-#include "dvq_common.cuh"
+#include "vq_exact.cuh"
 
 namespace dvq {
 namespace {
@@ -25,8 +23,7 @@ template <int DT, bool TRAIN, bool SMEM_E, typename ZT>
 __global__ void __launch_bounds__(RTHREADS, 1)
 vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K,
                  ZT* __restrict__ zq, int64_t* __restrict__ idx_out, unsigned long long* __restrict__ hist,
-                 double* __restrict__ sse, const int* __restrict__ row_list, const int* __restrict__ cand_list,
-                 const int* __restrict__ n_list, int gshift, const int* __restrict__ ovf_last, const int* __restrict__ n_ovf) {
+                 double* __restrict__ sse, RefineList L) {
   extern __shared__ __align__(16) float smem_f[];   // zbuf[warps][2][DT] (ZT) | es[K][DT+4] when SMEM_E
   constexpr int PITCH = DT + 4;
   constexpr int NW = RTHREADS / 32;
@@ -35,7 +32,7 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
   ZT* zbuf = reinterpret_cast<ZT*>(smem_f) + warp * 2 * DT;   // double-buffered z row of this warp
   float* es = reinterpret_cast<float*>(reinterpret_cast<ZT*>(smem_f) + NW * 2 * DT);
   // nothing listed (the usual case when the binned kernels ran first): leave before staging the codebook
-  if (*n_list == 0 && (n_ovf == nullptr || *n_ovf == 0)) return;
+  if (*L.n == 0 && (L.n_ovf == nullptr || *L.n_ovf == 0)) return;
   if (SMEM_E) {
     for (int i = tid; i < K * (DT / 4); i += RTHREADS) {
       const int k = i / (DT / 4), d = (i - k * (DT / 4)) * 4;
@@ -43,17 +40,15 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
     }
     __syncthreads();
   }
-  const int n = *n_list;
+  const int n = *L.n;
   const int wglobal = blockIdx.x * NW + warp;
   const int wtotal = gridDim.x * NW;
-  const bool list_mode = gshift < 0;   // candidates as up to three (sub-chunk index + 1) entries of 10 bits, see vq_tc_sm100.cu
   const int nsc = (K + 31) / 32;
-  const int groups = list_mode ? 0 : (nsc + (1 << gshift) - 1) >> gshift;   // candidate bits in use
   double lsse = 0.0;
   // cp.async prefetch of the next undecided row of this warp hides its (random-access) global latency
   auto prefetch = [&](int i, int buf) {
     if (i < n) {
-      const ZT* src = z + (int64_t)row_list[i] * DT;
+      const ZT* src = z + (int64_t)L.rows[i] * DT;
 #pragma unroll
       for (int v = lane; v < DT / ZE; v += 32) {
         const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zbuf + buf * DT + v * ZE);
@@ -62,20 +57,13 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
   };
-  // outputs of one row (vq_simt_fp32.cu's epilogue), executed by one warp
+  // outputs of one row, executed by one warp
   auto emit_row = [&](int64_t row, int bidx, const ZT* zsrc) {
     ZT* orow = zq + row * DT;
     const float* erow = E + (int64_t)bidx * DT;
     for (int c = lane * 4; c < DT; c += 128) {
-      const float4 e4 = ldg4(erow + c);
-      float4 o4 = e4;
-      if (TRAIN) {
-        const float4 z4 = zld4(zsrc + c);
-        const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
-        const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
-        lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
-        o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
-      }
+      float4 o4 = ldg4(erow + c);
+      if (TRAIN) o4 = st_step4(o4, zld4(zsrc + c), lsse);
       zst4(orow + c, o4);
     }
     if (lane == 0) {
@@ -89,68 +77,42 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
     prefetch(i + wtotal, buf ^ 1);
     asm volatile("cp.async.wait_group 1;" ::: "memory");
     __syncwarp();
-    const int64_t row = row_list[i];
-    const unsigned cand = (unsigned)cand_list[i];
+    const int64_t row = L.rows[i];
+    const uint32_t cand = (uint32_t)L.cand[i];
     const ZT* zb = zbuf + buf * DT;
-    float s2 = 0.f;   // ||z||^2 exactly as vq_simt_fp32.cu computes it
-#pragma unroll
-    for (int c = 0; c < DT; c += 32) {
-      if (c + lane < DT) { const float v = zf(zb[c + lane]); s2 = fmaf(v, v, s2); }
-    }
-    const float zz = warp_sum(s2);
-    float best = INFINITY;
-    int bidx = 0;
-    // candidate sub-chunks (32 codes each) in ascending code order, two at a time: one broadcast read of z
-    // feeds both dot products, and the two sequential FMA chains interleave
-    unsigned todo = 0u;
-    int g_sc = 0, g_end = 0, l0 = -1, l1 = -1, l2 = -1;
-    if (list_mode) {
-      if (cand == 0u || cand == 0x3fffffffu) { g_end = nsc; }   // overflow / degenerate: every code
-      else {
-        l0 = (int)(cand & 1023u) - 1; l1 = (int)((cand >> 10) & 1023u) - 1; l2 = (int)((cand >> 20) & 1023u) - 1;
-        // ascending order, empty entries (-1) last
-        const int big = 1 << 30;
-        int a0 = l0 < 0 ? big : l0, a1 = l1 < 0 ? big : l1, a2 = l2 < 0 ? big : l2;
-        int t;
-        if (a0 > a1) { t = a0; a0 = a1; a1 = t; }
-        if (a1 > a2) { t = a1; a1 = a2; a2 = t; }
-        if (a0 > a1) { t = a0; a0 = a1; a1 = t; }
-        l0 = a0 == big ? -1 : a0; l1 = a1 == big ? -1 : a1; l2 = a2 == big ? -1 : a2;
-      }
+    const float zz = warp_sum(sq_partial<DT>(zb, lane));
+    unsigned long long best = ~0ull;   // (distance key, code) minimum so far
+    // candidate sub-chunks (32 codes each) in ascending code order (the tie-break relies on it), two at a time: one
+    // broadcast read of z feeds both dot products, and the two sequential FMA chains interleave
+    unsigned todo = 0u;                          // mask mode: the candidate bits
+    int g_sc = 0, g_end = 0;                     // every code: sub-chunks g_sc .. g_end - 1
+    int l0 = -1, l1 = -1, l2 = -1;               // list mode: the entries
+    if (cand_is_all(cand, L.list_mode)) {
+      g_end = nsc;
+    } else if (L.list_mode) {
+      // ascending order, empty entries (-1) last
+      const int big = 1 << 30;
+      const int e0 = cand_entry(cand, 0), e1 = cand_entry(cand, 1), e2 = cand_entry(cand, 2);
+      int a0 = e0 < 0 ? big : e0, a1 = e1 < 0 ? big : e1, a2 = e2 < 0 ? big : e2;
+      int t;
+      if (a0 > a1) { t = a0; a0 = a1; a1 = t; }
+      if (a1 > a2) { t = a1; a1 = a2; a2 = t; }
+      if (a0 > a1) { t = a0; a0 = a1; a1 = t; }
+      l0 = a0 == big ? -1 : a0; l1 = a1 == big ? -1 : a1; l2 = a2 == big ? -1 : a2;
     } else {
-      todo = cand ? cand : 0xffffffffu;
-      if (groups < 32) todo &= (1u << groups) - 1u;
+      todo = cand;
     }
     auto next_sc = [&]() -> int {   // warp-uniform; -1 when exhausted
-      for (;;) {
-        if (g_sc < g_end) {
-          const int r = g_sc++;
-          if (r * 32 < K) return r;
-          g_sc = g_end;
-          continue;
-        }
-        if (list_mode) {
-          const int r = l0;
-          l0 = l1; l1 = l2; l2 = -1;
-          return (r >= 0 && r * 32 < K) ? r : -1;
-        }
-        if (!todo) return -1;
-        const int g = __ffs(todo) - 1;
-        todo &= todo - 1u;
-        g_sc = g << gshift;
-        g_end = (g + 1) << gshift;
+      if (g_sc < g_end) return g_sc++;
+      if (L.list_mode) {
+        const int r = l0;
+        l0 = l1; l1 = l2; l2 = -1;
+        return r < nsc ? r : -1;
       }
-    };
-    // lexicographic (distance, code) minimum over the warp: monotone integer image of the distance, one
-    // REDUX.MIN, then the lowest lane holding the minimum (= lowest code: exact ties keep the first index)
-    auto warp_argmin = [&](float dist, int sc, float& best_, int& bidx_) {
-      const uint32_t b = __float_as_uint(dist);
-      const uint32_t key = (b & 0x80000000u) ? ~b : (b | 0x80000000u);   // NaN-free input: order-preserving
-      const uint32_t kmin = __reduce_min_sync(0xffffffffu, key);
-      const unsigned who = __ballot_sync(0xffffffffu, key == kmin);
-      const int src = __ffs(who) - 1;
-      const float dmin = __shfl_sync(0xffffffffu, dist, src);
-      if (dmin < best_) { best_ = dmin; bidx_ = sc * 32 + src; }
+      if (!todo) return -1;
+      const int g = __ffs(todo) - 1;
+      todo &= todo - 1u;
+      return g;
     };
     for (;;) {
       const int sa = next_sc();
@@ -197,37 +159,26 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
           acc_a = fmaf(z4.w, a4.w, acc_a); acc_b = fmaf(z4.w, b4.w, acc_b);
         }
       }
-      const float dist_a = va ? __fmaf_rn(-2.0f, acc_a, __fadd_rn(zz, __ldg(ee + code_a))) : INFINITY;
-      warp_argmin(dist_a, sa, best, bidx);
-      if (sb >= 0) {
-        const float dist_b = vb ? __fmaf_rn(-2.0f, acc_b, __fadd_rn(zz, __ldg(ee + code_b))) : INFINITY;
-        warp_argmin(dist_b, sb, best, bidx);
-      }
+      best = min(best, warp_argmin(dist_key(va ? exact_dist(acc_a, zz, __ldg(ee + code_a)) : INFINITY), sa * 32));
+      if (sb >= 0) best = min(best, warp_argmin(dist_key(vb ? exact_dist(acc_b, zz, __ldg(ee + code_b)) : INFINITY), sb * 32));
     }
-    emit_row(row, bidx, zbuf + buf * DT);
+    emit_row(row, packed_winner(best), zbuf + buf * DT);
     __syncwarp();   // everyone is done with zbuf[buf] before the next-but-one prefetch overwrites it
   }
   asm volatile("cp.async.wait_group 0;" ::: "memory");
   // ---- overflow rows (list mode: more than three candidate sub-chunks, degenerate rows): one CTA per row, the
   //      warps split the sub-chunks of the whole codebook, lexicographic (distance, code) minimum across warps ----
-  if (n_ovf != nullptr) {
-    __shared__ float red_d[NW];
-    __shared__ int red_k[NW];
-    const int n2 = *n_ovf;
+  if (L.n_ovf != nullptr) {
+    __shared__ unsigned long long red[NW];
+    const int n2 = *L.n_ovf;
     ZT* zrow = reinterpret_cast<ZT*>(smem_f);   // every warp is done with its z buffers after the barrier below
     for (int j = blockIdx.x; j < n2; j += gridDim.x) {
       __syncthreads();
-      const int64_t row = ovf_last[-(int64_t)j];   // the list is stored downwards from the end of the buffer
+      const int64_t row = L.ovf_last[-(int64_t)j];
       for (int v = tid; v < DT / ZE; v += RTHREADS) reinterpret_cast<uint4*>(zrow)[v] = __ldg(reinterpret_cast<const uint4*>(z + row * DT) + v);
       __syncthreads();
-      float s2 = 0.f;
-#pragma unroll
-      for (int c = 0; c < DT; c += 32) {
-        if (c + lane < DT) { const float v = zf(zrow[c + lane]); s2 = fmaf(v, v, s2); }
-      }
-      const float zz = warp_sum(s2);
-      float best = INFINITY;
-      int bidx = 0x7fffffff;
+      const float zz = warp_sum(sq_partial<DT>(zrow, lane));
+      unsigned long long best = ~0ull;
       for (int sc = warp; sc < nsc; sc += NW) {
         const int code = sc * 32 + lane;
         float dist = INFINITY;
@@ -241,28 +192,17 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
             acc = fmaf(z4.x, e4.x, acc); acc = fmaf(z4.y, e4.y, acc);
             acc = fmaf(z4.z, e4.z, acc); acc = fmaf(z4.w, e4.w, acc);
           }
-          dist = __fmaf_rn(-2.0f, acc, __fadd_rn(zz, __ldg(ee + code)));
+          dist = exact_dist(acc, zz, __ldg(ee + code));
         }
-        const uint32_t b = __float_as_uint(dist);
-        const uint32_t key = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-        const uint32_t kmin = __reduce_min_sync(0xffffffffu, key);
-        const int src = __ffs(__ballot_sync(0xffffffffu, key == kmin)) - 1;
-        const float dmin = __shfl_sync(0xffffffffu, dist, src);
-        if (dmin < best) { best = dmin; bidx = sc * 32 + src; }
+        best = min(best, warp_argmin(dist_key(dist), sc * 32));
       }
-      if (lane == 0) { red_d[warp] = best; red_k[warp] = bidx; }
+      if (lane == 0) red[warp] = best;
       __syncthreads();
       if (warp == 0) {
-        float d = red_d[lane];
-        int k = red_k[lane];
+        unsigned long long b = red[lane];
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-          const float od = __shfl_xor_sync(0xffffffffu, d, o);
-          const int ok = __shfl_xor_sync(0xffffffffu, k, o);
-          if (od < d || (od == d && ok < k)) { d = od; k = ok; }
-        }
-        if (k == 0x7fffffff) k = 0;
-        emit_row(row, k, zrow);
+        for (int o = 16; o > 0; o >>= 1) b = min(b, __shfl_xor_sync(0xffffffffu, b, o));
+        emit_row(row, packed_winner(b), zrow);
       }
     }
   }
@@ -283,8 +223,7 @@ bool vq_refine_supported(int K, int D) { return (D == 16 || D == 32 || D == 64 |
 
 template <int DT, typename ZT>
 static int launch_refine_dt(const ZT* z, const float* E, const float* ee, int K, int train, ZT* z_q, int64_t* idx,
-                            unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                            const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, int sm_count, cudaStream_t s) {
+                            unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
   const size_t zbuf_bytes = (size_t)(RTHREADS / 32) * 2 * DT * sizeof(ZT);
   const size_t smem_e = (size_t)K * (DT + 4) * sizeof(float);
   const bool in_smem = vq_refine_codebook_in_smem(K, DT);
@@ -292,8 +231,7 @@ static int launch_refine_dt(const ZT* z, const float* E, const float* ee, int K,
   do {                                                                                                                   \
     const size_t bytes = zbuf_bytes + (SM_ ? smem_e : 0);                                                                \
     DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_refine_kernel<DT, TR_, SM_, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)); \
-    vq_refine_kernel<DT, TR_, SM_, ZT><<<sm_count, RTHREADS, bytes, s>>>(z, E, ee, K, z_q, idx, hist, sse, row_list,         \
-                                                                      cand_list, n_list, gshift, ovf_last, n_ovf);      \
+    vq_refine_kernel<DT, TR_, SM_, ZT><<<sm_count, RTHREADS, bytes, s>>>(z, E, ee, K, z_q, idx, hist, sse, list);         \
   } while (0)
   if (train) { if (in_smem) DVQ_LAUNCH_REFINE(true, true); else DVQ_LAUNCH_REFINE(true, false); }
   else       { if (in_smem) DVQ_LAUNCH_REFINE(false, true); else DVQ_LAUNCH_REFINE(false, false); }
@@ -305,30 +243,27 @@ static int launch_refine_dt(const ZT* z, const float* E, const float* ee, int K,
 
 template <typename ZT>
 static int launch_refine_t(const ZT* z, const float* E, const float* ee, int K, int D, int train, ZT* z_q, int64_t* idx,
-                           unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                           const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, const DeviceProps& dp, cudaStream_t s) {
+                           unsigned long long* hist, double* sse, const RefineList& list, const DeviceProps& dp, cudaStream_t s) {
   switch (D) {
-    case 16: return launch_refine_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
-    case 32: return launch_refine_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
-    case 64: return launch_refine_dt<64>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
-    case 128: return launch_refine_dt<128>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
-    case 256: return launch_refine_dt<256>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
-    case 512: return launch_refine_dt<512>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp.sm_count, s);
+    case 16: return launch_refine_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
+    case 32: return launch_refine_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
+    case 64: return launch_refine_dt<64>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
+    case 128: return launch_refine_dt<128>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
+    case 256: return launch_refine_dt<256>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
+    case 512: return launch_refine_dt<512>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
     default: return fail(DVQ_ERR_BAD_SHAPE, "candidate refine kernel is instantiated for e_dim 16..512 (powers of two) only");
   }
 }
 
 int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                     unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                     const int* n_list, int gshift, const int* ovf_last, const int* n_ovf, bool zbf, cudaStream_t s) {
+                     unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
   if (zbf)
     return launch_refine_t(static_cast<const __nv_bfloat16*>(z), E, ee, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
-                           row_list, cand_list, n_list, gshift, ovf_last, n_ovf, dp, s);
-  return launch_refine_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, row_list, cand_list,
-                         n_list, gshift, ovf_last, n_ovf, dp, s);
+                           list, dp, s);
+  return launch_refine_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list, dp, s);
 }
 
 }  // namespace dvq

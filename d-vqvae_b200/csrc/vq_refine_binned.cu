@@ -16,15 +16,13 @@
 //                          time against the warp's 32 codes, warp argmin, atomicMin on idx[row]
 //   refine_emit_kernel     one warp per listed row: winner -> idx, z_q, SSE, histogram
 //
-// Arithmetic is bit-identical to vq_simt_fp32.cu / vq_refine.cu: per (row, code) a sequential fmaf over
-// d = 0..D-1, zz = lane-strided fmaf partials + xor-shuffle tree, dist = fma(-2, dot, fl(zz + ee_k)), winner =
-// lexicographic minimum of (distance, code) — here as an unsigned 64-bit minimum of
-// (order-preserving image of the distance) << 32 | code, so the order in which pairs are processed is irrelevant.
+// Arithmetic: the contract of vq_exact.cuh; the (distance, code) minimum is an unsigned 64-bit minimum of
+// warp_argmin's packed values, so the order in which pairs are processed is irrelevant.
 //
 // Rows whose candidate record says "every code" (degenerate rows; list mode: more than three candidate
 // sub-chunks) are paired with every sub-chunk.  If the pairs do not fit the workspace (2 N entries) the
 // scatter kernel hands the whole list to vq_refine.cu instead (device-side switch, no host sync).
-#include "dvq_common.cuh"
+#include "vq_exact.cuh"
 
 namespace dvq {
 namespace {
@@ -33,11 +31,6 @@ constexpr int PREP_THREADS = 1024;
 constexpr int PAIR_THREADS = 384;
 constexpr int RB = 16;                 // rows per batch of the pairs kernel
 constexpr int MAX_BINS = 1024;         // K <= 32 768
-constexpr uint32_t CAND_ALL_LIST = 0x3fffffffu;
-
-// counters[] slots used here (zeroed per call by tc_cb_stats_kernel): [0] listed rows, [2] overflow rows,
-// [4] total pairs, [5] / [6] rows / overflow rows handed to the fallback kernel
-enum { C_N = 0, C_NOVF = 2, C_PAIRS = 4, C_FB_N = 5, C_FB_NOVF = 6 };
 
 struct BinTables {        // int arrays in the workspace
   int* count;             // [MAX_BINS]   pairs per sub-chunk            (zeroed per call)
@@ -46,29 +39,9 @@ struct BinTables {        // int arrays in the workspace
   int* item_start;        // [MAX_BINS+1] exclusive scan of ceil(count / ch); [MAX_BINS+1] = ch
 };
 
-__device__ __forceinline__ int64_t listed_row(int i, int n, const int* __restrict__ row_list, const int* __restrict__ ovf_last) {
-  return i < n ? row_list[i] : ovf_last[-(int64_t)(i - n)];   // the overflow list is stored downwards from the end
-}
-
-// candidate sub-chunks of a listed row, spread over a group of `gs` lanes (gl = lane inside the group)
-template <typename F>
-__device__ __forceinline__ void for_each_candidate(unsigned cand, bool all, bool list_mode, int nbins, int gl, int gs, F&& f) {
-  if (all) {
-    for (int b = gl; b < nbins; b += gs) f(b);
-  } else if (list_mode) {
-    for (int k = gl; k < 3; k += gs) {
-      const int e = (int)((cand >> (10 * k)) & 1023u) - 1;
-      if (e >= 0 && e < nbins) f(e);
-    }
-  } else {
-    for (int b = gl; b < 31 && b < nbins; b += gs)
-      if ((cand >> b) & 1u) f(b);
-  }
-}
-__device__ __forceinline__ bool cand_is_all(unsigned cand, bool listed_normal, bool list_mode) {
-  if (!listed_normal) return true;                       // overflow list
-  if (list_mode) return cand == 0u || cand == CAND_ALL_LIST;
-  return cand == 0u || cand == 0x7fffffffu;
+// listed row i: the refine list, then the overflow list
+__device__ __forceinline__ int64_t listed_row(int i, int n, const int* __restrict__ rows, const int* __restrict__ ovf_last) {
+  return i < n ? rows[i] : ovf_last[-(int64_t)(i - n)];
 }
 
 // ||z||^2 of a listed row is stashed as a float in the first 4 bytes of its z_q row (rewritten by the emit kernel): 2 D >= 32
@@ -79,27 +52,25 @@ __device__ __forceinline__ float* zz_stash(ZT* zq, int64_t row, int D) { return 
 template <typename ZT>
 __global__ void __launch_bounds__(PREP_THREADS, 1)
 refine_prep_kernel(const ZT* __restrict__ z, int D, int K, ZT* __restrict__ zq, unsigned long long* __restrict__ idx64,
-                   const int* __restrict__ row_list, const int* __restrict__ cand_list, const int* __restrict__ ovf_last,
-                   int* __restrict__ counters, BinTables bt, int list_mode) {
+                   RefineList L, int* __restrict__ counters, BinTables bt) {
   __shared__ int s_cnt[MAX_BINS];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int n = counters[C_N], n2 = list_mode ? counters[C_NOVF] : 0;
+  const int n = counters[CNT_LISTED], n2 = L.list_mode ? counters[CNT_OVF] : 0;
   if (n + n2 == 0) return;
   const int nbins = (K + 31) / 32;
   for (int b = tid; b < nbins; b += PREP_THREADS) s_cnt[b] = 0;
   __syncthreads();
-  // Four rows per warp (8 lanes each) so that four independent row fetches are in flight per warp.  ||z||^2 is
-  // bit-identical to vq_simt_fp32.cu's (lane l of a 32-lane warp accumulates elements l, l + 32, ... with fmaf,
-  // then an xor-shuffle tree): lane j of a group plays the virtual lanes j, j + 8, j + 16, j + 24; the first two
-  // tree levels (xor 16, xor 8) are in-thread sums of the same operand pairs, the last three are shuffles.
+  // Four rows per warp (8 lanes each) so that four independent row fetches are in flight per warp.  ||z||^2 is the
+  // 32-lane sum of vq_exact.cuh bit for bit: lane j of a group plays the virtual lanes j, j + 8, j + 16, j + 24; the
+  // first two tree levels (xor 16, xor 8) are in-thread sums of the same operand pairs, the last three are shuffles.
   const int wtotal = gridDim.x * (PREP_THREADS / 32);
   const int g = lane >> 3, j = lane & 7;
   int my_pairs = 0;
   for (int base = (blockIdx.x * (PREP_THREADS / 32) + warp) * 4; base < n + n2; base += wtotal * 4) {
     const int i = base + g;
     const bool active = i < n + n2;
-    const int64_t row = active ? listed_row(i, n, row_list, ovf_last) : 0;
-    const unsigned cand = (active && i < n) ? (unsigned)cand_list[i] : 0u;
+    const int64_t row = active ? (i < n ? L.rows[i] : L.ovf_last[-(int64_t)(i - n)]) : 0;
+    const uint32_t cand = (active && i < n) ? (uint32_t)L.cand[i] : 0u;
     const ZT* zr = z + row * D;
     float pm[4] = {0.f, 0.f, 0.f, 0.f};
     for (int c = 0; c < D; c += 32) {
@@ -118,8 +89,8 @@ refine_prep_kernel(const ZT* __restrict__ z, int D, int K, ZT* __restrict__ zq, 
         *zz_stash(zq, row, D) = zz;    // the row's z_q is rewritten by the emit kernel
         idx64[row] = ~0ull;
       }
-      const bool all = cand_is_all(cand, i < n, list_mode != 0);
-      for_each_candidate(cand, all, list_mode != 0, nbins, j, 8, [&](int b) { atomicAdd(&s_cnt[b], 1); ++my_pairs; });
+      const bool all = i >= n || cand_is_all(cand, L.list_mode);   // overflow rows: every code
+      for_each_candidate(cand, all, L.list_mode, nbins, j, 8, [&](int b) { atomicAdd(&s_cnt[b], 1); ++my_pairs; });
     }
   }
   __syncthreads();
@@ -128,7 +99,7 @@ refine_prep_kernel(const ZT* __restrict__ z, int D, int K, ZT* __restrict__ zq, 
     if (c) atomicAdd(bt.count + b, c);
   }
   my_pairs = (int)warp_sum((float)my_pairs);   // < 2^24 per warp: exact in FP32
-  if (lane == 0 && my_pairs) atomicAdd(counters + C_PAIRS, my_pairs);
+  if (lane == 0 && my_pairs) atomicAdd(counters + CNT_PAIRS, my_pairs);
 }
 
 // exclusive scan of v[0..n) (n <= MAX_BINS) by a 1024-thread block; out[n] = total
@@ -159,19 +130,19 @@ __device__ __forceinline__ void block_scan_1024(int v, int n, int* out, int* s_w
 }
 
 __global__ void __launch_bounds__(PREP_THREADS, 1)
-refine_scatter_kernel(int K, const int* __restrict__ cand_list, int* __restrict__ counters, BinTables bt, int* __restrict__ pairs,
-                      long long pair_cap, int list_mode, int pair_warps) {
+refine_scatter_kernel(int K, RefineList L, int* __restrict__ counters, BinTables bt, int* __restrict__ pairs, long long pair_cap,
+                      int pair_warps) {
   __shared__ int s_start[MAX_BINS + 1];
   __shared__ int s_items[MAX_BINS + 1];
   __shared__ int s_cnt[MAX_BINS];
   __shared__ int s_base[MAX_BINS];
   __shared__ int s_warp[32];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int n = counters[C_N], n2 = list_mode ? counters[C_NOVF] : 0;
+  const int n = counters[CNT_LISTED], n2 = L.list_mode ? counters[CNT_OVF] : 0;
   if (n + n2 == 0) return;
-  const long long total = counters[C_PAIRS];
+  const long long total = counters[CNT_PAIRS];
   if (total > pair_cap || total >= (1ll << 30)) {   // does not fit: the per-row kernel takes the whole list
-    if (blockIdx.x == 0 && tid == 0) { counters[C_FB_N] = n; counters[C_FB_NOVF] = n2; }
+    if (blockIdx.x == 0 && tid == 0) { counters[CNT_HANDBACK] = n; counters[CNT_HANDBACK_OVF] = n2; }
     return;
   }
   const int nbins = (K + 31) / 32;
@@ -196,9 +167,9 @@ refine_scatter_kernel(int K, const int* __restrict__ cand_list, int* __restrict_
     for (int ib = i0 + warp * 32; ib < i1; ib += PREP_THREADS) {
       const int i = ib + lane;
       const bool active = i < i1;
-      const unsigned cand = (active && i < n) ? (unsigned)cand_list[i] : 0u;
-      const bool all = active && cand_is_all(cand, i < n, list_mode != 0);
-      if (active && !all) for_each_candidate(cand, false, list_mode != 0, nbins, 0, 1, [&](int b) { f(b, i); });
+      const uint32_t cand = (active && i < n) ? (uint32_t)L.cand[i] : 0u;
+      const bool all = active && (i >= n || cand_is_all(cand, L.list_mode));
+      if (active && !all) for_each_candidate(cand, false, L.list_mode, nbins, 0, 1, [&](int b) { f(b, i); });
       unsigned am = __ballot_sync(0xffffffffu, all);
       while (am) {
         const int ii = ib + __ffs(am) - 1;
@@ -218,25 +189,18 @@ refine_scatter_kernel(int K, const int* __restrict__ cand_list, int* __restrict_
   sweep([&](int b, int i) { pairs[s_base[b] + atomicAdd(&s_cnt[b], 1)] = i; });
 }
 
-// order-preserving unsigned image of a float (NaN-free input)
-__device__ __forceinline__ uint32_t float_key(float d) {
-  const uint32_t b = __float_as_uint(d);
-  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-
 template <int DS, typename ZT>
 __global__ void __launch_bounds__(PAIR_THREADS, DS <= 32 ? 2 : 1)
 refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K, int D,
-                    ZT* __restrict__ zq, unsigned long long* __restrict__ idx64, const int* __restrict__ row_list,
-                    const int* __restrict__ ovf_last, const int* __restrict__ pairs, const int* __restrict__ counters,
-                    BinTables bt, long long pair_cap, int list_mode) {
+                    ZT* __restrict__ zq, unsigned long long* __restrict__ idx64, RefineList L, const int* __restrict__ pairs,
+                    const int* __restrict__ counters, BinTables bt, long long pair_cap) {
   extern __shared__ __align__(16) float smem_f[];   // zs[warps][2][RB][DS] (ZT: bf16 rows are staged as bf16) | es
   __shared__ int s_start[MAX_BINS + 1];
   __shared__ int s_items[MAX_BINS + 1];
   constexpr int NW = PAIR_THREADS / 32;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int n = counters[C_N], n2 = list_mode ? counters[C_NOVF] : 0;
-  const long long total = counters[C_PAIRS];
+  const int n = counters[CNT_LISTED], n2 = L.list_mode ? counters[CNT_OVF] : 0;
+  const long long total = counters[CNT_PAIRS];
   if (n + n2 == 0 || total == 0 || total > pair_cap || total >= (1ll << 30)) return;
   const int nbins = (K + 31) / 32;
   for (int b = tid; b <= nbins; b += PAIR_THREADS) { s_start[b] = bt.start[b]; s_items[b] = bt.item_start[b]; }
@@ -282,7 +246,7 @@ refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const
     auto fetch_rows = [&](int p, int64_t& row_, float& zz_) {
       row_ = -1; zz_ = 0.f;
       if (p < p1 && lane < min(RB, p1 - p)) {
-        row_ = listed_row(pairs[p + lane], n, row_list, ovf_last);
+        row_ = listed_row(pairs[p + lane], n, L.rows, L.ovf_last);
         zz_ = *zz_stash(zq, row_, D);
       }
     };
@@ -360,13 +324,9 @@ refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const
       for (int r = 0; r < RB; ++r) {
         if (r < nb) {   // warp-uniform
           const float zzr = __shfl_sync(0xffffffffu, zz, r);
-          float dist = __fmaf_rn(-2.0f, acc[r], __fadd_rn(zzr, eek));
-          if (!valid || !(dist == dist)) dist = INFINITY;
-          const uint32_t key = float_key(dist);
-          const uint32_t kmin = __reduce_min_sync(0xffffffffu, key);
-          const int src = __ffs(__ballot_sync(0xffffffffu, key == kmin)) - 1;   // lowest lane = lowest code
+          const unsigned long long best = warp_argmin(dist_key(valid ? exact_dist(acc[r], zzr, eek) : INFINITY), b * 32);
           const long long rr = __shfl_sync(0xffffffffu, (long long)row, r);
-          if (lane == 0) atomicMin(idx64 + rr, ((unsigned long long)kmin << 32) | (unsigned)(b * 32 + src));
+          if (lane == 0) atomicMin(idx64 + rr, best);
         }
       }
       row = row_n; zz = zz_n;
@@ -378,11 +338,10 @@ template <bool TRAIN, typename ZT>
 __global__ void __launch_bounds__(PREP_THREADS, 1)
 refine_emit_kernel(const ZT* __restrict__ z, const float* __restrict__ E, int D, ZT* __restrict__ zq,
                    unsigned long long* __restrict__ idx64, unsigned long long* __restrict__ hist, double* __restrict__ sse,
-                   const int* __restrict__ row_list, const int* __restrict__ ovf_last, const int* __restrict__ counters,
-                   long long pair_cap, int list_mode) {
+                   RefineList L, const int* __restrict__ counters, long long pair_cap) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int n = counters[C_N], n2 = list_mode ? counters[C_NOVF] : 0;
-  const long long total = counters[C_PAIRS];
+  const int n = counters[CNT_LISTED], n2 = L.list_mode ? counters[CNT_OVF] : 0;
+  const long long total = counters[CNT_PAIRS];
   if (n + n2 == 0 || total > pair_cap || total >= (1ll << 30)) return;
   const int wtotal = gridDim.x * (PREP_THREADS / 32);
   const int g = lane >> 3, j = lane & 7;   // four rows per warp, 8 lanes each: four independent fetch chains in flight
@@ -390,23 +349,15 @@ refine_emit_kernel(const ZT* __restrict__ z, const float* __restrict__ E, int D,
   for (int base = (blockIdx.x * (PREP_THREADS / 32) + warp) * 4; base < n + n2; base += wtotal * 4) {
     const int i = base + g;
     const bool active = i < n + n2;
-    const int64_t row = active ? listed_row(i, n, row_list, ovf_last) : 0;
-    const unsigned long long best = active ? idx64[row] : 0ull;
-    const int bidx = best == ~0ull ? 0 : (int)(best & 0xffffffffull);
+    const int64_t row = active ? listed_row(i, n, L.rows, L.ovf_last) : 0;
+    const int bidx = active ? packed_winner(idx64[row]) : 0;
     ZT* orow = zq + row * D;
     const float* erow = E + (int64_t)bidx * D;
     const ZT* zsrc = z + row * D;
     if (active) {
       for (int c = j * 4; c < D; c += 32) {
-        const float4 e4 = ldg4(erow + c);
-        float4 o4 = e4;
-        if (TRAIN) {
-          const float4 z4 = zldg4(zsrc + c);
-          const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
-          const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
-          lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
-          o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
-        }
+        float4 o4 = ldg4(erow + c);
+        if (TRAIN) o4 = st_step4(o4, zldg4(zsrc + c), lsse);
         zst4(orow + c, o4);
       }
     }
@@ -433,8 +384,8 @@ size_t vq_refine_binned_zero_bytes() { return sizeof(int) * 2 * MAX_BINS; }
 
 template <typename ZT>
 static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t N, int K, int D, int train, ZT* z_q,
-                           int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                           int* counters, int list_mode, void* ws, cudaStream_t s) {
+                           int64_t* idx, unsigned long long* hist, double* sse, const RefineList& L, int* counters, void* ws,
+                           cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
@@ -445,7 +396,6 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
   int* pairs = reinterpret_cast<int*>(static_cast<char*>(ws) + align_up(sizeof(int) * (size_t)(4 * MAX_BINS + 8), 256));
   const long long cap_override = refine_pair_cap_override();
   const long long pair_cap = (cap_override > 0 && cap_override < 2 * (long long)N) ? cap_override : 2 * (long long)N;
-  const int* ovf_last = row_list + (N - 1);
   unsigned long long* idx64 = reinterpret_cast<unsigned long long*>(idx);
   // slice width of the pairs kernel: a lane keeps DS floats of its code row in registers.  DS = 64 (168 registers, one CTA
   // of 12 warps per SM) re-reads a code row half as often, DS = 32 (80 registers) fits two CTAs per SM: measured at
@@ -458,16 +408,16 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
   const int pair_grid = dp.sm_count * (DS <= 32 && D >= 64 ? 2 : 1);
   const int pair_warps = pair_grid * (PAIR_THREADS / 32);
 
-  refine_prep_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(z, D, K, z_q, idx64, row_list, cand_list, ovf_last, counters, bt, list_mode);
+  refine_prep_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(z, D, K, z_q, idx64, L, counters, bt);
   DVQ_CUDA_CHECK(cudaGetLastError());
-  refine_scatter_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(K, cand_list, counters, bt, pairs, pair_cap, list_mode, pair_warps);
+  refine_scatter_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(K, L, counters, bt, pairs, pair_cap, pair_warps);
   DVQ_CUDA_CHECK(cudaGetLastError());
   const size_t smem = (size_t)(PAIR_THREADS / 32) * (2 * RB * DS * sizeof(ZT) + (D > DS ? 32 * (DS + 4) * sizeof(float) : 0));
 #define DVQ_LAUNCH_PAIRS(DS_)                                                                                              \
   do {                                                                                                                     \
     DVQ_CUDA_CHECK(cudaFuncSetAttribute(refine_pairs_kernel<DS_, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    refine_pairs_kernel<DS_, ZT><<<pair_grid, PAIR_THREADS, smem, s>>>(z, E, ee, K, D, z_q, idx64, row_list, ovf_last, pairs,  \
-                                                                   counters, bt, pair_cap, list_mode);                     \
+    refine_pairs_kernel<DS_, ZT><<<pair_grid, PAIR_THREADS, smem, s>>>(z, E, ee, K, D, z_q, idx64, L, pairs, counters, bt,      \
+                                                                   pair_cap);                                              \
   } while (0)
   if (DS == 64) DVQ_LAUNCH_PAIRS(64);
   else if (DS == 32) DVQ_LAUNCH_PAIRS(32);
@@ -476,22 +426,22 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
 #undef DVQ_LAUNCH_PAIRS
   DVQ_CUDA_CHECK(cudaGetLastError());
   if (train)
-    refine_emit_kernel<true, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, row_list, ovf_last, counters, pair_cap, list_mode);
+    refine_emit_kernel<true, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, L, counters, pair_cap);
   else
-    refine_emit_kernel<false, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, row_list, ovf_last, counters, pair_cap, list_mode);
+    refine_emit_kernel<false, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, L, counters, pair_cap);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch(4);
   return DVQ_OK;
 }
 
 int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                            int64_t* idx, unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                            int* counters, int list_mode, void* ws, bool zbf, cudaStream_t s) {
+                            int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
+                            void* ws, bool zbf, cudaStream_t s) {
   if (zbf)
     return launch_binned_t(static_cast<const __nv_bfloat16*>(z), E, ee, N, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
-                           row_list, cand_list, counters, list_mode, ws, s);
-  return launch_binned_t(static_cast<const float*>(z), E, ee, N, K, D, train, static_cast<float*>(z_q), idx, hist, sse, row_list,
-                         cand_list, counters, list_mode, ws, s);
+                           list, counters, ws, s);
+  return launch_binned_t(static_cast<const float*>(z), E, ee, N, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list, counters,
+                         ws, s);
 }
 
 }  // namespace dvq

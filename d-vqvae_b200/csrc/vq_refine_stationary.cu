@@ -2,7 +2,7 @@
 // every lane of a CTA can hold one code row in registers.  One warp per 32-code sub-chunk (K / 32 warps), lane = code;
 // the code rows are loaded once per CTA and the z rows stream past them.
 //
-// Each CTA takes a contiguous share of the filter's row list (sized on the device from *n_list) and stages it in
+// Each CTA takes a contiguous share of the filter's row list (sized on the device from its count) and stages it in
 // batches of SB rows: row ids and candidate masks by 4-byte cp.async two batches ahead, the z rows by 16-byte cp.async
 // one batch ahead (double-buffered, fp32 or bf16 as stored).  Per batch: ||z||^2 once per row (one warp per row), then
 // every warp evaluates the rows whose mask names its sub-chunk (mask 0 = degenerate row: every warp), four rows at a
@@ -12,29 +12,19 @@
 // takes the table's minimum and writes idx, and all threads write z_q / SSE as independent (row, 4-column) items; the
 // histogram is kept in shared memory and flushed once per CTA.
 //
-// Arithmetic is that of vq_refine.cu and vq_simt_fp32.cu bit for bit: zz = lane-strided fmaf partials + xor-shuffle
-// tree, dot = sequential fmaf over d = 0..D-1, dist = fma(-2, dot, fl(zz + ee_k)), winner = lexicographic (distance,
-// code) minimum; a row without a finite distance on its candidate codes gets code 0, as in those kernels.
-#include "dvq_common.cuh"
+// Arithmetic: the contract of vq_exact.cuh.
+#include "vq_exact.cuh"
 
 namespace dvq {
 namespace {
 
 constexpr int SB = 128;           // rows per staged batch
 constexpr int SMAX_WARPS = 31;    // mask mode: at most 31 sub-chunks
-constexpr uint32_t KEY_INF = 0xff800000u;   // image of +inf under dist_key
 
 // warps (sub-chunks) a CTA can hold with DT code floats per lane in registers: 1024 threads leave 64 registers a
 // thread, 512 leave 128, 256 leave 255
 template <int DT>
 constexpr int stationary_max_warps() { return DT <= 16 ? 31 : DT <= 64 ? 16 : DT == 128 ? 8 : 0; }
-
-// order-preserving unsigned image of a distance; NaN counts as +inf (never a winner)
-__device__ __forceinline__ uint32_t dist_key(float d) {
-  if (!(d == d)) d = INFINITY;
-  const uint32_t b = __float_as_uint(d);
-  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
 
 // distances of R staged rows (slots rs[0..R)) to this lane's code; the warp's (distance image, code) minimum of each row
 // goes to cand[row] (this warp's column of the per-row candidate table)
@@ -58,10 +48,8 @@ __device__ __forceinline__ void eval_rows(const float (&e)[DT], float eek, int s
   }
 #pragma unroll
   for (int i = 0; i < R; ++i) {
-    const uint32_t key = dist_key(__fmaf_rn(-2.0f, acc[i], __fadd_rn(s_zz[r[i]], eek)));
-    const uint32_t kmin = __reduce_min_sync(0xffffffffu, key);
-    const int src = __ffs(__ballot_sync(0xffffffffu, key == kmin)) - 1;   // lowest lane = lowest code
-    if (lane == 0) cand[r[i]] = ((unsigned long long)kmin << 32) | (unsigned)(sc_base + src);
+    const unsigned long long best = warp_argmin(dist_key(exact_dist(acc[i], s_zz[r[i]], eek)), sc_base);
+    if (lane == 0) cand[r[i]] = best;
   }
 }
 
@@ -70,8 +58,7 @@ template <int DT, typename ZT>
 __global__ void __launch_bounds__(stationary_max_warps<DT>() * 32, 1)
 vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee, int K, int train,
                             ZT* __restrict__ zq, int64_t* __restrict__ idx_out, unsigned long long* __restrict__ hist,
-                            double* __restrict__ sse, const int* __restrict__ row_list, const int* __restrict__ cand_list,
-                            const int* __restrict__ n_list) {
+                            double* __restrict__ sse, RefineList L) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ZT* zbuf = reinterpret_cast<ZT*>(smem_raw);   // [2][SB][DT]
   // [warps][SB]: each warp's (distance image << 32 | code) minimum per row, ~0 where the warp did not evaluate the row
@@ -90,7 +77,7 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   uint32_t lanemask_lt;
   asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lanemask_lt));
-  const int n = *n_list;
+  const int n = *L.n;
   const int start = (int)((int64_t)n * blockIdx.x / gridDim.x);
   const int end = (int)((int64_t)n * (blockIdx.x + 1) / gridDim.x);
   if (start >= end) return;
@@ -101,8 +88,8 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     for (int t = tid; t < cnt; t += nt) {
       const uint32_t dr = (uint32_t)__cvta_generic_to_shared(&s_row[b % 3][t]);
       const uint32_t dm = (uint32_t)__cvta_generic_to_shared(&s_mask[b % 3][t]);
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dr), "l"(row_list + i0 + t) : "memory");
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dm), "l"(cand_list + i0 + t) : "memory");
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dr), "l"(L.rows + i0 + t) : "memory");
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dm), "l"(L.cand + i0 + t) : "memory");
     }
   };
   auto stage_z = [&](int b) {     // z rows of batch b (ids landed and visible; no commit of its own)
@@ -149,18 +136,11 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     const ZT* zb = zbuf + (b & 1) * SB * DT;
     const int* rows = s_row[b % 3];
     const unsigned* masks = s_mask[b % 3];
-    // ||z||^2 exactly as vq_simt_fp32.cu computes it, four rows of a warp at a time (independent shuffle trees)
+    // ||z||^2, four rows of a warp at a time (independent shuffle trees)
     for (int r0 = warp; r0 < cnt; r0 += 4 * nw) {
       float s2[4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int r = min(r0 + u * nw, cnt - 1);
-        s2[u] = 0.f;
-#pragma unroll
-        for (int c = 0; c < DT; c += 32) {
-          if (c + lane < DT) { const float v = zf(zb[r * DT + c + lane]); s2[u] = fmaf(v, v, s2[u]); }
-        }
-      }
+      for (int u = 0; u < 4; ++u) s2[u] = sq_partial<DT>(zb + min(r0 + u * nw, cnt - 1) * DT, lane);
 #pragma unroll
       for (int u = 0; u < 4; ++u) s2[u] = warp_sum(s2[u]);
       if (lane == 0) {
@@ -177,7 +157,7 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     for (int g = 0; g < cnt; g += 32) {
       const int r = g + lane;
       const unsigned mk = r < cnt ? masks[r] : 1u;
-      const bool sel = r < cnt && (mk == 0u || ((mk >> warp) & 1u));
+      const bool sel = r < cnt && (cand_is_all(mk, false) || ((mk >> warp) & 1u));
       const unsigned bal = __ballot_sync(0xffffffffu, sel);
       if (sel) list[m + __popc(bal & lanemask_lt)] = (unsigned char)r;
       m += __popc(bal);
@@ -189,32 +169,23 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     if (j + 2 <= m) { eval_rows<2, DT>(e, eek, warp * 32, zb, list + j, s_zz, cand, lane); j += 2; }
     if (j < m) eval_rows<1, DT>(e, eek, warp * 32, zb, list + j, s_zz, cand, lane);
     __syncthreads();
-    // winner per row: lexicographic minimum over the warps' candidates; no finite distance -> code 0, as in the
-    // per-row and all-FP32 kernels
+    // winner per row: lexicographic minimum over the warps' candidates
     for (int r = tid; r < cnt; r += nt) {
       unsigned long long best = ~0ull;
       for (int w = 0; w < nw; ++w) best = min(best, s_cand[w * SB + r]);
-      const int bidx = (uint32_t)(best >> 32) >= KEY_INF ? 0 : (int)(uint32_t)best;
+      const int bidx = packed_winner(best);
       s_bidx[r] = bidx;
       idx_out[rows[r]] = (int64_t)bidx;
       if (train) atomicAdd(s_hist + bidx, 1u);
     }
     __syncthreads();
-    // z_q (and SSE) of the batch's rows as vq_simt_fp32.cu's epilogue computes them: every thread a few
-    // (row, 4-column) items, their loads independent
+    // z_q (and SSE) of the batch's rows: every thread a few (row, 4-column) items, their loads independent
     double lsse = 0.0;
 #pragma unroll 4
     for (int p = tid; p < cnt * C4; p += nt) {
       const int r = p / C4, c = (p - r * C4) * 4;
-      const float4 e4 = ldg4(E + (int64_t)s_bidx[r] * DT + c);
-      float4 o4 = e4;
-      if (train) {
-        const float4 z4 = zld4(zb + r * DT + c);
-        const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
-        const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
-        lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
-        o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
-      }
+      float4 o4 = ldg4(E + (int64_t)s_bidx[r] * DT + c);
+      if (train) o4 = st_step4(o4, zld4(zb + r * DT + c), lsse);
       zst4(zq + (int64_t)rows[r] * DT + c, o4);
     }
     if (train) {
@@ -232,15 +203,14 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
 
 template <int DT, typename ZT>
 int launch_stationary_dt(const ZT* z, const float* E, const float* ee, int K, int train, ZT* z_q, int64_t* idx,
-                         unsigned long long* hist, double* sse, const int* row_list, const int* cand_list, const int* n_list,
-                         int sm_count, cudaStream_t s) {
+                         unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
   auto kern = vq_refine_stationary_kernel<DT, ZT>;
   const int threads = K;   // one warp per 32-code sub-chunk
   const size_t bytes = (size_t)2 * SB * DT * sizeof(ZT) + (size_t)(K / 32) * SB * sizeof(unsigned long long);
   DVQ_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   int per_sm = 0;   // small codebooks (few warps) fit several CTAs per SM
   DVQ_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, bytes));
-  kern<<<sm_count * (per_sm > 0 ? per_sm : 1), threads, bytes, s>>>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list);
+  kern<<<sm_count * (per_sm > 0 ? per_sm : 1), threads, bytes, s>>>(z, E, ee, K, train, z_q, idx, hist, sse, list);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;
@@ -248,13 +218,12 @@ int launch_stationary_dt(const ZT* z, const float* E, const float* ee, int K, in
 
 template <typename ZT>
 int launch_stationary_t(const ZT* z, const float* E, const float* ee, int K, int D, int train, ZT* z_q, int64_t* idx,
-                        unsigned long long* hist, double* sse, const int* row_list, const int* cand_list, const int* n_list,
-                        int sm_count, cudaStream_t s) {
+                        unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
   switch (D) {
-    case 16: return launch_stationary_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, sm_count, s);
-    case 32: return launch_stationary_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, sm_count, s);
-    case 64: return launch_stationary_dt<64>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, sm_count, s);
-    case 128: return launch_stationary_dt<128>(z, E, ee, K, train, z_q, idx, hist, sse, row_list, cand_list, n_list, sm_count, s);
+    case 16: return launch_stationary_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
+    case 32: return launch_stationary_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
+    case 64: return launch_stationary_dt<64>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
+    case 128: return launch_stationary_dt<128>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
     default: return fail(DVQ_ERR_BAD_SHAPE, "code-stationary refine kernel is instantiated for e_dim 16..128 only");
   }
 }
@@ -270,7 +239,7 @@ bool vq_refine_stationary_supported(int K, int D) {
     case 128: max_warps = stationary_max_warps<128>(); break;
     default: return false;
   }
-  return vq_tc_cand_gshift(K) == 0 && K % 32 == 0 && K >= 32 && K / 32 <= max_warps;
+  return !cand_list_mode(K) && K % 32 == 0 && K >= 32 && K / 32 <= max_warps;
 }
 
 // Where the automatic choice takes it: K >= 128 (e_dim <= 64) and K = 256 at e_dim 128, the shapes where it measured faster
@@ -280,8 +249,7 @@ bool vq_refine_stationary_supported(int K, int D) {
 bool vq_refine_stationary_default(int K, int D) { return vq_refine_stationary_supported(K, D) && K >= (D <= 64 ? 128 : 256); }
 
 int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                                unsigned long long* hist, double* sse, const int* row_list, const int* cand_list,
-                                const int* n_list, bool zbf, cudaStream_t s) {
+                                unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {
   if (!vq_refine_stationary_supported(K, D))
     return fail(DVQ_ERR_BAD_SHAPE, "code-stationary refine: K=%d, e_dim %d does not fit (mask-mode K with K/32 warps x e_dim registers)", K, D);
   DeviceProps dp;
@@ -289,9 +257,9 @@ int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, 
   if (rc) return rc;
   if (zbf)
     return launch_stationary_t(static_cast<const __nv_bfloat16*>(z), E, ee, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist,
-                               sse, row_list, cand_list, n_list, dp.sm_count, s);
-  return launch_stationary_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, row_list,
-                             cand_list, n_list, dp.sm_count, s);
+                               sse, list, dp.sm_count, s);
+  return launch_stationary_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list,
+                             dp.sm_count, s);
 }
 
 }  // namespace dvq

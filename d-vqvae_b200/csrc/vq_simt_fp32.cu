@@ -6,15 +6,14 @@
 // the tcgen05 path — the same kernel driven by a device-side list of rows the tensor-core
 // filter could not decide rigorously.
 //
-// Numerics (SURVEY §0.4): per (row, code) dot = sequential fmaf over d = 0..D-1 in FP32,
-// zz = lane-strided fmaf partials + shuffle tree, d = fl(fl(zz + ee_k) - 2*dot) — the reference's structure —
-// and the winner is the lowest index among exact FP32 ties.
+// Numerics (SURVEY §0.4): the contract of vq_exact.cuh — the reference's structure, the winner is the lowest
+// index among exact FP32 ties.
 //
 // Tiling: CTA = 256 threads, 128 rows x 128 codes x 16-wide D chunks; each thread owns an
 // 8x8 register tile split 4+4 (rows ty*4.., 64+ty*4..; codes tx*4.., 64+tx*4..) so every
 // shared-memory read is a conflict-free 128-bit load.  Roofline: FP32 FMA pipe
 // (2*N*K*D flop); it is the *fallback*, the tensor path is the fast one.
-#include "dvq_common.cuh"
+#include "vq_exact.cuh"
 
 namespace dvq {
 
@@ -76,11 +75,7 @@ vq_simt_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const floa
     // for the main loop below)
     for (int r = warp; r < BM; r += NTHREADS / 32) {
       const int64_t grow = srow[r];
-      float s2 = 0.f;
-      if (grow >= 0) {
-        const ZT* zrow = z + grow * (int64_t)D;
-        for (int c = lane; c < D; c += 32) { const float v = zf(__ldg(zrow + c)); s2 = fmaf(v, v, s2); }
-      }
+      float s2 = grow >= 0 ? sq_partial_ldg(z + grow * (int64_t)D, D, lane) : 0.f;
       s2 = warp_sum(s2);
       if (lane == 0) szz[r] = s2;
     }
@@ -141,8 +136,7 @@ vq_simt_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const floa
           const float eev = __ldg(ee + c);
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
-            const float t = __fadd_rn(zz[i], eev);
-            const float dist = __fmaf_rn(-2.0f, acc[i][j], t);  // == fl(t - 2*dot): 2*dot is exact
+            const float dist = exact_dist(acc[i][j], zz[i], eev);
             if (dist < best[i]) { best[i] = dist; bidx[i] = c; }
           }
         }
@@ -176,27 +170,14 @@ vq_simt_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const floa
       ZT* orow = zq + grow * (int64_t)D;
       if (VEC) {
         for (int c = lane * 4; c < D; c += 128) {
-          const float4 e4 = ldg4(erow + c);
-          float4 o4 = e4;
-          if (train) {
-            const float4 z4 = zldg4(zrow + c);
-            const float dx = __fsub_rn(e4.x, z4.x), dy = __fsub_rn(e4.y, z4.y);
-            const float dz = __fsub_rn(e4.z, z4.z), dw = __fsub_rn(e4.w, z4.w);
-            lsse += (double)dx * dx + (double)dy * dy + (double)dz * dz + (double)dw * dw;
-            o4 = make_float4(__fadd_rn(z4.x, dx), __fadd_rn(z4.y, dy), __fadd_rn(z4.z, dz), __fadd_rn(z4.w, dw));
-          }
+          float4 o4 = ldg4(erow + c);
+          if (train) o4 = st_step4(o4, zldg4(zrow + c), lsse);
           zst4(orow + c, o4);
         }
       } else {
         for (int c = lane; c < D; c += 32) {
-          const float e1 = __ldg(erow + c);
-          float o1 = e1;
-          if (train) {
-            const float z1 = zf(__ldg(zrow + c));
-            const float dx = __fsub_rn(e1, z1);
-            lsse += (double)dx * dx;
-            o1 = __fadd_rn(z1, dx);
-          }
+          float o1 = __ldg(erow + c);
+          if (train) o1 = st_step1(o1, zf(__ldg(zrow + c)), lsse);
           zst1(orow + c, o1);
         }
       }
@@ -224,10 +205,7 @@ __global__ void code_norms_kernel(const float* __restrict__ E, int K, int D, flo
   // one warp per code: lane-strided fmaf partials, then a shuffle tree
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= K) return;
-  const float* row = E + (int64_t)warp * D;
-  float s = 0.f;
-  for (int c = lane; c < D; c += 32) { const float v = __ldg(row + c); s = fmaf(v, v, s); }
-  s = warp_sum(s);
+  const float s = warp_sum(sq_partial_ldg(E + (int64_t)warp * D, D, lane));
   if (lane == 0) ee[warp] = s;
 }
 }  // namespace

@@ -118,11 +118,10 @@ struct TcParams {
   int64_t* idx;
   unsigned long long* hist;
   double* sse;
-  int* counters;   // [0] refine-list length, [1] protocol error code
+  int* counters;        // CounterSlot (dvq_common.cuh)
   int* row_list;
-  int* cand_list;       // candidates of each listed row: group mask (bit g = codes [32*g<<gshift, ...)) or sub-chunk list
+  int* cand_list;       // candidate record of each listed row (dvq_common.cuh)
   int layout_ovr;       // smem_layout override (0 = automatic)
-  int cand_gshift;      // 0: mask mode (bit g = sub-chunk g); -1: list mode (see cand_union)
   unsigned long long* stats;   // optional wait-time accounting (DVQ_TC_STATS builds)
   int64_t ntiles;
 };
@@ -276,14 +275,14 @@ __global__ void tc_cb_stats_kernel(const float* __restrict__ ee, int K, int D, C
     c.delta_max = 0.f;
     c.magic = cb_magic(K, D, pair);
     *cb = c;
-    for (int i = 0; i < 64; ++i) counters[i] = 0;
+    for (int i = 0; i < CNT_WORDS; ++i) counters[i] = 0;
   }
 }
 
 // per-call reset when the codebook preparation is reused (DVQ_CODEBOOK_CACHED)
 __global__ void tc_reset_kernel(int* __restrict__ counters, int* __restrict__ zero_ints, int zero_n) {
   for (int i = threadIdx.x; i < zero_n; i += blockDim.x) zero_ints[i] = 0;
-  if (threadIdx.x < 64) counters[threadIdx.x] = 0;
+  if (threadIdx.x < CNT_WORDS) counters[threadIdx.x] = 0;
 }
 
 // byte offset of element (code k, column d) in the global operand image: one block per (256-code chunk,
@@ -507,11 +506,11 @@ struct RowState {   // per (row, column subset) running result of the filter
 };
 // Record that sub-chunk `gbit` held a key inside the band.  Mask mode: set its bit.  List mode: push its 10-bit entry
 // (newest in the low bits) and count; with more than three pushes the oldest entry has been shifted out and the
-// record becomes CAND_OVERFLOW when the tile is finished (filter_tile) — two predicated instructions per sub-chunk
+// record becomes CAND_LIST_OVERFLOW when the tile is finished (filter_tile) — two predicated instructions per sub-chunk
 // instead of the branchy cand_union, which is kept for the once-per-tile merge of the warps' records.
 template <bool LIST>
 __device__ __forceinline__ void cand_push(RowState& st, uint32_t gbit) {
-  if (LIST) { st.cand = (st.cand << 10) | gbit; ++st.ncand; }
+  if (LIST) { st.cand = (st.cand << CAND_ENTRY_BITS) | gbit; ++st.ncand; }
   else st.cand |= gbit;
 }
 // code index of a set bit of the mask (for a decided row the only set bit is the minimum itself)
@@ -520,17 +519,15 @@ __device__ __forceinline__ int row_state_col(const RowState& st) {
   return st.col0 + (zc < 16 ? 2 * zc : 2 * zc - 31);
 }
 
-// Candidate record of a row.  Mask mode (K <= 992): bit g <-> 32-code sub-chunk g held a key inside the band.
-// List mode (larger codebooks, where 31 bits would be too coarse): up to three 10-bit entries (sub-chunk index
-// + 1, 0 = empty, packed from the low bits); CAND_OVERFLOW = more than three -> the refine scans every code.
-constexpr uint32_t CAND_OVERFLOW = 0x3fffffffu;
+// Union of two candidate records (format: dvq_common.cuh); in list mode more than three entries become CAND_LIST_OVERFLOW.
 template <bool LIST>
 __device__ __forceinline__ uint32_t cand_union(uint32_t a, uint32_t b) {
   if (!LIST) return a | b;
-  if (a == CAND_OVERFLOW || b == CAND_OVERFLOW) return CAND_OVERFLOW;
-  const int na = a == 0u ? 0 : (a < 1024u ? 1 : (a < (1u << 20) ? 2 : 3));
-  const int nb = b == 0u ? 0 : (b < 1024u ? 1 : (b < (1u << 20) ? 2 : 3));
-  return na + nb > 3 ? CAND_OVERFLOW : (a | (b << (10 * na)));
+  if (a == CAND_LIST_OVERFLOW || b == CAND_LIST_OVERFLOW) return CAND_LIST_OVERFLOW;
+  constexpr uint32_t one = 1u << CAND_ENTRY_BITS, two = 1u << (2 * CAND_ENTRY_BITS);
+  const int na = a == 0u ? 0 : (a < one ? 1 : (a < two ? 2 : 3));
+  const int nb = b == 0u ? 0 : (b < one ? 1 : (b < two ? 2 : 3));
+  return na + nb > 3 ? CAND_LIST_OVERFLOW : (a | (b << (CAND_ENTRY_BITS * na)));
 }
 
 // packed f32x2 helpers (Blackwell FFMA2: two FP32 FMAs per issued instruction)
@@ -701,7 +698,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
   uint32_t bar0, smem0;
   asm volatile("mov.u32 %0, %1;" : "=r"(bar0) : "r"(tc::smem_u32(ctl.bars)));
   asm volatile("mov.u32 %0, %1;" : "=r"(smem0) : "r"(tc::smem_u32(smem)));
-  int* const err_out = p.counters + 1;
+  int* const err_out = p.counters + CNT_ERROR;
 
   const int D = DT > 0 ? DT : p.D;
   const int K = p.K;
@@ -761,7 +758,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
   // members when they are uneven (it also merges, writes idx and the histogram).  The sub-chunk loop is kept
   // rolled so that the filter stays inside the instruction cache; the TMEM-load latency is covered by the other
   // warps of the sub-partition.  Mask mode: one candidate bit per 32-code sub-chunk (K <= 992, see
-  // vq_tc_cand_gshift); list mode: sub-chunk index + 1.
+  // cand_list_mode); list mode: sub-chunk index + 1.
   auto filter_tile = [&](int64_t it, uint32_t& q, int wq, int r, RowState& st, float& band) {
     const uint32_t lane_addr = (uint32_t)(r & ~31) << 16;
     st.m1 = __uint_as_float(0x7f800000u); st.cnt = 0; st.bits = 0u; st.col0 = 0; st.cand = 0u; st.ncand = 0;
@@ -821,7 +818,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
       }
       if (wq == 1 && r < 32) TRACE(2, 3, c & 1);   // (stats builds) after the stage was handed back
     }
-    if (LIST && st.ncand > 3) st.cand = CAND_OVERFLOW;   // an entry was shifted out: the refine scans every code of this row
+    if (LIST && st.ncand > 3) st.cand = CAND_LIST_OVERFLOW;   // an entry was shifted out: the refine scans every code of this row
   };
   // a helper hands its partial result of the tile to the owner warp of the same rows (single slot per helper)
   auto helper_handoff = [&](int64_t it, int wq, int r, const RowState& st) {
@@ -1271,14 +1268,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
         }
         if (it + 1 < my_tiles) nb_arrive(NB_FIN_EMPTY, NB_FIN_THREADS);
         flag = flag || (cnt > 0);
-        if (band < 0.f) { flag = true; cand = LIST ? CAND_OVERFLOW : 0x7fffffffu; }   // degenerate row: every code is a candidate
+        if (band < 0.f) { flag = true; cand = LIST ? CAND_LIST_OVERFLOW : CAND_MASK_ALL; }   // degenerate row: every code is a candidate
         const bool valid = r < rows;
         flag = flag && valid;
         if (it >= 2) { STAT_T0(); nb_sync(NB_SIDX_EMPTY + slot, NB_SIDX_THREADS); STAT_ADD(3); }
         // code for the gather warps: byte offset of the code row in E, or — sign bit set — "undecided" with the
         // candidate-group mask in the low 31 bits (the gather warps append such rows to the refine list; the
         // exact kernel rewrites their z_q row and accounts their SSE / histogram contribution)
-        reinterpret_cast<int*>(smem + L.sidx)[slot * TM + r] = flag ? (int)(cand | 0x80000000u) : col * D * 4;
+        reinterpret_cast<int*>(smem + L.sidx)[slot * TM + r] = flag ? (int)(cand | CAND_UNDECIDED) : col * D * 4;
         nb_arrive(NB_SIDX_FULL + slot, NB_SIDX_THREADS);
         if (w == 0) TRACE(1, 3, 0);
         if (valid && !flag) {
@@ -1348,23 +1345,23 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
         // against the whole codebook (a one-warp scan of a large codebook would take milliseconds).
         const int code = reinterpret_cast<const int*>(smem + L.sidx)[slot * TM + gw * rows_per_warp + lane];
         const bool und = code < 0 && lane < rows_per_warp && gw * rows_per_warp + lane < rows;
-        const bool ovf = LIST && und && ((uint32_t)code & CAND_OVERFLOW) == CAND_OVERFLOW;
+        const bool ovf = LIST && und && ((uint32_t)code & CAND_LIST_OVERFLOW) == CAND_LIST_OVERFLOW;
         const unsigned bal = __ballot_sync(0xffffffffu, und && !ovf);
         if (bal) {
           int base = 0;
-          if (lane == 0) base = atomicAdd(p.counters, __popc(bal));
+          if (lane == 0) base = atomicAdd(p.counters + CNT_LISTED, __popc(bal));
           base = __shfl_sync(0xffffffffu, base, 0);
           if (und && !ovf) {
             const int pos = base + __popc(bal & ((1u << lane) - 1u));
             p.row_list[pos] = (int)(row0 + gw * rows_per_warp + lane);
-            p.cand_list[pos] = code & 0x7fffffff;
+            p.cand_list[pos] = (int)((uint32_t)code & ~CAND_UNDECIDED);
           }
         }
         if (LIST) {
           const unsigned bal2 = __ballot_sync(0xffffffffu, ovf);
           if (bal2) {
             int base = 0;
-            if (lane == 0) base = atomicAdd(p.counters + 2, __popc(bal2));
+            if (lane == 0) base = atomicAdd(p.counters + CNT_OVF, __popc(bal2));
             base = __shfl_sync(0xffffffffu, base, 0);
             if (ovf) p.row_list[p.N - 1 - (base + __popc(bal2 & ((1u << lane) - 1u)))] = (int)(row0 + gw * rows_per_warp + lane);
           }
@@ -1578,10 +1575,6 @@ void vq_tc_layout_info(int K, int D, int* out8, int zbytes) {
   out8[6] = (int)L.total + 128; out8[7] = (int)L.hist_in_smem;
 }
 
-int vq_tc_cand_gshift(int K) {   // 31 candidate bits (bit 31 is the "undecided" flag of the hand-off word), one per 32-code sub-chunk
-  return K <= 992 ? 0 : -1;      // -1 = list mode: up to three exact sub-chunk indices instead of a mask
-}
-
 size_t vq_tc_operand_bytes(int K, int D) {
   const SmemLayout L = smem_layout(K, D);
   return align_up(sizeof(CbMeta), 256) + align_up((size_t)((K + 255) / 256) * L.ns * L.bchunk_bytes, 256);
@@ -1644,9 +1637,9 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
     if (rc) return rc;
   }
   p.z = z; p.E = E; p.bimg = bimg; p.cb = cb; p.N = N; p.K = K; p.D = D; p.train = train;
-  p.zq = z_q; p.idx = idx; p.hist = hist; p.sse = sse; p.counters = counters; p.row_list = row_list; p.cand_list = cand_list; p.cand_gshift = vq_tc_cand_gshift(K);
+  p.zq = z_q; p.idx = idx; p.hist = hist; p.sse = sse; p.counters = counters; p.row_list = row_list; p.cand_list = cand_list;
   p.layout_ovr = pair ? pair_ovr : ovr;
-  p.stats = reinterpret_cast<unsigned long long*>(counters + 8);
+  p.stats = reinterpret_cast<unsigned long long*>(counters + CNT_STATS);
   p.ntiles = (N + TM - 1) / TM;
   const size_t smem = L.total + 128;
   int64_t grid = p.ntiles < dp.sm_count ? p.ntiles : dp.sm_count;
@@ -1692,7 +1685,7 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
   // two-sub-chunk filter with the epilogue-heavy register split (DVQ_TC_ST=1; streamed codebooks only).  Measured
   // within +-2 % of the default at every K >= 2048 shape of the sweep, so it is not selected automatically.
   const bool st = !zbf && streamed && st_env && st_env[0] == '1';
-  const bool list = p.cand_gshift < 0;
+  const bool list = cand_list_mode(K);
   if (zbf) {
     if (D == 64 && !list && !streamed) {
       if (train) DVQ_LAUNCH_TC(64, true, false, false, false, __nv_bfloat16); else DVQ_LAUNCH_TC(64, false, false, false, false, __nv_bfloat16);

@@ -391,44 +391,63 @@ def test_degenerate_rows_and_duplicate_codes_take_the_exact_path(K, D):
     assert np.array_equal(out["tc"][1].view(np.uint32), out["simt"][1].view(np.uint32))
 
 
+def _bits_equal_nan(a, b):
+    """Bit equality of two uint32 views of fp32 arrays; positions where both are NaN count as equal."""
+    nan_a, nan_b = np.isnan(a.view(np.float32)), np.isnan(b.view(np.float32))
+    return np.array_equal(nan_a, nan_b) and np.array_equal(a[~nan_a], b[~nan_b])
+
+
 @pytest.mark.parametrize("K,D", [(512, 64), (2048, 64), (1024, 256), (128, 256)])
 def test_refine_variants_give_identical_results(K, D):
-    """The exact refine stage of the tcgen05 path has two implementations (one warp per undecided row;
-    (row, sub-chunk) pairs bucketed by sub-chunk) plus a device-side hand-back from the second to the first
-    when the pair list overflows.  All three must produce the same idx / z_q / histogram bit for bit — they
-    evaluate the same FP32 expression and take the same lexicographic (distance, code) minimum — and equal
-    the all-FP32 kernel.  Input: default-init codebook (a few % undecided rows) plus zero / huge rows (paired
-    with every sub-chunk)."""
+    """The exact refine stage of the tcgen05 path has three implementations (one warp per undecided row;
+    (row, sub-chunk) pairs bucketed by sub-chunk; code-stationary, for the mask-mode shapes it covers) plus a
+    device-side hand-back from the binned kernels to the per-row kernel when the pair list overflows.  All must
+    produce the same idx / z_q / histogram bit for bit — they evaluate the same FP32 expression and take the same
+    lexicographic (distance, code) minimum — and equal the all-FP32 kernel.  Inputs: default-init codebook (a few %
+    undecided rows) plus zero / huge rows (paired with every sub-chunk); and the same rows with some made non-finite
+    (+inf, -inf, a single NaN element), whose distances are NaN or inf on every code."""
     from dvq import _cabi
     N = 50000 + 13
     E = vo.default_codebook(K, D, 41)
     z = vo.normal_latents(N, D, 42)
     z[::211] = 0.0
     z[3::307] *= 1e18
-    zt = torch.from_numpy(z).cuda()
+    z_nf = z.copy()
+    z_nf[11::401] = np.inf
+    z_nf[13::409, 3] = np.nan
+    z_nf[17::419, :2] = -np.inf
+    inputs = {"finite": torch.from_numpy(z).cuda(), "nonfinite": torch.from_numpy(z_nf).cuda()}
+    arms = [("simt", _cabi.DVQ_PATH_SIMT, 0, 0), ("per_row", _cabi.DVQ_PATH_TC, 1, 0), ("binned", _cabi.DVQ_PATH_TC, 2, 0),
+            ("handback", _cabi.DVQ_PATH_TC, 2, 64)]
+    if (K, D) == (512, 64):                                        # the one shape here the code-stationary kernel covers
+        arms.append(("stationary", _cabi.DVQ_PATH_TC, 3, 0))
     res = {}
     try:
-        for name, path, mode, cap in (("simt", _cabi.DVQ_PATH_SIMT, 0, 0), ("per_row", _cabi.DVQ_PATH_TC, 1, 0),
-                                      ("binned", _cabi.DVQ_PATH_TC, 2, 0), ("handback", _cabi.DVQ_PATH_TC, 2, 64)):
+        for name, path, mode, cap in arms:
             _cabi.check(_cabi.lib.dvq_vq_set_refine(mode, cap), "dvq_vq_set_refine")
             m = _module(E, 1.0, 0.25, path)
             m.onehot_limit_bytes = 0
-            with torch.no_grad():
-                loss, zq, ppl, _, idx = m(zt, True)
-            n_ref, err = m.last_counters(N)
-            assert err == 0
-            if name != "simt":
-                assert n_ref > 0                                   # the refine stage did run
-            res[name] = (idx.cpu().numpy().reshape(-1), zq.cpu().numpy().view(np.uint32), m.last_stats[:K].cpu().numpy(),
-                         loss.item(), ppl.item())
+            for which, zt in inputs.items():
+                with torch.no_grad():
+                    loss, zq, ppl, _, idx = m(zt, True)
+                n_ref, err = m.last_counters(N)
+                assert err == 0
+                if name != "simt":
+                    assert n_ref > 0                               # the refine stage did run
+                res[name, which] = (idx.cpu().numpy().reshape(-1), zq.cpu().numpy().view(np.uint32), m.last_stats[:K].cpu().numpy(),
+                                    loss.item(), ppl.item())
     finally:
         _cabi.check(_cabi.lib.dvq_vq_set_refine(0, 0), "dvq_vq_set_refine")
-    for name in ("binned", "handback"):
-        assert np.array_equal(res[name][0], res["per_row"][0]), name
-        assert np.array_equal(res[name][1], res["per_row"][1]), name
-        assert np.array_equal(res[name][2], res["per_row"][2]), name
-        assert rel_err(res[name][3], res["per_row"][3]) < 1e-7 and rel_err(res[name][4], res["per_row"][4]) < 1e-7
-    n_mis, n_bad, worst = vo.allowed_index_mismatch(z, E, res["binned"][0], res["simt"][0])
+    for name in [a[0] for a in arms if a[0] not in ("simt", "per_row")]:
+        for which in inputs:
+            got, want = res[name, which], res["per_row", which]
+            assert np.array_equal(got[0], want[0]), (name, which)
+            assert _bits_equal_nan(got[1], want[1]), (name, which)
+            assert np.array_equal(got[2], want[2]), (name, which)
+            assert rel_err(got[4], want[4]) < 1e-7
+        got, want = res[name, "finite"], res["per_row", "finite"]
+        assert rel_err(got[3], want[3]) < 1e-7                      # (the SSE of a non-finite row is NaN)
+    n_mis, n_bad, worst = vo.allowed_index_mismatch(z, E, res["binned", "finite"][0], res["simt", "finite"][0])
     assert n_bad == 0, (n_mis, worst)
 
 
