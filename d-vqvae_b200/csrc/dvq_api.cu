@@ -435,6 +435,47 @@ int dvq_mano_backward(const DvqManoModel* model, const float* betas, const float
                               grad_hand_pose, grad_transl, static_cast<cudaStream_t>(stream));
 }
 
+// the contact kernels index within a call in 32 bits: every [B, n, 3] tensor they touch must have fewer than 2^31 elements
+static int check_nn_shape(int B, int N1, int N2) {
+  if (B < 0 || N1 < 0 || N2 <= 0) return fail(DVQ_ERR_BAD_SHAPE, "need B >= 0, N1 >= 0, N2 > 0 (got B=%d N1=%d N2=%d)", B, N1, N2);
+  if ((long long)B * (N1 > N2 ? N1 : N2) * 3 >= (1LL << 31))
+    return fail(DVQ_ERR_BAD_SHAPE, "B * max(N1, N2) * 3 = %lld must be below 2^31; split the batch", (long long)B * (N1 > N2 ? N1 : N2) * 3);
+  return DVQ_OK;
+}
+
+int dvq_nn_forward(const float* src, const float* trg, int B, int N1, int N2, const float* trg_normals, float* dist, int64_t* idx,
+                   uint8_t* interior, void* stream) {
+  int rc = check_nn_shape(B, N1, N2);
+  if (rc) return rc;
+  const bool work = (long long)B * N1 > 0;    // empty tensors may have NULL data pointers
+  if (work && (!src || !trg || !dist || !idx)) return fail(DVQ_ERR_BAD_ARG, "src, trg, dist and idx must not be NULL");
+  if (work && !trg_normals != !interior) return fail(DVQ_ERR_BAD_ARG, "trg_normals and interior go together (both NULL or both set)");
+  rc = require_sm100();
+  if (rc) return rc;
+  return launch_nn_forward(src, trg, B, N1, N2, trg_normals, dist, idx, interior, static_cast<cudaStream_t>(stream));
+}
+
+int dvq_nn_backward(const float* src, const float* trg, const int64_t* idx, const float* g_dist, int B, int N1, int N2, float* g_src,
+                    float* g_trg, void* stream) {
+  int rc = check_nn_shape(B, N1, N2);
+  if (rc) return rc;
+  if ((long long)B * N1 > 0 && (!src || !trg || !idx || !g_dist)) return fail(DVQ_ERR_BAD_ARG, "src, trg, idx and g_dist must not be NULL");
+  rc = require_sm100();
+  if (rc) return rc;
+  return launch_nn_backward(src, trg, idx, g_dist, B, N1, N2, g_src, g_trg, static_cast<cudaStream_t>(stream));
+}
+
+int dvq_vertex_normals(const float* verts, int B, int V, const int* faces, int F, const int* vf_offsets, const int* vf_faces,
+                       float* normals, void* stream) {
+  if (B < 0 || V <= 0 || F < 0) return fail(DVQ_ERR_BAD_SHAPE, "need B >= 0, V > 0, F >= 0 (got B=%d V=%d F=%d)", B, V, F);
+  if ((long long)B * V * 3 >= (1LL << 31) || (long long)F * 3 >= (1LL << 31))
+    return fail(DVQ_ERR_BAD_SHAPE, "B * V * 3 and F * 3 must be below 2^31; split the batch");
+  if (!vf_offsets || (B > 0 && (!verts || !normals)) || (F > 0 && (!faces || !vf_faces))) return fail(DVQ_ERR_BAD_ARG, "NULL argument");
+  int rc = require_sm100();
+  if (rc) return rc;
+  return launch_vertex_normals(verts, B, V, faces, vf_offsets, vf_faces, normals, static_cast<cudaStream_t>(stream));
+}
+
 int dvq_pcnn_gemm(const DvqPcnnGemm* g, void* stream) {
   int rc = require_sm100();
   if (rc) return rc;

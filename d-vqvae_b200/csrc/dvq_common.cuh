@@ -179,6 +179,14 @@ int launch_mano_backward(const DvqManoModel* m, const float* betas, const float*
                          const float* grad_vertices, const float* grad_joints, float* grad_betas, float* grad_global_orient,
                          float* grad_hand_pose, float* grad_transl, cudaStream_t s);
 
+// hand-object nearest-point search (contact_sm100.cu)
+int launch_nn_forward(const float* src, const float* trg, int B, int N1, int N2, const float* trg_normals, float* dist, int64_t* idx,
+                      uint8_t* interior, cudaStream_t s);
+int launch_nn_backward(const float* src, const float* trg, const int64_t* idx, const float* g_dist, int B, int N1, int N2,
+                       float* g_src, float* g_trg, cudaStream_t s);
+int launch_vertex_normals(const float* verts, int B, int V, const int* faces, const int* vf_offsets, const int* vf_faces,
+                          float* normals, cudaStream_t s);
+
 // PointNet
 size_t pointnet_workspace_bytes(int B, int C, int P, int flags);
 int launch_pointnet(const float* x, const DvqPointNetWeights* w, int B, int C, int P, int flags, float* feat,

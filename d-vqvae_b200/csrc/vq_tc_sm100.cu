@@ -47,6 +47,7 @@
 #include <cstring>
 
 #include "dvq_common.cuh"
+#include "f32x2.cuh"
 #include "tc_prims.cuh"
 
 namespace dvq {
@@ -528,37 +529,6 @@ __device__ __forceinline__ uint32_t cand_union(uint32_t a, uint32_t b) {
   const int na = a == 0u ? 0 : (a < one ? 1 : (a < two ? 2 : 3));
   const int nb = b == 0u ? 0 : (b < one ? 1 : (b < two ? 2 : 3));
   return na + nb > 3 ? CAND_LIST_OVERFLOW : (a | (b << (CAND_ENTRY_BITS * na)));
-}
-
-// packed f32x2 helpers (Blackwell FFMA2: two FP32 FMAs per issued instruction)
-__device__ __forceinline__ uint64_t pack_f32x2(float lo, float hi) {
-  uint64_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ void unpack_f32x2(uint64_t v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ uint64_t ffma2(uint64_t a, uint64_t b, uint64_t c) {
-  uint64_t r;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-  return r;
-}
-// FADD2 / FMUL2: each half is an ordinary IEEE round-to-nearest FP32 operation (no contraction possible)
-__device__ __forceinline__ uint64_t fadd2(uint64_t a, uint64_t b) {
-  uint64_t r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-__device__ __forceinline__ uint64_t fsub2(uint64_t a, uint64_t b) {
-  uint64_t r;
-  asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-__device__ __forceinline__ uint64_t fmul2(uint64_t a, uint64_t b) {
-  uint64_t r;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
 }
 
 // One 32-column sub-chunk of raw accumulators (all >= 0, so float order == bit order):

@@ -67,6 +67,9 @@ SYMBOLS = {
     "dvq_allreduce_stats": (_i, [_vp, _vp, _vp, _i, _vp]),
     "dvq_mano_forward": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "dvq_mano_backward": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dvq_nn_forward": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "dvq_nn_backward": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "dvq_vertex_normals": (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp]),
 }
 
 

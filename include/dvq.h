@@ -248,6 +248,27 @@ DVQ_API int dvq_mano_backward(const DvqManoModel* model, const float* betas, con
                               int B, const float* grad_vertices, const float* grad_joints, float* grad_betas,
                               float* grad_global_orient, float* grad_hand_pose, float* grad_transl, void* stream);
 
+/* ---- hand-object nearest-point search (grasp refinement: pytorch3d knn_points(K=1), Meshes.verts_normals_packed and
+ * GraspTTA's interior test) — the exact FP32 contract is stated in csrc/contact_exact.cuh.
+ * Points are fp32 [B, n, 3], contiguous; item b's src points are searched against item b's trg points only.  Each entry is
+ * an ordinary stream launch (no host synchronisation, no allocation; CUDA-graph capturable).  Shapes: B, N1 >= 0, N2 > 0
+ * (DVQ_ERR_BAD_SHAPE otherwise), and B * max(N1, N2) * 3 < 2^31, which keeps the kernels' index arithmetic in 32 bits.
+ * B = 0 or N1 = 0 launches nothing. */
+/* src [B,N1,3], trg [B,N2,3] -> dist [B,N1] (squared distance to the nearest trg point), idx [B,N1] (its index, lowest
+ * among exact ties); with trg_normals [B,N2,3] (unit vertex normals) also interior [B,N1] (1 when the offset from the src
+ * point to its nearest trg point points along that point's normal), else interior may be NULL. */
+DVQ_API int dvq_nn_forward(const float* src, const float* trg, int B, int N1, int N2, const float* trg_normals, float* dist,
+                           int64_t* idx, uint8_t* interior, void* stream);
+/* Gradient of dist with respect to src and trg, given the forward's idx and the upstream g_dist [B,N1].  g_src [B,N1,3]
+ * and g_trg [B,N2,3] are each written when non-NULL.  Deterministic: g_trg sums in ascending src index, no atomics. */
+DVQ_API int dvq_nn_backward(const float* src, const float* trg, const int64_t* idx, const float* g_dist, int B, int N1, int N2,
+                            float* g_src, float* g_trg, void* stream);
+/* Area-weighted unit vertex normals of a triangle mesh: verts [B,V,3], faces [F,3] (int32 ids in [0, V)), vf_offsets [V+1]
+ * and vf_faces [vf_offsets[V]] list the faces of each vertex in ascending order, once per occurrence -> normals [B,V,3].
+ * Needs V > 0, F >= 0, B * V * 3 < 2^31 and F * 3 < 2^31. */
+DVQ_API int dvq_vertex_normals(const float* verts, int B, int V, const int* faces, int F, const int* vf_offsets,
+                               const int* vf_faces, float* normals, void* stream);
+
 /* Host-buffer (end-to-end) form of the same forward: z_host/E_host/zq_host/idx_host are
  * HOST pointers (pinned for full overlap).  Rows are streamed through the GPU in chunks on
  * three internal streams (H2D, compute, D2H).  loss/perplexity are host floats (train only). */
