@@ -50,7 +50,6 @@ void count_launch(int n) { __atomic_fetch_add(&g_launches, (long long)n, __ATOMI
 
 static int g_refine_mode = 0;            // dvq_vq_set_refine
 static long long g_refine_pair_cap = 0;
-long long refine_pair_cap_override() { return __atomic_load_n(&g_refine_pair_cap, __ATOMIC_RELAXED); }
 
 static const int kStages = 4;
 static const int kProfSlots = 128;  // event pairs per stage between enable and read-out
@@ -240,50 +239,23 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
                         reinterpret_cast<int*>(ws + w.off_binned), (int)(vq_refine_binned_zero_bytes() / sizeof(int)), cached, zbf, s);
       profile_mark(1, false, s);
       if (rc) return rc;
-      // exact FP32 refine of the rows the filter flagged (device-side count, no host sync): restricted to
-      // the recorded candidate groups when that kernel covers the shape, else the full FP32 kernel on the list
-      profile_mark(2, true, s);
-      // (large codebooks: rows with too many candidates for the list record, and degenerate rows, sit in a second
-      //  list stored downwards from the end of the same buffer; both kernels re-evaluate them against every code)
+      // exact FP32 refine of the rows the filter flagged (device-side counts, no host sync), restricted to their recorded
+      // candidate sub-chunks.  Large codebooks: rows with too many candidates for the list record, and degenerate rows,
+      // sit in a second list stored downwards from the end of the same buffer and are re-evaluated against every code.
       const bool list_mode = cand_list_mode(K);
       const RefineList list{row_list, cand_list, counters + CNT_LISTED, list_mode ? row_list + (N - 1) : nullptr,
                             list_mode ? counters + CNT_OVF : nullptr, list_mode};
-      if (vq_refine_supported(K, D)) {
-        // Three exact refine paths with identical results.  The code-stationary kernel (code rows register-resident, one
-        // warp per 32-code sub-chunk, z rows streamed past them) covers mask-mode codebooks whose K/32 warps hold e_dim
-        // floats per lane; the automatic choice takes it where it measured faster than the per-row kernel
-        // (vq_refine_stationary_default: K >= 128 up to e_dim 64, K = 256 at e_dim 128; config 2: 0.077 vs 0.101 ms).
-        // Otherwise the per-row kernel (one warp per undecided row) while the FP32 codebook fits its shared memory
-        // (measured at K = 512, e_dim = 64: 0.105 vs 0.128 ms for 108 k rows against the binned kernels); beyond that the
-        // binned kernels win by 2-5x (code rows register-resident per bucket instead of re-read from L2 per row).  The
-        // binned path hands its list back to the per-row kernel through the hand-back counters when the pairs do not
-        // fit its workspace (normally both stay zero and the per-row kernel exits at once).  dvq_vq_set_refine /
-        // DVQ_REFINE_PER_ROW / DVQ_REFINE_BINNED force one path.
-        static const bool env_per_row = getenv("DVQ_REFINE_PER_ROW") != nullptr;
-        static const bool env_binned = getenv("DVQ_REFINE_BINNED") != nullptr;
-        const int mode = __atomic_load_n(&g_refine_mode, __ATOMIC_RELAXED);
-        const bool force_per_row = env_per_row || mode == 1, force_binned = env_binned || mode == 2;
-        const bool stationary = mode == 3 || (!force_per_row && !force_binned && vq_refine_stationary_default(K, D));
-        const bool per_row_only = force_per_row || (!force_binned && vq_refine_codebook_in_smem(K, D));
-        RefineList handback = list;
-        handback.n = counters + CNT_HANDBACK;
-        if (list_mode) handback.n_ovf = counters + CNT_HANDBACK_OVF;
-        if (stationary)
-          rc = launch_vq_refine_stationary(z, E, ee, K, D, train, z_q, idx, hist, sse, list, zbf, s);
-        else if (!per_row_only)
-          rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list, counters, ws + w.off_binned, zbf, s);
-        if (!rc && !stationary)
-          rc = launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, per_row_only ? list : handback, zbf, s);
-      } else {
-        rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list.rows, list.n, 1, zbf, s);
-        if (!rc && list_mode)
-          rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list.ovf_last, list.n_ovf, -1, zbf, s);
-      }
+      // a mode set by dvq_vq_set_refine wins; under mode 0, DVQ_REFINE_PER_ROW (any value) selects the per-row kernel
+      static const int env_mode = getenv("DVQ_REFINE_PER_ROW") != nullptr ? 1 : 0;
+      const int set_mode = __atomic_load_n(&g_refine_mode, __ATOMIC_RELAXED);
+      profile_mark(2, true, s);
+      rc = launch_vq_refine_stage(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list, counters, ws + w.off_binned,
+                                  set_mode != 0 ? set_mode : env_mode, __atomic_load_n(&g_refine_pair_cap, __ATOMIC_RELAXED), zbf, s);
       profile_mark(2, false, s);
       if (rc) return rc;
     } else {
       profile_mark(1, true, s);
-      rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, nullptr, nullptr, 1, zbf, s);
+      rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, zbf, s);
       profile_mark(1, false, s);
       if (rc) return rc;
     }

@@ -111,12 +111,10 @@ struct RefineList {
 // ee[k] = sum_d E[k,d]^2
 int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s);
 
-// Exact FP32 CUDA-core path.  row_list == nullptr: rows [0,N).  Otherwise rows
-// row_list[0 .. *n_list) (device-side count), used as the refine stage of the tcgen05 path.
+// Exact FP32 CUDA-core path over rows [0, N): every shape, the path when the tcgen05 kernel does not run.
 // zbf: z / z_q are bf16 rows (DVQ_Z_BF16), else fp32 — every VQ kernel below computes in fp32 on the upcast rows
 int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse,
-                   const int* row_list, const int* n_list, int list_stride, bool zbf, cudaStream_t s);
+                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse, bool zbf, cudaStream_t s);
 
 // tcgen05 filter kernel (vq_tc_sm100.cu); supported(K,D) says whether the shape is handled.
 bool vq_tc_supported(int64_t N, int K, int D);
@@ -130,27 +128,27 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
                  void* bop, int* counters, int* row_list, int* cand_list, int* zero_ints, int zero_n,
                  bool codebook_cached, bool zbf, cudaStream_t s);
 
-// candidate-restricted exact refine (vq_refine.cu): one warp per listed row
-bool vq_refine_supported(int K, int D);
-bool vq_refine_codebook_in_smem(int K, int D);
-int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                     unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s);
+// The exact refine stage of the tcgen05 path (vq_refine.cu): re-evaluates the rows of the filter's refine list with the
+// refine kernels its plan picks for the shape.  mode and pair_cap as in dvq_vq_set_refine (0 = automatic / default);
+// binned_ws: the VqWorkspace::off_binned area.
+int launch_vq_refine_stage(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
+                           int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
+                           void* binned_ws, int mode, long long pair_cap, bool zbf, cudaStream_t s);
 
 // code-stationary exact refine (vq_refine_stationary.cu): mask-mode codebooks whose K/32 warps hold e_dim code floats
 // per lane in registers
 bool vq_refine_stationary_supported(int K, int D);
-bool vq_refine_stationary_default(int K, int D);   // the subset the automatic refine choice gives it (measured faster)
 int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
                                 unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s);
 
-// binned exact refine (vq_refine_binned.cu): (row, sub-chunk) pairs bucketed by sub-chunk; hands the list to
-// launch_vq_refine through counters[CNT_HANDBACK] / [CNT_HANDBACK_OVF] when the pairs do not fit its workspace
-long long refine_pair_cap_override();   // dvq_vq_set_refine (dvq_api.cu); 0 = default
+// binned exact refine (vq_refine_binned.cu): (row, sub-chunk) pairs bucketed by sub-chunk; hands the list to the per-row
+// kernel through counters[CNT_HANDBACK] / [CNT_HANDBACK_OVF] when the pairs do not fit min(pair_cap, 2 N) (pair_cap 0:
+// 2 N, the workspace's capacity)
 size_t vq_refine_binned_bytes(int64_t N);
 size_t vq_refine_binned_zero_bytes();
 int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
                             int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
-                            void* ws, bool zbf, cudaStream_t s);
+                            void* ws, long long pair_cap, bool zbf, cudaStream_t s);
 
 int launch_onehot(const int64_t* idx, int64_t N, int K, float* onehot, cudaStream_t s);
 int launch_finalize(const unsigned long long* hist, const double* sse, int64_t N, int K, int D, float al,
@@ -225,6 +223,25 @@ __device__ __forceinline__ void zstcs4(float* p, float4 v) { __stcs(reinterpret_
 __device__ __forceinline__ void zstcs4(__nv_bfloat16* p, float4 v) { __stcs(reinterpret_cast<uint2*>(p), f4_to_bf4(v)); }
 __device__ __forceinline__ void zst1(float* p, float v) { *p = v; }
 __device__ __forceinline__ void zst1(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+
+// cp.async global -> shared copies (dst: shared-window address, (uint32_t)__cvta_generic_to_shared(p)): .ca caches in L1,
+// .cg only in L2; with src_bytes (16 or 0) the copy reads that many bytes and zero-fills the rest of the 16.  Completion:
+// cp_async_commit() closes a group, cp_async_wait<N>() waits until at most N of this thread's groups are pending.
+__device__ __forceinline__ void cp_async_ca4(uint32_t dst, const void* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_ca16(uint32_t dst, const void* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_cg16(uint32_t dst, const void* src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_cg16(uint32_t dst, const void* src, uint32_t src_bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

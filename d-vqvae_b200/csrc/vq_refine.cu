@@ -52,10 +52,10 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
 #pragma unroll
       for (int v = lane; v < DT / ZE; v += 32) {
         const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zbuf + buf * DT + v * ZE);
-        asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src + v * ZE) : "memory");
+        cp_async_ca16(dst, src + v * ZE);
       }
     }
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
   };
   // outputs of one row, executed by one warp
   auto emit_row = [&](int64_t row, int bidx, const ZT* zsrc) {
@@ -75,7 +75,7 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
   int buf = 0;
   for (int i = wglobal; i < n; i += wtotal, buf ^= 1) {
     prefetch(i + wtotal, buf ^ 1);
-    asm volatile("cp.async.wait_group 1;" ::: "memory");
+    cp_async_wait<1>();
     __syncwarp();
     const int64_t row = L.rows[i];
     const uint32_t cand = (uint32_t)L.cand[i];
@@ -165,7 +165,7 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
     emit_row(row, packed_winner(best), zbuf + buf * DT);
     __syncwarp();   // everyone is done with zbuf[buf] before the next-but-one prefetch overwrites it
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait<0>();
   // ---- overflow rows (list mode: more than three candidate sub-chunks, degenerate rows): one CTA per row, the
   //      warps split the sub-chunks of the whole codebook, lexicographic (distance, code) minimum across warps ----
   if (L.n_ovf != nullptr) {
@@ -215,18 +215,16 @@ vq_refine_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const fl
 }  // namespace
 
 // true when the per-row kernel can keep the whole FP32 codebook in shared memory (its fast regime)
-bool vq_refine_codebook_in_smem(int K, int D) {
+static bool codebook_in_smem(int K, int D) {
   return (size_t)K * (D + 4) * sizeof(float) + (size_t)(RTHREADS / 32) * 2 * D * sizeof(float) <= 200 * 1024;
 }
-
-bool vq_refine_supported(int K, int D) { return (D == 16 || D == 32 || D == 64 || D == 128 || D == 256 || D == 512) && K >= 32; }
 
 template <int DT, typename ZT>
 static int launch_refine_dt(const ZT* z, const float* E, const float* ee, int K, int train, ZT* z_q, int64_t* idx,
                             unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
   const size_t zbuf_bytes = (size_t)(RTHREADS / 32) * 2 * DT * sizeof(ZT);
   const size_t smem_e = (size_t)K * (DT + 4) * sizeof(float);
-  const bool in_smem = vq_refine_codebook_in_smem(K, DT);
+  const bool in_smem = codebook_in_smem(K, DT);
 #define DVQ_LAUNCH_REFINE(TR_, SM_)                                                                                      \
   do {                                                                                                                   \
     const size_t bytes = zbuf_bytes + (SM_ ? smem_e : 0);                                                                \
@@ -255,8 +253,8 @@ static int launch_refine_t(const ZT* z, const float* E, const float* ee, int K, 
   }
 }
 
-int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                     unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {
+static int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
+                            unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
@@ -264,6 +262,35 @@ int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int 
     return launch_refine_t(static_cast<const __nv_bfloat16*>(z), E, ee, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
                            list, dp, s);
   return launch_refine_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list, dp, s);
+}
+
+// The refine plan.  The three refine kernels give identical results; the automatic choice (mode 0) takes the one that
+// measured fastest for the shape (NVIDIA B200, 1000 W power limit, refine stage):
+//  - code-stationary (code rows register-resident, one warp per 32-code sub-chunk, z rows streamed past them) where it covers
+//    the shape and K >= 128 up to e_dim 64, K >= 256 at e_dim 128: N = 4M, K = 512 / e_dim 64 (config 2) 0.077 vs 0.101 ms
+//    for the per-row kernel, K = 128 / e_dim 64 0.062 vs 0.077, K = 256 / e_dim 128 0.149 vs 0.185.  With fewer sub-chunks a
+//    CTA has too few warps to hide the FMA chains' latency (K = 64 / e_dim 64: 0.072 vs 0.065 ms; K = 128 / e_dim 128: 0.169
+//    vs 0.162 ms);
+//  - otherwise per-row (one warp per listed row) while the FP32 codebook fits its shared memory: K = 512 / e_dim 64, 108 k
+//    rows, 0.105 vs 0.128 ms for the binned kernels;
+//  - otherwise binned, 2-5x faster than per-row reading its code rows from L2 (code rows register-resident per bucket).  The
+//    per-row kernel then runs on the hand-back list, which the binned kernels fill when their pairs do not fit the pair list
+//    (normally both hand-back counts stay zero and it exits at once).
+int launch_vq_refine_stage(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
+                           int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
+                           void* binned_ws, int mode, long long pair_cap, bool zbf, cudaStream_t s) {
+  if (mode == 0) {
+    const bool stationary = vq_refine_stationary_supported(K, D) && K >= (D <= 64 ? 128 : 256);
+    mode = stationary ? 3 : codebook_in_smem(K, D) ? 1 : 2;
+  }
+  if (mode == 3) return launch_vq_refine_stationary(z, E, ee, K, D, train, z_q, idx, hist, sse, list, zbf, s);
+  if (mode == 1) return launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, list, zbf, s);
+  const int rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list, counters, binned_ws, pair_cap, zbf, s);
+  if (rc) return rc;
+  RefineList handback = list;
+  handback.n = counters + CNT_HANDBACK;
+  if (list.list_mode) handback.n_ovf = counters + CNT_HANDBACK_OVF;
+  return launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, handback, zbf, s);
 }
 
 }  // namespace dvq

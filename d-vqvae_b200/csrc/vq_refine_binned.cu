@@ -258,7 +258,7 @@ refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const
         const bool cv = b * 32 + cl < K;
         const float* src = E + (size_t)(cv ? b * 32 + cl : 0) * D + sl * DS + c4 * 4;
         const uint32_t dst = (uint32_t)__cvta_generic_to_shared(es + cl * EP + c4 * 4);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(cv ? 16 : 0) : "memory");
+        cp_async_cg16(dst, src, cv ? 16 : 0);
       }
     };
     auto stage_z = [&](int64_t row_, int sl, int buf) {
@@ -269,9 +269,9 @@ refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const
         const long long rr = __shfl_sync(0xffffffffu, (long long)row_, r);
         const ZT* src = rr >= 0 ? z + rr * D + sl * DS + c4 * ZE : z;
         const uint32_t dst = (uint32_t)__cvta_generic_to_shared(zs + buf * RB * DS + r * DS + c4 * ZE);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(rr >= 0 ? 16 : 0) : "memory");
+        cp_async_cg16(dst, src, rr >= 0 ? 16 : 0);
       }
-      asm volatile("cp.async.commit_group;" ::: "memory");
+      cp_async_commit();
     };
     int64_t row, row_n;
     float zz, zz_n;
@@ -289,8 +289,8 @@ refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const
         __syncwarp();   // the previous step's reads of the other half are done
         if (sl + 1 < ns) stage_z(row, sl + 1, buf ^ 1);
         else if (p + RB < p1) stage_z(row_n, 0, buf ^ 1);
-        else asm volatile("cp.async.commit_group;" ::: "memory");   // keep one group per step
-        asm volatile("cp.async.wait_group 1;" ::: "memory");         // this step's rows (and code slices) have landed
+        else cp_async_commit();   // keep one group per step
+        cp_async_wait<1>();       // this step's rows (and code slices) have landed
         __syncwarp();
         if (ns > 1) {
           const float* eb = es + lane * EP;
@@ -303,7 +303,7 @@ refine_pairs_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const
                           // the next step's z group, so that step's wait_group 1 covers it)
           if (sl + 1 < ns || p + RB < p1) {
             stage_e(sl + 1 < ns ? sl + 1 : 0);
-            asm volatile("cp.async.commit_group;" ::: "memory");
+            cp_async_commit();
           }
         }
         const ZT* zb = zs + buf * RB * DS;
@@ -385,7 +385,7 @@ size_t vq_refine_binned_zero_bytes() { return sizeof(int) * 2 * MAX_BINS; }
 template <typename ZT>
 static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t N, int K, int D, int train, ZT* z_q,
                            int64_t* idx, unsigned long long* hist, double* sse, const RefineList& L, int* counters, void* ws,
-                           cudaStream_t s) {
+                           long long pair_cap, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
@@ -394,8 +394,7 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
   BinTables bt;
   bt.count = wi; bt.cursor = wi + MAX_BINS; bt.start = wi + 2 * MAX_BINS; bt.item_start = wi + 3 * MAX_BINS + 1;
   int* pairs = reinterpret_cast<int*>(static_cast<char*>(ws) + align_up(sizeof(int) * (size_t)(4 * MAX_BINS + 8), 256));
-  const long long cap_override = refine_pair_cap_override();
-  const long long pair_cap = (cap_override > 0 && cap_override < 2 * (long long)N) ? cap_override : 2 * (long long)N;
+  if (pair_cap <= 0 || pair_cap > 2 * (long long)N) pair_cap = 2 * (long long)N;   // the pair list holds 2 N entries
   unsigned long long* idx64 = reinterpret_cast<unsigned long long*>(idx);
   // slice width of the pairs kernel: a lane keeps DS floats of its code row in registers.  DS = 64 (168 registers, one CTA
   // of 12 warps per SM) re-reads a code row half as often, DS = 32 (80 registers) fits two CTAs per SM: measured at
@@ -436,12 +435,12 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
 
 int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
                             int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
-                            void* ws, bool zbf, cudaStream_t s) {
+                            void* ws, long long pair_cap, bool zbf, cudaStream_t s) {
   if (zbf)
     return launch_binned_t(static_cast<const __nv_bfloat16*>(z), E, ee, N, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
-                           list, counters, ws, s);
+                           list, counters, ws, pair_cap, s);
   return launch_binned_t(static_cast<const float*>(z), E, ee, N, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list, counters,
-                         ws, s);
+                         ws, pair_cap, s);
 }
 
 }  // namespace dvq

@@ -88,8 +88,8 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     for (int t = tid; t < cnt; t += nt) {
       const uint32_t dr = (uint32_t)__cvta_generic_to_shared(&s_row[b % 3][t]);
       const uint32_t dm = (uint32_t)__cvta_generic_to_shared(&s_mask[b % 3][t]);
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dr), "l"(L.rows + i0 + t) : "memory");
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dm), "l"(L.cand + i0 + t) : "memory");
+      cp_async_ca4(dr, L.rows + i0 + t);
+      cp_async_ca4(dm, L.cand + i0 + t);
     }
   };
   auto stage_z = [&](int b) {     // z rows of batch b (ids landed and visible; no commit of its own)
@@ -99,12 +99,12 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     for (int p = tid; p < cnt * PPR; p += nt) {
       const int r = p / PPR, c = p - r * PPR;
       const uint32_t dst = (uint32_t)__cvta_generic_to_shared(dst0 + r * DT + c * ZE);
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(z + (int64_t)rows[r] * DT + c * ZE) : "memory");
+      cp_async_cg16(dst, z + (int64_t)rows[r] * DT + c * ZE);
     }
   };
 
   stage_ids(0);
-  asm volatile("cp.async.commit_group;" ::: "memory");
+  cp_async_commit();
   // the code rows (loaded once) and the histogram reset overlap the first ids' round trip
   const int code = warp * 32 + lane;            // K is a multiple of 32: every lane holds a code
   float e[DT];
@@ -118,21 +118,21 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
     for (int k = tid; k < K; k += nt) s_hist[k] = 0u;
     if (lane == 0) s_sse[warp] = 0.0;
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait<0>();
   __syncthreads();
   stage_z(0);
   if (nb > 1) stage_ids(1);
-  asm volatile("cp.async.commit_group;" ::: "memory");
+  cp_async_commit();
 
   for (int b = 0; b < nb; ++b) {
     const int cnt = min(SB, end - (start + b * SB));
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
+    cp_async_wait<0>();
     __syncthreads();   // batch b's z rows and batch b+1's ids have landed; batch b-1 is written out (its buffers are free)
     if (b + 1 < nb) {
       stage_z(b + 1);
       if (b + 2 < nb) stage_ids(b + 2);
     }
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
     const ZT* zb = zbuf + (b & 1) * SB * DT;
     const int* rows = s_row[b % 3];
     const unsigned* masks = s_mask[b % 3];
@@ -241,12 +241,6 @@ bool vq_refine_stationary_supported(int K, int D) {
   }
   return !cand_list_mode(K) && K % 32 == 0 && K >= 32 && K / 32 <= max_warps;
 }
-
-// Where the automatic choice takes it: K >= 128 (e_dim <= 64) and K = 256 at e_dim 128, the shapes where it measured faster
-// than the per-row kernel (NVIDIA B200, 1000 W, N = 4M, refine stage: K = 512 / e_dim 64 0.077 vs 0.101 ms, K = 128 / e_dim
-// 64 0.062 vs 0.077, K = 256 / e_dim 128 0.149 vs 0.185).  With fewer sub-chunks a CTA has too few warps to hide the FMA
-// chains' latency (K = 64 / e_dim 64: 0.072 vs 0.065 ms; K = 128 / e_dim 128: 0.169 vs 0.162 ms).
-bool vq_refine_stationary_default(int K, int D) { return vq_refine_stationary_supported(K, D) && K >= (D <= 64 ? 128 : 256); }
 
 int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
                                 unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {

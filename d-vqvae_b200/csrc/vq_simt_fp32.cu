@@ -2,9 +2,7 @@
 // straight-through / SSE / usage histogram.  Replaces network/vqvae/quantizer.py:36-43,56-60
 // without materialising the N x K distance matrix.
 //
-// Role in the design: (1) the always-correct path for any (N, K, D); (2) the *refine* stage of
-// the tcgen05 path — the same kernel driven by a device-side list of rows the tensor-core
-// filter could not decide rigorously.
+// Role in the design: the always-correct path for any (N, K, D).
 //
 // Numerics (SURVEY §0.4): the contract of vq_exact.cuh — the reference's structure, the winner is the lowest
 // index among exact FP32 ties.
@@ -45,8 +43,7 @@ template <bool VEC, typename ZT>
 __global__ void __launch_bounds__(NTHREADS, 2)
 vq_simt_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const float* __restrict__ ee,
                int64_t N, int K, int D, int train, ZT* __restrict__ zq, int64_t* __restrict__ idx_out,
-               unsigned long long* __restrict__ hist, double* __restrict__ sse,
-               const int* __restrict__ row_list, const int* __restrict__ n_list, int list_stride) {
+               unsigned long long* __restrict__ hist, double* __restrict__ sse) {
   __shared__ __align__(16) float zs[BK][LDT];
   __shared__ __align__(16) float es[BK][LDT];
   __shared__ int64_t srow[BM];
@@ -60,13 +57,12 @@ vq_simt_kernel(const ZT* __restrict__ z, const float* __restrict__ E, const floa
   const int lk = (tid & 3) * 4;    // loader: offset inside the 16-wide D chunk
   const int warp = tid >> 5, lane = tid & 31;
 
-  const int64_t nrows = row_list ? (int64_t)(*n_list) : N;
-  const int64_t ntiles = (nrows + BM - 1) / BM;
+  const int64_t ntiles = (N + BM - 1) / BM;
 
   for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     if (tid < BM) {
-      int64_t r = tile * BM + tid;
-      srow[tid] = r < nrows ? (row_list ? (int64_t)row_list[r * list_stride] : r) : (int64_t)-1;
+      const int64_t r = tile * BM + tid;
+      srow[tid] = r < N ? r : (int64_t)-1;
     }
     __syncthreads();
     const int64_t grow0 = srow[lrow], grow1 = srow[lrow + 64];
@@ -220,21 +216,20 @@ int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s) {
 }
 
 int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse, const int* row_list,
-                   const int* n_list, int list_stride, bool zbf, cudaStream_t s) {
+                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse, bool zbf, cudaStream_t s) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
   const int64_t tiles = (N + BM - 1) / BM;
   int64_t grid = (int64_t)dp.sm_count * 2;
-  if (!row_list && tiles < grid) grid = tiles;
+  if (tiles < grid) grid = tiles;
   if (grid < 1) grid = 1;
   // 128-bit codebook loads; z / z_q rows move 4 elements at a time (16 bytes fp32, 8 bytes bf16)
   const bool vec = (D % 4 == 0) && reinterpret_cast<uintptr_t>(E) % 16 == 0 &&
                    (reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(z_q)) % (zbf ? 8 : 16) == 0;
 #define DVQ_LAUNCH_SIMT(V_, T_)                                                                                             \
   vq_simt_kernel<V_, T_><<<(unsigned)grid, NTHREADS, 0, s>>>(static_cast<const T_*>(z), E, ee, N, K, D, train,          \
-                                                             static_cast<T_*>(z_q), idx, hist, sse, row_list, n_list, list_stride)
+                                                             static_cast<T_*>(z_q), idx, hist, sse)
   if (zbf) { if (vec) DVQ_LAUNCH_SIMT(true, __nv_bfloat16); else DVQ_LAUNCH_SIMT(false, __nv_bfloat16); }
   else     { if (vec) DVQ_LAUNCH_SIMT(true, float); else DVQ_LAUNCH_SIMT(false, float); }
 #undef DVQ_LAUNCH_SIMT

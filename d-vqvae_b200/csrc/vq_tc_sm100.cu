@@ -1,7 +1,7 @@
 // tcgen05 VQ kernel: tensor-core distance filter fused with the row argmin, the codebook gather,
 // the straight-through / SSE reduction and the usage histogram.  The rows whose winner the filter
 // cannot decide *rigorously* are appended to a device-side list and re-evaluated by the exact
-// FP32 kernel (vq_simt_fp32.cu) — "filter and refine" (SURVEY §7.4).
+// FP32 refine kernels (launch_vq_refine_stage, vq_refine.cu) — "filter and refine" (SURVEY §7.4).
 //
 // Contraction.  For a 128-row tile the accumulator is
 //     acc[n,k] = g_n * (B_n + ee_k) - 2 z'_n . e'_k        (z' = s_n z, e' = s_E e, g_n = s_n s_E)

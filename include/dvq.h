@@ -84,7 +84,8 @@ DVQ_API int dvq_profile_mean(float* ms, int* count, int n);
  * kernels otherwise), 1 = per-row kernel only, 2 = binned kernels, 3 = code-stationary kernel
  * (dvq_vq_forward fails with DVQ_ERR_BAD_SHAPE on a shape it does not cover); pair_cap > 0 overrides the capacity
  * of the binned (row, sub-chunk) pair list (default 2 N) so that tests can exercise the device-side
- * hand-back to the per-row kernel, <= 0 restores the default.  Process-wide. */
+ * hand-back to the per-row kernel, <= 0 restores the default.  Process-wide.  A non-zero mode takes precedence over the
+ * environment variable DVQ_REFINE_PER_ROW, which selects mode 1 while the mode set here is 0. */
 DVQ_API int dvq_vq_set_refine(int mode, long long pair_cap);
 
 /* Diagnostic (host-only, no GPU needed): the shared-memory plan the tcgen05 VQ kernel would use for a codebook
