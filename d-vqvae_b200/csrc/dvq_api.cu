@@ -117,23 +117,21 @@ int dvq_vq_set_refine(int mode, long long pair_cap) {
 int dvq_debug_tc_layout(int K, int D, int* out8) {
   if (!out8) return fail(DVQ_ERR_BAD_ARG, "out8 is NULL");
   if (K <= 0 || D <= 0) return fail(DVQ_ERR_BAD_SHAPE, "need K > 0, D > 0");
-  vq_tc_layout_info(K, D, out8);
+  vq_tc_plan_info(1, K, D, 4, 0, out8);
   return DVQ_OK;
 }
 
 int dvq_debug_tc_pair_layout(long long N, int K, int D, int* out8) {
   if (!out8) return fail(DVQ_ERR_BAD_ARG, "out8 is NULL");
   if (K <= 0 || D <= 0) return fail(DVQ_ERR_BAD_SHAPE, "need K > 0, D > 0");
-  vq_tc_pair_layout_info((int64_t)N, K, D, out8);
+  vq_tc_plan_info((int64_t)N, K, D, 4, 1, out8);
   return DVQ_OK;
 }
 
 int dvq_debug_tc_layout_ex(long long N, int K, int D, int flags, int* out8) {
   if (!out8) return fail(DVQ_ERR_BAD_ARG, "out8 is NULL");
   if (K <= 0 || D <= 0) return fail(DVQ_ERR_BAD_SHAPE, "need K > 0, D > 0");
-  const int zbytes = (flags & DVQ_Z_BF16) ? 2 : 4;
-  if (vq_tc_pair_selected((int64_t)N, K, D)) vq_tc_pair_layout_info((int64_t)N, K, D, out8, zbytes);
-  else vq_tc_layout_info(K, D, out8, zbytes);
+  vq_tc_plan_info((int64_t)N, K, D, (flags & DVQ_Z_BF16) ? 2 : 4, -1, out8);
   return DVQ_OK;
 }
 

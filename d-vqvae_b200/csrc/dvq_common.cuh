@@ -116,13 +116,12 @@ int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s);
 int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
                    void* z_q, int64_t* idx, unsigned long long* hist, double* sse, bool zbf, cudaStream_t s);
 
-// tcgen05 filter kernel (vq_tc_sm100.cu); supported(K,D) says whether the shape is handled.
+// tcgen05 filter kernel (vq_tc_sm100.cu, whose plan_vq_tc makes every decision below); supported(N,K,D) says whether the shape is handled.
 bool vq_tc_supported(int64_t N, int K, int D);
-void vq_tc_layout_info(int K, int D, int* out8, int zbytes = 4);   // dvq_debug_tc_layout (zbytes: size of a z element)
-bool vq_tc_pair_selected(int64_t N, int K, int D);   // CTA-pair (cta_group::2) kernel for this shape?
-void vq_tc_pair_layout_info(int64_t N, int K, int D, int* out8, int zbytes = 4);   // dvq_debug_tc_pair_layout
-long long vq_tc_image_offset(int k, int d, int K, int D, int pair, long long* image_bytes);   // dvq_debug_tc_image_offset
 size_t vq_tc_operand_bytes(int K, int D);
+// dvq_debug_tc_layout (kernel 0), _pair_layout (1), _layout_ex (-1); zbytes: size of a z element
+void vq_tc_plan_info(int64_t N, int K, int D, int zbytes, int kernel, int* out8);
+long long vq_tc_image_offset(int k, int d, int K, int D, int pair, long long* image_bytes);   // dvq_debug_tc_image_offset
 int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
                  void* z_q, int64_t* idx, unsigned long long* hist, double* sse,
                  void* bop, int* counters, int* row_list, int* cand_list, int* zero_ints, int zero_n,

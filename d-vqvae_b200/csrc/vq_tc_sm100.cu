@@ -45,6 +45,7 @@
 #include <cstddef>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 #include "dvq_common.cuh"
 #include "f32x2.cuh"
@@ -163,7 +164,7 @@ __host__ __device__ inline uint32_t smem_place(SmemLayout& L, int K) {
 // (experiments: DVQ_TC_LAYOUT; the launch passes it to the kernel so that both sides agree)
 // `pair`: layout of the CTA-pair kernel (cta_group::2) — always streamed, a ring slot holds this CTA's half (128 codes) of a block
 // `zbytes`: size of a z element (4 fp32, 2 bf16): a staging slot holds 128 rows of one slice.  Which kernel and layout class a shape
-// gets is decided on the fp32 plan (vq_tc_supported, vq_tc_pair_selected); the smaller bf16 slots only re-run the search below.
+// gets is decided on the fp32 layouts (plan_vq_tc); the smaller bf16 slots only re-run the search below.
 __host__ __device__ inline SmemLayout smem_layout(int K, int D, int ovr = 0, bool pair = false, int zbytes = 4) {
   SmemLayout L;
   L.ds = (uint32_t)slice_width(D);
@@ -1446,108 +1447,186 @@ __global__ void __launch_bounds__(NTHREADS, 1) vq_tc_kernel(const __grid_constan
 
 }  // namespace
 
-// z [N, D] fp32 / bf16 row-major as a 2-D tensor map with box (ds columns, TM rows), no swizzle: a slice of a row tile lands as
-// [row][ds elements], the layout the converter warps read
-static int encode_ztile(CUtensorMap* map, const void* z, int64_t N, int D, int ds, bool zbf) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                               const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    DVQ_CUDA_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    if (!fn || qres != cudaDriverEntryPointSuccess) return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
-    encode = reinterpret_cast<EncodeFn>(fn);
-  }
-  const cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)N};
-  const cuuint64_t strides[1] = {(cuuint64_t)D * (zbf ? 2u : 4u)};
-  const cuuint32_t box[2] = {(cuuint32_t)ds, (cuuint32_t)TM};
-  const cuuint32_t estr[2] = {1u, 1u};
-  const CUresult r = encode(map, zbf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(z), dims, strides,
-                            box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for z [%lld, %d]", (int)r, (long long)N, D);
-  return DVQ_OK;
+// ------------------------------------------------------------------------------------------------
+// host: the plan of a call (kernel, variant, layout, image size) and its launch
+// ------------------------------------------------------------------------------------------------
+
+// Process-wide switches for A/B runs and tests, read once:
+//   DVQ_TC_PAIR=0 / 1           the CTA-pair kernel never / for every streamed shape (otherwise the rule in plan_vq_tc)
+//   DVQ_TC_LAYOUT=<a><st><sl>   streamed layout override, e.g. 123 = 1 A image, 2 z staging slots, 3 ring slots (layout_override)
+//   DVQ_TC_CE=1, DVQ_TC_ST=1    the CE / ST filter variants (TcVariant)
+struct TcSwitches {
+  int pair, layout;   // pair: -1 automatic, 0 never, 1 every streamed shape; layout: the DVQ_TC_LAYOUT digits, 0 = unset
+  bool ce, st;
+};
+
+static const TcSwitches& tc_switches() {
+  static const TcSwitches sw = [] {
+    const char* pair = getenv("DVQ_TC_PAIR");
+    const char* layout = getenv("DVQ_TC_LAYOUT");
+    const char* ce = getenv("DVQ_TC_CE");
+    const char* st = getenv("DVQ_TC_ST");
+    return TcSwitches{pair && pair[0] == '0' ? 0 : (pair && pair[0] == '1' ? 1 : -1), layout ? atoi(layout) : 0,
+                      ce && ce[0] == '1', st && st[0] == '1'};
+  }();
+  return sw;
 }
 
-// the operand image as a [bytes / 1024, 256] int32 tensor, box = (256, rows): one half block lands densely in its ring slot
-static int encode_bimg(CUtensorMap* map, const uint8_t* bimg, size_t image_bytes, uint32_t box_rows) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                               const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    DVQ_CUDA_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    if (!fn || qres != cudaDriverEntryPointSuccess) return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
-    encode = reinterpret_cast<EncodeFn>(fn);
-  }
-  const cuuint64_t dims[2] = {256, (cuuint64_t)(image_bytes / 1024)};
-  const cuuint64_t strides[1] = {1024};
-  const cuuint32_t box[2] = {256, box_rows};
-  const cuuint32_t estr[2] = {1u, 1u};
-  const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<uint8_t*>(bimg), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for the operand image (%zu bytes, box rows %u)", (int)r, image_bytes, box_rows);
-  return DVQ_OK;
+// Filter kernel variant (the DT / CE / ST template arguments of vq_tc_kernel):
+//   Generic     DT = 0, e_dim at run time.
+//   Resident64  DT = 64: the resident mask-mode e_dim 64 shapes (config 2).
+//   CE          converters join the filter as a fourth warp per TMEM lane quarter (DVQ_TC_CE=1; streamed image, two A
+//               images).  It paid +4 % at e_dim 64, K >= 4096 while the filter was the bound; with the list-mode early-out
+//               the filter is cheap and the variant is 5 % behind the default there, so it is not selected automatically.
+//   ST          two-sub-chunk filter with the epilogue-heavy register split (DVQ_TC_ST=1; streamed image).  Measured within
+//               +-2 % of the default at every K >= 2048 shape of the sweep, so it is not selected automatically.
+// CE and ST are built for fp32 z only: a bf16 call ignores the switches.
+enum class TcVariant { Generic, Resident64, CE, ST };
+
+// Everything the host decides for one call of the filter kernel.  It depends on (N, K, D, z element size) and the
+// switches alone, so the debug entries report exactly what dvq_vq_forward launches.
+struct TcPlan {
+  bool supported;       // the tcgen05 path handles the shape (the fields below are zero otherwise)
+  bool pair;            // CTA-pair kernel (cta_group::2)
+  bool streamed;        // operand image streamed through the ring (else resident in the two slots)
+  bool list;            // cand_list_mode(K): candidate records are sub-chunk lists
+  TcVariant variant;
+  int layout_ovr;       // validated DVQ_TC_LAYOUT, passed to the kernel (TcParams::layout_ovr) so that both sides agree
+  SmemLayout L;         // shared-memory layout of the kernel that runs
+  size_t image_bytes;   // global operand image (the same for both image layouts)
+};
+
+// DVQ_TC_LAYOUT as one kernel kind accepts it, else 0 (automatic layout): streamed images only (a resident image keeps its
+// layout; the pair kernel runs on streamed images only), 1-2 A images, 1-2 z staging slots, a ring of 2..MAX_BSLOTS_SOLO
+// slots for the single-CTA kernel or of 2..MAX_BSLOTS for the CTA pair, and only if the layout fits shared memory
+static int layout_override(int K, int D, int zbytes, bool pair, bool streamed) {
+  const int ovr = tc_switches().layout;
+  const int a = ovr / 100, st = ovr / 10 % 10, sl = ovr % 10;
+  const bool ok = streamed && a >= 1 && a <= 2 && st >= 1 && st <= 2 && sl >= 2 && sl <= (pair ? MAX_BSLOTS : MAX_BSLOTS_SOLO);
+  return ok && smem_layout(K, D, ovr, pair, zbytes).total <= SMEM_LIMIT ? ovr : 0;
 }
 
-bool vq_tc_supported(int64_t N, int K, int D) {
-  if (N <= 0 || N > 2147483647LL - 256) return false;
-  if (D < 16 || D > 512 || (D & (D - 1)) != 0) return false;   // power of two: index math is masks/shifts
-  if (USE_ZL && D > DSLICE) return false;
-  if (K % 32 != 0 || K < 32 || K > 32704) return false;   // list-mode candidate entries are 10 bits (sub-chunk index + 1 <= 1023)
-  return smem_layout(K, D).total <= SMEM_LIMIT;
+// The plan of one kernel kind for a codebook shape, whatever the row count
+static TcPlan plan_kernel(int K, int D, int zbytes, bool pair) {
+  TcPlan P = {};
+  if (D < 16 || D > 512 || (D & (D - 1)) != 0) return P;   // power of two: index math is masks/shifts
+  if (USE_ZL && D > DSLICE) return P;
+  if (K % 32 != 0 || K < 32 || K > 32704) return P;   // list-mode candidate entries are 10 bits (sub-chunk index + 1 <= 1023)
+  const SmemLayout L1 = smem_layout(K, D);   // the fp32 single-CTA layout decides support for both z types
+  if (L1.total > SMEM_LIMIT) return P;
+  const int nchunks = (K + 255) / 256;
+  P.supported = true;
+  P.pair = pair;
+  P.streamed = nchunks * (int)L1.ns > 2;
+  P.list = cand_list_mode(K);
+  P.image_bytes = (size_t)nchunks * L1.ns * L1.bchunk_bytes;
+  P.layout_ovr = layout_override(K, D, zbytes, pair, P.streamed);
+  P.L = smem_layout(K, D, P.layout_ovr, pair, zbytes);
+  const TcSwitches& sw = tc_switches();
+  const bool fp32 = zbytes == 4;
+  if (D == 64 && !P.list && !P.streamed) P.variant = TcVariant::Resident64;
+  else if (fp32 && P.streamed && sw.st) P.variant = TcVariant::ST;
+  else if (fp32 && P.streamed && sw.ce && P.L.a_bufs == 2) P.variant = TcVariant::CE;
+  else P.variant = TcVariant::Generic;
+  return P;
 }
+
+// The plan of a call of N rows.  CTA-pair kernel for streamed codebooks only.  Measured at N = 16.8M against the single-CTA
+// kernel, whole call (profiles/README.md): e_dim 512 1.05x (K = 512) .. 1.67x (K = 16 384); e_dim 256 1.11-1.27x from
+// K = 2048 on, 0.93x at K = 1024; e_dim 128 1.06-1.09x from K = 2048 on, 0.91x at K = 512; e_dim 64 0.98-1.00x (one slice
+// per chunk: the accumulator hand-off between the SMs costs what the halved operand stream saves).  Hence: e_dim 512
+// always, e_dim 128 / 256 from K = 2048 on, and at least two row tiles.  The z type plays no part in the choice.
+static TcPlan plan_vq_tc(int64_t N, int K, int D, int zbytes) {
+  if (N <= 0 || N > 2147483647LL - 256) return TcPlan{};
+  const TcPlan single = plan_kernel(K, D, zbytes, false);
+  const int sw = tc_switches().pair;
+  const bool pair = single.supported && single.streamed && N > TM && (sw == 1 || (sw < 0 && (D >= 512 || (D >= 128 && K >= 2048)))) &&
+                    smem_layout(K, D, 0, true).total <= SMEM_LIMIT;
+  return pair ? plan_kernel(K, D, zbytes, true) : single;
+}
+
+bool vq_tc_supported(int64_t N, int K, int D) { return plan_vq_tc(N, K, D, 4).supported; }
+
+size_t vq_tc_operand_bytes(int K, int D) { return align_up(sizeof(CbMeta), 256) + align_up(plan_vq_tc(1, K, D, 4).image_bytes, 256); }
 
 // dvq_debug_tc_image_offset: byte offset of (code k, column d; d in [D, D + 16) = fold columns) in the global operand image of
 // either layout, and the image size (host-only; tests/test_cabi_symbols.py checks that the maps are injective and in range)
 long long vq_tc_image_offset(int k, int d, int K, int D, int pair, long long* image_bytes) {
-  const SmemLayout L1 = smem_layout(K, D);
-  if (image_bytes) *image_bytes = (long long)((K + 255) / 256) * L1.ns * L1.bchunk_bytes;
+  if (image_bytes) *image_bytes = (long long)plan_vq_tc(1, K, D, 4).image_bytes;
   return (long long)bimg_offset(k, d, D, K, pair != 0);
 }
 
-// CTA-pair kernel (cta_group::2) for this call?  Streamed codebooks only.  Measured at N = 16.8M against the single-CTA
-// kernel, whole call (profiles/README.md): e_dim 512 1.05x (K = 512) .. 1.67x (K = 16 384); e_dim 256 1.11-1.27x from
-// K = 2048 on, 0.93x at K = 1024; e_dim 128 1.06-1.09x from K = 2048 on, 0.91x at K = 512; e_dim 64 0.98-1.00x (one slice
-// per chunk: the accumulator hand-off between the SMs costs what the halved operand stream saves).  Hence: e_dim 512
-// always, e_dim 128 / 256 from K = 2048 on.  DVQ_TC_PAIR=0 turns it off, DVQ_TC_PAIR=1 selects it for every streamed shape.
-bool vq_tc_pair_selected(int64_t N, int K, int D) {
-  static const char* pair_env = getenv("DVQ_TC_PAIR");
-  if (pair_env && pair_env[0] == '0') return false;
-  if (!vq_tc_supported(N, K, D)) return false;
-  const SmemLayout L1 = smem_layout(K, D);
-  if (((K + 255) / 256) * (int)L1.ns <= 2) return false;                 // resident image: the single-CTA kernel
-  if (!(pair_env && pair_env[0] == '1') && !(D >= 512 || (D >= 128 && K >= 2048))) return false;
-  if (smem_layout(K, D, 0, true).total > SMEM_LIMIT) return false;
-  return N > TM;                                                         // at least two tiles
+// out8 of the debug entries (dvq.h): kernel = 0 the single-CTA kernel's plan (dvq_debug_tc_layout), 1 the CTA pair's
+// (dvq_debug_tc_pair_layout), -1 that of the kernel a call of N rows launches (dvq_debug_tc_layout_ex)
+void vq_tc_plan_info(int64_t N, int K, int D, int zbytes, int kernel, int* out8) {
+  const bool selected = plan_vq_tc(N, K, D, zbytes).pair;
+  const TcPlan P = plan_kernel(K, D, zbytes, kernel < 0 ? selected : kernel == 1);
+  const SmemLayout& L = P.L;
+  const int info[8] = {P.pair ? (int)selected : 1, (int)L.ds, (int)L.ns, (int)L.a_bufs, (int)L.nslots, (int)L.nstage, (int)L.total + 128,
+                       P.pair ? (int)L.bcodes : (int)L.hist_in_smem};
+  for (int i = 0; i < 8; ++i) out8[i] = P.supported ? info[i] : 0;
 }
 
-// dvq_debug_tc_pair_layout: out8 = { CTA-pair kernel selected for (N, K, D) (0/1), slice width, slices, A images, ring
-// slots, z staging slots, dynamic shared memory, codes per ring slot } of the pair layout (host-only)
-void vq_tc_pair_layout_info(int64_t N, int K, int D, int* out8, int zbytes) {
-  for (int i = 0; i < 8; ++i) out8[i] = 0;
-  if (!vq_tc_supported(N > 0 ? N : 1, K, D)) return;
-  const SmemLayout L = smem_layout(K, D, 0, true, zbytes);
-  out8[0] = vq_tc_pair_selected(N, K, D) ? 1 : 0;
-  out8[1] = (int)L.ds; out8[2] = (int)L.ns; out8[3] = (int)L.a_bufs; out8[4] = (int)L.nslots; out8[5] = (int)L.nstage;
-  out8[6] = (int)L.total + 128; out8[7] = (int)L.bcodes;
+// A 2-D tensor map without swizzle over `rows` rows of `cols` elements, `row_bytes` apart, box (box_cols, box_rows).
+// cuTensorMapEncodeTiled is fetched once through cudaGetDriverEntryPoint (no libcuda link dependency).
+static int encode_2d(CUtensorMap* map, CUtensorMapDataType type, const void* base, uint64_t cols, uint64_t rows, uint64_t row_bytes,
+                     uint32_t box_cols, uint32_t box_rows) {
+  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
+                               const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  static EncodeFn encode = nullptr;
+  if (!encode) {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    DVQ_CUDA_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+    if (!fn || qres != cudaDriverEntryPointSuccess) return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
+    encode = reinterpret_cast<EncodeFn>(fn);
+  }
+  const cuuint64_t dims[2] = {cols, rows};
+  const cuuint64_t strides[1] = {row_bytes};
+  const cuuint32_t box[2] = {box_cols, box_rows};
+  const cuuint32_t estr[2] = {1u, 1u};
+  const CUresult r = encode(map, type, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS)
+    return fail(DVQ_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a [%llu, %llu] tensor with box [%u, %u]", (int)r,
+                (unsigned long long)rows, (unsigned long long)cols, box_rows, box_cols);
+  return DVQ_OK;
 }
 
-void vq_tc_layout_info(int K, int D, int* out8, int zbytes) {
-  const bool shape_ok = D >= 16 && D <= 512 && (D & (D - 1)) == 0 && K % 32 == 0 && K >= 32 && K <= 32704;
-  for (int i = 0; i < 8; ++i) out8[i] = 0;
-  if (!shape_ok) return;
-  const SmemLayout L = smem_layout(K, D, 0, false, zbytes);
-  out8[0] = L.total <= SMEM_LIMIT ? 1 : 0;
-  out8[1] = (int)L.ds; out8[2] = (int)L.ns; out8[3] = (int)L.a_bufs; out8[4] = (int)L.nslots; out8[5] = (int)L.nstage;
-  out8[6] = (int)L.total + 128; out8[7] = (int)L.hist_in_smem;
+// One vq_tc_kernel instance: the shared-memory attribute, then a plain launch or, for the pair kernel, a launch in clusters of two
+template <int DT, bool TRAIN, bool LIST, bool CE, bool ST, bool PAIR, typename ZT>
+static int launch_filter(const TcParams& p, unsigned grid, size_t smem, cudaStream_t s) {
+  DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<DT, TRAIN, LIST, CE, ST, PAIR, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (!PAIR) {
+    vq_tc_kernel<DT, TRAIN, LIST, CE, ST, PAIR, ZT><<<grid, NTHREADS, smem, s>>>(p);
+    return DVQ_OK;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  cfg.attrs = at; cfg.numAttrs = 1;
+  DVQ_CUDA_CHECK(cudaLaunchKernelEx(&cfg, vq_tc_kernel<DT, TRAIN, LIST, CE, ST, PAIR, ZT>, p));
+  return DVQ_OK;
 }
 
-size_t vq_tc_operand_bytes(int K, int D) {
-  const SmemLayout L = smem_layout(K, D);
-  return align_up(sizeof(CbMeta), 256) + align_up((size_t)((K + 255) / 256) * L.ns * L.bchunk_bytes, 256);
+template <bool TRAIN, bool LIST, bool PAIR, typename ZT>
+static int launch_generic(TcVariant v, const TcParams& p, unsigned grid, size_t smem, cudaStream_t s) {
+  if constexpr (std::is_same<ZT, float>::value) {
+    if (v == TcVariant::CE) return launch_filter<0, TRAIN, LIST, true, false, PAIR, ZT>(p, grid, smem, s);
+    if (v == TcVariant::ST) return launch_filter<0, TRAIN, LIST, false, true, PAIR, ZT>(p, grid, smem, s);
+  }
+  return launch_filter<0, TRAIN, LIST, false, false, PAIR, ZT>(p, grid, smem, s);
+}
+
+// The plan's kernel.  Per z type and TRAIN this instantiates DT = 64 plus (mask / list mode) x (single CTA / pair) x
+// (generic, and for fp32 CE and ST): 36 kernels in all.
+template <bool TRAIN, typename ZT>
+static int launch_planned(const TcPlan& P, const TcParams& p, unsigned grid, size_t smem, cudaStream_t s) {
+  if (P.variant == TcVariant::Resident64) return launch_filter<64, TRAIN, false, false, false, false, ZT>(p, grid, smem, s);
+  if (P.list) return P.pair ? launch_generic<TRAIN, true, true, ZT>(P.variant, p, grid, smem, s) : launch_generic<TRAIN, true, false, ZT>(P.variant, p, grid, smem, s);
+  return P.pair ? launch_generic<TRAIN, false, true, ZT>(P.variant, p, grid, smem, s) : launch_generic<TRAIN, false, false, ZT>(P.variant, p, grid, smem, s);
 }
 
 int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
@@ -1558,27 +1637,10 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
   if (rc) return rc;
   if ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(E) | reinterpret_cast<uintptr_t>(z_q)) % 16 != 0)
     return fail(DVQ_ERR_BAD_ALIGN, "tcgen05 path needs 16-byte aligned z / E / z_q");
+  const int zbytes = zbf ? 2 : 4;
+  const TcPlan P = plan_vq_tc(N, K, D, zbytes);
   CbMeta* cb = static_cast<CbMeta*>(bop);
   uint8_t* bimg = static_cast<uint8_t*>(bop) + align_up(sizeof(CbMeta), 256);
-  static const char* lay_env = getenv("DVQ_TC_LAYOUT");   // experiment: "a st sl" digits, e.g. 123 = 1 A image, 2 staging slots, 3 ring slots
-  int ovr = lay_env ? atoi(lay_env) : 0;
-  const int zbytes = zbf ? 2 : 4;
-  if (ovr && (((K + 255) / 256) * (D / slice_width(D)) <= 2 || smem_layout(K, D, ovr, false, zbytes).total > SMEM_LIMIT || ovr / 100 < 1 || ovr / 100 > 2 ||
-              ovr / 10 % 10 < 1 || ovr / 10 % 10 > 2 || ovr % 10 < 2 || ovr % 10 > MAX_BSLOTS_SOLO))
-    ovr = 0;   // resident images keep their layout; impossible requests are ignored
-  // CTA-pair kernel (cta_group::2) for streamed codebooks: on by default, DVQ_TC_PAIR=0 selects the single-CTA kernel (A/B runs).
-  // It needs an even number of SMs to pair up and at least one full pair of tiles.
-  static const char* ce_env = getenv("DVQ_TC_CE");
-  static const char* st_env = getenv("DVQ_TC_ST");
-  int pair_ovr = lay_env ? atoi(lay_env) : 0;   // the pair kernel accepts rings of up to MAX_BSLOTS slots
-  if (pair_ovr && (pair_ovr / 100 < 1 || pair_ovr / 100 > 2 || pair_ovr / 10 % 10 < 1 || pair_ovr / 10 % 10 > 2 || pair_ovr % 10 < 2 || pair_ovr % 10 > MAX_BSLOTS ||
-                   smem_layout(K, D, pair_ovr, true, zbytes).total > SMEM_LIMIT))
-    pair_ovr = 0;
-  const SmemLayout L1 = smem_layout(K, D, ovr, false, zbytes);
-  const bool streamed = ((K + 255) / 256) * (int)L1.ns > 2;
-  const bool pair = vq_tc_pair_selected(N, K, D) && dp.sm_count >= 2;   // chosen on (N, K, D) alone, whatever the z type
-  const SmemLayout L = pair ? smem_layout(K, D, pair_ovr, true, zbytes) : L1;
-  const size_t image_bytes = (size_t)((K + 255) / 256) * L1.ns * L1.bchunk_bytes;   // the same for both image layouts
   if (codebook_cached) {
     // DVQ_CODEBOOK_CACHED: CbMeta and the operand image in `bop` are those of this codebook; only the per-call
     // counters and bin tables are reset
@@ -1586,95 +1648,41 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
     DVQ_CUDA_CHECK(cudaGetLastError());
     count_launch();
   } else {
-    tc_cb_stats_kernel<<<1, 256, 0, s>>>(ee, K, D, cb, counters, zero_ints, zero_n, pair);
+    tc_cb_stats_kernel<<<1, 256, 0, s>>>(ee, K, D, cb, counters, zero_ints, zero_n, P.pair);
     DVQ_CUDA_CHECK(cudaGetLastError());
-    DVQ_CUDA_CHECK(cudaMemsetAsync(bimg, 0, image_bytes, s));
-    tc_cb_image_kernel<<<(K * 32 + 255) / 256, 256, 0, s>>>(E, ee, K, D, cb, bimg, pair);
+    DVQ_CUDA_CHECK(cudaMemsetAsync(bimg, 0, P.image_bytes, s));
+    tc_cb_image_kernel<<<(K * 32 + 255) / 256, 256, 0, s>>>(E, ee, K, D, cb, bimg, P.pair);
     DVQ_CUDA_CHECK(cudaGetLastError());
     count_launch(2);
   }
 
   TcParams p;
   memset(&p.ztile, 0, sizeof(p.ztile));
-  if (D > DSLICE) {
-    rc = encode_ztile(&p.ztile, z, N, D, (int)L.ds, zbf);
+  if (D > DSLICE) {   // z [N, D] row-major, box (slice columns, TM rows): a slice of a row tile lands as [row][ds elements], as the converters read it
+    rc = encode_2d(&p.ztile, zbf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, z, (uint64_t)D, (uint64_t)N,
+                   (uint64_t)D * zbytes, P.L.ds, TM);
     if (rc) return rc;
   }
   memset(p.bmap, 0, sizeof(p.bmap));
-  if (pair) {
-    rc = encode_bimg(&p.bmap[0], bimg, image_bytes, L.bslice_bytes / 1024);
-    if (!rc) rc = encode_bimg(&p.bmap[1], bimg, image_bytes, L.bchunk_bytes / 1024);
+  if (P.pair) {   // the operand image as [bytes / 1024, 256] int32: one half block without / with the fold columns lands densely in its ring slot
+    rc = encode_2d(&p.bmap[0], CU_TENSOR_MAP_DATA_TYPE_INT32, bimg, 256, P.image_bytes / 1024, 1024, 256, P.L.bslice_bytes / 1024);
+    if (!rc) rc = encode_2d(&p.bmap[1], CU_TENSOR_MAP_DATA_TYPE_INT32, bimg, 256, P.image_bytes / 1024, 1024, 256, P.L.bchunk_bytes / 1024);
     if (rc) return rc;
   }
   p.z = z; p.E = E; p.bimg = bimg; p.cb = cb; p.N = N; p.K = K; p.D = D; p.train = train;
   p.zq = z_q; p.idx = idx; p.hist = hist; p.sse = sse; p.counters = counters; p.row_list = row_list; p.cand_list = cand_list;
-  p.layout_ovr = pair ? pair_ovr : ovr;
+  p.layout_ovr = P.layout_ovr;
   p.stats = reinterpret_cast<unsigned long long*>(counters + CNT_STATS);
   p.ntiles = (N + TM - 1) / TM;
-  const size_t smem = L.total + 128;
+  const size_t smem = P.L.total + 128;
   int64_t grid = p.ntiles < dp.sm_count ? p.ntiles : dp.sm_count;
-  if (pair) {   // clusters of two CTAs: one per tile pair, at most one per TPC
+  if (P.pair) {   // clusters of two CTAs: one per tile pair, at most one per TPC
     const int64_t units = (p.ntiles + 1) / 2;
     grid = 2 * (units < dp.sm_count / 2 ? units : dp.sm_count / 2);
   }
-  // Converters join the filter as a fourth warp per TMEM lane quarter (DVQ_TC_CE=1; needs a streamed codebook and a
-  // double-buffered A image).  It paid +4 % at e_dim 64, K >= 4096 while the filter was the bound; with the list-mode
-  // early-out the filter is cheap and the variant is 5 % behind the default there, so it is not selected automatically.
-  // (the bf16 kernels are instantiated without the CE / ST experiment variants: a bf16 call ignores DVQ_TC_CE / DVQ_TC_ST)
-  const bool ce = !zbf && streamed && L.a_bufs == 2 && ce_env && ce_env[0] == '1';
-#define DVQ_LAUNCH_TC(DT_, TR_, LS_, CE_, ST_, ZT_)                                                                         \
-  do {                                                                                                                 \
-    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<DT_, TR_, LS_, CE_, ST_, false, ZT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    vq_tc_kernel<DT_, TR_, LS_, CE_, ST_, false, ZT_><<<(unsigned)grid, NTHREADS, smem, s>>>(p);                           \
-  } while (0)
-#define DVQ_LAUNCH_TC_PAIR(TR_, LS_, CE_, ST_, ZT_)                                                                         \
-  do {                                                                                                                 \
-    DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_tc_kernel<0, TR_, LS_, CE_, ST_, true, ZT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    cudaLaunchConfig_t cfg = {};                                                                                       \
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;     \
-    cudaLaunchAttribute at[1];                                                                                         \
-    at[0].id = cudaLaunchAttributeClusterDimension;                                                                    \
-    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;                                 \
-    cfg.attrs = at; cfg.numAttrs = 1;                                                                                  \
-    DVQ_CUDA_CHECK(cudaLaunchKernelEx(&cfg, vq_tc_kernel<0, TR_, LS_, CE_, ST_, true, ZT_>, p));                        \
-  } while (0)
-#define DVQ_LAUNCH_TC_GENERIC(TR_, LS_)                                      \
-  do {                                                                       \
-    if (pair && st) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, true, float);        \
-    else if (pair && ce) DVQ_LAUNCH_TC_PAIR(TR_, LS_, true, false, float);   \
-    else if (pair) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, false, float);        \
-    else if (st) DVQ_LAUNCH_TC(0, TR_, LS_, false, true, float);             \
-    else if (ce) DVQ_LAUNCH_TC(0, TR_, LS_, true, false, float);             \
-    else DVQ_LAUNCH_TC(0, TR_, LS_, false, false, float);                    \
-  } while (0)
-#define DVQ_LAUNCH_TC_GENERIC_BF16(TR_, LS_)                                 \
-  do {                                                                       \
-    if (pair) DVQ_LAUNCH_TC_PAIR(TR_, LS_, false, false, __nv_bfloat16);     \
-    else DVQ_LAUNCH_TC(0, TR_, LS_, false, false, __nv_bfloat16);            \
-  } while (0)
-  // two-sub-chunk filter with the epilogue-heavy register split (DVQ_TC_ST=1; streamed codebooks only).  Measured
-  // within +-2 % of the default at every K >= 2048 shape of the sweep, so it is not selected automatically.
-  const bool st = !zbf && streamed && st_env && st_env[0] == '1';
-  const bool list = cand_list_mode(K);
-  if (zbf) {
-    if (D == 64 && !list && !streamed) {
-      if (train) DVQ_LAUNCH_TC(64, true, false, false, false, __nv_bfloat16); else DVQ_LAUNCH_TC(64, false, false, false, false, __nv_bfloat16);
-    } else if (!list) {
-      if (train) DVQ_LAUNCH_TC_GENERIC_BF16(true, false); else DVQ_LAUNCH_TC_GENERIC_BF16(false, false);
-    } else {
-      if (train) DVQ_LAUNCH_TC_GENERIC_BF16(true, true); else DVQ_LAUNCH_TC_GENERIC_BF16(false, true);
-    }
-  } else if (D == 64 && !list && !streamed) {
-    if (train) DVQ_LAUNCH_TC(64, true, false, false, false, float); else DVQ_LAUNCH_TC(64, false, false, false, false, float);
-  } else if (!list) {
-    if (train) DVQ_LAUNCH_TC_GENERIC(true, false); else DVQ_LAUNCH_TC_GENERIC(false, false);
-  } else {
-    if (train) DVQ_LAUNCH_TC_GENERIC(true, true); else DVQ_LAUNCH_TC_GENERIC(false, true);
-  }
-#undef DVQ_LAUNCH_TC_GENERIC_BF16
-#undef DVQ_LAUNCH_TC_GENERIC
-#undef DVQ_LAUNCH_TC_PAIR
-#undef DVQ_LAUNCH_TC
+  if (zbf) rc = train ? launch_planned<true, __nv_bfloat16>(P, p, (unsigned)grid, smem, s) : launch_planned<false, __nv_bfloat16>(P, p, (unsigned)grid, smem, s);
+  else rc = train ? launch_planned<true, float>(P, p, (unsigned)grid, smem, s) : launch_planned<false, float>(P, p, (unsigned)grid, smem, s);
+  if (rc) return rc;
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;

@@ -88,24 +88,26 @@ DVQ_API int dvq_profile_mean(float* ms, int* count, int n);
  * environment variable DVQ_REFINE_PER_ROW, which selects mode 1 while the mode set here is 0. */
 DVQ_API int dvq_vq_set_refine(int mode, long long pair_cap);
 
-/* Diagnostic (host-only, no GPU needed): the shared-memory plan the tcgen05 VQ kernel would use for a codebook
- * shape.  out8 = { handled by the tensor-core path (0/1), e_dim slice width, slices per row, A images (1-2),
+/* Diagnostic (host-only, no GPU needed): the shared-memory plan the tcgen05 VQ kernel (single-CTA kernel) would use for
+ * a codebook shape.  out8 = { handled by the tensor-core path (0/1), e_dim slice width, slices per row, A images (1-2),
  * operand ring slots (2-4), z staging slots (1-2), dynamic shared memory in bytes, histogram kept in shared
- * memory (0/1) }.  Used by tests/test_cabi_symbols.py to pin the per-shape choices. */
+ * memory (0/1) }.  Used by tests/test_cabi_symbols.py to pin the per-shape choices.  This entry and the two below come
+ * from the planner the launch uses: they honour DVQ_TC_PAIR and the DVQ_TC_LAYOUT override exactly as a launch does. */
 DVQ_API int dvq_debug_tc_layout(int K, int D, int* out8);
 
 /* Diagnostic (host-only): streamed codebooks (the operand image does not fit shared memory) with e_dim 512, or e_dim
  * 128 / 256 from K = 2048 on, run on CTA pairs (clusters of two CTAs, tcgen05 cta_group::2: one M = 256 MMA over both
  * SMs' row tiles, each CTA streaming half of every operand block).  out8 = { pair kernel selected for (N, K, D) (0/1;
  * honours DVQ_TC_PAIR=0/1), e_dim slice width, slices per row, A images, ring slots (2-8), z staging slots, dynamic
- * shared memory in bytes, codes per ring slot (128) } of the pair kernel's plan. */
+ * shared memory in bytes, codes per ring slot (128) } of the pair kernel's plan (with DVQ_TC_LAYOUT where the pair
+ * kernel accepts it). */
 DVQ_API int dvq_debug_tc_pair_layout(long long N, int K, int D, int* out8);
 
 /* Diagnostic (host-only): the plan of the tcgen05 kernel variant dvq_vq_forward would launch for (N, K, D, flags) (flags:
- * DVQ_Z_BF16 or 0; other bits are ignored).  When the CTA-pair kernel is selected, out8 is filled as by
- * dvq_debug_tc_pair_layout, otherwise as by dvq_debug_tc_layout — with flags = 0 exactly their output — with the plan
- * of the z element type: the dynamic shared memory out8[6] includes the z staging slots of 128 rows x (slice width)
- * x (4 bytes fp32 / 2 bytes bf16) each. */
+ * DVQ_Z_BF16 or 0; other bits are ignored), DVQ_TC_PAIR and DVQ_TC_LAYOUT included.  When the CTA-pair kernel is
+ * selected, out8 is filled as by dvq_debug_tc_pair_layout, otherwise as by dvq_debug_tc_layout — with flags = 0 exactly
+ * their output — with the plan of the z element type: the dynamic shared memory out8[6] includes the z staging slots of
+ * 128 rows x (slice width) x (4 bytes fp32 / 2 bytes bf16) each. */
 DVQ_API int dvq_debug_tc_layout_ex(long long N, int K, int D, int flags, int* out8);
 
 /* Diagnostic (host-only): byte offset of element (code k, column d) of the FP16 operand image the tcgen05 VQ kernel keeps in
