@@ -67,14 +67,21 @@ void profile_mark(int stage, bool begin, cudaStream_t s) {
   if (!begin) g_prof_n[stage] = slot + 1;
 }
 
-static int require_sm100() {
+static int require_sm100(DeviceProps* out = nullptr) {
   DeviceProps dp;
   int rc = device_props(&dp);
   if (rc) return rc;
   if (dp.cc_major != 10)
     return fail(DVQ_ERR_UNSUPPORTED_ARCH, "libdvq_sm100 is built for sm_100a only; device is sm_%d%d",
                 dp.cc_major, dp.cc_minor);
+  if (out) *out = dp;
   return DVQ_OK;
+}
+
+// Whether the tcgen05 path may run for a call: its workspace areas exist and its counters are read.  A call runs it
+// when z / E / z_q are also 16-byte aligned (dvq_vq_forward).
+static bool vq_tc_may_run(int64_t N, int K, int D, int flags) {
+  return (flags & DVQ_PATH_MASK) != DVQ_PATH_SIMT && vq_tc_supported(N, K, D);
 }
 
 VqWorkspace vq_workspace_layout(int64_t N, int K, int D, int flags) {
@@ -84,9 +91,11 @@ VqWorkspace vq_workspace_layout(int64_t N, int K, int D, int flags) {
   off = align_up(off + sizeof(float) * (size_t)K, 256);
   w.off_counters = off;
   off = align_up(off + sizeof(int) * CNT_WORDS, 256);
-  const bool may_tc = (flags & DVQ_PATH_MASK) != DVQ_PATH_SIMT && vq_tc_supported(N, K, D);
+  const bool may_tc = vq_tc_may_run(N, K, D, flags);
   w.off_rowlist = off;
-  if (may_tc) off = align_up(off + 2 * align_up(sizeof(int) * (size_t)N, 256), 256);
+  if (may_tc) off = align_up(off + sizeof(int) * (size_t)N, 256);
+  w.off_candlist = off;
+  if (may_tc) off = align_up(off + sizeof(int) * (size_t)N, 256);
   w.off_bop = off;
   if (may_tc) off = align_up(off + vq_tc_operand_bytes(K, D), 1024);
   w.off_binned = off;
@@ -206,63 +215,56 @@ int dvq_vq_forward(const float* z, const float* E, int64_t N, int K, int D, int 
   const VqWorkspace w = vq_workspace_layout(N, K, D, flags);
   if (workspace_bytes < w.total)
     return fail(DVQ_ERR_WORKSPACE, "workspace too small: %zu < %zu bytes", workspace_bytes, w.total);
-  rc = require_sm100();
+  DeviceProps dp;
+  rc = require_sm100(&dp);
   if (rc) return rc;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  char* ws = static_cast<char*>(workspace);
-  float* ee = reinterpret_cast<float*>(ws + w.off_ee);
-
   const int path = flags & DVQ_PATH_MASK;
-  const bool tc_ok = vq_tc_supported(N, K, D);
+  const bool tc_ok = vq_tc_may_run(N, K, D, flags);
   if (path == DVQ_PATH_TC && !tc_ok)
     return fail(DVQ_ERR_BAD_SHAPE, "DVQ_PATH_TC: shape N=%lld K=%d D=%d is not handled by the tcgen05 kernel", (long long)N, K, D);
-  // the tcgen05 kernel moves rows with bulk copies / 128-bit accesses: AUTO falls back to the FP32 kernel for a
-  // (valid) 4-byte-aligned view such as a contiguous tensor with an odd storage offset; an explicit DVQ_PATH_TC
-  // request errors in launch_vq_tc
+  // the tcgen05 kernel moves rows with bulk copies / 128-bit accesses: AUTO runs the FP32 kernel on a (valid)
+  // 4-byte-aligned view such as a contiguous tensor with an odd storage offset, an explicit DVQ_PATH_TC request fails
   const bool aligned16 = (reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(E) | reinterpret_cast<uintptr_t>(z_q)) % 16 == 0;
-  const bool use_tc = tc_ok && path != DVQ_PATH_SIMT && (aligned16 || path == DVQ_PATH_TC);
+  if (path == DVQ_PATH_TC && !aligned16) return fail(DVQ_ERR_BAD_ALIGN, "tcgen05 path needs 16-byte aligned z / E / z_q");
+  const bool use_tc = tc_ok && aligned16;
+
+  char* ws = static_cast<char*>(workspace);
+  VqCall c;
+  c.z = z; c.E = E; c.z_q = z_q; c.idx = idx; c.hist = hist; c.sse = sse;
+  c.N = N; c.K = K; c.D = D; c.train = train; c.zbf = zbf;
+  c.s = static_cast<cudaStream_t>(stream);
+  c.sm_count = dp.sm_count;
+  c.ee = reinterpret_cast<float*>(ws + w.off_ee);
+  c.counters = reinterpret_cast<int*>(ws + w.off_counters);
+  c.row_list = reinterpret_cast<int*>(ws + w.off_rowlist);
+  c.cand_list = reinterpret_cast<int*>(ws + w.off_candlist);
+  c.bop = ws + w.off_bop;
+  c.binned = ws + w.off_binned;
 
   const bool cached = (flags & DVQ_CODEBOOK_CACHED) != 0;   // the caller vouches for ee / CbMeta / operand image in the workspace
-  profile_mark(0, true, s);
-  if (!cached) rc = launch_code_norms(E, K, D, ee, s);
-  profile_mark(0, false, s);
+  profile_mark(0, true, c.s);
+  if (!cached) rc = launch_code_norms(E, K, D, c.ee, c.s);
+  profile_mark(0, false, c.s);
   if (rc) return rc;
-  if (N > 0) {
-    if (use_tc) {
-      int* counters = reinterpret_cast<int*>(ws + w.off_counters);
-      int* row_list = reinterpret_cast<int*>(ws + w.off_rowlist);
-      int* cand_list = reinterpret_cast<int*>(ws + w.off_rowlist + align_up(sizeof(int) * (size_t)N, 256));
-      profile_mark(1, true, s);
-      rc = launch_vq_tc(z, E, ee, N, K, D, train, z_q, idx, hist, sse, ws + w.off_bop, counters, row_list, cand_list,
-                        reinterpret_cast<int*>(ws + w.off_binned), (int)(vq_refine_binned_zero_bytes() / sizeof(int)), cached, zbf, s);
-      profile_mark(1, false, s);
-      if (rc) return rc;
-      // exact FP32 refine of the rows the filter flagged (device-side counts, no host sync), restricted to their recorded
-      // candidate sub-chunks.  Large codebooks: rows with too many candidates for the list record, and degenerate rows,
-      // sit in a second list stored downwards from the end of the same buffer and are re-evaluated against every code.
-      const bool list_mode = cand_list_mode(K);
-      const RefineList list{row_list, cand_list, counters + CNT_LISTED, list_mode ? row_list + (N - 1) : nullptr,
-                            list_mode ? counters + CNT_OVF : nullptr, list_mode};
-      // a mode set by dvq_vq_set_refine wins; under mode 0, DVQ_REFINE_PER_ROW (any value) selects the per-row kernel
-      static const int env_mode = getenv("DVQ_REFINE_PER_ROW") != nullptr ? 1 : 0;
-      const int set_mode = __atomic_load_n(&g_refine_mode, __ATOMIC_RELAXED);
-      profile_mark(2, true, s);
-      rc = launch_vq_refine_stage(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list, counters, ws + w.off_binned,
-                                  set_mode != 0 ? set_mode : env_mode, __atomic_load_n(&g_refine_pair_cap, __ATOMIC_RELAXED), zbf, s);
-      profile_mark(2, false, s);
-      if (rc) return rc;
-    } else {
-      profile_mark(1, true, s);
-      rc = launch_vq_simt(z, E, ee, N, K, D, train, z_q, idx, hist, sse, zbf, s);
-      profile_mark(1, false, s);
-      if (rc) return rc;
-    }
-    if (flags & DVQ_WRITE_ONEHOT) {
-      profile_mark(3, true, s);
-      rc = launch_onehot(idx, N, K, onehot, s);
-      profile_mark(3, false, s);
-      if (rc) return rc;
-    }
+  if (N == 0) return DVQ_OK;
+  profile_mark(1, true, c.s);
+  rc = use_tc ? launch_vq_tc(c, cached) : launch_vq_simt(c);
+  profile_mark(1, false, c.s);
+  if (rc) return rc;
+  if (use_tc) {
+    // a mode set by dvq_vq_set_refine wins; under mode 0, DVQ_REFINE_PER_ROW (any value) selects the per-row kernel
+    static const int env_mode = getenv("DVQ_REFINE_PER_ROW") != nullptr ? 1 : 0;
+    const int set_mode = __atomic_load_n(&g_refine_mode, __ATOMIC_RELAXED);
+    profile_mark(2, true, c.s);
+    rc = launch_vq_refine_stage(c, set_mode != 0 ? set_mode : env_mode, __atomic_load_n(&g_refine_pair_cap, __ATOMIC_RELAXED));
+    profile_mark(2, false, c.s);
+    if (rc) return rc;
+  }
+  if (flags & DVQ_WRITE_ONEHOT) {
+    profile_mark(3, true, c.s);
+    rc = launch_onehot(idx, N, K, onehot, c.s);
+    profile_mark(3, false, c.s);
+    if (rc) return rc;
   }
   return DVQ_OK;
 }
@@ -272,41 +274,12 @@ int dvq_vq_read_counters(const void* workspace, int64_t N, int K, int D, int fla
   int rc = check_vq_shape(N, K, D);
   if (rc) return rc;
   out4[0] = out4[1] = out4[2] = out4[3] = 0;
-  const bool use_tc = vq_tc_supported(N, K, D) && (flags & DVQ_PATH_MASK) != DVQ_PATH_SIMT;
-  if (!use_tc) return DVQ_OK;
+  if (!vq_tc_may_run(N, K, D, flags)) return DVQ_OK;
   const VqWorkspace w = vq_workspace_layout(N, K, D, flags);
-  DVQ_CUDA_CHECK(cudaMemcpy(out4, static_cast<const char*>(workspace) + w.off_counters, 4 * sizeof(int), cudaMemcpyDeviceToHost));
-  if (getenv("DVQ_TC_STATS_PRINT")) {
-    unsigned long long st[17];
-    DVQ_CUDA_CHECK(cudaMemcpy(st, static_cast<const char*>(workspace) + w.off_counters + CNT_STATS * sizeof(int), sizeof(st),
-                              cudaMemcpyDeviceToHost));
-    static const char* names[17] = {"producer.wait_stage_empty", "mma.wait_a_full", "mma.wait_acc_empty", "mma.total",
-                                    "conv.wait_stage_full", "conv.wait_a_empty", "conv.total", "epi0.wait_acc_full",
-                                    "epi4.wait_fin_empty", "epi0.wait_fin_full", "epi0.wait_sidx_empty", "epi0.total",
-                                    "gather.wait_sidx_full", "gather.total", "mma.wait_b_full", "(unused)", "mma.wait_peer_acc_empty"};
-    for (int i = 0; i < 17; ++i) fprintf(stderr, "[dvq tc stats] %-28s %14llu cycles (sum over CTAs)\n", names[i], st[i]);
-    if (N >= 65536) {   // pipeline timeline of CTA 3, tiles 8..11 (see TRACE in vq_tc_sm100.cu)
-      static long long tr[5 * 8 * 8];
-      DVQ_CUDA_CHECK(cudaMemcpy(tr, static_cast<const char*>(workspace) + w.off_rowlist + (size_t)(N - 8192) * sizeof(int), sizeof(tr),
-                                cudaMemcpyDeviceToHost));
-      static const char* ev[5][4] = {{"mma.a_full", "mma.acc_empty", "mma.issued", "mma.complete"},
-                                     {"own.acc_full", "own.chunk_done", "own.fin_full", "own.sidx_out"},
-                                     {"hlp.acc_full", "hlp.chunk_done", "hlp.fin_out", "hlp.stage_freed"},
-                                     {"cnv.stage_full", "cnv.pass1_done", "cnv.a_empty", "cnv.a_full_out"},
-                                     {"gth.sidx_full", "gth.done", "", ""}};
-      long long base = tr[(0 * 8 + 0) * 8 + 0];
-      for (int role = 0; role < 5; ++role)
-        for (int e = 0; e < 4; ++e) {
-          if (!ev[role][e][0]) continue;
-          fprintf(stderr, "[dvq tc trace] %-16s", ev[role][e]);
-          for (int k = 0; k < 8; ++k) {
-            const long long v = tr[(role * 8 + e) * 8 + k];
-            fprintf(stderr, " %7lld", v ? v - base : -1);
-          }
-          fprintf(stderr, "\n");
-        }
-    }
-  }
+  const char* ws = static_cast<const char*>(workspace);
+  DVQ_CUDA_CHECK(cudaMemcpy(out4, ws + w.off_counters, 4 * sizeof(int), cudaMemcpyDeviceToHost));
+  if (getenv("DVQ_TC_STATS_PRINT"))
+    return vq_tc_print_stats(reinterpret_cast<const int*>(ws + w.off_counters), reinterpret_cast<const int*>(ws + w.off_rowlist), N);
   return DVQ_OK;
 }
 

@@ -37,10 +37,12 @@ void profile_mark(int stage, bool begin, cudaStream_t s);  // no-op unless dvq_p
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // ---- workspace layout of dvq_vq_forward (all offsets 256-byte aligned) -------------------
+// The areas after the counters exist only when the tcgen05 path may run for the call.
 struct VqWorkspace {
   size_t off_ee;        // float [K]            ||e_k||^2
   size_t off_counters;  // int   [CNT_WORDS]    see CounterSlot
-  size_t off_rowlist;   // int   [2][N]         rows the tensor-core filter could not decide + their candidate records
+  size_t off_rowlist;   // int   [N]            rows the tensor-core filter could not decide (RefineList)
+  size_t off_candlist;  // int   [N]            their candidate records
   size_t off_bop;       // operand image of the codebook for the tcgen05 path
   size_t off_binned;    // bin tables + (row, sub-chunk) pair list of the binned refine (vq_refine_binned.cu)
   size_t total;
@@ -107,14 +109,41 @@ struct RefineList {
   bool list_mode;
 };
 
+// ---- one dvq_vq_forward call, as its launchers see it ------------------------------------
+// Filled once by dvq_vq_forward after validation; the workspace views are the VqWorkspace areas.
+struct VqCall {
+  const void* z;                // [N, D] fp32, or bf16 when zbf (DVQ_Z_BF16): every VQ kernel computes in fp32 on the upcast rows
+  const float* E;               // [K, D]
+  void* z_q;                    // [N, D], the type of z
+  int64_t* idx;                 // [N]
+  unsigned long long* hist;     // [K]   train only
+  double* sse;                  //       train only
+  int64_t N;
+  int K, D, train;
+  bool zbf;
+  cudaStream_t s;
+  int sm_count;                 // of the current device
+  float* ee;
+  int* counters;
+  int* row_list;
+  int* cand_list;
+  void* bop;
+  void* binned;
+};
+
+// f(z, z_q) with z / z_q typed as the call's element type: const float* / float*, or the __nv_bfloat16 pair
+template <typename F>
+int with_z_type(const VqCall& c, F&& f) {
+  if (c.zbf) return f(static_cast<const __nv_bfloat16*>(c.z), static_cast<__nv_bfloat16*>(c.z_q));
+  return f(static_cast<const float*>(c.z), static_cast<float*>(c.z_q));
+}
+
 // ---- kernels launched by the API layer ---------------------------------------------------
 // ee[k] = sum_d E[k,d]^2
 int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s);
 
 // Exact FP32 CUDA-core path over rows [0, N): every shape, the path when the tcgen05 kernel does not run.
-// zbf: z / z_q are bf16 rows (DVQ_Z_BF16), else fp32 — every VQ kernel below computes in fp32 on the upcast rows
-int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse, bool zbf, cudaStream_t s);
+int launch_vq_simt(const VqCall& c);
 
 // tcgen05 filter kernel (vq_tc_sm100.cu, whose plan_vq_tc makes every decision below); supported(N,K,D) says whether the shape is handled.
 bool vq_tc_supported(int64_t N, int K, int D);
@@ -122,32 +151,26 @@ size_t vq_tc_operand_bytes(int K, int D);
 // dvq_debug_tc_layout (kernel 0), _pair_layout (1), _layout_ex (-1); zbytes: size of a z element
 void vq_tc_plan_info(int64_t N, int K, int D, int zbytes, int kernel, int* out8);
 long long vq_tc_image_offset(int k, int d, int K, int D, int pair, long long* image_bytes);   // dvq_debug_tc_image_offset
-int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                 void* z_q, int64_t* idx, unsigned long long* hist, double* sse,
-                 void* bop, int* counters, int* row_list, int* cand_list, int* zero_ints, int zero_n,
-                 bool codebook_cached, bool zbf, cudaStream_t s);
+// z, E and z_q 16-byte aligned
+int launch_vq_tc(const VqCall& c, bool codebook_cached);
+// DVQ_TC_STATS_PRINT: prints the filter's wait-time sums and pipeline timeline, which DVQ_TC_STATS builds record
+int vq_tc_print_stats(const int* counters, const int* row_list, int64_t N);
 
 // The exact refine stage of the tcgen05 path (vq_refine.cu): re-evaluates the rows of the filter's refine list with the
-// refine kernels its plan picks for the shape.  mode and pair_cap as in dvq_vq_set_refine (0 = automatic / default);
-// binned_ws: the VqWorkspace::off_binned area.
-int launch_vq_refine_stage(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                           int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
-                           void* binned_ws, int mode, long long pair_cap, bool zbf, cudaStream_t s);
+// refine kernels its plan picks for the shape.  mode and pair_cap as in dvq_vq_set_refine (0 = automatic / default).
+int launch_vq_refine_stage(const VqCall& c, int mode, long long pair_cap);
 
 // code-stationary exact refine (vq_refine_stationary.cu): mask-mode codebooks whose K/32 warps hold e_dim code floats
 // per lane in registers
 bool vq_refine_stationary_supported(int K, int D);
-int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                                unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s);
+int launch_vq_refine_stationary(const VqCall& c, const RefineList& list);
 
 // binned exact refine (vq_refine_binned.cu): (row, sub-chunk) pairs bucketed by sub-chunk; hands the list to the per-row
 // kernel through counters[CNT_HANDBACK] / [CNT_HANDBACK_OVF] when the pairs do not fit min(pair_cap, 2 N) (pair_cap 0:
 // 2 N, the workspace's capacity)
 size_t vq_refine_binned_bytes(int64_t N);
 size_t vq_refine_binned_zero_bytes();
-int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                            int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
-                            void* ws, long long pair_cap, bool zbf, cudaStream_t s);
+int launch_vq_refine_binned(const VqCall& c, const RefineList& list, long long pair_cap);
 
 int launch_onehot(const int64_t* idx, int64_t N, int K, float* onehot, cudaStream_t s);
 int launch_finalize(const unsigned long long* hist, const double* sse, int64_t N, int K, int D, float al,

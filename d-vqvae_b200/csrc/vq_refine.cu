@@ -220,48 +220,37 @@ static bool codebook_in_smem(int K, int D) {
 }
 
 template <int DT, typename ZT>
-static int launch_refine_dt(const ZT* z, const float* E, const float* ee, int K, int train, ZT* z_q, int64_t* idx,
-                            unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
+static int launch_refine_dt(const ZT* z, ZT* z_q, const VqCall& c, const RefineList& list) {
   const size_t zbuf_bytes = (size_t)(RTHREADS / 32) * 2 * DT * sizeof(ZT);
-  const size_t smem_e = (size_t)K * (DT + 4) * sizeof(float);
-  const bool in_smem = codebook_in_smem(K, DT);
+  const size_t smem_e = (size_t)c.K * (DT + 4) * sizeof(float);
+  const bool in_smem = codebook_in_smem(c.K, DT);
 #define DVQ_LAUNCH_REFINE(TR_, SM_)                                                                                      \
   do {                                                                                                                   \
     const size_t bytes = zbuf_bytes + (SM_ ? smem_e : 0);                                                                \
     DVQ_CUDA_CHECK(cudaFuncSetAttribute(vq_refine_kernel<DT, TR_, SM_, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)); \
-    vq_refine_kernel<DT, TR_, SM_, ZT><<<sm_count, RTHREADS, bytes, s>>>(z, E, ee, K, z_q, idx, hist, sse, list);         \
+    vq_refine_kernel<DT, TR_, SM_, ZT><<<c.sm_count, RTHREADS, bytes, c.s>>>(z, c.E, c.ee, c.K, z_q, c.idx, c.hist, c.sse, list); \
   } while (0)
-  if (train) { if (in_smem) DVQ_LAUNCH_REFINE(true, true); else DVQ_LAUNCH_REFINE(true, false); }
-  else       { if (in_smem) DVQ_LAUNCH_REFINE(false, true); else DVQ_LAUNCH_REFINE(false, false); }
+  if (c.train) { if (in_smem) DVQ_LAUNCH_REFINE(true, true); else DVQ_LAUNCH_REFINE(true, false); }
+  else         { if (in_smem) DVQ_LAUNCH_REFINE(false, true); else DVQ_LAUNCH_REFINE(false, false); }
 #undef DVQ_LAUNCH_REFINE
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;
 }
 
-template <typename ZT>
-static int launch_refine_t(const ZT* z, const float* E, const float* ee, int K, int D, int train, ZT* z_q, int64_t* idx,
-                           unsigned long long* hist, double* sse, const RefineList& list, const DeviceProps& dp, cudaStream_t s) {
-  switch (D) {
-    case 16: return launch_refine_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
-    case 32: return launch_refine_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
-    case 64: return launch_refine_dt<64>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
-    case 128: return launch_refine_dt<128>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
-    case 256: return launch_refine_dt<256>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
-    case 512: return launch_refine_dt<512>(z, E, ee, K, train, z_q, idx, hist, sse, list, dp.sm_count, s);
-    default: return fail(DVQ_ERR_BAD_SHAPE, "candidate refine kernel is instantiated for e_dim 16..512 (powers of two) only");
-  }
-}
-
-static int launch_vq_refine(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                            unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {
-  DeviceProps dp;
-  int rc = device_props(&dp);
-  if (rc) return rc;
-  if (zbf)
-    return launch_refine_t(static_cast<const __nv_bfloat16*>(z), E, ee, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
-                           list, dp, s);
-  return launch_refine_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list, dp, s);
+// the per-row kernel on `list`: the filter's refine list, or the binned kernels' hand-back list
+static int launch_vq_refine(const VqCall& c, const RefineList& list) {
+  return with_z_type(c, [&](auto z, auto z_q) {
+    switch (c.D) {
+      case 16: return launch_refine_dt<16>(z, z_q, c, list);
+      case 32: return launch_refine_dt<32>(z, z_q, c, list);
+      case 64: return launch_refine_dt<64>(z, z_q, c, list);
+      case 128: return launch_refine_dt<128>(z, z_q, c, list);
+      case 256: return launch_refine_dt<256>(z, z_q, c, list);
+      case 512: return launch_refine_dt<512>(z, z_q, c, list);
+      default: return fail(DVQ_ERR_BAD_SHAPE, "candidate refine kernel is instantiated for e_dim 16..512 (powers of two) only");
+    }
+  });
 }
 
 // The refine plan.  The three refine kernels give identical results; the automatic choice (mode 0) takes the one that
@@ -276,21 +265,24 @@ static int launch_vq_refine(const void* z, const float* E, const float* ee, int 
 //  - otherwise binned, 2-5x faster than per-row reading its code rows from L2 (code rows register-resident per bucket).  The
 //    per-row kernel then runs on the hand-back list, which the binned kernels fill when their pairs do not fit the pair list
 //    (normally both hand-back counts stay zero and it exits at once).
-int launch_vq_refine_stage(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                           int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
-                           void* binned_ws, int mode, long long pair_cap, bool zbf, cudaStream_t s) {
+int launch_vq_refine_stage(const VqCall& c, int mode, long long pair_cap) {
+  // the filter's list: rows [0, counters[CNT_LISTED]) with their candidate records; in list mode (large codebooks) also the
+  // overflow list (too many candidates for a record, degenerate rows), stored downwards from the end of the row list
+  const bool lm = cand_list_mode(c.K);
+  const RefineList list{c.row_list, c.cand_list, c.counters + CNT_LISTED, lm ? c.row_list + (c.N - 1) : nullptr,
+                        lm ? c.counters + CNT_OVF : nullptr, lm};
   if (mode == 0) {
-    const bool stationary = vq_refine_stationary_supported(K, D) && K >= (D <= 64 ? 128 : 256);
-    mode = stationary ? 3 : codebook_in_smem(K, D) ? 1 : 2;
+    const bool stationary = vq_refine_stationary_supported(c.K, c.D) && c.K >= (c.D <= 64 ? 128 : 256);
+    mode = stationary ? 3 : codebook_in_smem(c.K, c.D) ? 1 : 2;
   }
-  if (mode == 3) return launch_vq_refine_stationary(z, E, ee, K, D, train, z_q, idx, hist, sse, list, zbf, s);
-  if (mode == 1) return launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, list, zbf, s);
-  const int rc = launch_vq_refine_binned(z, E, ee, N, K, D, train, z_q, idx, hist, sse, list, counters, binned_ws, pair_cap, zbf, s);
+  if (mode == 3) return launch_vq_refine_stationary(c, list);
+  if (mode == 1) return launch_vq_refine(c, list);
+  const int rc = launch_vq_refine_binned(c, list, pair_cap);
   if (rc) return rc;
   RefineList handback = list;
-  handback.n = counters + CNT_HANDBACK;
-  if (list.list_mode) handback.n_ovf = counters + CNT_HANDBACK_OVF;
-  return launch_vq_refine(z, E, ee, K, D, train, z_q, idx, hist, sse, handback, zbf, s);
+  handback.n = c.counters + CNT_HANDBACK;
+  if (lm) handback.n_ovf = c.counters + CNT_HANDBACK_OVF;
+  return launch_vq_refine(c, handback);
 }
 
 }  // namespace dvq

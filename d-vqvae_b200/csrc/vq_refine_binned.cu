@@ -383,19 +383,15 @@ size_t vq_refine_binned_bytes(int64_t N) {
 size_t vq_refine_binned_zero_bytes() { return sizeof(int) * 2 * MAX_BINS; }
 
 template <typename ZT>
-static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t N, int K, int D, int train, ZT* z_q,
-                           int64_t* idx, unsigned long long* hist, double* sse, const RefineList& L, int* counters, void* ws,
-                           long long pair_cap, cudaStream_t s) {
-  DeviceProps dp;
-  int rc = device_props(&dp);
-  if (rc) return rc;
+static int launch_binned_t(const ZT* z, ZT* z_q, const VqCall& c, const RefineList& L, long long pair_cap) {
+  const int K = c.K, D = c.D;
   if (K > 32 * MAX_BINS) return fail(DVQ_ERR_BAD_SHAPE, "binned refine handles K <= %d", 32 * MAX_BINS);
-  int* wi = static_cast<int*>(ws);
+  int* wi = static_cast<int*>(c.binned);
   BinTables bt;
   bt.count = wi; bt.cursor = wi + MAX_BINS; bt.start = wi + 2 * MAX_BINS; bt.item_start = wi + 3 * MAX_BINS + 1;
-  int* pairs = reinterpret_cast<int*>(static_cast<char*>(ws) + align_up(sizeof(int) * (size_t)(4 * MAX_BINS + 8), 256));
-  if (pair_cap <= 0 || pair_cap > 2 * (long long)N) pair_cap = 2 * (long long)N;   // the pair list holds 2 N entries
-  unsigned long long* idx64 = reinterpret_cast<unsigned long long*>(idx);
+  int* pairs = reinterpret_cast<int*>(static_cast<char*>(c.binned) + align_up(sizeof(int) * (size_t)(4 * MAX_BINS + 8), 256));
+  if (pair_cap <= 0 || pair_cap > 2 * (long long)c.N) pair_cap = 2 * (long long)c.N;   // the pair list holds 2 N entries
+  unsigned long long* idx64 = reinterpret_cast<unsigned long long*>(c.idx);
   // slice width of the pairs kernel: a lane keeps DS floats of its code row in registers.  DS = 64 (168 registers, one CTA
   // of 12 warps per SM) re-reads a code row half as often, DS = 32 (80 registers) fits two CTAs per SM: measured at
   // N = 2M-4M, refine stage: e_dim 128 / 256 / 512 at K = 16 384 / 16 384 / 4096: 0.60 -> 0.44, 1.85 -> 1.37, 2.32 -> 1.71 ms
@@ -404,19 +400,19 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
   static const char* ds_env = getenv("DVQ_REFINE_DS");
   const int ds_want = ds_env ? atoi(ds_env) : (D >= 128 ? 32 : 64);
   const int DS = D < 64 ? D : (ds_want == 32 ? 32 : 64);
-  const int pair_grid = dp.sm_count * (DS <= 32 && D >= 64 ? 2 : 1);
+  const int pair_grid = c.sm_count * (DS <= 32 && D >= 64 ? 2 : 1);
   const int pair_warps = pair_grid * (PAIR_THREADS / 32);
 
-  refine_prep_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(z, D, K, z_q, idx64, L, counters, bt);
+  refine_prep_kernel<<<c.sm_count, PREP_THREADS, 0, c.s>>>(z, D, K, z_q, idx64, L, c.counters, bt);
   DVQ_CUDA_CHECK(cudaGetLastError());
-  refine_scatter_kernel<<<dp.sm_count, PREP_THREADS, 0, s>>>(K, L, counters, bt, pairs, pair_cap, pair_warps);
+  refine_scatter_kernel<<<c.sm_count, PREP_THREADS, 0, c.s>>>(K, L, c.counters, bt, pairs, pair_cap, pair_warps);
   DVQ_CUDA_CHECK(cudaGetLastError());
   const size_t smem = (size_t)(PAIR_THREADS / 32) * (2 * RB * DS * sizeof(ZT) + (D > DS ? 32 * (DS + 4) * sizeof(float) : 0));
 #define DVQ_LAUNCH_PAIRS(DS_)                                                                                              \
   do {                                                                                                                     \
     DVQ_CUDA_CHECK(cudaFuncSetAttribute(refine_pairs_kernel<DS_, ZT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    refine_pairs_kernel<DS_, ZT><<<pair_grid, PAIR_THREADS, smem, s>>>(z, E, ee, K, D, z_q, idx64, L, pairs, counters, bt,      \
-                                                                   pair_cap);                                              \
+    refine_pairs_kernel<DS_, ZT><<<pair_grid, PAIR_THREADS, smem, c.s>>>(z, c.E, c.ee, K, D, z_q, idx64, L, pairs, c.counters, \
+                                                                     bt, pair_cap);                                        \
   } while (0)
   if (DS == 64) DVQ_LAUNCH_PAIRS(64);
   else if (DS == 32) DVQ_LAUNCH_PAIRS(32);
@@ -424,23 +420,17 @@ static int launch_binned_t(const ZT* z, const float* E, const float* ee, int64_t
   else return fail(DVQ_ERR_BAD_SHAPE, "binned refine needs e_dim 16, 32 or a multiple of 64");
 #undef DVQ_LAUNCH_PAIRS
   DVQ_CUDA_CHECK(cudaGetLastError());
-  if (train)
-    refine_emit_kernel<true, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, L, counters, pair_cap);
+  if (c.train)
+    refine_emit_kernel<true, ZT><<<c.sm_count, PREP_THREADS, 0, c.s>>>(z, c.E, D, z_q, idx64, c.hist, c.sse, L, c.counters, pair_cap);
   else
-    refine_emit_kernel<false, ZT><<<dp.sm_count, PREP_THREADS, 0, s>>>(z, E, D, z_q, idx64, hist, sse, L, counters, pair_cap);
+    refine_emit_kernel<false, ZT><<<c.sm_count, PREP_THREADS, 0, c.s>>>(z, c.E, D, z_q, idx64, c.hist, c.sse, L, c.counters, pair_cap);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch(4);
   return DVQ_OK;
 }
 
-int launch_vq_refine_binned(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                            int64_t* idx, unsigned long long* hist, double* sse, const RefineList& list, int* counters,
-                            void* ws, long long pair_cap, bool zbf, cudaStream_t s) {
-  if (zbf)
-    return launch_binned_t(static_cast<const __nv_bfloat16*>(z), E, ee, N, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist, sse,
-                           list, counters, ws, pair_cap, s);
-  return launch_binned_t(static_cast<const float*>(z), E, ee, N, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list, counters,
-                         ws, pair_cap, s);
+int launch_vq_refine_binned(const VqCall& c, const RefineList& list, long long pair_cap) {
+  return with_z_type(c, [&](auto z, auto z_q) { return launch_binned_t(z, z_q, c, list, pair_cap); });
 }
 
 }  // namespace dvq

@@ -202,30 +202,17 @@ vq_refine_stationary_kernel(const ZT* __restrict__ z, const float* __restrict__ 
 }
 
 template <int DT, typename ZT>
-int launch_stationary_dt(const ZT* z, const float* E, const float* ee, int K, int train, ZT* z_q, int64_t* idx,
-                         unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
+int launch_stationary_dt(const ZT* z, ZT* z_q, const VqCall& c, const RefineList& list) {
   auto kern = vq_refine_stationary_kernel<DT, ZT>;
-  const int threads = K;   // one warp per 32-code sub-chunk
-  const size_t bytes = (size_t)2 * SB * DT * sizeof(ZT) + (size_t)(K / 32) * SB * sizeof(unsigned long long);
+  const int threads = c.K;   // one warp per 32-code sub-chunk
+  const size_t bytes = (size_t)2 * SB * DT * sizeof(ZT) + (size_t)(c.K / 32) * SB * sizeof(unsigned long long);
   DVQ_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   int per_sm = 0;   // small codebooks (few warps) fit several CTAs per SM
   DVQ_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, bytes));
-  kern<<<sm_count * (per_sm > 0 ? per_sm : 1), threads, bytes, s>>>(z, E, ee, K, train, z_q, idx, hist, sse, list);
+  kern<<<c.sm_count * (per_sm > 0 ? per_sm : 1), threads, bytes, c.s>>>(z, c.E, c.ee, c.K, c.train, z_q, c.idx, c.hist, c.sse, list);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;
-}
-
-template <typename ZT>
-int launch_stationary_t(const ZT* z, const float* E, const float* ee, int K, int D, int train, ZT* z_q, int64_t* idx,
-                        unsigned long long* hist, double* sse, const RefineList& list, int sm_count, cudaStream_t s) {
-  switch (D) {
-    case 16: return launch_stationary_dt<16>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
-    case 32: return launch_stationary_dt<32>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
-    case 64: return launch_stationary_dt<64>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
-    case 128: return launch_stationary_dt<128>(z, E, ee, K, train, z_q, idx, hist, sse, list, sm_count, s);
-    default: return fail(DVQ_ERR_BAD_SHAPE, "code-stationary refine kernel is instantiated for e_dim 16..128 only");
-  }
 }
 
 }  // namespace
@@ -242,18 +229,18 @@ bool vq_refine_stationary_supported(int K, int D) {
   return !cand_list_mode(K) && K % 32 == 0 && K >= 32 && K / 32 <= max_warps;
 }
 
-int launch_vq_refine_stationary(const void* z, const float* E, const float* ee, int K, int D, int train, void* z_q, int64_t* idx,
-                                unsigned long long* hist, double* sse, const RefineList& list, bool zbf, cudaStream_t s) {
-  if (!vq_refine_stationary_supported(K, D))
-    return fail(DVQ_ERR_BAD_SHAPE, "code-stationary refine: K=%d, e_dim %d does not fit (mask-mode K with K/32 warps x e_dim registers)", K, D);
-  DeviceProps dp;
-  int rc = device_props(&dp);
-  if (rc) return rc;
-  if (zbf)
-    return launch_stationary_t(static_cast<const __nv_bfloat16*>(z), E, ee, K, D, train, static_cast<__nv_bfloat16*>(z_q), idx, hist,
-                               sse, list, dp.sm_count, s);
-  return launch_stationary_t(static_cast<const float*>(z), E, ee, K, D, train, static_cast<float*>(z_q), idx, hist, sse, list,
-                             dp.sm_count, s);
+int launch_vq_refine_stationary(const VqCall& c, const RefineList& list) {
+  if (!vq_refine_stationary_supported(c.K, c.D))
+    return fail(DVQ_ERR_BAD_SHAPE, "code-stationary refine: K=%d, e_dim %d does not fit (mask-mode K with K/32 warps x e_dim registers)", c.K, c.D);
+  return with_z_type(c, [&](auto z, auto z_q) {
+    switch (c.D) {
+      case 16: return launch_stationary_dt<16>(z, z_q, c, list);
+      case 32: return launch_stationary_dt<32>(z, z_q, c, list);
+      case 64: return launch_stationary_dt<64>(z, z_q, c, list);
+      case 128: return launch_stationary_dt<128>(z, z_q, c, list);
+      default: return fail(DVQ_ERR_BAD_SHAPE, "code-stationary refine kernel is instantiated for e_dim 16..128 only");
+    }
+  });
 }
 
 }  // namespace dvq

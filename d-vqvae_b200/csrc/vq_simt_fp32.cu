@@ -11,6 +11,8 @@
 // 8x8 register tile split 4+4 (rows ty*4.., 64+ty*4..; codes tx*4.., 64+tx*4..) so every
 // shared-memory read is a conflict-free 128-bit load.  Roofline: FP32 FMA pipe
 // (2*N*K*D flop); it is the *fallback*, the tensor path is the fast one.
+#include <type_traits>
+
 #include "vq_exact.cuh"
 
 namespace dvq {
@@ -215,24 +217,20 @@ int launch_code_norms(const float* E, int K, int D, float* ee, cudaStream_t s) {
   return DVQ_OK;
 }
 
-int launch_vq_simt(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train,
-                   void* z_q, int64_t* idx, unsigned long long* hist, double* sse, bool zbf, cudaStream_t s) {
-  DeviceProps dp;
-  int rc = device_props(&dp);
-  if (rc) return rc;
-  const int64_t tiles = (N + BM - 1) / BM;
-  int64_t grid = (int64_t)dp.sm_count * 2;
+int launch_vq_simt(const VqCall& c) {
+  const int64_t tiles = (c.N + BM - 1) / BM;
+  int64_t grid = (int64_t)c.sm_count * 2;
   if (tiles < grid) grid = tiles;
   if (grid < 1) grid = 1;
   // 128-bit codebook loads; z / z_q rows move 4 elements at a time (16 bytes fp32, 8 bytes bf16)
-  const bool vec = (D % 4 == 0) && reinterpret_cast<uintptr_t>(E) % 16 == 0 &&
-                   (reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(z_q)) % (zbf ? 8 : 16) == 0;
-#define DVQ_LAUNCH_SIMT(V_, T_)                                                                                             \
-  vq_simt_kernel<V_, T_><<<(unsigned)grid, NTHREADS, 0, s>>>(static_cast<const T_*>(z), E, ee, N, K, D, train,          \
-                                                             static_cast<T_*>(z_q), idx, hist, sse)
-  if (zbf) { if (vec) DVQ_LAUNCH_SIMT(true, __nv_bfloat16); else DVQ_LAUNCH_SIMT(false, __nv_bfloat16); }
-  else     { if (vec) DVQ_LAUNCH_SIMT(true, float); else DVQ_LAUNCH_SIMT(false, float); }
-#undef DVQ_LAUNCH_SIMT
+  const bool vec = (c.D % 4 == 0) && reinterpret_cast<uintptr_t>(c.E) % 16 == 0 &&
+                   (reinterpret_cast<uintptr_t>(c.z) | reinterpret_cast<uintptr_t>(c.z_q)) % (c.zbf ? 8 : 16) == 0;
+  with_z_type(c, [&](auto z, auto z_q) {
+    using ZT = std::remove_pointer_t<decltype(z_q)>;
+    auto kern = vec ? vq_simt_kernel<true, ZT> : vq_simt_kernel<false, ZT>;
+    kern<<<(unsigned)grid, NTHREADS, 0, c.s>>>(z, c.E, c.ee, c.N, c.K, c.D, c.train, z_q, c.idx, c.hist, c.sse);
+    return DVQ_OK;
+  });
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;

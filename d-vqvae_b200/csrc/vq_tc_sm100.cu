@@ -439,7 +439,7 @@ __device__ __forceinline__ void wait_or_trap_cluster(uint32_t bar, uint32_t pari
 #define STAT_FLUSH(n, base)
 #endif
 // Pipeline timeline (DVQ_TC_STATS builds): clock64 stamps of one CTA for tiles 8..11, written to the unused
-// tail of the refine row list (role, event, tile, chunk); printed by dvq_vq_read_counters.
+// tail of the refine row list (role, event, tile, chunk).  vq_tc_print_stats prints both (DVQ_TC_STATS_PRINT).
 #ifdef DVQ_TC_STATS
 #define TRACE(role, ev, c_)                                                                                         \
   do {                                                                                                              \
@@ -449,6 +449,42 @@ __device__ __forceinline__ void wait_or_trap_cluster(uint32_t bar, uint32_t pari
 #else
 #define TRACE(role, ev, c_)
 #endif
+
+}  // namespace
+
+int vq_tc_print_stats(const int* counters, const int* row_list, int64_t N) {
+  unsigned long long st[17];
+  DVQ_CUDA_CHECK(cudaMemcpy(st, counters + CNT_STATS, sizeof(st), cudaMemcpyDeviceToHost));
+  // the STAT_ADD sites, in the order of the STAT_FLUSH slots
+  static const char* names[17] = {"producer.wait_stage_empty", "mma.wait_a_full", "mma.wait_acc_empty", "mma.total",
+                                  "conv.wait_stage_full", "conv.wait_a_empty", "conv.total", "epi0.wait_acc_full",
+                                  "epi4.wait_fin_empty", "epi0.wait_fin_full", "epi0.wait_sidx_empty", "epi0.total",
+                                  "gather.wait_sidx_full", "gather.total", "mma.wait_b_full", "(unused)", "mma.wait_peer_acc_empty"};
+  for (int i = 0; i < 17; ++i) fprintf(stderr, "[dvq tc stats] %-28s %14llu cycles (sum over CTAs)\n", names[i], st[i]);
+  if (N >= 65536) {   // the TRACE timeline, [role][event][tile 8..11][chunk]
+    static long long tr[5 * 8 * 8];
+    DVQ_CUDA_CHECK(cudaMemcpy(tr, row_list + (N - 8192), sizeof(tr), cudaMemcpyDeviceToHost));
+    static const char* ev[5][4] = {{"mma.a_full", "mma.acc_empty", "mma.issued", "mma.complete"},
+                                   {"own.acc_full", "own.chunk_done", "own.fin_full", "own.sidx_out"},
+                                   {"hlp.acc_full", "hlp.chunk_done", "hlp.fin_out", "hlp.stage_freed"},
+                                   {"cnv.stage_full", "cnv.pass1_done", "cnv.a_empty", "cnv.a_full_out"},
+                                   {"gth.sidx_full", "gth.done", "", ""}};
+    long long base = tr[(0 * 8 + 0) * 8 + 0];
+    for (int role = 0; role < 5; ++role)
+      for (int e = 0; e < 4; ++e) {
+        if (!ev[role][e][0]) continue;
+        fprintf(stderr, "[dvq tc trace] %-16s", ev[role][e]);
+        for (int k = 0; k < 8; ++k) {
+          const long long v = tr[(role * 8 + e) * 8 + k];
+          fprintf(stderr, " %7lld", v ? v - base : -1);
+        }
+        fprintf(stderr, "\n");
+      }
+  }
+  return DVQ_OK;
+}
+
+namespace {
 
 // float(h) - a in one FHADD (PTX mixed-precision sub, sm_100+): h is one half of a packed pair
 __device__ __forceinline__ float half_minus_float(uint32_t h16, float a) {
@@ -1629,38 +1665,34 @@ static int launch_planned(const TcPlan& P, const TcParams& p, unsigned grid, siz
   return P.pair ? launch_generic<TRAIN, false, true, ZT>(P.variant, p, grid, smem, s) : launch_generic<TRAIN, false, false, ZT>(P.variant, p, grid, smem, s);
 }
 
-int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int K, int D, int train, void* z_q,
-                 int64_t* idx, unsigned long long* hist, double* sse, void* bop, int* counters, int* row_list,
-                 int* cand_list, int* zero_ints, int zero_n, bool codebook_cached, bool zbf, cudaStream_t s) {
-  DeviceProps dp;
-  int rc = device_props(&dp);
-  if (rc) return rc;
-  if ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(E) | reinterpret_cast<uintptr_t>(z_q)) % 16 != 0)
-    return fail(DVQ_ERR_BAD_ALIGN, "tcgen05 path needs 16-byte aligned z / E / z_q");
-  const int zbytes = zbf ? 2 : 4;
-  const TcPlan P = plan_vq_tc(N, K, D, zbytes);
-  CbMeta* cb = static_cast<CbMeta*>(bop);
-  uint8_t* bimg = static_cast<uint8_t*>(bop) + align_up(sizeof(CbMeta), 256);
+int launch_vq_tc(const VqCall& c, bool codebook_cached) {
+  const int zbytes = c.zbf ? 2 : 4;
+  const TcPlan P = plan_vq_tc(c.N, c.K, c.D, zbytes);
+  CbMeta* cb = static_cast<CbMeta*>(c.bop);
+  uint8_t* bimg = static_cast<uint8_t*>(c.bop) + align_up(sizeof(CbMeta), 256);
+  int* zero_ints = static_cast<int*>(c.binned);   // the bin tables of the binned refine, zeroed on every call
+  const int zero_n = (int)(vq_refine_binned_zero_bytes() / sizeof(int));
   if (codebook_cached) {
     // DVQ_CODEBOOK_CACHED: CbMeta and the operand image in `bop` are those of this codebook; only the per-call
     // counters and bin tables are reset
-    tc_reset_kernel<<<1, 256, 0, s>>>(counters, zero_ints, zero_n);
+    tc_reset_kernel<<<1, 256, 0, c.s>>>(c.counters, zero_ints, zero_n);
     DVQ_CUDA_CHECK(cudaGetLastError());
     count_launch();
   } else {
-    tc_cb_stats_kernel<<<1, 256, 0, s>>>(ee, K, D, cb, counters, zero_ints, zero_n, P.pair);
+    tc_cb_stats_kernel<<<1, 256, 0, c.s>>>(c.ee, c.K, c.D, cb, c.counters, zero_ints, zero_n, P.pair);
     DVQ_CUDA_CHECK(cudaGetLastError());
-    DVQ_CUDA_CHECK(cudaMemsetAsync(bimg, 0, P.image_bytes, s));
-    tc_cb_image_kernel<<<(K * 32 + 255) / 256, 256, 0, s>>>(E, ee, K, D, cb, bimg, P.pair);
+    DVQ_CUDA_CHECK(cudaMemsetAsync(bimg, 0, P.image_bytes, c.s));
+    tc_cb_image_kernel<<<(c.K * 32 + 255) / 256, 256, 0, c.s>>>(c.E, c.ee, c.K, c.D, cb, bimg, P.pair);
     DVQ_CUDA_CHECK(cudaGetLastError());
     count_launch(2);
   }
 
+  int rc = DVQ_OK;
   TcParams p;
   memset(&p.ztile, 0, sizeof(p.ztile));
-  if (D > DSLICE) {   // z [N, D] row-major, box (slice columns, TM rows): a slice of a row tile lands as [row][ds elements], as the converters read it
-    rc = encode_2d(&p.ztile, zbf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, z, (uint64_t)D, (uint64_t)N,
-                   (uint64_t)D * zbytes, P.L.ds, TM);
+  if (c.D > DSLICE) {   // z [N, D] row-major, box (slice columns, TM rows): a slice of a row tile lands as [row][ds elements], as the converters read it
+    rc = encode_2d(&p.ztile, c.zbf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, c.z, (uint64_t)c.D, (uint64_t)c.N,
+                   (uint64_t)c.D * zbytes, P.L.ds, TM);
     if (rc) return rc;
   }
   memset(p.bmap, 0, sizeof(p.bmap));
@@ -1669,19 +1701,21 @@ int launch_vq_tc(const void* z, const float* E, const float* ee, int64_t N, int 
     if (!rc) rc = encode_2d(&p.bmap[1], CU_TENSOR_MAP_DATA_TYPE_INT32, bimg, 256, P.image_bytes / 1024, 1024, 256, P.L.bchunk_bytes / 1024);
     if (rc) return rc;
   }
-  p.z = z; p.E = E; p.bimg = bimg; p.cb = cb; p.N = N; p.K = K; p.D = D; p.train = train;
-  p.zq = z_q; p.idx = idx; p.hist = hist; p.sse = sse; p.counters = counters; p.row_list = row_list; p.cand_list = cand_list;
+  p.z = c.z; p.E = c.E; p.bimg = bimg; p.cb = cb; p.N = c.N; p.K = c.K; p.D = c.D; p.train = c.train;
+  p.zq = c.z_q; p.idx = c.idx; p.hist = c.hist; p.sse = c.sse; p.counters = c.counters; p.row_list = c.row_list; p.cand_list = c.cand_list;
   p.layout_ovr = P.layout_ovr;
-  p.stats = reinterpret_cast<unsigned long long*>(counters + CNT_STATS);
-  p.ntiles = (N + TM - 1) / TM;
+  p.stats = reinterpret_cast<unsigned long long*>(c.counters + CNT_STATS);
+  p.ntiles = (c.N + TM - 1) / TM;
   const size_t smem = P.L.total + 128;
-  int64_t grid = p.ntiles < dp.sm_count ? p.ntiles : dp.sm_count;
+  int64_t grid = p.ntiles < c.sm_count ? p.ntiles : c.sm_count;
   if (P.pair) {   // clusters of two CTAs: one per tile pair, at most one per TPC
     const int64_t units = (p.ntiles + 1) / 2;
-    grid = 2 * (units < dp.sm_count / 2 ? units : dp.sm_count / 2);
+    grid = 2 * (units < c.sm_count / 2 ? units : c.sm_count / 2);
   }
-  if (zbf) rc = train ? launch_planned<true, __nv_bfloat16>(P, p, (unsigned)grid, smem, s) : launch_planned<false, __nv_bfloat16>(P, p, (unsigned)grid, smem, s);
-  else rc = train ? launch_planned<true, float>(P, p, (unsigned)grid, smem, s) : launch_planned<false, float>(P, p, (unsigned)grid, smem, s);
+  rc = with_z_type(c, [&](auto, auto z_q) {
+    using ZT = std::remove_pointer_t<decltype(z_q)>;
+    return c.train ? launch_planned<true, ZT>(P, p, (unsigned)grid, smem, c.s) : launch_planned<false, ZT>(P, p, (unsigned)grid, smem, c.s);
+  });
   if (rc) return rc;
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
