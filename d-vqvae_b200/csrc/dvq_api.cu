@@ -419,6 +419,46 @@ int dvq_vertex_normals(const float* verts, int B, int V, const int* faces, int F
   return launch_vertex_normals(verts, B, V, faces, vf_offsets, vf_faces, normals, static_cast<cudaStream_t>(stream));
 }
 
+// The mesh kernels index within a call in 32 bits.  Bm and Bp are each 1 or B (B = the other one when one of them is 1),
+// the mesh's and the queries' [n, V or Q, 3] tensors, the [B, Q] outputs and faces [F, 3] must each have fewer than 2^31
+// elements.  On success *B is the broadcast batch.
+static int check_mesh_shape(int Bm, int V, int F, int Bp, int Q, int* B) {
+  if (Bm < 0 || Bp < 0 || V <= 0 || F < 0 || Q < 0)
+    return fail(DVQ_ERR_BAD_SHAPE, "need Bm >= 0, Bp >= 0, V > 0, F >= 0, Q >= 0 (got Bm=%d Bp=%d V=%d F=%d Q=%d)", Bm, Bp, V, F, Q);
+  *B = Bm == 1 ? Bp : Bm;
+  if (Bp != *B && Bp != 1) return fail(DVQ_ERR_BAD_SHAPE, "Bm and Bp must each be 1 or the batch size (got Bm=%d Bp=%d)", Bm, Bp);
+  if ((long long)Bm * V * 3 >= (1LL << 31) || (long long)Bp * Q * 3 >= (1LL << 31) || (long long)*B * Q * 3 >= (1LL << 31) ||
+      (long long)F * 3 >= (1LL << 31))
+    return fail(DVQ_ERR_BAD_SHAPE, "Bm * V * 3, Bp * Q * 3, B * Q * 3 and F * 3 must be below 2^31; split the batch");
+  return DVQ_OK;
+}
+
+int dvq_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, float* w,
+                     int* inside_count, void* stream) {
+  int B = 0;
+  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  if (rc) return rc;
+  if (!w && !inside_count) return fail(DVQ_ERR_BAD_ARG, "w and inside_count must not both be NULL");
+  if ((long long)B * Q > 0 && (!verts || !pts || (F > 0 && !faces)))   // empty tensors may have NULL data pointers
+    return fail(DVQ_ERR_BAD_ARG, "verts, faces and pts must not be NULL");
+  rc = require_sm100();
+  if (rc) return rc;
+  return launch_mesh_winding(verts, Bm, V, faces, F, pts, Bp, Q, B, w, inside_count, static_cast<cudaStream_t>(stream));
+}
+
+int dvq_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, float* dist2,
+                      int64_t* face, void* stream) {
+  int B = 0;
+  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  if (rc) return rc;
+  if (F == 0) return fail(DVQ_ERR_BAD_SHAPE, "dvq_mesh_distance needs F > 0");
+  if ((long long)B * Q > 0 && (!verts || !faces || !pts || !dist2 || !face))
+    return fail(DVQ_ERR_BAD_ARG, "verts, faces, pts, dist2 and face must not be NULL");
+  rc = require_sm100();
+  if (rc) return rc;
+  return launch_mesh_distance(verts, Bm, V, faces, F, pts, Bp, Q, B, dist2, face, static_cast<cudaStream_t>(stream));
+}
+
 int dvq_pcnn_gemm(const DvqPcnnGemm* g, void* stream) {
   int rc = require_sm100();
   if (rc) return rc;

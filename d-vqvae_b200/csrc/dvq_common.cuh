@@ -207,6 +207,12 @@ int launch_nn_backward(const float* src, const float* trg, const int64_t* idx, c
 int launch_vertex_normals(const float* verts, int B, int V, const int* faces, const int* vf_offsets, const int* vf_faces,
                           float* normals, cudaStream_t s);
 
+// mesh winding numbers and point-to-mesh distances (mesh_sm100.cu); B = the broadcast batch of Bm and Bp
+int launch_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B, float* w,
+                        int* inside_count, cudaStream_t s);
+int launch_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
+                         float* dist2, int64_t* face, cudaStream_t s);
+
 // PointNet
 size_t pointnet_workspace_bytes(int B, int C, int P, int flags);
 int launch_pointnet(const float* x, const DvqPointNetWeights* w, int B, int C, int P, int flags, float* feat,

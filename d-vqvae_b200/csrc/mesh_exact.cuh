@@ -1,0 +1,110 @@
+// The FP32 contract of the mesh kernels (mesh_sm100.cu): generalised winding number, point-to-mesh distance and the grasp
+// metrics built on them.  oracle/mesh_oracle.py restates it in float64 numpy; the tests compare the kernels with that
+// restatement within bars that cover the fp32 rounding of the arithmetic below.
+//
+// A mesh is fp32 vertices [V, 3] plus int32 faces [F, 3].  A face with a vertex id outside [0, V) contributes nothing.
+//
+//   winding    a = fl(v0 - q), b = fl(v1 - q), c = fl(v2 - q) (componentwise),
+//              Omega_f = 2 atan2(a . (b x c), |a||b||c| + (a . b)|c| + (b . c)|a| + (c . a)|b|) (Van Oosterom-Strackee),
+//              w(q) = fl(S / fl(4 pi)), S = the sum of Omega_f over ascending f from +0, one fp32 add per face, in the query's
+//              owner thread (deterministic).  atan2f / sqrtf are CUDA's accurate functions, not fast-math intrinsics.
+//              For an outward-oriented closed mesh w = 1 inside and 0 outside (-1 inside a flipped one).
+//   inside     w >= 0.5, the robust rule for open meshes such as MANO's hand (open at the wrist).  NaN is outside.
+//   box rule   a query outside the axis-aligned box of its mesh item's V vertices gets w = 0 without being evaluated: exact
+//              for a closed mesh, and what makes the kernel's culling legal.  The box is the per-axis min / max over the
+//              item's vertices with NaN coordinates ignored (fminf / fmaxf); a query is inside it when lo <= q <= hi holds on
+//              every axis, so a NaN query is outside.
+//   distance   dist2(q) = min over f of the squared distance from q to the closest point of triangle f (Ericson, Real-Time
+//              Collision Detection 5.1.5, written as closest = a + v ab + w ac, dist2 = |ap - v ab - w ac|^2).  A triangle
+//              whose fp32 area^2 = |ab x ac|^2 is 0 is taken as its three edge segments (no 0/0 in the interior region).
+//   face       the lowest f among exact fp32 minima of dist2; NaN counts as +inf (so a triangle with a non-finite corner
+//              never wins).  When no face gives a finite distance, face = 0 and dist2 = +inf.
+//
+// Grasp metrics of hand b against one object (dvq.GraspQuality; the last reductions are device-side torch on the kernels'
+// outputs):
+//   voxels     lo = the object's vertex min, n = max(1, ceil((hi - lo) / pitch)) cells per axis (sized on the host once),
+//              centre c = fl(lo + fl((i + 0.5) pitch)), kept when inside the object: an fp32 list [M, 3] in (i, j, k) order,
+//              k fastest, so consecutive query tiles are spatially compact (and mostly culled by the box rule).
+//   volume[b]  = count[b] pitch^3, count[b] = the number of voxel centres inside hand b (one integer atomicAdd per CTA).
+//   depth[b]   = max of sqrt(dist2) over the hand vertices inside the object, 0 if there are none.
+//   contact[b] = some hand vertex is inside the object or has dist2 <= contact_tol^2.
+#pragma once
+
+#include <math.h>
+
+#include "f32x2.cuh"
+
+namespace dvq {
+
+constexpr float MESH_4PI = 12.566370614359172f;     // fl(4 pi)
+
+__device__ __forceinline__ uint64_t dot2(uint64_t ax, uint64_t ay, uint64_t az, uint64_t bx, uint64_t by, uint64_t bz) {
+  return ffma2(az, bz, ffma2(ay, by, fmul2(ax, bx)));
+}
+
+// Omega_f of one face for two queries at once: packed corner offsets a = fl(v0 - q), b, c of the two queries
+__device__ __forceinline__ void solid_angle2(uint64_t ax, uint64_t ay, uint64_t az, uint64_t bx, uint64_t by, uint64_t bz,
+                                             uint64_t cx, uint64_t cy, uint64_t cz, float& o0, float& o1) {
+  const uint64_t rx = fsub2(fmul2(by, cz), fmul2(bz, cy));
+  const uint64_t ry = fsub2(fmul2(bz, cx), fmul2(bx, cz));
+  const uint64_t rz = fsub2(fmul2(bx, cy), fmul2(by, cx));
+  const uint64_t det = dot2(ax, ay, az, rx, ry, rz);
+  float a0, a1, b0, b1, c0, c1;
+  unpack_f32x2(dot2(ax, ay, az, ax, ay, az), a0, a1);
+  unpack_f32x2(dot2(bx, by, bz, bx, by, bz), b0, b1);
+  unpack_f32x2(dot2(cx, cy, cz, cx, cy, cz), c0, c1);
+  const uint64_t la = pack_f32x2(sqrtf(a0), sqrtf(a1)), lb = pack_f32x2(sqrtf(b0), sqrtf(b1)), lc = pack_f32x2(sqrtf(c0), sqrtf(c1));
+  const uint64_t den = ffma2(dot2(cx, cy, cz, ax, ay, az), lb,
+                             ffma2(dot2(bx, by, bz, cx, cy, cz), la, ffma2(dot2(ax, ay, az, bx, by, bz), lc, fmul2(fmul2(la, lb), lc))));
+  float d0, d1, n0, n1;
+  unpack_f32x2(det, n0, n1);
+  unpack_f32x2(den, d0, d1);
+  o0 = 2.f * atan2f(n0, d0);
+  o1 = 2.f * atan2f(n1, d1);
+}
+
+// Ericson's region cascade for one query: (v, w) of the closest point a + v ab + w ac, from d1 = ab . ap, d2 = ac . ap and
+// the face's aa = ab . ab, cc = ac . ac, bc = ab . ac (so d3 = ab . bp = d1 - aa, d4 = ac . bp = d2 - bc, d5 = ab . cp =
+// d1 - bc, d6 = ac . cp = d2 - cc).  A NaN anywhere falls through to the interior case and gives NaN.
+__device__ __forceinline__ void closest_vw(float d1, float d2, float aa, float cc, float bc, float& v, float& w) {
+  const float d3 = d1 - aa, d4 = d2 - bc, d5 = d1 - bc, d6 = d2 - cc;
+  const float vc = d1 * d4 - d3 * d2, vb = d5 * d2 - d1 * d6, va = d3 * d6 - d5 * d4;
+  float nv, nw, den = 1.f;
+  if (d1 <= 0.f && d2 <= 0.f) {                              // vertex a
+    nv = 0.f, nw = 0.f;
+  } else if (d3 >= 0.f && d4 <= d3) {                        // vertex b
+    nv = 1.f, nw = 0.f;
+  } else if (vc <= 0.f && d1 >= 0.f && d3 <= 0.f) {          // edge ab
+    nv = d1, nw = 0.f, den = d1 - d3;
+  } else if (d6 >= 0.f && d5 <= d6) {                        // vertex c
+    nv = 0.f, nw = 1.f;
+  } else if (vb <= 0.f && d2 >= 0.f && d6 <= 0.f) {          // edge ac
+    nv = 0.f, nw = d2, den = d2 - d6;
+  } else if (va <= 0.f && d4 - d3 >= 0.f && d5 - d6 >= 0.f) {  // edge bc: b + t (c - b) = a + (1 - t) ab + t ac
+    nv = d5 - d6, nw = d4 - d3, den = (d4 - d3) + (d5 - d6);
+  } else {                                                   // interior
+    nv = vb, nw = vc, den = va + vb + vc;
+  }
+  const float r = 1.f / den;
+  v = nv * r;
+  w = nw * r;
+}
+
+// |ab x ac|^2 of the edges ab = fl(v1 - v0), ac = fl(v2 - v0), every operation rounded (no FMA), so the degenerate-face
+// decision is reproducible bit for bit
+__device__ __forceinline__ float area2(const float* e1, const float* e2) {
+  const float nx = __fsub_rn(__fmul_rn(e1[1], e2[2]), __fmul_rn(e1[2], e2[1]));
+  const float ny = __fsub_rn(__fmul_rn(e1[2], e2[0]), __fmul_rn(e1[0], e2[2]));
+  const float nz = __fsub_rn(__fmul_rn(e1[0], e2[1]), __fmul_rn(e1[1], e2[0]));
+  return __fadd_rn(__fadd_rn(__fmul_rn(nx, nx), __fmul_rn(ny, ny)), __fmul_rn(nz, nz));
+}
+
+// squared distance from p = a + ap to the segment a + t e, t in [0, 1] (a zero-length segment is its point)
+__device__ __forceinline__ float segment_dist2(float px, float py, float pz, float ex, float ey, float ez) {
+  const float ee = ex * ex + ey * ey + ez * ez, pe = px * ex + py * ey + pz * ez;
+  const float t = ee > 0.f ? fminf(fmaxf(pe / ee, 0.f), 1.f) : 0.f;
+  const float dx = px - t * ex, dy = py - t * ey, dz = pz - t * ez;
+  return dx * dx + dy * dy + dz * dz;
+}
+
+}  // namespace dvq

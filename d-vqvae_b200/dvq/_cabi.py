@@ -70,6 +70,8 @@ SYMBOLS = {
     "dvq_nn_forward": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "dvq_nn_backward": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "dvq_vertex_normals": (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp]),
+    "dvq_mesh_winding": (_i, [_vp, _i, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
+    "dvq_mesh_distance": (_i, [_vp, _i, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
 }
 
 

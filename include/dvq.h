@@ -272,6 +272,23 @@ DVQ_API int dvq_nn_backward(const float* src, const float* trg, const int64_t* i
 DVQ_API int dvq_vertex_normals(const float* verts, int B, int V, const int* faces, int F, const int* vf_offsets,
                                const int* vf_faces, float* normals, void* stream);
 
+/* ---- mesh queries for grasp scoring (penetration volume, depth, contact) — the FP32 contract (winding number, box rule,
+ * distance, tie rule) is stated in csrc/mesh_exact.cuh.
+ * A mesh is verts [Bm, V, 3] fp32 plus faces [F, 3] int32 shared by every item (a face with an id outside [0, V)
+ * contributes nothing); the queries are pts [Bp, Q, 3] fp32.  Bm and Bp are each 1 or B (a batch of 1 is broadcast), and
+ * query row b is tested against mesh item b.  Shapes: Bm, Bp, F, Q >= 0, V > 0, and Bm * V * 3, Bp * Q * 3, B * Q * 3 and
+ * F * 3 below 2^31 (DVQ_ERR_BAD_SHAPE otherwise).  B = 0 or Q = 0 launches nothing.  Each entry is an ordinary stream
+ * launch (no host synchronisation, no allocation; CUDA-graph capturable) and deterministic. */
+/* Generalised winding number w [B,Q] of each query (0 for a query outside its mesh item's vertex box); with inside_count
+ * [B] (int32), the number of queries with w >= 0.5 is ADDED to inside_count[b] (the caller zeroes it first).  w and
+ * inside_count may each be NULL, but not both. */
+DVQ_API int dvq_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
+                             float* w, int* inside_count, void* stream);
+/* Squared distance dist2 [B,Q] from each query to its mesh item and the index face [B,Q] (int64) of the closest face
+ * (the lowest among exact ties; 0 with dist2 = +inf when no face gives a finite distance).  Needs F > 0. */
+DVQ_API int dvq_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
+                              float* dist2, int64_t* face, void* stream);
+
 /* Host-buffer (end-to-end) form of the same forward: z_host/E_host/zq_host/idx_host are
  * HOST pointers (pinned for full overlap).  Rows are streamed through the GPU in chunks on
  * three internal streams (H2D, compute, D2H).  loss/perplexity are host floats (train only). */
