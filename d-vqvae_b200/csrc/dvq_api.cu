@@ -459,6 +459,35 @@ int dvq_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F
   return launch_mesh_distance(verts, Bm, V, faces, F, pts, Bp, Q, B, dist2, face, static_cast<cudaStream_t>(stream));
 }
 
+int dvq_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, float* depth2,
+                         int64_t* face, void* stream) {
+  int B = 0;
+  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  if (rc) return rc;
+  if (F == 0) return fail(DVQ_ERR_BAD_SHAPE, "dvq_mesh_penetration needs F > 0");
+  if ((long long)B * Q > 0 && (!verts || !faces || !pts || !depth2 || !face))
+    return fail(DVQ_ERR_BAD_ARG, "verts, faces, pts, depth2 and face must not be NULL");
+  rc = require_sm100();
+  if (rc) return rc;
+  return launch_mesh_penetration(verts, Bm, V, faces, F, pts, Bp, Q, B, depth2, face, static_cast<cudaStream_t>(stream));
+}
+
+int dvq_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
+                               const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, void* stream) {
+  int B = 0;
+  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  if (rc) return rc;
+  if (!g_pts && !g_verts) return fail(DVQ_ERR_BAD_ARG, "g_pts and g_verts must not both be NULL");
+  if (g_verts && (long long)B * V * 3 >= (1LL << 31))
+    return fail(DVQ_ERR_BAD_SHAPE, "B * V * 3 = %lld must be below 2^31 for g_verts; split the batch", (long long)B * V * 3);
+  if ((long long)B * Q > 0 && (!verts || !pts || !face || !g_dist2 || (F > 0 && !faces)))
+    return fail(DVQ_ERR_BAD_ARG, "verts, faces, pts, face and g_dist2 must not be NULL");
+  rc = require_sm100();
+  if (rc) return rc;
+  return launch_mesh_distance_backward(verts, Bm, V, faces, F, pts, Bp, Q, B, face, g_dist2, g_pts, g_verts,
+                                       static_cast<cudaStream_t>(stream));
+}
+
 int dvq_pcnn_gemm(const DvqPcnnGemm* g, void* stream) {
   int rc = require_sm100();
   if (rc) return rc;

@@ -207,11 +207,16 @@ int launch_nn_backward(const float* src, const float* trg, const int64_t* idx, c
 int launch_vertex_normals(const float* verts, int B, int V, const int* faces, const int* vf_offsets, const int* vf_faces,
                           float* normals, cudaStream_t s);
 
-// mesh winding numbers and point-to-mesh distances (mesh_sm100.cu); B = the broadcast batch of Bm and Bp
+// mesh winding numbers, point-to-mesh distances, penetration and the distance gradient (mesh_sm100.cu); B = the broadcast
+// batch of Bm and Bp
 int launch_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B, float* w,
                         int* inside_count, cudaStream_t s);
 int launch_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
                          float* dist2, int64_t* face, cudaStream_t s);
+int launch_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
+                            float* depth2, int64_t* face, cudaStream_t s);
+int launch_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
+                                  const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, cudaStream_t s);
 
 // PointNet
 size_t pointnet_workspace_bytes(int B, int C, int P, int flags);

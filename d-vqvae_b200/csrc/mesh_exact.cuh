@@ -19,6 +19,21 @@
 //              whose fp32 area^2 = |ab x ac|^2 is 0 is taken as its three edge segments (no 0/0 in the interior region).
 //   face       the lowest f among exact fp32 minima of dist2; NaN counts as +inf (so a triangle with a non-finite corner
 //              never wins).  When no face gives a finite distance, face = 0 and dist2 = +inf.
+//   penetration  per query: depth2 = dist2 and face = the closest face when w >= 0.5, else depth2 = +0 and face = -1, with w,
+//              dist2 and face exactly the winding and distance values above (so sqrt(depth2) maxed over a hand's vertices
+//              is GraspQuality's depth, bit for bit).
+//
+// Gradient of dist2 (envelope theorem: the closest point's barycentrics are held fixed), for a query with its face f:
+//   offset     triangle (fp32 area^2 != 0): from the forward's staged a = v0, ab = fl(v1 - v0), ac = fl(v2 - v0), aa, cc,
+//              bc and ap = fl(q - a): (v, w) = closest_vw, d = ap - v ab - w ac in tri_offset2's FMA order, so
+//              fma(dz, dz, fma(dy, dy, dx dx)) is the forward's dist2 bit for bit; lambda = (fl(fl(1 - v) - w), v, w).
+//              Degenerate face: the first of the segments ab, ac, bc whose segment_dist2 equals the forward's minimum over
+//              the three, its t and offset from segment_offset, its two endpoints weighted (fl(1 - t), t), the third 0.
+//   g_pts      = fl(2 g) d per component, g the upstream gradient of dist2.
+//   g_verts    corner k of face f gets the term -fl(lambda_k g_pts); g_verts[b, vertex] is the sum of its terms in
+//              ascending (query, corner) order from +0 (no atomics).
+//   nothing    a query contributes nothing (g_pts = 0, no term) when face = -1, face is outside [0, F), its face has a
+//              vertex id outside [0, V), or its recomputed offset is not finite.
 //
 // Grasp metrics of hand b against one object (dvq.GraspQuality; the last reductions are device-side torch on the kernels'
 // outputs):
@@ -99,11 +114,50 @@ __device__ __forceinline__ float area2(const float* e1, const float* e2) {
   return __fadd_rn(__fadd_rn(__fmul_rn(nx, nx), __fmul_rn(ny, ny)), __fmul_rn(nz, nz));
 }
 
-// squared distance from p = a + ap to the segment a + t e, t in [0, 1] (a zero-length segment is its point)
-__device__ __forceinline__ float segment_dist2(float px, float py, float pz, float ex, float ey, float ez) {
+// The face data both the distance and its gradient stage: a = v0, ab = fl(v1 - v0), ac = fl(v2 - v0) from the corners
+// p0, p1, p2, and aa = ab . ab, cc = ac . ac, bc = ab . ac.
+__device__ __forceinline__ void face_frame(const float* p0, const float* p1, const float* p2, float (&a)[3], float (&e1)[3],
+                                           float (&e2)[3], float& aa, float& cc, float& bc) {
+#pragma unroll
+  for (int d = 0; d < 3; ++d) {
+    a[d] = p0[d];
+    e1[d] = p1[d] - a[d];
+    e2[d] = p2[d] - a[d];
+  }
+  aa = e1[0] * e1[0] + e1[1] * e1[1] + e1[2] * e1[2];
+  cc = e2[0] * e2[0] + e2[1] * e2[1] + e2[2] * e2[2];
+  bc = e1[0] * e2[0] + e1[1] * e2[1] + e1[2] * e2[2];
+}
+
+// Triangle offset d = ap - v ab - w ac of two queries (packed ap; packed ab = e[0..2], ac = e[3..5]); (v, w) per query
+// from closest_vw.  dist2 = dot2(d, d).
+__device__ __forceinline__ void tri_offset2(uint64_t px, uint64_t py, uint64_t pz, const uint64_t* e, float aa, float cc, float bc,
+                                            float (&vv)[2], float (&ww)[2], uint64_t& dx, uint64_t& dy, uint64_t& dz) {
+  float d1[2], d2[2];
+  unpack_f32x2(dot2(e[0], e[1], e[2], px, py, pz), d1[0], d1[1]);
+  unpack_f32x2(dot2(e[3], e[4], e[5], px, py, pz), d2[0], d2[1]);
+#pragma unroll
+  for (int h = 0; h < 2; ++h) closest_vw(d1[h], d2[h], aa, cc, bc, vv[h], ww[h]);
+  const uint64_t nv = pack_f32x2(-vv[0], -vv[1]), nw = pack_f32x2(-ww[0], -ww[1]);
+  dx = ffma2(nw, e[3], ffma2(nv, e[0], px));
+  dy = ffma2(nw, e[4], ffma2(nv, e[1], py));
+  dz = ffma2(nw, e[5], ffma2(nv, e[2], pz));
+}
+
+// Offset d = p - t e from p = a + ap to the closest point of the segment a + t e, t in [0, 1] (a zero-length segment is
+// its point); returns t.
+__device__ __forceinline__ float segment_offset(float px, float py, float pz, float ex, float ey, float ez, float& dx, float& dy,
+                                                float& dz) {
   const float ee = ex * ex + ey * ey + ez * ez, pe = px * ex + py * ey + pz * ez;
   const float t = ee > 0.f ? fminf(fmaxf(pe / ee, 0.f), 1.f) : 0.f;
-  const float dx = px - t * ex, dy = py - t * ey, dz = pz - t * ez;
+  dx = px - t * ex, dy = py - t * ey, dz = pz - t * ez;
+  return t;
+}
+
+// squared distance from p = a + ap to the segment a + t e
+__device__ __forceinline__ float segment_dist2(float px, float py, float pz, float ex, float ey, float ez) {
+  float dx, dy, dz;
+  segment_offset(px, py, pz, ex, ey, ez, dx, dy, dz);
   return dx * dx + dy * dy + dz * dz;
 }
 

@@ -1,13 +1,15 @@
-// Batched mesh queries for grasp scoring (dvq_mesh_winding / dvq_mesh_distance): generalised winding numbers (inside
-// tests, voxel volumes) and point-to-mesh distances, on the FP32 SIMT pipe.  The arithmetic is mesh_exact.cuh's contract.
+// Batched mesh queries for grasp scoring and refinement (dvq_mesh_winding / dvq_mesh_distance / dvq_mesh_penetration /
+// dvq_mesh_distance_backward): generalised winding numbers (inside tests, voxel volumes), point-to-mesh distances, the
+// fused penetration query and the gradient of the distance, on the FP32 SIMT pipe.  The arithmetic is mesh_exact.cuh's
+// contract.
 //
-// Both kernels share one layout: one CTA per (batch item, tile of MESH_TILE queries).  A thread keeps MESH_Q queries in
-// registers as packed x / y / z pairs, so one broadcast shared-memory read of a face's data serves MESH_Q queries and the
-// polynomial part of the arithmetic runs as f32x2 instructions (two queries per instruction); sqrtf, atan2f and the
-// region selection of the distance run per query.  The item's faces are staged in shared memory MESH_STAGE at a time as
-// structure-of-arrays, each value duplicated into both halves of a 64-bit word (the packed operand), with one flag per
-// face (skip: a vertex id outside [0, V); triangle; or degenerate: area^2 = 0, taken as three segments).  The flag is the
-// same for every thread, so its branch never diverges.
+// The forward kernels share one layout: one CTA per (batch item, tile of MESH_TILE queries).  A thread keeps MESH_Q
+// queries in registers as packed x / y / z pairs, so one broadcast shared-memory read of a face's data serves MESH_Q
+// queries and the polynomial part of the arithmetic runs as f32x2 instructions (two queries per instruction); sqrtf, atan2f
+// and the region selection of the distance run per query.  The item's faces are staged in shared memory MESH_STAGE at a
+// time as structure-of-arrays, each value duplicated into both halves of a 64-bit word (the packed operand), with one flag
+// per face (skip: a vertex id outside [0, V); triangle; or degenerate: area^2 = 0, taken as three segments).  The flag is
+// the same for every thread, so its branch never diverges.
 //
 // Mesh batch Bm and query batch Bp are each 1 or B: the item's mesh is verts[Bm == 1 ? 0 : b], its queries
 // pts[Bp == 1 ? 0 : b] (an object's voxel list shared by every hand, or every hand's vertices against one object).
@@ -15,6 +17,9 @@
 // mesh_winding_kernel first reduces the item's vertex box over the CTA; a query outside it gets w = 0 (the box rule), and
 // a CTA none of whose queries lies inside exits before staging a face: that keeps the voxel-volume pass proportional to
 // the hand/object overlap rather than to (voxels x hands).  The per-CTA inside count is one integer atomicAdd.
+//
+// mesh_penetration_kernel runs the winding sweep, compacts the CTA's inside queries into a shared-memory list and runs the
+// distance sweep over that list only; a CTA with no inside query never stages a face for distances.
 #include "dvq_common.cuh"
 #include "mesh_exact.cuh"
 
@@ -29,6 +34,17 @@ constexpr int MESH_STAGE = 256;                        // faces per shared-memor
 constexpr int MESH_WARPS = MESH_THREADS / 32;
 
 enum : uint8_t { FACE_SKIP = 0, FACE_TRI = 1, FACE_SEGS = 2 };
+
+struct WindingStage {
+  uint64_t sv[9][MESH_STAGE];                          // corners v0 x y z, v1 x y z, v2 x y z (18 KB)
+  uint8_t sflag[MESH_STAGE];
+};
+
+struct DistanceStage {
+  uint64_t sv[9][MESH_STAGE];                          // a x y z, ab x y z, ac x y z (18 KB)
+  float sd[3][MESH_STAGE];                             // ab . ab, ac . ac, ab . ac
+  uint8_t sflag[MESH_STAGE];
+};
 
 __device__ __forceinline__ bool face_ids(const int* __restrict__ faces, int f, int V, int& i0, int& i1, int& i2) {
   i0 = __ldg(faces + (size_t)f * 3);
@@ -88,12 +104,163 @@ __device__ void mesh_box(const float* __restrict__ P, int V, float* box, float (
   __syncthreads();
 }
 
+// The box rule for the thread's queries (inbox[p]); returns whether any query of the CTA is inside the box.
+__device__ __forceinline__ bool box_rule(const float* __restrict__ P, int V, int Q, int i0, const float (&c)[MESH_Q][3],
+                                         bool (&inbox)[MESH_Q], float* box, float (*red)[6]) {
+  mesh_box(P, V, box, red);
+  bool any = false;
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) {
+    inbox[p] = i0 + p * MESH_THREADS < Q && box[0] <= c[p][0] && c[p][0] <= box[3] && box[1] <= c[p][1] && c[p][1] <= box[4] &&
+               box[2] <= c[p][2] && c[p][2] <= box[5];
+    any |= inbox[p];
+  }
+  return __syncthreads_or(any);
+}
+
+// S = the sum of Omega_f over ascending f for the thread's MESH_Q queries; every face is staged through st.
+__device__ __forceinline__ void winding_sum(const float* __restrict__ P, int V, const int* __restrict__ faces, int F,
+                                            const uint64_t (&qx)[MESH_PAIRS], const uint64_t (&qy)[MESH_PAIRS],
+                                            const uint64_t (&qz)[MESH_PAIRS], float (&acc)[MESH_Q], WindingStage& st) {
+  const int tid = threadIdx.x;
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) acc[p] = 0.f;
+  for (int f0 = 0; f0 < F; f0 += MESH_STAGE) {
+    const int n = min(MESH_STAGE, F - f0);
+    __syncthreads();
+    for (int k = tid; k < n; k += MESH_THREADS) {
+      int id[3];
+      const bool ok = face_ids(faces, f0 + k, V, id[0], id[1], id[2]);
+      st.sflag[k] = ok ? FACE_TRI : FACE_SKIP;
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+#pragma unroll
+        for (int d = 0; d < 3; ++d) {
+          const float x = ok ? __ldg(P + (size_t)id[j] * 3 + d) : 0.f;
+          st.sv[j * 3 + d][k] = pack_f32x2(x, x);
+        }
+      }
+    }
+    __syncthreads();
+    for (int k = 0; k < n; ++k) {
+      if (st.sflag[k] == FACE_SKIP) continue;
+      uint64_t v[9];
+#pragma unroll
+      for (int j = 0; j < 9; ++j) v[j] = st.sv[j][k];
+#pragma unroll
+      for (int q = 0; q < MESH_PAIRS; ++q) {
+        float o0, o1;
+        solid_angle2(fsub2(v[0], qx[q]), fsub2(v[1], qy[q]), fsub2(v[2], qz[q]), fsub2(v[3], qx[q]), fsub2(v[4], qy[q]),
+                     fsub2(v[5], qz[q]), fsub2(v[6], qx[q]), fsub2(v[7], qy[q]), fsub2(v[8], qz[q]), o0, o1);
+        acc[2 * q] = __fadd_rn(acc[2 * q], o0);
+        acc[2 * q + 1] = __fadd_rn(acc[2 * q + 1], o1);
+      }
+    }
+  }
+}
+
+// Stages faces f0 .. f0 + n - 1 of P for the distance: a, ab, ac packed, the three dot products and the flag.
+__device__ __forceinline__ void distance_stage(const float* __restrict__ P, int V, const int* __restrict__ faces, int f0, int n,
+                                               DistanceStage& st) {
+  for (int k = threadIdx.x; k < n; k += MESH_THREADS) {
+    int id[3];
+    const bool ok = face_ids(faces, f0 + k, V, id[0], id[1], id[2]);
+    float p[3][3] = {{0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
+    if (ok) {
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+#pragma unroll
+        for (int d = 0; d < 3; ++d) p[j][d] = __ldg(P + (size_t)id[j] * 3 + d);
+      }
+    }
+    float a[3], e1[3], e2[3];
+    face_frame(p[0], p[1], p[2], a, e1, e2, st.sd[0][k], st.sd[1][k], st.sd[2][k]);
+    st.sflag[k] = !ok ? FACE_SKIP : (area2(e1, e2) == 0.f ? FACE_SEGS : FACE_TRI);
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+      st.sv[d][k] = pack_f32x2(a[d], a[d]);
+      st.sv[3 + d][k] = pack_f32x2(e1[d], e1[d]);
+      st.sv[6 + d][k] = pack_f32x2(e2[d], e2[d]);
+    }
+  }
+}
+
+// dist2 of one staged face (flag != FACE_SKIP) for a packed query pair with offsets (px, py, pz) = fl(q - a)
+__device__ __forceinline__ void face_dist2(uint8_t flag, const uint64_t (&v)[9], float aa, float cc, float bc, uint64_t px,
+                                           uint64_t py, uint64_t pz, float (&d)[2]) {
+  if (flag == FACE_TRI) {
+    float vv[2], ww[2];
+    uint64_t dx, dy, dz;
+    tri_offset2(px, py, pz, v + 3, aa, cc, bc, vv, ww, dx, dy, dz);
+    unpack_f32x2(dot2(dx, dy, dz, dx, dy, dz), d[0], d[1]);
+  } else {                                           // degenerate: the three edges ab, ac, bc
+    float ap[2][3], e1[3], e2[3], unused;
+    unpack_f32x2(px, ap[0][0], ap[1][0]);
+    unpack_f32x2(py, ap[0][1], ap[1][1]);
+    unpack_f32x2(pz, ap[0][2], ap[1][2]);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+      unpack_f32x2(v[3 + j], e1[j], unused);
+      unpack_f32x2(v[6 + j], e2[j], unused);
+    }
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const float sab = segment_dist2(ap[h][0], ap[h][1], ap[h][2], e1[0], e1[1], e1[2]);
+      const float sac = segment_dist2(ap[h][0], ap[h][1], ap[h][2], e2[0], e2[1], e2[2]);
+      const float sbc = segment_dist2(ap[h][0] - e1[0], ap[h][1] - e1[1], ap[h][2] - e1[2], e2[0] - e1[0], e2[1] - e1[1],
+                                      e2[2] - e1[2]);
+      d[h] = fminf(fminf(sab, sac), sbc);
+    }
+  }
+}
+
+// The distance sweep: best / bf = the smallest dist2 over ascending f and its lowest face for the thread's packed pairs
+// q < pairs (pairs is the same for the whole CTA).  Every thread joins the staging barriers; an inactive one skips the
+// arithmetic.
+__device__ __forceinline__ void distance_sweep(const float* __restrict__ P, int V, const int* __restrict__ faces, int F,
+                                               const uint64_t (&qx)[MESH_PAIRS], const uint64_t (&qy)[MESH_PAIRS],
+                                               const uint64_t (&qz)[MESH_PAIRS], int pairs, bool active, float (&best)[MESH_Q],
+                                               int (&bf)[MESH_Q], DistanceStage& st) {
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) {
+    best[p] = INFINITY;
+    bf[p] = 0;
+  }
+  for (int f0 = 0; f0 < F; f0 += MESH_STAGE) {
+    const int n = min(MESH_STAGE, F - f0);
+    __syncthreads();
+    distance_stage(P, V, faces, f0, n, st);
+    __syncthreads();
+    if (!active) continue;
+    for (int k = 0; k < n; ++k) {
+      const uint8_t flag = st.sflag[k];
+      if (flag == FACE_SKIP) continue;
+      uint64_t v[9];
+#pragma unroll
+      for (int j = 0; j < 9; ++j) v[j] = st.sv[j][k];
+      const float aa = st.sd[0][k], cc = st.sd[1][k], bc = st.sd[2][k];
+#pragma unroll
+      for (int q = 0; q < MESH_PAIRS; ++q) {
+        if (q >= pairs) break;
+        float d[2];
+        face_dist2(flag, v, aa, cc, bc, fsub2(qx[q], v[0]), fsub2(qy[q], v[1]), fsub2(qz[q], v[2]), d);
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          if (d[h] < best[2 * q + h]) {                  // strict, ascending f: the lowest f among exact minima; NaN never wins
+            best[2 * q + h] = d[h];
+            bf[2 * q + h] = f0 + k;
+          }
+        }
+      }
+    }
+  }
+}
+
 __global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(const float* __restrict__ verts, int Bm, int V,
                                                                      const int* __restrict__ faces, int F, const float* __restrict__ pts,
                                                                      int Bp, int Q, int tiles, float* __restrict__ w,
                                                                      int* __restrict__ inside_count) {
-  __shared__ __align__(16) uint64_t sv[9][MESH_STAGE];     // corners v0 x y z, v1 x y z, v2 x y z (18 KB)
-  __shared__ uint8_t sflag[MESH_STAGE];
+  __shared__ __align__(16) WindingStage st;
   __shared__ float red[MESH_WARPS][6];
   __shared__ float box[6];
   const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x;
@@ -101,18 +268,11 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(const float*
   const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
   const int i0 = tile * MESH_TILE + tid;
 
-  mesh_box(P, V, box, red);
   float c[MESH_Q][3];
   uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
   load_queries(S, Q, i0, c, qx, qy, qz);
-  bool inbox[MESH_Q], any = false;
-#pragma unroll
-  for (int p = 0; p < MESH_Q; ++p) {
-    inbox[p] = i0 + p * MESH_THREADS < Q && box[0] <= c[p][0] && c[p][0] <= box[3] && box[1] <= c[p][1] && c[p][1] <= box[4] &&
-               box[2] <= c[p][2] && c[p][2] <= box[5];
-    any |= inbox[p];
-  }
-  if (!__syncthreads_or(any)) {                 // the whole tile is outside the box: w = 0, nothing inside
+  bool inbox[MESH_Q];
+  if (!box_rule(P, V, Q, i0, c, inbox, box, red)) {   // the whole tile is outside the box: w = 0, nothing inside
     if (w) {
 #pragma unroll
       for (int p = 0; p < MESH_Q; ++p) {
@@ -124,41 +284,7 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(const float*
   }
 
   float acc[MESH_Q];
-#pragma unroll
-  for (int p = 0; p < MESH_Q; ++p) acc[p] = 0.f;
-  for (int f0 = 0; f0 < F; f0 += MESH_STAGE) {
-    const int n = min(MESH_STAGE, F - f0);
-    __syncthreads();
-    for (int k = tid; k < n; k += MESH_THREADS) {
-      int id[3];
-      const bool ok = face_ids(faces, f0 + k, V, id[0], id[1], id[2]);
-      sflag[k] = ok ? FACE_TRI : FACE_SKIP;
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-#pragma unroll
-        for (int d = 0; d < 3; ++d) {
-          const float x = ok ? __ldg(P + (size_t)id[j] * 3 + d) : 0.f;
-          sv[j * 3 + d][k] = pack_f32x2(x, x);
-        }
-      }
-    }
-    __syncthreads();
-    for (int k = 0; k < n; ++k) {
-      if (sflag[k] == FACE_SKIP) continue;
-      uint64_t v[9];
-#pragma unroll
-      for (int j = 0; j < 9; ++j) v[j] = sv[j][k];
-#pragma unroll
-      for (int q = 0; q < MESH_PAIRS; ++q) {
-        float o0, o1;
-        solid_angle2(fsub2(v[0], qx[q]), fsub2(v[1], qy[q]), fsub2(v[2], qz[q]), fsub2(v[3], qx[q]), fsub2(v[4], qy[q]),
-                     fsub2(v[5], qz[q]), fsub2(v[6], qx[q]), fsub2(v[7], qy[q]), fsub2(v[8], qz[q]), o0, o1);
-        acc[2 * q] = __fadd_rn(acc[2 * q], o0);
-        acc[2 * q + 1] = __fadd_rn(acc[2 * q + 1], o1);
-      }
-    }
-  }
-
+  winding_sum(P, V, faces, F, qx, qy, qz, acc, st);
   int mine[MESH_Q];
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
@@ -179,9 +305,7 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_distance_kernel(const float
                                                                       const int* __restrict__ faces, int F, const float* __restrict__ pts,
                                                                       int Bp, int Q, int tiles, float* __restrict__ dist2,
                                                                       int64_t* __restrict__ face) {
-  __shared__ __align__(16) uint64_t sv[9][MESH_STAGE];     // a x y z, ab x y z, ac x y z (18 KB)
-  __shared__ float sd[3][MESH_STAGE];                      // ab . ab, ac . ac, ab . ac
-  __shared__ uint8_t sflag[MESH_STAGE];
+  __shared__ __align__(16) DistanceStage st;
   const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x;
   const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
   const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
@@ -192,89 +316,7 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_distance_kernel(const float
   load_queries(S, Q, i0, c, qx, qy, qz);
   float best[MESH_Q];
   int bf[MESH_Q];
-#pragma unroll
-  for (int p = 0; p < MESH_Q; ++p) {
-    best[p] = INFINITY;
-    bf[p] = 0;
-  }
-
-  for (int f0 = 0; f0 < F; f0 += MESH_STAGE) {
-    const int n = min(MESH_STAGE, F - f0);
-    __syncthreads();
-    for (int k = tid; k < n; k += MESH_THREADS) {
-      int id[3];
-      const bool ok = face_ids(faces, f0 + k, V, id[0], id[1], id[2]);
-      float a[3] = {0.f, 0.f, 0.f}, e1[3] = {0.f, 0.f, 0.f}, e2[3] = {0.f, 0.f, 0.f};
-      if (ok) {
-#pragma unroll
-        for (int d = 0; d < 3; ++d) {
-          a[d] = __ldg(P + (size_t)id[0] * 3 + d);
-          e1[d] = __ldg(P + (size_t)id[1] * 3 + d) - a[d];
-          e2[d] = __ldg(P + (size_t)id[2] * 3 + d) - a[d];
-        }
-      }
-      sflag[k] = !ok ? FACE_SKIP : (area2(e1, e2) == 0.f ? FACE_SEGS : FACE_TRI);
-#pragma unroll
-      for (int d = 0; d < 3; ++d) {
-        sv[d][k] = pack_f32x2(a[d], a[d]);
-        sv[3 + d][k] = pack_f32x2(e1[d], e1[d]);
-        sv[6 + d][k] = pack_f32x2(e2[d], e2[d]);
-      }
-      sd[0][k] = e1[0] * e1[0] + e1[1] * e1[1] + e1[2] * e1[2];
-      sd[1][k] = e2[0] * e2[0] + e2[1] * e2[1] + e2[2] * e2[2];
-      sd[2][k] = e1[0] * e2[0] + e1[1] * e2[1] + e1[2] * e2[2];
-    }
-    __syncthreads();
-    for (int k = 0; k < n; ++k) {
-      const uint8_t flag = sflag[k];
-      if (flag == FACE_SKIP) continue;
-      uint64_t v[9];
-#pragma unroll
-      for (int j = 0; j < 9; ++j) v[j] = sv[j][k];
-      const float aa = sd[0][k], cc = sd[1][k], bc = sd[2][k];
-#pragma unroll
-      for (int q = 0; q < MESH_PAIRS; ++q) {
-        const uint64_t px = fsub2(qx[q], v[0]), py = fsub2(qy[q], v[1]), pz = fsub2(qz[q], v[2]);
-        float d[2];
-        if (flag == FACE_TRI) {
-          float d1[2], d2[2], vv[2], ww[2];
-          unpack_f32x2(dot2(v[3], v[4], v[5], px, py, pz), d1[0], d1[1]);
-          unpack_f32x2(dot2(v[6], v[7], v[8], px, py, pz), d2[0], d2[1]);
-#pragma unroll
-          for (int h = 0; h < 2; ++h) closest_vw(d1[h], d2[h], aa, cc, bc, vv[h], ww[h]);
-          const uint64_t nv = pack_f32x2(-vv[0], -vv[1]), nw = pack_f32x2(-ww[0], -ww[1]);
-          const uint64_t dx = ffma2(nw, v[6], ffma2(nv, v[3], px)), dy = ffma2(nw, v[7], ffma2(nv, v[4], py)),
-                         dz = ffma2(nw, v[8], ffma2(nv, v[5], pz));
-          unpack_f32x2(dot2(dx, dy, dz, dx, dy, dz), d[0], d[1]);
-        } else {                                           // degenerate: the three edges ab, ac, bc
-          float ap[2][3], e1[3], e2[3], unused;
-          unpack_f32x2(px, ap[0][0], ap[1][0]);
-          unpack_f32x2(py, ap[0][1], ap[1][1]);
-          unpack_f32x2(pz, ap[0][2], ap[1][2]);
-#pragma unroll
-          for (int j = 0; j < 3; ++j) {
-            unpack_f32x2(v[3 + j], e1[j], unused);
-            unpack_f32x2(v[6 + j], e2[j], unused);
-          }
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const float sab = segment_dist2(ap[h][0], ap[h][1], ap[h][2], e1[0], e1[1], e1[2]);
-            const float sac = segment_dist2(ap[h][0], ap[h][1], ap[h][2], e2[0], e2[1], e2[2]);
-            const float sbc = segment_dist2(ap[h][0] - e1[0], ap[h][1] - e1[1], ap[h][2] - e1[2], e2[0] - e1[0], e2[1] - e1[1],
-                                            e2[2] - e1[2]);
-            d[h] = fminf(fminf(sab, sac), sbc);
-          }
-        }
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          if (d[h] < best[2 * q + h]) {                  // strict, ascending f: the lowest f among exact minima; NaN never wins
-            best[2 * q + h] = d[h];
-            bf[2 * q + h] = f0 + k;
-          }
-        }
-      }
-    }
-  }
+  distance_sweep(P, V, faces, F, qx, qy, qz, MESH_PAIRS, true, best, bf, st);
 
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
@@ -282,6 +324,239 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_distance_kernel(const float
     if (i >= Q) continue;
     dist2[(size_t)b * Q + i] = best[p];
     face[(size_t)b * Q + i] = bf[p];
+  }
+}
+
+// Phase 1 is mesh_winding_kernel's box rule and sum.  Phase 2 compacts the inside queries, in ascending query order, into
+// slist; list entry j is held by thread (j mod 256) / 2 in half j mod 2 of pair j / 256, so n inside queries occupy the
+// first ceil(n / 64) warps and one pair per thread while n <= 256.  The distance faces are staged into the same shared
+// memory as the winding faces.
+__global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const float* __restrict__ verts, int Bm, int V,
+                                                                         const int* __restrict__ faces, int F,
+                                                                         const float* __restrict__ pts, int Bp, int Q, int tiles,
+                                                                         float* __restrict__ depth2, int64_t* __restrict__ face) {
+  __shared__ __align__(16) union {
+    WindingStage w;
+    DistanceStage d;
+  } st;
+  __shared__ float red[MESH_WARPS][6];
+  __shared__ float box[6];
+  __shared__ float slist[3][MESH_TILE];
+  __shared__ int sidx[MESH_TILE];
+  __shared__ int wcount[MESH_Q][MESH_WARPS];
+  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
+  const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
+  const int i0 = tile * MESH_TILE + tid;
+  float* D = depth2 + (size_t)b * Q;
+  int64_t* FC = face + (size_t)b * Q;
+
+  bool inside[MESH_Q];
+  {
+    float c[MESH_Q][3];
+    uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
+    load_queries(S, Q, i0, c, qx, qy, qz);
+    bool inbox[MESH_Q];
+    const bool any = box_rule(P, V, Q, i0, c, inbox, box, red);
+#pragma unroll
+    for (int p = 0; p < MESH_Q; ++p) inside[p] = false;
+    if (any) {
+      float acc[MESH_Q];
+      winding_sum(P, V, faces, F, qx, qy, qz, acc, st.w);
+#pragma unroll
+      for (int p = 0; p < MESH_Q; ++p) inside[p] = inbox[p] && __fdiv_rn(acc[p], MESH_4PI) >= 0.5f;
+    }
+#pragma unroll
+    for (int p = 0; p < MESH_Q; ++p) {
+      const int i = i0 + p * MESH_THREADS;
+      if (i < Q && !inside[p]) {
+        D[i] = 0.f;
+        FC[i] = -1;
+      }
+    }
+    if (!any) return;                                  // CTA-uniform: box_rule's vote
+  }
+
+  unsigned m[MESH_Q];
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) {
+    m[p] = __ballot_sync(0xffffffffu, inside[p]);
+    if (lane == 0) wcount[p][warp] = __popc(m[p]);
+  }
+  __syncthreads();
+  int n_in = 0, off[MESH_Q];
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) {
+#pragma unroll
+    for (int j = 0; j < MESH_WARPS; ++j) {
+      if (j == warp) off[p] = n_in;
+      n_in += wcount[p][j];
+    }
+  }
+  if (n_in == 0) return;                               // CTA-uniform
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) {
+    if (inside[p]) {
+      const int j = off[p] + __popc(m[p] & ((1u << lane) - 1u)), i = i0 + p * MESH_THREADS;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) slist[k][j] = __ldg(S + (size_t)i * 3 + k);
+      sidx[j] = i;
+    }
+  }
+  __syncthreads();
+
+  uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
+#pragma unroll
+  for (int q = 0; q < MESH_PAIRS; ++q) {
+    float c[2][3];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int j = q * 2 * MESH_THREADS + 2 * tid + h;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) c[h][k] = j < n_in ? slist[k][j] : 0.f;
+    }
+    qx[q] = pack_f32x2(c[0][0], c[1][0]);
+    qy[q] = pack_f32x2(c[0][1], c[1][1]);
+    qz[q] = pack_f32x2(c[0][2], c[1][2]);
+  }
+  const int pairs = (n_in + 2 * MESH_THREADS - 1) / (2 * MESH_THREADS);
+  const bool active = warp * 64 < n_in;
+  float best[MESH_Q];
+  int bf[MESH_Q];
+  distance_sweep(P, V, faces, F, qx, qy, qz, pairs, active, best, bf, st.d);
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) {
+    const int j = (p >> 1) * 2 * MESH_THREADS + 2 * tid + (p & 1);
+    if (j < n_in) {
+      const int i = sidx[j];
+      D[i] = best[p];
+      FC[i] = bf[p];
+    }
+  }
+}
+
+// One warp per broadcast item b, which owns (zero-fills, then accumulates) the item's g_verts rows: no races, no atomics.
+// The warp walks the item's queries 32 at a time; each lane recomputes its query's offset at its face (mesh_exact.cuh)
+// and writes g_pts.  The chunk's 96 (query, corner) terms go to shared memory in ascending (query, corner) order and are
+// added in three passes of 32 slots: in each, __match_any_sync groups the slots that share a vertex and the group's lowest
+// lane adds them into g_verts in ascending slot order, so every vertex's terms are summed in ascending (query, corner)
+// order.
+constexpr int BW_WARPS = 4;
+
+__global__ void __launch_bounds__(BW_WARPS * 32) mesh_distance_backward_kernel(
+    const float* __restrict__ verts, int Bm, int V, const int* __restrict__ faces, int F, const float* __restrict__ pts, int Bp,
+    int Q, int B, const int64_t* __restrict__ face, const float* __restrict__ g_dist2, float* __restrict__ g_pts,
+    float* __restrict__ g_verts) {
+  __shared__ float term[BW_WARPS][3][96];
+  __shared__ int tvert[BW_WARPS][96];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, b = blockIdx.x * BW_WARPS + w;
+  if (b >= B) return;
+  const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
+  const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
+  const int64_t* I = face + (size_t)b * Q;
+  const float* G = g_dist2 + (size_t)b * Q;
+  float* GP = g_pts ? g_pts + (size_t)b * Q * 3 : nullptr;
+  float* GV = g_verts ? g_verts + (size_t)b * V * 3 : nullptr;
+  if (GV) {
+    for (int k = lane; k < V * 3; k += 32) GV[k] = 0.f;
+    __syncwarp();
+  }
+  for (int c0 = 0; c0 < Q; c0 += 32) {
+    const int i = c0 + lane;
+    int id[3] = {-1, -1, -1};
+    float lam[3] = {0.f, 0.f, 0.f}, t[3] = {0.f, 0.f, 0.f};
+    bool valid = false;
+    const int64_t f64 = i < Q ? I[i] : -1;
+    if (f64 >= 0 && f64 < F && face_ids(faces, (int)f64, V, id[0], id[1], id[2])) {
+      float p[3][3], q[3];
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) p[j][k] = __ldg(P + (size_t)id[j] * 3 + k);
+      }
+#pragma unroll
+      for (int k = 0; k < 3; ++k) q[k] = __ldg(S + (size_t)i * 3 + k);
+      float a[3], e1[3], e2[3], aa, cc, bc, d[3];
+      face_frame(p[0], p[1], p[2], a, e1, e2, aa, cc, bc);
+      if (area2(e1, e2) != 0.f) {                       // the forward's packed arithmetic, both halves the same query
+        uint64_t e[6];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          e[k] = pack_f32x2(e1[k], e1[k]);
+          e[3 + k] = pack_f32x2(e2[k], e2[k]);
+        }
+        float vv[2], ww[2], unused;
+        uint64_t dx, dy, dz;
+        tri_offset2(fsub2(pack_f32x2(q[0], q[0]), pack_f32x2(a[0], a[0])), fsub2(pack_f32x2(q[1], q[1]), pack_f32x2(a[1], a[1])),
+                    fsub2(pack_f32x2(q[2], q[2]), pack_f32x2(a[2], a[2])), e, aa, cc, bc, vv, ww, dx, dy, dz);
+        unpack_f32x2(dx, d[0], unused);
+        unpack_f32x2(dy, d[1], unused);
+        unpack_f32x2(dz, d[2], unused);
+        lam[0] = __fsub_rn(__fsub_rn(1.f, vv[0]), ww[0]);
+        lam[1] = vv[0];
+        lam[2] = ww[0];
+      } else {                                          // degenerate: the first segment attaining the forward's minimum
+        float ap[3], bp[3], ebc[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          ap[k] = q[k] - a[k];
+          bp[k] = ap[k] - e1[k];
+          ebc[k] = e2[k] - e1[k];
+        }
+        const float sab = segment_dist2(ap[0], ap[1], ap[2], e1[0], e1[1], e1[2]);
+        const float sac = segment_dist2(ap[0], ap[1], ap[2], e2[0], e2[1], e2[2]);
+        const float sbc = segment_dist2(bp[0], bp[1], bp[2], ebc[0], ebc[1], ebc[2]);
+        const float m = fminf(fminf(sab, sac), sbc);
+        if (sab == m) {
+          const float s = segment_offset(ap[0], ap[1], ap[2], e1[0], e1[1], e1[2], d[0], d[1], d[2]);
+          lam[0] = __fsub_rn(1.f, s), lam[1] = s;
+        } else if (sac == m) {
+          const float s = segment_offset(ap[0], ap[1], ap[2], e2[0], e2[1], e2[2], d[0], d[1], d[2]);
+          lam[0] = __fsub_rn(1.f, s), lam[2] = s;
+        } else {
+          const float s = segment_offset(bp[0], bp[1], bp[2], ebc[0], ebc[1], ebc[2], d[0], d[1], d[2]);
+          lam[1] = __fsub_rn(1.f, s), lam[2] = s;
+        }
+      }
+      valid = isfinite(d[0]) && isfinite(d[1]) && isfinite(d[2]);
+      if (valid) {
+        const float g2 = __fmul_rn(2.f, G[i]);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) t[k] = __fmul_rn(g2, d[k]);
+      }
+    }
+    if (GP && i < Q) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k) GP[(size_t)i * 3 + k] = t[k];
+    }
+    if (GV && __ballot_sync(0xffffffffu, valid)) {     // warp-uniform
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+        tvert[w][3 * lane + j] = valid ? id[j] : -1;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) term[w][k][3 * lane + j] = -__fmul_rn(lam[j], t[k]);
+      }
+      __syncwarp();
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const int v = tvert[w][32 * r + lane];
+        const unsigned vmask = __ballot_sync(0xffffffffu, v >= 0);
+        if (v >= 0) {
+          const unsigned peers = __match_any_sync(vmask, v);
+          if (lane == __ffs(peers) - 1) {
+            float acc[3] = {GV[(size_t)v * 3], GV[(size_t)v * 3 + 1], GV[(size_t)v * 3 + 2]};
+            for (unsigned rest = peers; rest; rest &= rest - 1) {
+              const int l = 32 * r + __ffs(rest) - 1;
+#pragma unroll
+              for (int k = 0; k < 3; ++k) acc[k] = __fadd_rn(acc[k], term[w][k][l]);
+            }
+#pragma unroll
+            for (int k = 0; k < 3; ++k) GV[(size_t)v * 3 + k] = acc[k];
+          }
+        }
+        __syncwarp();
+      }
+    }
   }
 }
 
@@ -304,6 +579,27 @@ int launch_mesh_distance(const float* verts, int Bm, int V, const int* faces, in
   const int tiles = (Q + MESH_TILE - 1) / MESH_TILE;
   mesh_distance_kernel<<<(unsigned)((long long)B * tiles), MESH_THREADS, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, tiles, dist2,
                                                                                  face);
+  DVQ_CUDA_CHECK(cudaGetLastError());
+  count_launch();
+  return DVQ_OK;
+}
+
+int launch_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
+                            float* depth2, int64_t* face, cudaStream_t s) {
+  if (B == 0 || Q == 0) return DVQ_OK;
+  const int tiles = (Q + MESH_TILE - 1) / MESH_TILE;
+  mesh_penetration_kernel<<<(unsigned)((long long)B * tiles), MESH_THREADS, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, tiles,
+                                                                                    depth2, face);
+  DVQ_CUDA_CHECK(cudaGetLastError());
+  count_launch();
+  return DVQ_OK;
+}
+
+int launch_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
+                                  const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, cudaStream_t s) {
+  if (B == 0 || (Q == 0 && !g_verts)) return DVQ_OK;
+  mesh_distance_backward_kernel<<<(B + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, B, face,
+                                                                                         g_dist2, g_pts, g_verts);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;

@@ -5,7 +5,7 @@ from . import _cabi  # noqa: F401  (fails loudly when the CUDA library is missin
 from . import dist  # noqa: F401
 from .contact import HandObjectContact, nearest_points  # noqa: F401
 from .grasp import GraspGenerator  # noqa: F401
-from .grasp_quality import GraspQuality, point_mesh_distance, winding_number  # noqa: F401
+from .grasp_quality import GraspQuality, penetration_depth, point_mesh_distance, winding_number  # noqa: F401
 from .host import HostQuantizer  # noqa: F401
 from .mano import ManoLayer  # noqa: F401
 from .pointnet import PointNetEncoder, STN3d  # noqa: F401
@@ -13,4 +13,4 @@ from .quantizer import LazyOneHot, VectorQuantizer  # noqa: F401
 from .vqvae import VQVAE  # noqa: F401
 
 __all__ = ["VectorQuantizer", "VQVAE", "PointNetEncoder", "STN3d", "LazyOneHot", "HostQuantizer", "GraspGenerator", "ManoLayer", "HandObjectContact", "nearest_points",
-           "GraspQuality", "winding_number", "point_mesh_distance", "dist"]
+           "GraspQuality", "winding_number", "point_mesh_distance", "penetration_depth", "dist"]

@@ -72,6 +72,8 @@ SYMBOLS = {
     "dvq_vertex_normals": (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp]),
     "dvq_mesh_winding": (_i, [_vp, _i, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
     "dvq_mesh_distance": (_i, [_vp, _i, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
+    "dvq_mesh_penetration": (_i, [_vp, _i, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
+    "dvq_mesh_distance_backward": (_i, [_vp, _i, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -3,13 +3,18 @@ the metrics the reference scripts compute per grasp on the CPU (``intersection_e
 trimesh voxelisation and containment, igl distances).
 
 - ``winding_number(points, verts, faces)``: generalised winding numbers (``w >= 0.5`` is "inside").
-- ``point_mesh_distance(points, verts, faces)``: squared distance to the mesh and the closest face.
+- ``point_mesh_distance(points, verts, faces, differentiable=False)``: squared distance to the mesh and the closest face.
+- ``penetration_depth(points, verts, faces)``: the squared distance of the points inside the mesh (0 outside) and their
+  closest face, in one fused launch; differentiable.
 - ``GraspQuality(obj_verts, obj_faces, hand_faces, pitch, contact_tol)``: ``forward(hand_verts) -> (volume, depth,
   contact)``.
 
 The contract (winding number, box rule, distance, tie rule, voxel centres, metrics) is stated once in
-``csrc/mesh_exact.cuh`` and restated in float64 in ``oracle/mesh_oracle.py``.  CUDA fp32 only, no autograd: the metrics are
-step functions and maxima used for scoring, so inputs that require grad are detached.
+``csrc/mesh_exact.cuh`` and restated in float64 in ``oracle/mesh_oracle.py``.  CUDA fp32 only.  ``GraspQuality`` and
+``winding_number`` have no autograd (the metrics are step functions and maxima used for scoring, so inputs that require
+grad are detached); ``penetration_depth`` and ``point_mesh_distance(differentiable=True)`` carry the gradient of the
+squared distance to the points and the mesh vertices, with the closest point's barycentrics held fixed (the envelope
+theorem, as pytorch3d's ``point_mesh_face_distance``), for refinement losses.
 
 The voxelisation is filled and centre-sampled: a cell counts when its centre is inside the object, and a cell of the
 object counts for hand b when its centre is inside hand b.  trimesh's ``voxelized()`` marks the cells the surface passes
@@ -26,6 +31,7 @@ import math
 import numpy as np
 import torch
 from torch import nn
+from torch.autograd.function import once_differentiable
 
 from . import _cabi
 from .quantizer import _stream_ptr
@@ -33,7 +39,7 @@ from .quantizer import _stream_ptr
 MAX_CELLS = 1 << 24         # voxel grid cap: above it the pitch is almost certainly a unit mistake (mm vs m)
 
 
-def _points(x, name, what):
+def _points(x, name, what, detach=True):
     if not isinstance(x, torch.Tensor):
         raise TypeError("%s must be a torch.Tensor" % name)
     if x.dtype != torch.float32:
@@ -42,7 +48,7 @@ def _points(x, name, what):
         raise ValueError("%s has no CPU path: %s must be a CUDA tensor" % (what, name))
     if x.dim() != 3 or x.shape[2] != 3:
         raise ValueError("%s must be [B, n, 3]; got %s" % (name, tuple(x.shape)))
-    return x.detach().contiguous()
+    return (x.detach() if detach else x).contiguous()
 
 
 def check_faces(faces, num_verts=None, name="faces"):
@@ -63,8 +69,8 @@ def _broadcast(Bm, Bp):
     return Bp if Bm == 1 else Bm
 
 
-def _prepare(points, verts, faces, what):
-    points, verts = _points(points, "points", what), _points(verts, "verts", what)
+def _prepare(points, verts, faces, what, detach=True):
+    points, verts = _points(points, "points", what, detach), _points(verts, "verts", what, detach)
     if points.device != verts.device:
         raise ValueError("points are on %s, verts on %s" % (points.device, verts.device))
     if verts.shape[1] == 0:
@@ -102,14 +108,86 @@ def winding_number(points, verts, faces):
     return w
 
 
-def point_mesh_distance(points, verts, faces):
+def _penetration(points, verts, faces, B):
+    depth2 = torch.empty(B, points.shape[1], device=points.device, dtype=torch.float32)
+    face = torch.empty(B, points.shape[1], device=points.device, dtype=torch.int64)
+    with torch.cuda.device(points.device):
+        _cabi.check(_cabi.lib.dvq_mesh_penetration(verts.data_ptr(), verts.shape[0], verts.shape[1], faces.data_ptr(), faces.shape[0],
+                                                   points.data_ptr(), points.shape[0], points.shape[1], depth2.data_ptr(),
+                                                   face.data_ptr(), _stream_ptr(points.device)), "dvq_mesh_penetration")
+    return depth2, face
+
+
+class _MeshDistance(torch.autograd.Function):
+    """(points, verts, faces) -> (dist2, face) through ``dvq_mesh_distance`` or, with ``fused``, ``dvq_mesh_penetration``;
+    the backward is ``dvq_mesh_distance_backward`` from the saved inputs and ``face``.  Its gradients are per broadcast
+    item: an input given with a batch of 1 gets their sum over b, which the [B, ., 3] temporary exists for."""
+
+    @staticmethod
+    def forward(ctx, points, verts, faces, B, fused):
+        dist2, face = (_penetration if fused else _distance)(points, verts, faces, B)
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(points, verts, faces, face)
+        ctx.B = B
+        ctx.mark_non_differentiable(face)
+        return dist2, face
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_dist2, _g_face):
+        points, verts, faces, face = ctx.saved_tensors
+        want_pts, want_verts = ctx.needs_input_grad[:2]
+        if g_dist2 is None or not (want_pts or want_verts):
+            return None, None, None, None, None
+        B, Q, V = ctx.B, points.shape[1], verts.shape[1]
+        g = g_dist2.to(torch.float32).contiguous()
+        g_pts = torch.empty(B, Q, 3, device=points.device, dtype=torch.float32) if want_pts else None
+        g_verts = torch.empty(B, V, 3, device=verts.device, dtype=torch.float32) if want_verts else None
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        with torch.cuda.device(points.device):
+            _cabi.check(_cabi.lib.dvq_mesh_distance_backward(verts.data_ptr(), verts.shape[0], V, faces.data_ptr(), faces.shape[0],
+                                                             points.data_ptr(), points.shape[0], Q, face.data_ptr(), g.data_ptr(),
+                                                             ptr(g_pts), ptr(g_verts), _stream_ptr(points.device)),
+                        "dvq_mesh_distance_backward")
+        if g_pts is not None and points.shape[0] != B:
+            g_pts = g_pts.sum(0, keepdim=True)
+        if g_verts is not None and verts.shape[0] != B:
+            g_verts = g_verts.sum(0, keepdim=True)
+        return g_pts, g_verts, None, None, None
+
+
+def point_mesh_distance(points, verts, faces, differentiable=False):
     """``points [Bp,Q,3]``, ``verts [Bm,V,3]`` (fp32 CUDA; Bm, Bp each 1 or B), ``faces [F,3]`` int, F > 0 -> ``(dist2 [B,Q]
     fp32, face [B,Q] int64)``: the squared distance from each point to the closest point of its batch item's mesh and the
-    closest face (the lowest index among exact ties).  ``faces`` is validated on the host."""
-    points, verts, faces, B = _prepare(points, verts, faces, "dvq.point_mesh_distance")
+    closest face (the lowest index among exact ties).  ``faces`` is validated on the host.
+
+    By default the inputs are detached.  With ``differentiable=True``, ``dist2`` carries gradients to ``points`` and
+    ``verts`` (the closest point's barycentrics held fixed; deterministic); ``face`` is not differentiable.  An input
+    given with a batch of 1 gets the sum over b of the per-item gradients (the same bits autograd gives an explicit
+    ``expand``)."""
+    points, verts, faces, B = _prepare(points, verts, faces, "dvq.point_mesh_distance", detach=not differentiable)
     if faces.shape[0] == 0:
         raise ValueError("faces must hold at least one face")
-    return _distance(points, verts, faces, B)
+    if not differentiable:
+        return _distance(points, verts, faces, B)
+    return _MeshDistance.apply(points, verts, faces, B, False)
+
+
+def penetration_depth(points, verts, faces):
+    """``points [Bp,Q,3]``, ``verts [Bm,V,3]`` (fp32 CUDA; Bm, Bp each 1 or B), ``faces [F,3]`` int, F > 0 -> ``(depth2
+    [B,Q] fp32, face [B,Q] int64)``: for a point inside its batch item's mesh (winding number >= 0.5), the squared distance
+    to the mesh and the closest face, exactly as ``point_mesh_distance`` gives them; 0 and -1 for any other point.  One
+    launch: the distance sweep runs only for the inside points.
+
+    ``depth2`` is differentiable with respect to ``points`` and ``verts`` like ``point_mesh_distance(...,
+    differentiable=True)``; the inside test (a step function) has no gradient.  Hand vertices [B,778,3] against an object
+    mesh [1,V,3] give ``sqrt(depth2).amax(1)`` = ``GraspQuality``'s depth; an object's points or ``GraspQuality.centres``
+    [1,M,3] against the hand meshes [B,778,3] with ``ManoLayer.faces`` (open at the wrist: the winding rule handles it)
+    give, summed over the points, a differentiable counterpart of the penetration volume."""
+    points, verts, faces, B = _prepare(points, verts, faces, "dvq.penetration_depth", detach=False)
+    if faces.shape[0] == 0:
+        raise ValueError("faces must hold at least one face")
+    return _MeshDistance.apply(points, verts, faces, B, True)
 
 
 def voxel_grid(lo, hi, pitch):

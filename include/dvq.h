@@ -288,6 +288,19 @@ DVQ_API int dvq_mesh_winding(const float* verts, int Bm, int V, const int* faces
  * (the lowest among exact ties; 0 with dist2 = +inf when no face gives a finite distance).  Needs F > 0. */
 DVQ_API int dvq_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
                               float* dist2, int64_t* face, void* stream);
+/* Penetration query, the winding number and the distance fused: for a query with w >= 0.5, depth2 [B,Q] = dist2 and face
+ * [B,Q] (int64) = the closest face, exactly as dvq_mesh_winding / dvq_mesh_distance give them; for any other query
+ * depth2 = +0 and face = -1.  The distance sweep runs only for the inside queries.  Needs F > 0. */
+DVQ_API int dvq_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
+                                 float* depth2, int64_t* face, void* stream);
+/* Gradient of dist2 (of dvq_mesh_distance or depth2 of dvq_mesh_penetration) given the forward's face [B,Q] and the
+ * upstream g_dist2 [B,Q]: g_pts [B,Q,3] and g_verts [B,V,3], each written when non-NULL (not both NULL), per broadcast
+ * item b (the caller sums over b for an input given with a batch of 1).  The closest point's barycentrics are held fixed
+ * (csrc/mesh_exact.cuh); a query whose face is -1, outside [0, F), or has a vertex id outside [0, V) contributes nothing.
+ * Deterministic: g_verts sums each vertex's terms in ascending (query, corner) order, no atomics.  Also needs B * V * 3
+ * below 2^31 when g_verts is set. */
+DVQ_API int dvq_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
+                                       const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, void* stream);
 
 /* Host-buffer (end-to-end) form of the same forward: z_host/E_host/zq_host/idx_host are
  * HOST pointers (pinned for full overlap).  Rows are streamed through the GPU in chunks on
