@@ -34,6 +34,7 @@ int device_props(DeviceProps* out) {
   if (dev < 0 || dev >= 64) return fail(DVQ_ERR_CUDA, "device ordinal %d out of range", dev);
   if (!have[dev]) {
     DeviceProps p;
+    p.ordinal = dev;
     DVQ_CUDA_CHECK(cudaDeviceGetAttribute(&p.sm_count, cudaDevAttrMultiProcessorCount, dev));
     DVQ_CUDA_CHECK(cudaDeviceGetAttribute(&p.cc_major, cudaDevAttrComputeCapabilityMajor, dev));
     DVQ_CUDA_CHECK(cudaDeviceGetAttribute(&p.cc_minor, cudaDevAttrComputeCapabilityMinor, dev));

@@ -23,6 +23,7 @@ int fail(int code, const char* fmt, ...);
   } while (0)
 
 struct DeviceProps {
+  int ordinal;  // the current device, 0 <= ordinal < 64
   int sm_count;
   int cc_major;
   int cc_minor;

@@ -76,6 +76,12 @@ __device__ __forceinline__ float2 unpack_f16x2(uint32_t v) {
   return __half22float2(h);
 }
 
+// segment s contributes to the tiles of grid column col (the producer, MMA and epilogue warps all decide with this)
+__device__ __forceinline__ bool seg_valid(const PcParams& p, int s, int col) {
+  const int sc = col + p.seg[s].col_shift;
+  return sc >= 0 && sc < p.ncols_src;
+}
+
 __global__ void __launch_bounds__(PC_THREADS, 1) pcnn_gemm_kernel(const __grid_constant__ PcParams p) {
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar_full[PSTAGES], bar_empty[PSTAGES], bar_acc_full[2], bar_acc_empty[2];
@@ -107,9 +113,8 @@ __global__ void __launch_bounds__(PC_THREADS, 1) pcnn_gemm_kernel(const __grid_c
         const int mt = tile / p.n_tiles, nt = tile - mt * p.n_tiles;
         const int col = mt / p.tiles_per_col;
         for (int s = 0; ok && s < p.nseg; ++s) {
+          if (!seg_valid(p, s, col)) continue;
           const PcSeg& sg = p.seg[s];
-          const int sc = col + sg.col_shift;
-          if (sc < 0 || sc >= p.ncols_src) continue;
           const uint8_t* a = sg.a_img + (size_t)(mt + sg.tile_shift) * sg.a_kd * 256;
           const uint8_t* w = sg.w_img + (size_t)nt * sg.ks * 512;
           for (int k0 = 0; k0 < sg.ks; k0 += PKS, ++it) {
@@ -136,9 +141,8 @@ __global__ void __launch_bounds__(PC_THREADS, 1) pcnn_gemm_kernel(const __grid_c
       tc::tc_fence_after();
       uint32_t acc = 0;
       for (int s = 0; s < p.nseg; ++s) {
+        if (!seg_valid(p, s, col)) continue;
         const PcSeg& sg = p.seg[s];
-        const int sc = col + sg.col_shift;
-        if (sc < 0 || sc >= p.ncols_src) continue;
         for (int k0 = 0; k0 < sg.ks; k0 += PKS, ++it) {
           const uint32_t st = it % PSTAGES, ph = (it / PSTAGES) & 1u;
           if (!tc::mbar_wait(&bar_full[st], ph, errw, 3)) { acc = 0xffffffffu; break; }
@@ -169,10 +173,19 @@ __global__ void __launch_bounds__(PC_THREADS, 1) pcnn_gemm_kernel(const __grid_c
     const int quarter = warp & 3;                       // TMEM lanes this warp may access
     const int r = quarter * 32 + lane;                  // row inside the tile
     const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-    uint32_t q = 0;
+    uint32_t q = 0, live_bits = 0;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++q) {
       const int mt = tile / p.n_tiles, nt = tile - mt * p.n_tiles;
       const uint32_t t = q & 1u;
+      // A tile with no valid segment got no MMA: its TMEM stage still holds an earlier tile and is cleared below.  Lane k
+      // decides for the CTA's tile q + k, 32 tiles at a time, so the test stays off the per-tile path.
+      if ((q & 31u) == 0) {
+        const long long lt = tile + (long long)lane * gridDim.x;
+        bool live = false;
+        if (lt < ntiles)
+          for (int s = 0; s < p.nseg && !live; ++s) live = seg_valid(p, s, (int)lt / p.n_tiles / p.tiles_per_col);
+        live_bits = __ballot_sync(0xffffffffu, live);
+      }
       // bias of this tile -> shared memory (the four epilogue warps: 2 floats per thread)
       {
         const int et = ew * 32 + lane;
@@ -183,6 +196,10 @@ __global__ void __launch_bounds__(PC_THREADS, 1) pcnn_gemm_kernel(const __grid_c
       if (!tc::mbar_wait(&bar_acc_full[t], (q >> 1) & 1u, errw, 4)) break;
       tc::tc_fence_after();
       const uint32_t tbase = tmem + lane_addr + t * PTN;
+      if (!((live_bits >> (q & 31u)) & 1u)) {
+        for (int c = 0; c < PTN; c += 32) tc::tmem_st32_zero(tbase + (uint32_t)c);
+        tc::tmem_st_wait();
+      }
       const float* bs = sbias[t];
       if (p.mode == PC_GATE) {
         const int f0 = nt * 128;                        // first gated feature of this tile
@@ -361,10 +378,11 @@ int launch_pcnn_gemm(const DvqPcnnGemm* g, cudaStream_t s) {
   const int ntiles = p.m_tiles * p.n_tiles;
   const int grid = ntiles < dp.sm_count ? ntiles : dp.sm_count;
   const size_t smem = (size_t)PSTAGES * STAGE_BYTES + 128;
-  static bool attr_set = false;
-  if (!attr_set) {
+  // the opt-in applies to the current device only; set once per device, not per launch (hundreds per sample grid)
+  static bool attr_set[64] = {};
+  if (!attr_set[dp.ordinal]) {
     DVQ_CUDA_CHECK(cudaFuncSetAttribute(pcnn_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
+    attr_set[dp.ordinal] = true;
   }
   pcnn_gemm_kernel<<<grid, PC_THREADS, smem, s>>>(p);
   DVQ_CUDA_CHECK(cudaGetLastError());

@@ -96,6 +96,15 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
       : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// 0 -> 32 lanes x 32 consecutive columns (thread = TMEM lane); complete with tmem_st_wait() before reading them back
+__device__ __forceinline__ void tmem_st32_zero(uint32_t taddr) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+      "{%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, "
+      "%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1};" ::"r"(taddr), "r"(0u)
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // the same wait carrying a register dependence on the loaded values, so that the compiler cannot schedule their
 // consumers above it
 __device__ __forceinline__ void tmem_ld_wait_dep32(uint32_t (&v)[32]) {

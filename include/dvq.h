@@ -189,7 +189,8 @@ DVQ_API int dvq_onehot(const int64_t* idx, int64_t N, int K, float* out, void* s
  * C[m,n] = sum_s A_s[m + 128*tile_shift_s, :] . W_s[:, n], FP16 operands, FP32 accumulation.  Activations are FP16
  * operand images: rows in tiles of 128, a tile stored [K/8][128][8 halfs]; weights are images [n/256][K/8][256][8].
  * A grid row's rows are ordered column-major (m = column * B + b), so a convolution tap is a K-segment with a
- * whole-tile shift; a segment is skipped for tiles whose grid column + col_shift falls outside [0, ncols_src).
+ * whole-tile shift; a segment is skipped for tiles whose grid column + col_shift falls outside [0, ncols_src).  A tile
+ * none of whose segments is valid has C = 0 and receives the epilogue of the bias alone (+ residual / cond as below).
  * mode 0 GATE: 128 'a' + 128 'b' columns per tile, out = tanh(a + bias + cond_a) * sigmoid(b + bias + cond_b) -> FP16 image
  *   (out_kd = d wide) and, if pre_img, the raw a|b pre-activations (+ bias) -> FP16 image (2 d wide); cond_img: FP16 image
  *   [B, 2 d] of the class-conditional rows (may be NULL); d_gate = d.

@@ -160,3 +160,81 @@ def test_tc_kernel_sampler_matches_reference_logits():
     _, lg3 = m.generate(xb, lb, shape=(3, 3), batch_size=B2, forced=xb, return_logits=True)
     for n in range(9):
         assert float((lg2[n] - lg3[n]).abs().max()) < 2e-2 * float(lg3[n].abs().max()), n
+
+
+@pytest.fixture(scope="module")
+def bench_prior():
+    """The grasp benchmark's prior, GatedPixelCNN(512, 512, 15, 128) sampled with precision = "fp16_tc" at B = 4096
+    (seeded random biases, forced random grid and labels), its float64 copy, and a 256-row subset spread over the batch."""
+    import copy
+    torch.manual_seed(13)
+    m = GatedPixelCNN(512, 512, 15, 128).eval()
+    with torch.no_grad():
+        for n, p in m.named_parameters():
+            if n.endswith("bias"):
+                p.copy_(0.05 * torch.randn_like(p))
+    m = m.cuda()
+    m64 = copy.deepcopy(m).double()
+    m.precision = "fp16_tc"
+    B = 4096
+    gen = torch.Generator(device="cuda").manual_seed(14)
+    x = torch.randint(0, 512, (B, 3, 3), device="cuda", generator=gen)
+    label = torch.randint(0, 128, (B,), device="cuda", generator=gen)
+    _, logits = m.generate(None, label, shape=(3, 3), batch_size=B, forced=x, return_logits=True)
+    m._tc_sampler.check()
+    rows = torch.randperm(B, device="cuda", generator=gen)[:256].sort().values
+    return dict(m=m, m64=m64, x=x, label=label, logits=logits, rows=rows, gen=gen)
+
+
+def _same_bits(a, b):
+    return torch.equal(a.view(torch.int32), b.view(torch.int32))
+
+
+@pytest.mark.gpu
+def test_tc_sampler_at_bench_shape_is_equivariant_under_batch_permutation(bench_prior):
+    """A row's logits do not depend on which tile or CTA computed them: permuting the batch permutes all 9 steps' logits
+    bit for bit (every row of the multi-tile launches: 384-tile vertical stacks, 256-tile head)."""
+    p = bench_prior
+    perm = torch.randperm(p["x"].shape[0], device="cuda", generator=p["gen"])
+    _, lp = p["m"].generate(None, p["label"][perm], shape=(3, 3), batch_size=len(perm), forced=p["x"][perm], return_logits=True)
+    p["m"]._tc_sampler.check()
+    for n in range(9):
+        assert _same_bits(lp[n], p["logits"][n][perm]), n
+
+
+@pytest.mark.gpu
+def test_tc_sampler_at_bench_shape_does_not_depend_on_batch_size(bench_prior):
+    """256 rows spread over the batch, sampled alone (B = 256: 2 row tiles per grid column), equal their rows of the
+    B = 4096 run bit for bit."""
+    p = bench_prior
+    r = p["rows"]
+    _, ls = p["m"].generate(None, p["label"][r], shape=(3, 3), batch_size=len(r), forced=p["x"][r], return_logits=True)
+    p["m"]._tc_sampler.check()
+    for n in range(9):
+        assert _same_bits(ls[n], p["logits"][n][r]), n
+
+
+@pytest.mark.gpu
+def test_tc_sampler_at_bench_shape_matches_float64_forward(bench_prior):
+    """The fp16_tc logits of 256 rows of the B = 4096 run against the float64 reference forward of the grid as the
+    sampler sees it at step (i, j) (later positions 0), over 15 gated layers and the head.
+    Bar: 3e-3 of the logit scale, about 4x the error measured on a B200 (7.2e-4; worst step printed)."""
+    p = bench_prior
+    r = p["rows"]
+    x, label = p["x"][r], p["label"][r]
+    grids = []
+    for i in range(3):
+        for j in range(3):
+            g = torch.zeros_like(x)
+            g.view(len(r), 9)[:, :3 * i + j] = x.view(len(r), 9)[:, :3 * i + j]
+            grids.append(g)
+    with torch.no_grad():
+        full = p["m64"](torch.cat(grids), label.repeat(9))
+    worst = 0.0
+    for n in range(9):
+        i, j = divmod(n, 3)
+        ref = full[n * len(r):(n + 1) * len(r), :, i, j]
+        err = float((p["logits"][n][r].double() - ref).abs().max() / ref.abs().max())
+        worst = max(worst, err)
+    print("fp16_tc sampler, GatedPixelCNN(512, 512, 15): worst relative logit error %.2e vs float64" % worst)
+    assert worst < 3e-3, worst
