@@ -133,9 +133,8 @@ __global__ void __launch_bounds__(NN_THREADS) nn_forward_kernel(const float* __r
 }
 
 // One warp per batch item.  g_src is elementwise; g_trg is the ascending-i segmented sum: the warp walks its item's src
-// points 32 at a time, __match_any_sync groups the lanes that share a j, and the group's lowest lane adds the group's
-// terms into g_trg[b, j] in ascending lane order.  The warp owns the item's g_trg rows (zero-filled first, negated last),
-// so there are no races and no atomics.  An idx outside [0, N2) contributes nothing.
+// points 32 at a time and adds each chunk's terms into the item's g_trg rows with one warp_add_rows pass; the rows are
+// negated last.  An idx outside [0, N2) contributes nothing.
 constexpr int BW_WARPS = 4;
 
 __global__ void __launch_bounds__(BW_WARPS * 32) nn_backward_kernel(const float* __restrict__ src, const float* __restrict__ trg,
@@ -151,10 +150,7 @@ __global__ void __launch_bounds__(BW_WARPS * 32) nn_backward_kernel(const float*
   const float* G = g_dist + (size_t)b * N1;
   float* GS = g_src ? g_src + (size_t)b * N1 * 3 : nullptr;
   float* GT = g_trg ? g_trg + (size_t)b * N2 * 3 : nullptr;
-  if (GT) {
-    for (int k = lane; k < N2 * 3; k += 32) GT[k] = 0.f;
-    __syncwarp();
-  }
+  if (GT) warp_zero_rows(GT, N2);
   for (int c0 = 0; c0 < N1; c0 += 32) {
     const int i = c0 + lane;
     const int64_t j64 = i < N1 ? I[i] : -1;
@@ -173,22 +169,8 @@ __global__ void __launch_bounds__(BW_WARPS * 32) nn_backward_kernel(const float*
     if (GT) {
 #pragma unroll
       for (int k = 0; k < 3; ++k) term[w][k][lane] = t[k];
-      const unsigned vmask = __ballot_sync(0xffffffffu, valid);
       __syncwarp();
-      if (valid) {
-        const unsigned peers = __match_any_sync(vmask, j);
-        if (lane == __ffs(peers) - 1) {
-          float a[3] = {GT[j * 3], GT[j * 3 + 1], GT[j * 3 + 2]};
-          for (unsigned r = peers; r; r &= r - 1) {
-            const int l = __ffs(r) - 1;
-#pragma unroll
-            for (int k = 0; k < 3; ++k) a[k] = __fadd_rn(a[k], term[w][k][l]);
-          }
-#pragma unroll
-          for (int k = 0; k < 3; ++k) GT[j * 3 + k] = a[k];
-        }
-      }
-      __syncwarp();
+      warp_add_rows(GT, valid ? j : -1, term[w], 0);
     }
   }
   if (GT) {
@@ -207,11 +189,11 @@ __global__ void __launch_bounds__(128) vertex_normals_kernel(const float* __rest
   const float* P = verts + (size_t)b * V * 3;
   float3 acc = make_float3(0.f, 0.f, 0.f);
   for (int e = vf_offsets[v], e1 = vf_offsets[v + 1]; e < e1; ++e) {
-    const int f = vf_faces[e];
-    const int a = faces[f * 3], c = faces[f * 3 + 1], d = faces[f * 3 + 2];
-    if ((unsigned)a >= (unsigned)V || (unsigned)c >= (unsigned)V || (unsigned)d >= (unsigned)V) continue;
-    const float3 n = face_normal(make_float3(P[a * 3], P[a * 3 + 1], P[a * 3 + 2]), make_float3(P[c * 3], P[c * 3 + 1], P[c * 3 + 2]),
-                                 make_float3(P[d * 3], P[d * 3 + 1], P[d * 3 + 2]));
+    int id[3];
+    if (!face_ids(faces, vf_faces[e], V, id)) continue;
+    const float3 n = face_normal(make_float3(P[id[0] * 3], P[id[0] * 3 + 1], P[id[0] * 3 + 2]),
+                                 make_float3(P[id[1] * 3], P[id[1] * 3 + 1], P[id[1] * 3 + 2]),
+                                 make_float3(P[id[2] * 3], P[id[2] * 3 + 1], P[id[2] * 3 + 2]));
     acc = make_float3(__fadd_rn(acc.x, n.x), __fadd_rn(acc.y, n.y), __fadd_rn(acc.z, n.z));
   }
   const float3 r = normalize_eps(acc);

@@ -422,71 +422,71 @@ int dvq_vertex_normals(const float* verts, int B, int V, const int* faces, int F
 
 // The mesh kernels index within a call in 32 bits.  Bm and Bp are each 1 or B (B = the other one when one of them is 1),
 // the mesh's and the queries' [n, V or Q, 3] tensors, the [B, Q] outputs and faces [F, 3] must each have fewer than 2^31
-// elements.  On success *B is the broadcast batch.
-static int check_mesh_shape(int Bm, int V, int F, int Bp, int Q, int* B) {
+// elements.  On success *m describes the call.
+static int check_mesh_shape(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, MeshQuery* m) {
   if (Bm < 0 || Bp < 0 || V <= 0 || F < 0 || Q < 0)
     return fail(DVQ_ERR_BAD_SHAPE, "need Bm >= 0, Bp >= 0, V > 0, F >= 0, Q >= 0 (got Bm=%d Bp=%d V=%d F=%d Q=%d)", Bm, Bp, V, F, Q);
-  *B = Bm == 1 ? Bp : Bm;
-  if (Bp != *B && Bp != 1) return fail(DVQ_ERR_BAD_SHAPE, "Bm and Bp must each be 1 or the batch size (got Bm=%d Bp=%d)", Bm, Bp);
-  if ((long long)Bm * V * 3 >= (1LL << 31) || (long long)Bp * Q * 3 >= (1LL << 31) || (long long)*B * Q * 3 >= (1LL << 31) ||
+  const int B = Bm == 1 ? Bp : Bm;
+  if (Bp != B && Bp != 1) return fail(DVQ_ERR_BAD_SHAPE, "Bm and Bp must each be 1 or the batch size (got Bm=%d Bp=%d)", Bm, Bp);
+  if ((long long)Bm * V * 3 >= (1LL << 31) || (long long)Bp * Q * 3 >= (1LL << 31) || (long long)B * Q * 3 >= (1LL << 31) ||
       (long long)F * 3 >= (1LL << 31))
     return fail(DVQ_ERR_BAD_SHAPE, "Bm * V * 3, Bp * Q * 3, B * Q * 3 and F * 3 must be below 2^31; split the batch");
+  *m = MeshQuery{verts, Bm, V, faces, F, pts, Bp, Q, B};
   return DVQ_OK;
 }
 
 int dvq_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, float* w,
                      int* inside_count, void* stream) {
-  int B = 0;
-  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  MeshQuery m;
+  int rc = check_mesh_shape(verts, Bm, V, faces, F, pts, Bp, Q, &m);
   if (rc) return rc;
   if (!w && !inside_count) return fail(DVQ_ERR_BAD_ARG, "w and inside_count must not both be NULL");
-  if ((long long)B * Q > 0 && (!verts || !pts || (F > 0 && !faces)))   // empty tensors may have NULL data pointers
+  if ((long long)m.B * Q > 0 && (!verts || !pts || (F > 0 && !faces)))   // empty tensors may have NULL data pointers
     return fail(DVQ_ERR_BAD_ARG, "verts, faces and pts must not be NULL");
   rc = require_sm100();
   if (rc) return rc;
-  return launch_mesh_winding(verts, Bm, V, faces, F, pts, Bp, Q, B, w, inside_count, static_cast<cudaStream_t>(stream));
+  return launch_mesh_winding(m, w, inside_count, static_cast<cudaStream_t>(stream));
 }
 
 int dvq_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, float* dist2,
                       int64_t* face, void* stream) {
-  int B = 0;
-  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  MeshQuery m;
+  int rc = check_mesh_shape(verts, Bm, V, faces, F, pts, Bp, Q, &m);
   if (rc) return rc;
   if (F == 0) return fail(DVQ_ERR_BAD_SHAPE, "dvq_mesh_distance needs F > 0");
-  if ((long long)B * Q > 0 && (!verts || !faces || !pts || !dist2 || !face))
+  if ((long long)m.B * Q > 0 && (!verts || !faces || !pts || !dist2 || !face))
     return fail(DVQ_ERR_BAD_ARG, "verts, faces, pts, dist2 and face must not be NULL");
   rc = require_sm100();
   if (rc) return rc;
-  return launch_mesh_distance(verts, Bm, V, faces, F, pts, Bp, Q, B, dist2, face, static_cast<cudaStream_t>(stream));
+  return launch_mesh_distance(m, dist2, face, static_cast<cudaStream_t>(stream));
 }
 
 int dvq_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, float* depth2,
                          int64_t* face, void* stream) {
-  int B = 0;
-  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  MeshQuery m;
+  int rc = check_mesh_shape(verts, Bm, V, faces, F, pts, Bp, Q, &m);
   if (rc) return rc;
   if (F == 0) return fail(DVQ_ERR_BAD_SHAPE, "dvq_mesh_penetration needs F > 0");
-  if ((long long)B * Q > 0 && (!verts || !faces || !pts || !depth2 || !face))
+  if ((long long)m.B * Q > 0 && (!verts || !faces || !pts || !depth2 || !face))
     return fail(DVQ_ERR_BAD_ARG, "verts, faces, pts, depth2 and face must not be NULL");
   rc = require_sm100();
   if (rc) return rc;
-  return launch_mesh_penetration(verts, Bm, V, faces, F, pts, Bp, Q, B, depth2, face, static_cast<cudaStream_t>(stream));
+  return launch_mesh_penetration(m, depth2, face, static_cast<cudaStream_t>(stream));
 }
 
 int dvq_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q,
                                const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, void* stream) {
-  int B = 0;
-  int rc = check_mesh_shape(Bm, V, F, Bp, Q, &B);
+  MeshQuery m;
+  int rc = check_mesh_shape(verts, Bm, V, faces, F, pts, Bp, Q, &m);
   if (rc) return rc;
   if (!g_pts && !g_verts) return fail(DVQ_ERR_BAD_ARG, "g_pts and g_verts must not both be NULL");
-  if (g_verts && (long long)B * V * 3 >= (1LL << 31))
-    return fail(DVQ_ERR_BAD_SHAPE, "B * V * 3 = %lld must be below 2^31 for g_verts; split the batch", (long long)B * V * 3);
-  if ((long long)B * Q > 0 && (!verts || !pts || !face || !g_dist2 || (F > 0 && !faces)))
+  if (g_verts && (long long)m.B * V * 3 >= (1LL << 31))
+    return fail(DVQ_ERR_BAD_SHAPE, "B * V * 3 = %lld must be below 2^31 for g_verts; split the batch", (long long)m.B * V * 3);
+  if ((long long)m.B * Q > 0 && (!verts || !pts || !face || !g_dist2 || (F > 0 && !faces)))
     return fail(DVQ_ERR_BAD_ARG, "verts, faces, pts, face and g_dist2 must not be NULL");
   rc = require_sm100();
   if (rc) return rc;
-  return launch_mesh_distance_backward(verts, Bm, V, faces, F, pts, Bp, Q, B, face, g_dist2, g_pts, g_verts,
-                                       static_cast<cudaStream_t>(stream));
+  return launch_mesh_distance_backward(m, face, g_dist2, g_pts, g_verts, static_cast<cudaStream_t>(stream));
 }
 
 int dvq_pcnn_gemm(const DvqPcnnGemm* g, void* stream) {

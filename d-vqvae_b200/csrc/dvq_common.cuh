@@ -208,16 +208,28 @@ int launch_nn_backward(const float* src, const float* trg, const int64_t* idx, c
 int launch_vertex_normals(const float* verts, int B, int V, const int* faces, const int* vf_offsets, const int* vf_faces,
                           float* normals, cudaStream_t s);
 
-// mesh winding numbers, point-to-mesh distances, penetration and the distance gradient (mesh_sm100.cu); B = the broadcast
-// batch of Bm and Bp
-int launch_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B, float* w,
-                        int* inside_count, cudaStream_t s);
-int launch_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
-                         float* dist2, int64_t* face, cudaStream_t s);
-int launch_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
-                            float* depth2, int64_t* face, cudaStream_t s);
-int launch_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
-                                  const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, cudaStream_t s);
+// ---- one mesh query call (mesh_sm100.cu), as its launchers and kernels see it -------------
+// Filled by check_mesh_shape.  Mesh batch Bm and query batch Bp are each 1 or B: item b's mesh is verts[Bm == 1 ? 0 : b],
+// its queries pts[Bp == 1 ? 0 : b] (an object's voxel list shared by every hand, or every hand's vertices against one
+// object).
+struct MeshQuery {
+  const float* verts;   // [Bm, V, 3]
+  int Bm, V;
+  const int* faces;     // [F, 3]
+  int F;
+  const float* pts;     // [Bp, Q, 3]
+  int Bp, Q;
+  int B;                // the broadcast batch
+  __host__ __device__ const float* mesh(int b) const { return verts + (size_t)(Bm == 1 ? 0 : b) * V * 3; }
+  __host__ __device__ const float* queries(int b) const { return pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3; }
+};
+
+// mesh winding numbers, point-to-mesh distances, penetration and the distance gradient (mesh_sm100.cu)
+int launch_mesh_winding(const MeshQuery& m, float* w, int* inside_count, cudaStream_t s);
+int launch_mesh_distance(const MeshQuery& m, float* dist2, int64_t* face, cudaStream_t s);
+int launch_mesh_penetration(const MeshQuery& m, float* depth2, int64_t* face, cudaStream_t s);
+int launch_mesh_distance_backward(const MeshQuery& m, const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts,
+                                  cudaStream_t s);
 
 // PointNet
 size_t pointnet_workspace_bytes(int B, int C, int P, int flags);
@@ -286,6 +298,41 @@ __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
+}
+
+// the vertex ids of face f of faces [F, 3]; false when one of them lies outside [0, V), which skips the face
+__device__ __forceinline__ bool face_ids(const int* __restrict__ faces, int f, int V, int (&id)[3]) {
+#pragma unroll
+  for (int j = 0; j < 3; ++j) id[j] = __ldg(faces + (size_t)f * 3 + j);
+  return (unsigned)id[0] < (unsigned)V && (unsigned)id[1] < (unsigned)V && (unsigned)id[2] < (unsigned)V;
+}
+
+// Ordered, atomic-free row sums of a warp (the backward kernels' scatter of per-slot terms into [n_rows, 3] rows).  The
+// warp owns its item's rows, so there are no races and no atomics: warp_zero_rows zero-fills them, then each
+// warp_add_rows pass takes 32 slots, slot l (lane l) adding terms term[0..2][base + l] into row `row` (-1: nothing).
+// __match_any_sync groups the slots that share a row and the group's lowest lane adds them in ascending slot order, so
+// over passes in ascending base every row's terms are summed in ascending slot order from +0.
+__device__ __forceinline__ void warp_zero_rows(float* rows, int n_rows) {
+  for (int k = threadIdx.x & 31; k < n_rows * 3; k += 32) rows[k] = 0.f;
+  __syncwarp();
+}
+template <int N>
+__device__ __forceinline__ void warp_add_rows(float* rows, int row, const float (&term)[3][N], int base) {
+  const unsigned vmask = __ballot_sync(0xffffffffu, row >= 0);
+  if (row >= 0) {
+    const unsigned peers = __match_any_sync(vmask, row);
+    if ((threadIdx.x & 31) == __ffs(peers) - 1) {
+      float acc[3] = {rows[(size_t)row * 3], rows[(size_t)row * 3 + 1], rows[(size_t)row * 3 + 2]};
+      for (unsigned rest = peers; rest; rest &= rest - 1) {
+        const int l = base + __ffs(rest) - 1;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) acc[k] = __fadd_rn(acc[k], term[k][l]);
+      }
+#pragma unroll
+      for (int k = 0; k < 3; ++k) rows[(size_t)row * 3 + k] = acc[k];
+    }
+  }
+  __syncwarp();
 }
 
 }  // namespace dvq

@@ -16,7 +16,8 @@
 //              every axis, so a NaN query is outside.
 //   distance   dist2(q) = min over f of the squared distance from q to the closest point of triangle f (Ericson, Real-Time
 //              Collision Detection 5.1.5, written as closest = a + v ab + w ac, dist2 = |ap - v ab - w ac|^2).  A triangle
-//              whose fp32 area^2 = |ab x ac|^2 is 0 is taken as its three edge segments (no 0/0 in the interior region).
+//              whose fp32 area^2 = |ab x ac|^2 is 0 is degenerate (no 0/0 in the interior region): it is its three edge
+//              segments ab, ac, bc, in that order (face_segments), and its dist2 is the minimum of their segment_dist2.
 //   face       the lowest f among exact fp32 minima of dist2; NaN counts as +inf (so a triangle with a non-finite corner
 //              never wins).  When no face gives a finite distance, face = 0 and dist2 = +inf.
 //   penetration  per query: depth2 = dist2 and face = the closest face when w >= 0.5, else depth2 = +0 and face = -1, with w,
@@ -27,8 +28,8 @@
 //   offset     triangle (fp32 area^2 != 0): from the forward's staged a = v0, ab = fl(v1 - v0), ac = fl(v2 - v0), aa, cc,
 //              bc and ap = fl(q - a): (v, w) = closest_vw, d = ap - v ab - w ac in tri_offset2's FMA order, so
 //              fma(dz, dz, fma(dy, dy, dx dx)) is the forward's dist2 bit for bit; lambda = (fl(fl(1 - v) - w), v, w).
-//              Degenerate face: the first of the segments ab, ac, bc whose segment_dist2 equals the forward's minimum over
-//              the three, its t and offset from segment_offset, its two endpoints weighted (fl(1 - t), t), the third 0.
+//              Degenerate face: the first of its segments whose segment_dist2 equals that minimum, its t and offset from
+//              segment_offset, its two endpoints weighted (fl(1 - t), t), the third 0.
 //   g_pts      = fl(2 g) d per component, g the upstream gradient of dist2.
 //   g_verts    corner k of face f gets the term -fl(lambda_k g_pts); g_verts[b, vertex] is the sum of its terms in
 //              ascending (query, corner) order from +0 (no atomics).
@@ -159,6 +160,21 @@ __device__ __forceinline__ float segment_dist2(float px, float py, float pz, flo
   float dx, dy, dz;
   segment_offset(px, py, pz, ex, ey, ez, dx, dy, dz);
   return dx * dx + dy * dy + dz * dz;
+}
+
+// The segments of a degenerate face, k = 0 ab, 1 ac, 2 bc, from the query's offset ap = fl(q - a) and the face's ab = e1,
+// ac = e2: segment k is a' + t e[k] with p[k] = fl(q - a') -- (ap, ab), (ap, ac), (fl(ap - ab), fl(ac - ab)) -- and s[k] =
+// its segment_dist2.
+__device__ __forceinline__ void face_segments(const float (&ap)[3], const float (&e1)[3], const float (&e2)[3], float (&p)[3][3],
+                                              float (&e)[3][3], float (&s)[3]) {
+#pragma unroll
+  for (int d = 0; d < 3; ++d) {
+    p[0][d] = ap[d], e[0][d] = e1[d];
+    p[1][d] = ap[d], e[1][d] = e2[d];
+    p[2][d] = ap[d] - e1[d], e[2][d] = e2[d] - e1[d];
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) s[k] = segment_dist2(p[k][0], p[k][1], p[k][2], e[k][0], e[k][1], e[k][2]);
 }
 
 }  // namespace dvq

@@ -11,14 +11,12 @@
 // per face (skip: a vertex id outside [0, V); triangle; or degenerate: area^2 = 0, taken as three segments).  The flag is
 // the same for every thread, so its branch never diverges.
 //
-// Mesh batch Bm and query batch Bp are each 1 or B: the item's mesh is verts[Bm == 1 ? 0 : b], its queries
-// pts[Bp == 1 ? 0 : b] (an object's voxel list shared by every hand, or every hand's vertices against one object).
+// The winding phase (winding_phase) first reduces the item's vertex box over the CTA; a query outside it gets w = 0 (the
+// box rule), and a CTA none of whose queries lies inside stages no face: that keeps the voxel-volume pass proportional to
+// the hand/object overlap rather than to (voxels x hands).  mesh_winding_kernel's per-CTA inside count is one integer
+// atomicAdd.
 //
-// mesh_winding_kernel first reduces the item's vertex box over the CTA; a query outside it gets w = 0 (the box rule), and
-// a CTA none of whose queries lies inside exits before staging a face: that keeps the voxel-volume pass proportional to
-// the hand/object overlap rather than to (voxels x hands).  The per-CTA inside count is one integer atomicAdd.
-//
-// mesh_penetration_kernel runs the winding sweep, compacts the CTA's inside queries into a shared-memory list and runs the
+// mesh_penetration_kernel runs the winding phase, compacts the CTA's inside queries into a shared-memory list and runs the
 // distance sweep over that list only; a CTA with no inside query never stages a face for distances.
 #include "dvq_common.cuh"
 #include "mesh_exact.cuh"
@@ -45,13 +43,6 @@ struct DistanceStage {
   float sd[3][MESH_STAGE];                             // ab . ab, ac . ac, ab . ac
   uint8_t sflag[MESH_STAGE];
 };
-
-__device__ __forceinline__ bool face_ids(const int* __restrict__ faces, int f, int V, int& i0, int& i1, int& i2) {
-  i0 = __ldg(faces + (size_t)f * 3);
-  i1 = __ldg(faces + (size_t)f * 3 + 1);
-  i2 = __ldg(faces + (size_t)f * 3 + 2);
-  return (unsigned)i0 < (unsigned)V && (unsigned)i1 < (unsigned)V && (unsigned)i2 < (unsigned)V;
-}
 
 // The CTA's queries: thread tid holds i0 + p * MESH_THREADS, p < MESH_Q, as packed pairs (2q, 2q + 1); past Q -> 0.
 __device__ __forceinline__ void load_queries(const float* __restrict__ S, int Q, int i0, float (&c)[MESH_Q][3], uint64_t (&qx)[MESH_PAIRS],
@@ -130,7 +121,7 @@ __device__ __forceinline__ void winding_sum(const float* __restrict__ P, int V, 
     __syncthreads();
     for (int k = tid; k < n; k += MESH_THREADS) {
       int id[3];
-      const bool ok = face_ids(faces, f0 + k, V, id[0], id[1], id[2]);
+      const bool ok = face_ids(faces, f0 + k, V, id);
       st.sflag[k] = ok ? FACE_TRI : FACE_SKIP;
 #pragma unroll
       for (int j = 0; j < 3; ++j) {
@@ -159,12 +150,32 @@ __device__ __forceinline__ void winding_sum(const float* __restrict__ P, int V, 
   }
 }
 
+// The winding phase of the CTA's queries (P, S: the item's mesh and queries): per query of the thread, w = 0 outside the
+// item's vertex box, fl(S / fl(4 pi)) inside it; returns box_rule's vote (false: the CTA staged no face).
+__device__ __forceinline__ bool winding_phase(const MeshQuery& m, const float* P, const float* S, int i0, float (&w)[MESH_Q],
+                                              float* box, float (*red)[6], WindingStage& st) {
+  float c[MESH_Q][3];
+  uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
+  load_queries(S, m.Q, i0, c, qx, qy, qz);
+  bool inbox[MESH_Q];
+  if (!box_rule(P, m.V, m.Q, i0, c, inbox, box, red)) {
+#pragma unroll
+    for (int p = 0; p < MESH_Q; ++p) w[p] = 0.f;
+    return false;
+  }
+  float acc[MESH_Q];
+  winding_sum(P, m.V, m.faces, m.F, qx, qy, qz, acc, st);
+#pragma unroll
+  for (int p = 0; p < MESH_Q; ++p) w[p] = inbox[p] ? __fdiv_rn(acc[p], MESH_4PI) : 0.f;
+  return true;
+}
+
 // Stages faces f0 .. f0 + n - 1 of P for the distance: a, ab, ac packed, the three dot products and the flag.
 __device__ __forceinline__ void distance_stage(const float* __restrict__ P, int V, const int* __restrict__ faces, int f0, int n,
                                                DistanceStage& st) {
   for (int k = threadIdx.x; k < n; k += MESH_THREADS) {
     int id[3];
-    const bool ok = face_ids(faces, f0 + k, V, id[0], id[1], id[2]);
+    const bool ok = face_ids(faces, f0 + k, V, id);
     float p[3][3] = {{0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
     if (ok) {
 #pragma unroll
@@ -193,7 +204,7 @@ __device__ __forceinline__ void face_dist2(uint8_t flag, const uint64_t (&v)[9],
     uint64_t dx, dy, dz;
     tri_offset2(px, py, pz, v + 3, aa, cc, bc, vv, ww, dx, dy, dz);
     unpack_f32x2(dot2(dx, dy, dz, dx, dy, dz), d[0], d[1]);
-  } else {                                           // degenerate: the three edges ab, ac, bc
+  } else {                                           // degenerate: its three segments
     float ap[2][3], e1[3], e2[3], unused;
     unpack_f32x2(px, ap[0][0], ap[1][0]);
     unpack_f32x2(py, ap[0][1], ap[1][1]);
@@ -205,11 +216,9 @@ __device__ __forceinline__ void face_dist2(uint8_t flag, const uint64_t (&v)[9],
     }
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
-      const float sab = segment_dist2(ap[h][0], ap[h][1], ap[h][2], e1[0], e1[1], e1[2]);
-      const float sac = segment_dist2(ap[h][0], ap[h][1], ap[h][2], e2[0], e2[1], e2[2]);
-      const float sbc = segment_dist2(ap[h][0] - e1[0], ap[h][1] - e1[1], ap[h][2] - e1[2], e2[0] - e1[0], e2[1] - e1[1],
-                                      e2[2] - e1[2]);
-      d[h] = fminf(fminf(sab, sac), sbc);
+      float p[3][3], e[3][3], s[3];
+      face_segments(ap[h], e1, e2, p, e, s);
+      d[h] = fminf(fminf(s[0], s[1]), s[2]);
     }
   }
 }
@@ -256,23 +265,16 @@ __device__ __forceinline__ void distance_sweep(const float* __restrict__ P, int 
   }
 }
 
-__global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(const float* __restrict__ verts, int Bm, int V,
-                                                                     const int* __restrict__ faces, int F, const float* __restrict__ pts,
-                                                                     int Bp, int Q, int tiles, float* __restrict__ w,
-                                                                     int* __restrict__ inside_count) {
+__global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(__grid_constant__ const MeshQuery m, int tiles,
+                                                                     float* __restrict__ w, int* __restrict__ inside_count) {
   __shared__ __align__(16) WindingStage st;
   __shared__ float red[MESH_WARPS][6];
   __shared__ float box[6];
-  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x;
-  const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
-  const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
+  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x, Q = m.Q;
   const int i0 = tile * MESH_TILE + tid;
 
-  float c[MESH_Q][3];
-  uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
-  load_queries(S, Q, i0, c, qx, qy, qz);
-  bool inbox[MESH_Q];
-  if (!box_rule(P, V, Q, i0, c, inbox, box, red)) {   // the whole tile is outside the box: w = 0, nothing inside
+  float wv[MESH_Q];
+  if (!winding_phase(m, m.mesh(b), m.queries(b), i0, wv, box, red, st)) {   // the whole tile is outside the box: w = 0
     if (w) {
 #pragma unroll
       for (int p = 0; p < MESH_Q; ++p) {
@@ -282,16 +284,12 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(const float*
     }
     return;
   }
-
-  float acc[MESH_Q];
-  winding_sum(P, V, faces, F, qx, qy, qz, acc, st);
   int mine[MESH_Q];
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
     const int i = i0 + p * MESH_THREADS;
-    const float wv = inbox[p] ? __fdiv_rn(acc[p], MESH_4PI) : 0.f;
-    mine[p] = i < Q && wv >= 0.5f;
-    if (w && i < Q) w[(size_t)b * Q + i] = wv;
+    mine[p] = i < Q && wv[p] >= 0.5f;
+    if (w && i < Q) w[(size_t)b * Q + i] = wv[p];
   }
   if (inside_count) {
     int total = 0;
@@ -301,22 +299,18 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_winding_kernel(const float*
   }
 }
 
-__global__ void __launch_bounds__(MESH_THREADS) mesh_distance_kernel(const float* __restrict__ verts, int Bm, int V,
-                                                                      const int* __restrict__ faces, int F, const float* __restrict__ pts,
-                                                                      int Bp, int Q, int tiles, float* __restrict__ dist2,
-                                                                      int64_t* __restrict__ face) {
+__global__ void __launch_bounds__(MESH_THREADS) mesh_distance_kernel(__grid_constant__ const MeshQuery m, int tiles,
+                                                                      float* __restrict__ dist2, int64_t* __restrict__ face) {
   __shared__ __align__(16) DistanceStage st;
-  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x;
-  const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
-  const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
+  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x, Q = m.Q;
   const int i0 = tile * MESH_TILE + tid;
 
   float c[MESH_Q][3];
   uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
-  load_queries(S, Q, i0, c, qx, qy, qz);
+  load_queries(m.queries(b), Q, i0, c, qx, qy, qz);
   float best[MESH_Q];
   int bf[MESH_Q];
-  distance_sweep(P, V, faces, F, qx, qy, qz, MESH_PAIRS, true, best, bf, st);
+  distance_sweep(m.mesh(b), m.V, m.faces, m.F, qx, qy, qz, MESH_PAIRS, true, best, bf, st);
 
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
@@ -327,14 +321,12 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_distance_kernel(const float
   }
 }
 
-// Phase 1 is mesh_winding_kernel's box rule and sum.  Phase 2 compacts the inside queries, in ascending query order, into
-// slist; list entry j is held by thread (j mod 256) / 2 in half j mod 2 of pair j / 256, so n inside queries occupy the
-// first ceil(n / 64) warps and one pair per thread while n <= 256.  The distance faces are staged into the same shared
-// memory as the winding faces.
-__global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const float* __restrict__ verts, int Bm, int V,
-                                                                         const int* __restrict__ faces, int F,
-                                                                         const float* __restrict__ pts, int Bp, int Q, int tiles,
-                                                                         float* __restrict__ depth2, int64_t* __restrict__ face) {
+// Phase 1 is the winding phase.  Phase 2 compacts the inside queries, in ascending query order, into slist; list entry j
+// is held by thread (j mod 256) / 2 in half j mod 2 of pair j / 256, so n inside queries occupy the first ceil(n / 64)
+// warps and one pair per thread while n <= 256.  The distance faces are staged into the same shared memory as the winding
+// faces.  The bound of 6 CTAs per SM caps ptxas at 80 registers; without it, ptxas takes 94 (5 CTAs per SM).
+__global__ void __launch_bounds__(MESH_THREADS, 6) mesh_penetration_kernel(__grid_constant__ const MeshQuery m, int tiles,
+                                                                            float* __restrict__ depth2, int64_t* __restrict__ face) {
   __shared__ __align__(16) union {
     WindingStage w;
     DistanceStage d;
@@ -344,31 +336,21 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const fl
   __shared__ float slist[3][MESH_TILE];
   __shared__ int sidx[MESH_TILE];
   __shared__ int wcount[MESH_Q][MESH_WARPS];
-  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
-  const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
+  const int b = blockIdx.x / tiles, tile = blockIdx.x - b * tiles, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, Q = m.Q;
+  const float* P = m.mesh(b);
+  const float* S = m.queries(b);
   const int i0 = tile * MESH_TILE + tid;
   float* D = depth2 + (size_t)b * Q;
   int64_t* FC = face + (size_t)b * Q;
 
   bool inside[MESH_Q];
   {
-    float c[MESH_Q][3];
-    uint64_t qx[MESH_PAIRS], qy[MESH_PAIRS], qz[MESH_PAIRS];
-    load_queries(S, Q, i0, c, qx, qy, qz);
-    bool inbox[MESH_Q];
-    const bool any = box_rule(P, V, Q, i0, c, inbox, box, red);
-#pragma unroll
-    for (int p = 0; p < MESH_Q; ++p) inside[p] = false;
-    if (any) {
-      float acc[MESH_Q];
-      winding_sum(P, V, faces, F, qx, qy, qz, acc, st.w);
-#pragma unroll
-      for (int p = 0; p < MESH_Q; ++p) inside[p] = inbox[p] && __fdiv_rn(acc[p], MESH_4PI) >= 0.5f;
-    }
+    float wv[MESH_Q];
+    const bool any = winding_phase(m, P, S, i0, wv, box, red, st.w);
 #pragma unroll
     for (int p = 0; p < MESH_Q; ++p) {
       const int i = i0 + p * MESH_THREADS;
+      inside[p] = wv[p] >= 0.5f;
       if (i < Q && !inside[p]) {
         D[i] = 0.f;
         FC[i] = -1;
@@ -377,11 +359,11 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const fl
     if (!any) return;                                  // CTA-uniform: box_rule's vote
   }
 
-  unsigned m[MESH_Q];
+  unsigned mask[MESH_Q];
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
-    m[p] = __ballot_sync(0xffffffffu, inside[p]);
-    if (lane == 0) wcount[p][warp] = __popc(m[p]);
+    mask[p] = __ballot_sync(0xffffffffu, inside[p]);
+    if (lane == 0) wcount[p][warp] = __popc(mask[p]);
   }
   __syncthreads();
   int n_in = 0, off[MESH_Q];
@@ -397,7 +379,7 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const fl
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
     if (inside[p]) {
-      const int j = off[p] + __popc(m[p] & ((1u << lane) - 1u)), i = i0 + p * MESH_THREADS;
+      const int j = off[p] + __popc(mask[p] & ((1u << lane) - 1u)), i = i0 + p * MESH_THREADS;
 #pragma unroll
       for (int k = 0; k < 3; ++k) slist[k][j] = __ldg(S + (size_t)i * 3 + k);
       sidx[j] = i;
@@ -423,7 +405,7 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const fl
   const bool active = warp * 64 < n_in;
   float best[MESH_Q];
   int bf[MESH_Q];
-  distance_sweep(P, V, faces, F, qx, qy, qz, pairs, active, best, bf, st.d);
+  distance_sweep(P, m.V, m.faces, m.F, qx, qy, qz, pairs, active, best, bf, st.d);
 #pragma unroll
   for (int p = 0; p < MESH_Q; ++p) {
     const int j = (p >> 1) * 2 * MESH_THREADS + 2 * tid + (p & 1);
@@ -438,36 +420,32 @@ __global__ void __launch_bounds__(MESH_THREADS) mesh_penetration_kernel(const fl
 // One warp per broadcast item b, which owns (zero-fills, then accumulates) the item's g_verts rows: no races, no atomics.
 // The warp walks the item's queries 32 at a time; each lane recomputes its query's offset at its face (mesh_exact.cuh)
 // and writes g_pts.  The chunk's 96 (query, corner) terms go to shared memory in ascending (query, corner) order and are
-// added in three passes of 32 slots: in each, __match_any_sync groups the slots that share a vertex and the group's lowest
-// lane adds them into g_verts in ascending slot order, so every vertex's terms are summed in ascending (query, corner)
-// order.
+// added into g_verts by three warp_add_rows passes, so every vertex's terms are summed in ascending (query, corner) order.
 constexpr int BW_WARPS = 4;
 
-__global__ void __launch_bounds__(BW_WARPS * 32) mesh_distance_backward_kernel(
-    const float* __restrict__ verts, int Bm, int V, const int* __restrict__ faces, int F, const float* __restrict__ pts, int Bp,
-    int Q, int B, const int64_t* __restrict__ face, const float* __restrict__ g_dist2, float* __restrict__ g_pts,
-    float* __restrict__ g_verts) {
+__global__ void __launch_bounds__(BW_WARPS * 32) mesh_distance_backward_kernel(__grid_constant__ const MeshQuery m,
+                                                                               const int64_t* __restrict__ face,
+                                                                               const float* __restrict__ g_dist2,
+                                                                               float* __restrict__ g_pts, float* __restrict__ g_verts) {
   __shared__ float term[BW_WARPS][3][96];
   __shared__ int tvert[BW_WARPS][96];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, b = blockIdx.x * BW_WARPS + w;
-  if (b >= B) return;
-  const float* P = verts + (size_t)(Bm == 1 ? 0 : b) * V * 3;
-  const float* S = pts + (size_t)(Bp == 1 ? 0 : b) * Q * 3;
+  if (b >= m.B) return;
+  const int V = m.V, Q = m.Q;
+  const float* P = m.mesh(b);
+  const float* S = m.queries(b);
   const int64_t* I = face + (size_t)b * Q;
   const float* G = g_dist2 + (size_t)b * Q;
   float* GP = g_pts ? g_pts + (size_t)b * Q * 3 : nullptr;
   float* GV = g_verts ? g_verts + (size_t)b * V * 3 : nullptr;
-  if (GV) {
-    for (int k = lane; k < V * 3; k += 32) GV[k] = 0.f;
-    __syncwarp();
-  }
+  if (GV) warp_zero_rows(GV, V);
   for (int c0 = 0; c0 < Q; c0 += 32) {
     const int i = c0 + lane;
     int id[3] = {-1, -1, -1};
     float lam[3] = {0.f, 0.f, 0.f}, t[3] = {0.f, 0.f, 0.f};
     bool valid = false;
     const int64_t f64 = i < Q ? I[i] : -1;
-    if (f64 >= 0 && f64 < F && face_ids(faces, (int)f64, V, id[0], id[1], id[2])) {
+    if (f64 >= 0 && f64 < m.F && face_ids(m.faces, (int)f64, V, id)) {
       float p[3][3], q[3];
 #pragma unroll
       for (int j = 0; j < 3; ++j) {
@@ -496,26 +474,22 @@ __global__ void __launch_bounds__(BW_WARPS * 32) mesh_distance_backward_kernel(
         lam[1] = vv[0];
         lam[2] = ww[0];
       } else {                                          // degenerate: the first segment attaining the forward's minimum
-        float ap[3], bp[3], ebc[3];
+        float ap[3], sp[3][3], se[3][3], s[3];
 #pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          ap[k] = q[k] - a[k];
-          bp[k] = ap[k] - e1[k];
-          ebc[k] = e2[k] - e1[k];
-        }
-        const float sab = segment_dist2(ap[0], ap[1], ap[2], e1[0], e1[1], e1[2]);
-        const float sac = segment_dist2(ap[0], ap[1], ap[2], e2[0], e2[1], e2[2]);
-        const float sbc = segment_dist2(bp[0], bp[1], bp[2], ebc[0], ebc[1], ebc[2]);
-        const float m = fminf(fminf(sab, sac), sbc);
-        if (sab == m) {
-          const float s = segment_offset(ap[0], ap[1], ap[2], e1[0], e1[1], e1[2], d[0], d[1], d[2]);
-          lam[0] = __fsub_rn(1.f, s), lam[1] = s;
-        } else if (sac == m) {
-          const float s = segment_offset(ap[0], ap[1], ap[2], e2[0], e2[1], e2[2], d[0], d[1], d[2]);
-          lam[0] = __fsub_rn(1.f, s), lam[2] = s;
+        for (int k = 0; k < 3; ++k) ap[k] = q[k] - a[k];
+        face_segments(ap, e1, e2, sp, se, s);
+        const float mn = fminf(fminf(s[0], s[1]), s[2]);
+        auto take = [&](int k, int c0, int c1) {        // segment k, from corner c0 to corner c1
+          const float t = segment_offset(sp[k][0], sp[k][1], sp[k][2], se[k][0], se[k][1], se[k][2], d[0], d[1], d[2]);
+          lam[c0] = __fsub_rn(1.f, t);
+          lam[c1] = t;
+        };
+        if (s[0] == mn) {
+          take(0, 0, 1);
+        } else if (s[1] == mn) {
+          take(1, 0, 2);
         } else {
-          const float s = segment_offset(bp[0], bp[1], bp[2], ebc[0], ebc[1], ebc[2], d[0], d[1], d[2]);
-          lam[1] = __fsub_rn(1.f, s), lam[2] = s;
+          take(2, 1, 2);
         }
       }
       valid = isfinite(d[0]) && isfinite(d[1]) && isfinite(d[2]);
@@ -538,68 +512,40 @@ __global__ void __launch_bounds__(BW_WARPS * 32) mesh_distance_backward_kernel(
       }
       __syncwarp();
 #pragma unroll
-      for (int r = 0; r < 3; ++r) {
-        const int v = tvert[w][32 * r + lane];
-        const unsigned vmask = __ballot_sync(0xffffffffu, v >= 0);
-        if (v >= 0) {
-          const unsigned peers = __match_any_sync(vmask, v);
-          if (lane == __ffs(peers) - 1) {
-            float acc[3] = {GV[(size_t)v * 3], GV[(size_t)v * 3 + 1], GV[(size_t)v * 3 + 2]};
-            for (unsigned rest = peers; rest; rest &= rest - 1) {
-              const int l = 32 * r + __ffs(rest) - 1;
-#pragma unroll
-              for (int k = 0; k < 3; ++k) acc[k] = __fadd_rn(acc[k], term[w][k][l]);
-            }
-#pragma unroll
-            for (int k = 0; k < 3; ++k) GV[(size_t)v * 3 + k] = acc[k];
-          }
-        }
-        __syncwarp();
-      }
+      for (int r = 0; r < 3; ++r) warp_add_rows(GV, tvert[w][32 * r + lane], term[w], 32 * r);
     }
   }
 }
 
+// One CTA per (batch item, tile of MESH_TILE queries).
+template <typename... Out>
+int launch_mesh_tiles(void (*kernel)(MeshQuery, int, Out...), const MeshQuery& m, cudaStream_t s, Out... out) {
+  if (m.B == 0 || m.Q == 0) return DVQ_OK;
+  const int tiles = (m.Q + MESH_TILE - 1) / MESH_TILE;
+  kernel<<<(unsigned)((long long)m.B * tiles), MESH_THREADS, 0, s>>>(m, tiles, out...);
+  DVQ_CUDA_CHECK(cudaGetLastError());
+  count_launch();
+  return DVQ_OK;
+}
+
 }  // namespace
 
-int launch_mesh_winding(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B, float* w,
-                        int* inside_count, cudaStream_t s) {
-  if (B == 0 || Q == 0) return DVQ_OK;
-  const int tiles = (Q + MESH_TILE - 1) / MESH_TILE;
-  mesh_winding_kernel<<<(unsigned)((long long)B * tiles), MESH_THREADS, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, tiles, w,
-                                                                                inside_count);
-  DVQ_CUDA_CHECK(cudaGetLastError());
-  count_launch();
-  return DVQ_OK;
+int launch_mesh_winding(const MeshQuery& m, float* w, int* inside_count, cudaStream_t s) {
+  return launch_mesh_tiles(mesh_winding_kernel, m, s, w, inside_count);
 }
 
-int launch_mesh_distance(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
-                         float* dist2, int64_t* face, cudaStream_t s) {
-  if (B == 0 || Q == 0) return DVQ_OK;
-  const int tiles = (Q + MESH_TILE - 1) / MESH_TILE;
-  mesh_distance_kernel<<<(unsigned)((long long)B * tiles), MESH_THREADS, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, tiles, dist2,
-                                                                                 face);
-  DVQ_CUDA_CHECK(cudaGetLastError());
-  count_launch();
-  return DVQ_OK;
+int launch_mesh_distance(const MeshQuery& m, float* dist2, int64_t* face, cudaStream_t s) {
+  return launch_mesh_tiles(mesh_distance_kernel, m, s, dist2, face);
 }
 
-int launch_mesh_penetration(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
-                            float* depth2, int64_t* face, cudaStream_t s) {
-  if (B == 0 || Q == 0) return DVQ_OK;
-  const int tiles = (Q + MESH_TILE - 1) / MESH_TILE;
-  mesh_penetration_kernel<<<(unsigned)((long long)B * tiles), MESH_THREADS, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, tiles,
-                                                                                    depth2, face);
-  DVQ_CUDA_CHECK(cudaGetLastError());
-  count_launch();
-  return DVQ_OK;
+int launch_mesh_penetration(const MeshQuery& m, float* depth2, int64_t* face, cudaStream_t s) {
+  return launch_mesh_tiles(mesh_penetration_kernel, m, s, depth2, face);
 }
 
-int launch_mesh_distance_backward(const float* verts, int Bm, int V, const int* faces, int F, const float* pts, int Bp, int Q, int B,
-                                  const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts, cudaStream_t s) {
-  if (B == 0 || (Q == 0 && !g_verts)) return DVQ_OK;
-  mesh_distance_backward_kernel<<<(B + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, s>>>(verts, Bm, V, faces, F, pts, Bp, Q, B, face,
-                                                                                         g_dist2, g_pts, g_verts);
+int launch_mesh_distance_backward(const MeshQuery& m, const int64_t* face, const float* g_dist2, float* g_pts, float* g_verts,
+                                  cudaStream_t s) {
+  if (m.B == 0 || (m.Q == 0 && !g_verts)) return DVQ_OK;
+  mesh_distance_backward_kernel<<<(m.B + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, s>>>(m, face, g_dist2, g_pts, g_verts);
   DVQ_CUDA_CHECK(cudaGetLastError());
   count_launch();
   return DVQ_OK;

@@ -20,19 +20,8 @@ from torch import nn
 from torch.autograd.function import once_differentiable
 
 from . import _cabi
+from .grasp_quality import _points, check_faces
 from .quantizer import _stream_ptr
-
-
-def _points(x, name):
-    if not isinstance(x, torch.Tensor):
-        raise TypeError("%s must be a torch.Tensor" % name)
-    if x.dtype != torch.float32:
-        raise TypeError("%s must be fp32; got %s" % (name, x.dtype))
-    if not x.is_cuda:
-        raise ValueError("dvq.nearest_points has no CPU path: %s must be a CUDA tensor" % name)
-    if x.dim() != 3 or x.shape[2] != 3:
-        raise ValueError("%s must be [B, n, 3]; got %s" % (name, tuple(x.shape)))
-    return x.contiguous()
 
 
 class _NearestPoints(torch.autograd.Function):
@@ -75,7 +64,8 @@ class _NearestPoints(torch.autograd.Function):
 
 
 def _search(src, trg, trg_normals=None):
-    src, trg = _points(src, "src"), _points(trg, "trg")
+    src = _points(src, "src", "dvq.nearest_points", detach=False)
+    trg = _points(trg, "trg", "dvq.nearest_points", detach=False)
     if src.device != trg.device:
         raise ValueError("src is on %s, trg on %s" % (src.device, trg.device))
     if src.shape[0] != trg.shape[0]:
@@ -107,17 +97,10 @@ class HandObjectContact(nn.Module):
 
     def __init__(self, faces):
         super().__init__()
-        f = np.asarray(faces.detach().cpu() if isinstance(faces, torch.Tensor) else faces)
-        if f.dtype.kind not in "iu":
-            raise TypeError("faces must be an integer array; got %s" % f.dtype)
-        if f.ndim != 2 or f.shape[1] != 3:
-            raise ValueError("faces must be [F, 3]; got %s" % (f.shape,))
-        if f.size and (f.min() < 0 or f.max() >= 2 ** 31 - 1):
-            raise ValueError("face vertex ids must be in [0, V)")
-        f = f.astype(np.int64)
+        f = check_faces(faces, None)
         self.num_verts = int(f.max()) + 1 if f.size else 0     # the hand must have at least this many vertices
         offsets, vf_faces = vertex_face_csr(f, self.num_verts)
-        self.register_buffer("faces", torch.from_numpy(f.astype(np.int32)), persistent=False)
+        self.register_buffer("faces", torch.from_numpy(f), persistent=False)
         self.register_buffer("vf_offsets", torch.from_numpy(offsets), persistent=False)
         self.register_buffer("vf_faces", torch.from_numpy(vf_faces), persistent=False)
 
@@ -136,7 +119,7 @@ class HandObjectContact(nn.Module):
         return normals
 
     def forward(self, hand_verts, obj_pts):
-        hand = _points(hand_verts, "hand_verts")
+        hand = _points(hand_verts, "hand_verts", "dvq.nearest_points", detach=False)
         if self.faces.device != hand.device:
             raise ValueError("the module is on %s, hand_verts on %s: move it with .to(device)" % (self.faces.device, hand.device))
         normals = self.vertex_normals(hand.detach())

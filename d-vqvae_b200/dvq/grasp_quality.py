@@ -79,21 +79,24 @@ def _prepare(points, verts, faces, what, detach=True):
     return points, verts, f, _broadcast(verts.shape[0], points.shape[0])
 
 
-def _winding(points, verts, faces, w=None, count=None):
+def _mesh_call(entry, points, verts, faces, *tensors):
+    """Calls the C entry ``entry`` (one of the four ``dvq_mesh_*``) with the common mesh arguments (verts, Bm, V, faces, F,
+    pts, Bp, Q), then ``tensors`` (None is NULL) and the current stream of the points' device."""
     with torch.cuda.device(points.device):
-        _cabi.check(_cabi.lib.dvq_mesh_winding(verts.data_ptr(), verts.shape[0], verts.shape[1], faces.data_ptr(), faces.shape[0],
-                                               points.data_ptr(), points.shape[0], points.shape[1],
-                                               w.data_ptr() if w is not None else None, count.data_ptr() if count is not None else None,
-                                               _stream_ptr(points.device)), "dvq_mesh_winding")
+        _cabi.check(getattr(_cabi.lib, entry)(verts.data_ptr(), verts.shape[0], verts.shape[1], faces.data_ptr(), faces.shape[0],
+                                              points.data_ptr(), points.shape[0], points.shape[1],
+                                              *(t.data_ptr() if t is not None else None for t in tensors), _stream_ptr(points.device)),
+                    entry)
 
 
-def _distance(points, verts, faces, B):
+def _winding(points, verts, faces, w=None, count=None):
+    _mesh_call("dvq_mesh_winding", points, verts, faces, w, count)
+
+
+def _distance(points, verts, faces, B, entry="dvq_mesh_distance"):
     dist2 = torch.empty(B, points.shape[1], device=points.device, dtype=torch.float32)
     face = torch.empty(B, points.shape[1], device=points.device, dtype=torch.int64)
-    with torch.cuda.device(points.device):
-        _cabi.check(_cabi.lib.dvq_mesh_distance(verts.data_ptr(), verts.shape[0], verts.shape[1], faces.data_ptr(), faces.shape[0],
-                                                points.data_ptr(), points.shape[0], points.shape[1], dist2.data_ptr(), face.data_ptr(),
-                                                _stream_ptr(points.device)), "dvq_mesh_distance")
+    _mesh_call(entry, points, verts, faces, dist2, face)
     return dist2, face
 
 
@@ -109,13 +112,7 @@ def winding_number(points, verts, faces):
 
 
 def _penetration(points, verts, faces, B):
-    depth2 = torch.empty(B, points.shape[1], device=points.device, dtype=torch.float32)
-    face = torch.empty(B, points.shape[1], device=points.device, dtype=torch.int64)
-    with torch.cuda.device(points.device):
-        _cabi.check(_cabi.lib.dvq_mesh_penetration(verts.data_ptr(), verts.shape[0], verts.shape[1], faces.data_ptr(), faces.shape[0],
-                                                   points.data_ptr(), points.shape[0], points.shape[1], depth2.data_ptr(),
-                                                   face.data_ptr(), _stream_ptr(points.device)), "dvq_mesh_penetration")
-    return depth2, face
+    return _distance(points, verts, faces, B, "dvq_mesh_penetration")
 
 
 class _MeshDistance(torch.autograd.Function):
@@ -143,12 +140,7 @@ class _MeshDistance(torch.autograd.Function):
         g = g_dist2.to(torch.float32).contiguous()
         g_pts = torch.empty(B, Q, 3, device=points.device, dtype=torch.float32) if want_pts else None
         g_verts = torch.empty(B, V, 3, device=verts.device, dtype=torch.float32) if want_verts else None
-        ptr = lambda t: t.data_ptr() if t is not None else None
-        with torch.cuda.device(points.device):
-            _cabi.check(_cabi.lib.dvq_mesh_distance_backward(verts.data_ptr(), verts.shape[0], V, faces.data_ptr(), faces.shape[0],
-                                                             points.data_ptr(), points.shape[0], Q, face.data_ptr(), g.data_ptr(),
-                                                             ptr(g_pts), ptr(g_verts), _stream_ptr(points.device)),
-                        "dvq_mesh_distance_backward")
+        _mesh_call("dvq_mesh_distance_backward", points, verts, faces, face, g, g_pts, g_verts)
         if g_pts is not None and points.shape[0] != B:
             g_pts = g_pts.sum(0, keepdim=True)
         if g_verts is not None and verts.shape[0] != B:
